@@ -5,6 +5,7 @@ all-gather of the logits per step.
 
     python bench.py --gpus 1 --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host CPU (oracle port)
+    python bench.py ... --dump-outputs DIR                   # + DIR/probs.npy: what the last timed step returned
     torchrun ... bench.py --gpus N ...                       # N > 1, weak scaling (64 clips per GPU)
 
 Prints ONE JSON line (contract in the task statement): value = whole-job clips/s with inputs resident in HBM,
@@ -69,6 +70,7 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        self.proc.wait()
         sm, mx, reasons = [], None, set()
         for r in self.rows:
             try:
@@ -152,11 +154,26 @@ def cpu_forward_timed(cfg, model, clips, frames, crop, alpha, steps, warmup):
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        O.forward(cfg, sd, xs)
+        y = O.forward(cfg, sd, xs)
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
-    return clips * len(times) / sum(times), sum(times) / len(times)
+    return clips * len(times) / sum(times), sum(times) / len(times), y
+
+
+def dump_outputs(dirname, probs):
+    """Writes the class probabilities of the last timed step as dirname/probs.npy (float32), so that two builds run
+    with the same arguments (hence the same seeded weights and clips) can be compared output for output.  Above 64 MB
+    only a fixed, seeded sample of the rows is written."""
+    import numpy as np
+
+    a = probs.detach().float().cpu()
+    limit = 64 << 20
+    if a.numel() * 4 > limit:
+        keep = limit // (4 * a[0].numel())
+        a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "probs.npy"), a.numpy())
 
 
 def run_reference(args):
@@ -167,7 +184,9 @@ def run_reference(args):
     model = build_weights(cfg)
     clips = args.cpu_clips
     t_start = time.time()
-    value, sec = cpu_forward_timed(cfg, model, clips, args.frames, args.crop, args.alpha, args.steps, args.warmup)
+    value, sec, probs = cpu_forward_timed(cfg, model, clips, args.frames, args.crop, args.alpha, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, probs)
     cores = torch.get_num_threads()
     sample = "%d clip(s) of the workload per step (same shape, CPU FP32 oracle port of the reference forward)" % clips
     line = {
@@ -348,8 +367,10 @@ def run_extra_config(h, base_args, key, model_name, batch, frames, crop):
     steps = max(5, int(1000.0 / max(est, 1e-3)) + 1)
     sampler = ClockSampler(h.local_rank)
     sampler.start()
-    ms = h.timed(step, steps)
-    clocks = sampler.stop()
+    try:
+        ms = h.timed(step, steps)
+    finally:
+        clocks = sampler.stop()
     out = {"workload": workload_name(a), "value": a.batch * steps / (ms * 1e-3), "unit": UNIT, "steps": steps, "warmup": 5,
            "ms_per_step": ms / steps, "batch": a.batch, "launches_per_step": plan.launches_per_run,
            "arena_gb": round(plan.arena_bytes() / 1e9, 2), "clocks": clocks, "parity_check": par}
@@ -380,10 +401,13 @@ def run_gpu(args):
     B, T, S, alpha = args.batch, args.frames, args.crop, args.alpha
     K = cfg.MODEL.NUM_CLASSES
 
+    last = {}                                       # what the latest step returned, for --dump-outputs
+
     def step():
         out = model(ins)                            # graph replay; no staging copy (inputs are the static buffers)
         if world > 1:
-            return h.esf_dist.all_gather([out])[0]  # the only collective on the path (tools/test_net.py:95-98)
+            out = h.esf_dist.all_gather([out])[0]   # the only collective on the path (tools/test_net.py:95-98)
+        last["probs"] = out
         return out
 
     if args.profile_mode:
@@ -402,9 +426,13 @@ def run_gpu(args):
     sampler = ClockSampler(h.local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = h.timed(step, args.steps)
-    clocks = sampler.stop() if rank == 0 else None
+    try:
+        ms_total = h.timed(step, args.steps)
+    finally:                                        # the sampler's nvidia-smi must not outlive a failed step
+        clocks = sampler.stop() if rank == 0 else None
     value = world * B * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["probs"])
 
     # ---- end-to-end through the public API with pinned host inputs (H2D + forward + D2H per step)
     # ClipStream = the package's public host-side loop: per batch H2D from pinned memory -> model.forward ->
@@ -522,7 +550,7 @@ def run_gpu(args):
     cpu = None
     if world == 1 and not args.no_cpu_baseline:
         os.sched_setaffinity(0, h.affinity0)      # all host cores again (the NUMA binding was for the pinned buffers)
-        cv, csec = cpu_forward_timed(cfg, model, args.cpu_clips, T, S, alpha, steps=1, warmup=1)
+        cv, csec, _ = cpu_forward_timed(cfg, model, args.cpu_clips, T, S, alpha, steps=1, warmup=1)
         cpu = {"value": cv, "unit": UNIT, "cores": torch.get_num_threads(), "kind": "port",
                "sample": "%d clip(s) of the same workload, 1 warm-up + 1 timed oracle forward (%.1f s)" % (
                    args.cpu_clips, csec)}
@@ -561,7 +589,7 @@ def run_gpu(args):
         dist.destroy_process_group()
 
 
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -574,9 +602,11 @@ def main():
     ap.add_argument("--frames", type=int, default=32)
     ap.add_argument("--crop", type=int, default=224)
     ap.add_argument("--cpu-clips", type=int, default=1)
-    ap.add_argument("--e2e-steps", type=int, default=0, help="end-to-end steps (0: same as --steps)")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="end-to-end steps (0: --steps, at least 30)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--dump-ops", default="", help="write per-op device times (JSON lines) to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the probabilities of the last timed step to DIR/probs.npy (float32)")
     ap.add_argument("--precision", default="fp16", choices=["fp16", "bf16", "fp32"],
                     help="16-bit storage / tensor-core operand format (FP32 accumulation in both)")
     ap.add_argument("--e2e-depth", type=int, default=3, help="staging slots of the end-to-end ClipStream")
@@ -585,7 +615,11 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the rank to its GPU's NUMA node")
     ap.add_argument("--profile-mode", action="store_true",
                     help="for ncu: eager launches (no CUDA graph), 1 warm-up + --steps steps, nothing else")
-    args = ap.parse_args()
+    args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.profile_mode and args.dump_outputs:
+        ap.error("--dump-outputs writes the last timed step, and --profile-mode times none")
     args.alpha = 8 if args.model == "SlowFast" else 4
     if args.case:
         from efficient_slowfast_b200 import workloads as recipe
@@ -595,6 +629,11 @@ def main():
             args.alpha = 0
         elif args.model == "SlowFast":
             args.alpha = 8
+    return args
+
+
+def main():
+    args = parse_args()
     if args.impl == "reference":
         run_reference(args)
     else:

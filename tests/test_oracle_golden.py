@@ -47,6 +47,19 @@ def test_oracle_matches_reference_golden(name, tag):
         assert abs(y.sum(1) - 1).max() < 1e-5
 
 
+@pytest.mark.parametrize("name", sorted(recipe.CASES))
+def test_bn_buffers_match_reference_state_dict(name):
+    """Each fixture stores the reference model's BN running statistics under its state_dict keys, in its state_dict
+    order: the drop-in has the same BN buffers, in the same order and with the same shapes."""
+    import efficient_slowfast_b200 as esf
+
+    gold = helpers.load_golden(name)
+    ref = [(k[3:], tuple(v.shape)) for k, v in gold.items() if k.startswith("bn/")]
+    torch.manual_seed(0)
+    sd = esf.build_model(helpers.case_cfg(name)).state_dict()
+    assert [(k, tuple(v.shape)) for k, v in sd.items() if k.endswith((".running_mean", ".running_var"))] == ref
+
+
 def test_oracle_default_init_corner():
     """gamma = 0 and zero-initialised final BN (the reference's shipped init): attention/bottleneck branches vanish."""
     import efficient_slowfast_b200 as esf
