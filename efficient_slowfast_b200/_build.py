@@ -1,7 +1,8 @@
 """In-tree build of libesf_b200.so (hand-written sm_100a CUDA behind the C ABI in include/esf.h).
 
-nvcc cross-compiles for sm_100a without a GPU; the resulting .so lives next to the sources so that it travels
-with the repo snapshot to the GPU box (it is git-ignored, not gpurun-ignored).
+nvcc cross-compiles for sm_100a without a GPU; the resulting .so lives next to the sources (git-ignored), so that a
+copy of the built tree runs on a GPU machine without compiling again.  ESF_NVCC_EXTRA adds nvcc flags (instrumented
+builds such as -DESF_ATTN_TIMING); the library itself reads no environment variables at run time.
 """
 import hashlib
 import os
@@ -15,7 +16,7 @@ HEADERS = ["esf_common.cuh", "esf_host.h", os.path.join("..", "..", "include", "
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-DESF_NO_FAST_MATH",
-] + os.environ.get("ESF_NVCC_EXTRA", "").split()      # e.g. ESF_NVCC_EXTRA=-DESF_ATTN_TIMING for kernel phase timing
+] + os.environ.get("ESF_NVCC_EXTRA", "").split()
 
 
 def _nvcc():

@@ -55,8 +55,6 @@ struct __align__(64) AttnTcParams {
   uint32_t q_tile_bytes, k_tile_bytes, v_tile_bytes;
   int f16;  // 16-bit operands (Q~, K~, V^T, P) and the output are IEEE half instead of BF16
   int out_f32;  // the output view is FP32 (FP32-accurate path, esf_precise.cu); strides stay in elements
-  int pdbl;     // v2 kernel: two P buffers per (query tile, half) -- TMEM has the columns when DVp <= 32 (d < 32)
-  int qk_async; // v2 kernel: the Q.K^T issuer serves the two query tiles independently (no lock step)
   // split mode (v1 kernel, FP32-accurate plan): P and V are FP16 PAIRS, O += P_hi V_hi + P_lo V_hi + P_hi V_lo.  P_lo
   // lives 16 KB behind P_hi in shared memory, V_lo^T `v_half` bytes behind V^T inside a stage.
   int split;
@@ -419,59 +417,35 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_tc_kernel(const __grid_con
 // on 87 % of the tiles (~200 of ~1500 cycles) because one warp issued both MMAs and could only issue S_{j+1} after it
 // had waited for both halves of P_{j-1}; a Q.K^T issuer warp of its own removed that wait (-4 .. -8 %).
 // The FMA-pipe exponential was repeated with packed sm_100 arithmetic (FFMA2 / FADD2.RM, 5.5 issue slots per element
-// instead of ~8; template parameter POLY, knob ESF_ATTN_POLY = pairs of every 8): correct (kernel tests green at 2/8
-// and 4/8) but no faster -- d = 8: 3.26 / 3.16 / 3.07 / 3.31 / 3.05 Texp/s at 0 .. 4/8, d = 32: 2.97 / 2.96 / 2.93 /
-// 2.82 / 2.61 (8 clips, N = 25 088).  The scale FFMA of every pair is an FFMA2 since then.  Default stays MUFU only.
+// instead of ~8, on 1 .. 4 of every 8 element pairs): correct (kernel tests green at 2/8 and 4/8) but no faster --
+// d = 8: 3.26 / 3.16 / 3.07 / 3.31 / 3.05 Texp/s at 0 .. 4/8, d = 32: 2.97 / 2.96 / 2.93 / 2.82 / 2.61 (8 clips,
+// N = 25 088).  The scale FFMA of every pair is an FFMA2 since then; the polynomial was removed, MUFU only.
 // TMEM columns: S[q][buf] 4 x 64 | O[q][h] 4 x DVp (<= 48) | P[q][h] 4 x 16  = 512.
 // 16 softmax warps + TMA producer + Q.K^T issuer + 2 P.V issuers.  20 warps: ptxas sizes the register file for the
 // block rounded up to 128 threads, so 21 warps would cap the softmax threads at 80 registers (spills).
 constexpr int kV2Threads = 640;
 constexpr int kV2PCol = 448;     // first TMEM column of P
-constexpr int kV2DefaultPoly = 0;
-// Experiment (-DESF_ATTN_LATE_HANDOFF=1): issue the tcgen05.st of P, fetch the next scores, and complete the hand-over
-// (wait::st, fence, arrive p_full) half way through the next tile's exponentials, so that the ~200 cycles of store
-// latency are covered by MUFU work.  Measured with the dedicated Q.K^T issuer in place: correct, but 12 % SLOWER
-// (d = 8: 3.56 -> 3.12 Texp/s, d = 32: 3.25 -> 2.88) -- the P.V MMA then finishes after the next P is ready, and the
-// sync in the middle of the MUFU stream lets the pipe drain.
-#ifndef ESF_ATTN_LATE_HANDOFF
-#define ESF_ATTN_LATE_HANDOFF 0
-#endif
+// Tried and dropped: issue the tcgen05.st of P, fetch the next scores, and complete the hand-over (wait::st, fence,
+// arrive p_full) half way through the next tile's exponentials, so that the ~200 cycles of store latency are covered
+// by MUFU work.  Measured with the dedicated Q.K^T issuer in place: correct, but 12 % SLOWER (d = 8: 3.56 -> 3.12
+// Texp/s, d = 32: 3.25 -> 2.88) -- the P.V MMA then finishes after the next P is ready, and the sync in the middle of
+// the MUFU stream lets the pipe drain.  With a second P buffer still 9 % slower at d = 8 (2.993 -> 3.267 ms, 16 clips).
 // Also tried and dropped: P aliased onto the S tile it was computed from (FlashAttention-4 style; consecutive P tiles then
 // live in different TMEM buffers, the S buffer is released by the P.V commits and p_free is only consulted before an O
 // rescale).  No measurable gain (d = 8: 0.812 vs 0.814 ms, d = 32: 0.863 vs 0.860 ms at 4 clips) and the interaction
 // with the replay / rescale path was not yet right (one kernel test failed at 4x logits), so it is not in the tree.
 
-// exp2 of a pair on the FMA pipe (packed FFMA2 / FADD2, sm_100): Cody-Waite split x = floor(x) + f with the
-// round-down magic-number add, degree-3 minimax polynomial for 2^f on [0, 1) (max relative error 8.8e-5, below the
-// half-ulp of the 16-bit P it is rounded to), exponent inserted with an integer add.  x is clamped at -126: smaller
-// arguments would wrap the exponent field (2^-126 rounds to 0 in P).
-__device__ __forceinline__ float2 poly_exp2_pair(float2 x) {
-  x.x = fmaxf(x.x, -126.f);
-  x.y = fmaxf(x.y, -126.f);
-  const float2 t = __fadd2_rd(x, make_float2(12582912.f, 12582912.f));       // 1.5 * 2^23 + floor(x)
-  const float2 fl = __fadd2_rn(t, make_float2(-12582912.f, -12582912.f));
-  const float2 fr = __ffma2_rn(fl, make_float2(-1.f, -1.f), x);              // exact
-  float2 pl = __ffma2_rn(fr, make_float2(0.077119089663028717f, 0.077119089663028717f),
-                         make_float2(0.227564394474029541f, 0.227564394474029541f));
-  pl = __ffma2_rn(pl, fr, make_float2(0.695146143436431885f, 0.695146143436431885f));
-  pl = __ffma2_rn(pl, fr, make_float2(1.f, 1.f));
-  float2 r;
-  r.x = __int_as_float(__float_as_int(pl.x) + (__float_as_int(t.x) << 23));
-  r.y = __int_as_float(__float_as_int(pl.y) + (__float_as_int(t.y) << 23));
-  return r;
-}
-
-// POLY: how many of every 8 element pairs take the FMA-pipe exponential instead of MUFU.EX2 (0 = none)
-// KNOBS (compile time): the round-2 experiment paths (second P buffer, independent Q.K^T issue).  With the knobs as
-// run-time flags the DEFAULT path lost 4 - 6 % (88 instead of 96 registers, d = 8: 11.04 -> 11.68 ms, d = 32: 12.23 ->
-// 12.68 ms at batch 64 on one box, tools/sessions/r2_s18_attn_regress.sh), so they are a separate instantiation.
-// PIPE (compile time, experiment ESF_ATTN_PIPE=1): software-pipelined softmax loop.  The exponentials of tile j + 1 are
-// ISSUED before tile j is packed, stored and handed over, so a warp's hand-over work runs while its own MUFU
-// instructions are in flight (default loop: exps -> wait for them -> hand-over -> next tile; with the four warps of a
-// scheduler in similar phases the MUFU pipe idles ~23 % of the time).  Two tiles of values are live, so the softmax
-// warps take 112 registers from the four control warps with setmaxnreg (32 there: 512 x 112 + 128 x 32 = 640 x 96, the
-// pool the CTA was launched with -- asking for more never returns).
-template <bool F16, int POLY, bool KNOBS, bool PIPE = false>
+// Also measured, correct and removed again (profiles/r2_attention_experiments.md):
+//   * a second P buffer per (query tile, half) (d < 32: TMEM has the columns), so that the P store of tile j need not
+//     wait for the P.V MMA of tile j - 1, and an independent Q.K^T issue of the two query tiles instead of lock step:
+//     no change, d = 8 2.993 / 3.002 / 2.980 / 2.989 ms, d = 32 3.214 / 3.212 / 3.219 / 3.217 ms (16 clips,
+//     N = 25 088; neither, P, QK, both).  The waits they remove (ncu: 4.7 % + 6 % of the softmax warps' samples) are
+//     not what bounds the loop.  As run-time flags of this kernel they also cost the default path 4 - 6 % (88 instead
+//     of 96 registers, d = 8: 11.04 -> 11.68 ms, d = 32: 12.23 -> 12.68 ms at batch 64).
+//   * a software-pipelined softmax loop (the exponentials of tile j + 1 issued before tile j is packed, stored and
+//     handed over; two tiles of values live, so the softmax warps took 112 registers from the control warps with
+//     setmaxnreg): 3 % slower (d = 8: 2.832 -> 2.913 ms, d = 32: 3.112 -> 3.192 ms, 16 clips).
+template <bool F16>
 __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_constant__ AttnTcParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -485,7 +459,7 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
   uint64_t* kv_empty = kv_full + kTcMaxStages;
   uint64_t* s_full = kv_empty + kTcMaxStages;  // [q][buf]
   uint64_t* s_free = s_full + 4;
-  uint64_t* p_full = s_free + 4;               // [q][h][buffer]
+  uint64_t* p_full = s_free + 4;               // [q][h] (8 slots, 4 used)
   uint64_t* p_free = p_full + 8;
   uint64_t* o_full = p_free + 8;               // [q]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(o_full + 2);
@@ -496,12 +470,6 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
   const int row0 = blockIdx.x * 256;
   const int N = p.N;
   const int nt = (N + kTcBN - 1) / kTcBN;
-  // P buffers: one per (q, h) at columns 448.., or two (tile j uses buffer j & 1) at columns 384.. when O leaves room.
-  // With one buffer the P store of tile j waits for the P.V MMA of tile j - 1, which queues behind the Q.K^T MMAs of
-  // tile j + 1 on the in-order tensor pipe (ncu: 4.7 % of the softmax warps' samples sit in that wait).
-  const int pdbl = KNOBS ? p.pdbl : 0;
-  const uint32_t p_col0 = pdbl ? 384u : (uint32_t)kV2PCol;
-  const uint32_t p_qh_cols = pdbl ? 32u : 16u;
 
   if (threadIdx.x == 0) {
     mbar_init(q_full, 1);
@@ -537,7 +505,6 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
 
   if (warp == 16) {
     // ------------------------------------------------------------------ TMA producer
-    if constexpr (PIPE) asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
     if (elect_one()) {
       mbar_arrive_expect_tx(q_full, 2 * p.q_tile_bytes);
       for (int q = 0; q < 2; ++q) tma_load_3d(Qs + q * p.q_tile_bytes, &p.q_map, q_full, 0, row0 + q * 128, b);
@@ -560,9 +527,9 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
     }
   } else if (warp == 17) {
     // ------------------------------------------------------------------ Q.K^T issuer (both query tiles)
-    if constexpr (PIPE) asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
     // Separate from the P.V issuers: with one warp doing both, S_{j+1} could only be issued after that warp had waited
     // for BOTH halves of P_{j-1}, and the softmax warps found it missing on 87 % of the tiles (~200 cycles each).
+    // Truncating the step list (timing only) showed five of the six d = 32 MMAs per tile cost 6.8 % of the launch.
     const uint32_t idesc_s = make_idesc_16(128, kTcBN, F16);
     const uint32_t qk_hi = kmajor_desc_hi(p.sbo, p.layout_type);
     const uint32_t q_lo0 = kmajor_desc_lo(smem_u32(Qs));
@@ -571,101 +538,35 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
     const uint32_t k_stage_step = p.k_tile_bytes >> 4;
     mbar_wait(q_full, 0, 33);
     tc_fence_after();
-    if constexpr (!KNOBS) {
-      // round 1's loop, verbatim (the two query tiles in lock step)
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int c = 0; c < nt; ++c) {
-        const int buf = c & 1;
-        mbar_wait(&kv_full[stage], phase, 34);
+    // round 1's loop, verbatim (the two query tiles in lock step)
+    int stage = 0;
+    uint32_t phase = 0;
+    for (int c = 0; c < nt; ++c) {
+      const int buf = c & 1;
+      mbar_wait(&kv_full[stage], phase, 34);
 #pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          mbar_wait(&s_free[q * 2 + buf], ((c >> 1) & 1) ^ 1, 32);
-          tc_fence_after();
-          if (elect_one()) {
-            const uint32_t d_tmem = tmem_base + (q * 2 + buf) * kTcBN;
-            const uint32_t kb = k_lo + stage * k_stage_step;
-            const uint32_t q_lo = q_lo0 + q * q_step;
-#pragma unroll
-            for (int i = 0; i < 6; ++i)
-              if (i < p.nsteps2)
-                umma_bf16_lohi(d_tmem, q_lo + (p.steps2[i] & 0xffff), qk_hi, kb + (p.steps2[i] >> 16), qk_hi, idesc_s, i != 0);
-            umma_commit(&s_full[q * 2 + buf]);
-          }
-          __syncwarp();
-        }
-        if (++stage == p.stages) {
-          stage = 0;
-          phase ^= 1;
-        }
-      }
-    } else {
-      auto issue_s = [&](int q, int c, int stage) {
+      for (int q = 0; q < 2; ++q) {
+        mbar_wait(&s_free[q * 2 + buf], ((c >> 1) & 1) ^ 1, 32);
+        tc_fence_after();
         if (elect_one()) {
-          const uint32_t d_tmem = tmem_base + (q * 2 + (c & 1)) * kTcBN;
+          const uint32_t d_tmem = tmem_base + (q * 2 + buf) * kTcBN;
           const uint32_t kb = k_lo + stage * k_stage_step;
           const uint32_t q_lo = q_lo0 + q * q_step;
-  #pragma unroll
+#pragma unroll
           for (int i = 0; i < 6; ++i)
             if (i < p.nsteps2)
               umma_bf16_lohi(d_tmem, q_lo + (p.steps2[i] & 0xffff), qk_hi, kb + (p.steps2[i] >> 16), qk_hi, idesc_s, i != 0);
-          umma_commit(&s_full[q * 2 + (c & 1)]);
+          umma_commit(&s_full[q * 2 + buf]);
         }
         __syncwarp();
-      };
-      if (KNOBS && p.qk_async) {
-        // The two query tiles advance independently: whichever has its S buffer free (and its K tile landed) gets its
-        // next Q.K^T issued.  In lock step (the loop below) a late warp of one tile also delays the other tile's scores,
-        // and all sixteen softmax warps reach their MUFU phase together (ncu: 6 % of their samples wait for S).
-        int cq[2] = {0, 0}, stq[2] = {0, 0};
-        uint32_t phq[2] = {0, 0};
-        uint32_t spins = 0;
-        uint64_t t0 = 0;
-        while (cq[0] < nt || cq[1] < nt) {
-          bool progress = false;
-  #pragma unroll
-          for (int q = 0; q < 2; ++q) {
-            const int c = cq[q];
-            if (c >= nt) continue;
-            if (!mbar_try_wait(&kv_full[stq[q]], phq[q])) continue;
-            if (!mbar_try_wait(&s_free[q * 2 + (c & 1)], ((c >> 1) & 1) ^ 1)) continue;
-            tc_fence_after();
-            issue_s(q, c, stq[q]);
-            cq[q] = c + 1;
-            if (++stq[q] == p.stages) stq[q] = 0, phq[q] ^= 1;
-            progress = true;
-          }
-          if (!progress && ((++spins) & 0xfff) == 0) {   // bounded like mbar_wait: a pipeline bug traps instead of hanging
-            const uint64_t now = globaltimer_ns();
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > ESF_WAIT_TIMEOUT_NS) {
-              if (lane == 0) printf("[esf] attention Q.K issuer timeout: block %d tiles %d/%d of %d\n", (int)blockIdx.x, cq[0], cq[1], nt);
-              __trap();
-            }
-          }
-          if (progress) spins = 0, t0 = 0;
-        }
-      } else {
-        int stage = 0;
-        uint32_t phase = 0;
-        for (int c = 0; c < nt; ++c) {
-          mbar_wait(&kv_full[stage], phase, 34);
-  #pragma unroll
-          for (int q = 0; q < 2; ++q) {
-            mbar_wait(&s_free[q * 2 + (c & 1)], ((c >> 1) & 1) ^ 1, 32);
-            tc_fence_after();
-            issue_s(q, c, stage);
-          }
-          if (++stage == p.stages) {
-            stage = 0;
-            phase ^= 1;
-          }
-        }
+      }
+      if (++stage == p.stages) {
+        stage = 0;
+        phase ^= 1;
       }
     }
   } else if (warp == 18 || warp == 19) {
     // ------------------------------------------------------------------ P.V issuers (one per query tile)
-    if constexpr (PIPE) asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
     const int q = warp - 18;
     const uint32_t idesc_o = make_idesc_16(128, p.DVp, F16);
     const uint32_t pv_hi = kmajor_desc_hi(1024, 2);
@@ -676,18 +577,16 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
     for (int j = 0; j < nt; ++j) {
       mbar_wait(&kv_full[stage], phase, 35);   // already complete (S_j was computed from this stage): visibility only
       const uint32_t vl = v_lo + stage * v_stage_step;
-      const int pb = pdbl ? (j & 1) : 0;                       // P buffer of this tile
-      const uint32_t p_par = pdbl ? ((j >> 1) & 1) : (j & 1);   // parity of this use of the buffer
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
-        mbar_wait(KNOBS ? &p_full[(q * 2 + h) * 2 + pb] : &p_full[q * 2 + h], p_par, 36);
+        mbar_wait(&p_full[q * 2 + h], j & 1, 36);
         tc_fence_after();
         if (elect_one()) {
           const uint32_t o_tmem = tmem_base + 4 * kTcBN + (q * 2 + h) * p.DVp;
-          const uint32_t p_tmem = tmem_base + p_col0 + (q * 2 + h) * p_qh_cols + pb * 16;
+          const uint32_t p_tmem = tmem_base + kV2PCol + (q * 2 + h) * 16;
           umma_f16_ts(o_tmem, p_tmem, vl + 4 * h, pv_hi, idesc_o, j != 0);      // keys 32h .. 32h+15
           umma_f16_ts(o_tmem, p_tmem + 8, vl + 4 * h + 2, pv_hi, idesc_o, 1);  // keys 32h+16 .. 32h+31
-          umma_commit(KNOBS ? &p_free[(q * 2 + h) * 2 + pb] : &p_free[q * 2 + h]);
+          umma_commit(&p_free[q * 2 + h]);
           if (h == 1) {
             umma_commit(&kv_empty[stage]);
             if (j == nt - 1) umma_commit(&o_full[q]);
@@ -702,7 +601,6 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
     }
   } else {
     // ------------------------------------------------------------------ softmax: warp = q * 8 + h * 4 + quarter
-    if constexpr (PIPE) asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
     const int q = warp >> 3;
     const int h = (warp >> 2) & 1;
     const int quarter = warp & 3;
@@ -710,7 +608,7 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
     const int n = row0 + q * 128 + r;
     const uint32_t lane_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
     const uint32_t o_addr = lane_addr + 4 * kTcBN + (q * 2 + h) * p.DVp;
-    const uint32_t p_addr0 = lane_addr + p_col0 + (q * 2 + h) * p_qh_cols;
+    const uint32_t p_addr = lane_addr + kV2PCol + (q * 2 + h) * 16;
     const bool tail = (N % kTcBN) != 0;
     float m = -CUDART_INF_F;
     // 12 * ln 2: p = exp(s - m) stays <= 4096, inside FP16 and harmless in the FP32 sums; a larger window means
@@ -729,117 +627,6 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
 #else
 #define ESF_TICK(k)
 #endif
-    if constexpr (PIPE) {
-      float w[32];
-      float f = 1.f;
-      bool any_raise = false;
-      // raw scores of tile jj in x -> speculative exponentials in place, running maximum, S buffer released.  `prev`
-      // holds the exponentials of tile jj - 1, which are not stored yet: a raise rescales them too.
-      auto stage1 = [&](float (&x)[32], float (&prev)[32], int jj, bool has_prev) {
-        const int buf = jj & 1;
-        const uint32_t s_addr = lane_addr + (q * 2 + buf) * kTcBN + 32 * h;
-        const bool last_tail = tail && jj == nt - 1;
-        if (last_tail) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i)
-            if (jj * kTcBN + 32 * h + i >= N) x[i] = -CUDART_INF_F;
-        }
-        float ms = (m == -CUDART_INF_F) ? 0.f : m * kTcLog2e;
-        float mx0 = -CUDART_INF_F, mx1 = -CUDART_INF_F;
-        const float2 ms2 = make_float2(-ms, -ms), c2 = make_float2(kTcLog2e, kTcLog2e);
-#pragma unroll
-        for (int i = 0; i < 32; i += 4) {
-          mx0 = fmaxf(fmaxf(mx0, x[i]), x[i + 1]);
-          mx1 = fmaxf(fmaxf(mx1, x[i + 2]), x[i + 3]);
-#pragma unroll
-          for (int e = 0; e < 4; e += 2) {
-            const float2 y = __ffma2_rn(make_float2(x[i + e], x[i + e + 1]), c2, ms2);
-            x[i + e] = fast_exp2(y.x);
-            x[i + e + 1] = fast_exp2(y.y);
-          }
-        }
-        const float mx = fmaxf(mx0, mx1);
-        const bool raise = mx > m + kTau;
-        any_raise = __any_sync(0xffffffffu, raise);
-        f = 1.f;
-        if (any_raise) {
-          const float m_new = raise ? mx : m;
-          f = raise ? fast_exp2((m - m_new) * kTcLog2e) : 1.f;
-          const bool big = raise && !((mx - m) * kTcLog2e < 100.f);
-          m = m_new;
-          if (__any_sync(0xffffffffu, big)) {
-            tmem_ld32_nowait(s_addr, x);
-            tmem_wait_ld();
-            tmem_ld32_acquire(x);
-            if (last_tail) {
-#pragma unroll
-              for (int i = 0; i < 32; ++i)
-                if (jj * kTcBN + 32 * h + i >= N) x[i] = -CUDART_INF_F;
-            }
-            ms = (m == -CUDART_INF_F) ? 0.f : m * kTcLog2e;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) x[i] = fast_exp2(fmaf(x[i], kTcLog2e, -ms));
-          } else {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) x[i] *= f;
-          }
-          if (has_prev) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) prev[i] *= f;
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&s_free[q * 2 + buf]);
-      };
-      // exponentials of tile jj in x -> P in TMEM, handed to the P.V issuer; O is brought to the maximum P was scaled to
-      auto stage2 = [&](float (&x)[32], int jj, bool rescale) {
-        uint32_t pk[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) pk[i] = pack16x2(x[2 * i], x[2 * i + 1], F16);
-        mbar_wait(&p_free[q * 2 + h], (jj & 1) ^ 1, 38);   // P.V of tile jj - 1 has consumed the buffer (and left O alone)
-        tc_fence_after();
-        if (jj > 0 && rescale) {
-          for (int c0 = 0; c0 < p.DVp; c0 += 16) {
-            float o[16];
-            tmem_ld16(o_addr + c0, o);
-#pragma unroll
-            for (int k2 = 0; k2 < 16; ++k2) o[k2] *= f;
-            tmem_st16(o_addr + c0, o);
-          }
-        }
-        tmem_st16_b32(p_addr0, pk);
-        tmem_wait_st();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&p_full[q * 2 + h]);
-      };
-      auto fetch = [&](float (&x)[32], int jj) {
-        mbar_wait(&s_full[q * 2 + (jj & 1)], (jj >> 1) & 1, 37);
-        tc_fence_after();
-        tmem_ld32_nowait(lane_addr + (q * 2 + (jj & 1)) * kTcBN + 32 * h, x);
-        tmem_wait_ld();
-        tmem_ld32_acquire(x);
-      };
-      stage1(v, w, 0, false);
-      for (int j = 0; j < nt; j += 2) {
-        bool rs = false;
-        if (j + 1 < nt) {
-          fetch(w, j + 1);
-          stage1(w, v, j + 1, true);
-          rs = any_raise;
-        }
-        stage2(v, j, rs);
-        if (j + 1 >= nt) break;
-        rs = false;
-        if (j + 2 < nt) {
-          fetch(v, j + 2);
-          stage1(v, w, j + 2, true);
-          rs = any_raise;
-        }
-        stage2(w, j + 1, rs);
-      }
-    } else
     for (int j = 0; j < nt; ++j) {
       const int buf = j & 1;
       const uint32_t s_addr = lane_addr + (q * 2 + buf) * kTcBN + 32 * h;
@@ -856,26 +643,13 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
       const float2 ms2 = make_float2(-ms, -ms), c2 = make_float2(kTcLog2e, kTcLog2e);
 #pragma unroll
       for (int i = 0; i < 32; i += 4) {
-        if (ESF_ATTN_LATE_HANDOFF && i == 16 && j > 0) {
-          // P of the PREVIOUS tile: its tcgen05.st was issued before this tile's scores were fetched; the ~200 cycles
-          // until the store is visible are covered by the first half of this tile's exponentials
-          tmem_wait_st();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(KNOBS ? &p_full[(q * 2 + h) * 2 + (pdbl ? ((j - 1) & 1) : 0)] : &p_full[q * 2 + h]);
-        }
         mx0 = fmaxf(fmaxf(mx0, v[i]), v[i + 1]);
         mx1 = fmaxf(fmaxf(mx1, v[i + 2]), v[i + 3]);
 #pragma unroll
         for (int e = 0; e < 4; e += 2) {
-          const int k = (i + e) >> 1;   // pair index 0..15
           float2 x = __ffma2_rn(make_float2(v[i + e], v[i + e + 1]), c2, ms2);
-          if (POLY > 0 && ((k * POLY) & 7) < POLY) {
-            x = poly_exp2_pair(x);
-          } else {
-            x.x = fast_exp2(x.x);
-            x.y = fast_exp2(x.y);
-          }
+          x.x = fast_exp2(x.x);
+          x.y = fast_exp2(x.y);
           v[i + e] = x.x;
           v[i + e + 1] = x.y;
         }
@@ -920,19 +694,11 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
       for (int i = 0; i < 16; ++i) pk[i] = pack16x2(v[2 * i], v[2 * i + 1], F16);
       asm volatile("" ::"r"(pk[15]));
       ESF_TICK(3)   // pack
-      const int pb = pdbl ? (j & 1) : 0;
-      const uint32_t p_par = pdbl ? ((j >> 1) & 1) : (j & 1);
-      const uint32_t p_addr = p_addr0 + pb * 16;
-      mbar_wait(KNOBS ? &p_free[(q * 2 + h) * 2 + pb] : &p_free[q * 2 + h], p_par ^ 1, 38);   // previous use consumed
+      mbar_wait(&p_free[q * 2 + h], (j & 1) ^ 1, 38);   // previous use consumed
       tc_fence_after();
       ESF_TICK(4)   // wait p_free
       if (j > 0 && any_raise) {
-        // O may only be touched while no P.V MMA of this (q, h) is in flight: with two P buffers that also means the
-        // MMA of tile j - 1 (the other buffer)
-        if (pdbl) {
-          mbar_wait(&p_free[(q * 2 + h) * 2 + (pb ^ 1)], ((j - 1) >> 1) & 1, 40);
-          tc_fence_after();
-        }
+        // O may only be touched while no P.V MMA of this (q, h) is in flight
         for (int c0 = 0; c0 < p.DVp; c0 += 16) {
           float o[16];
           tmem_ld16(o_addr + c0, o);
@@ -942,12 +708,10 @@ __global__ void __launch_bounds__(kV2Threads, 1) attn_tc_v2_kernel(const __grid_
         }
       }
       tmem_st16_b32(p_addr, pk);
-      if (!ESF_ATTN_LATE_HANDOFF || j + 1 == nt) {   // otherwise handed over from inside the next tile's exponentials
-        tmem_wait_st();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(KNOBS ? &p_full[(q * 2 + h) * 2 + pb] : &p_full[q * 2 + h]);
-      }
+      tmem_wait_st();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&p_full[q * 2 + h]);
       ESF_TICK(5)   // O rescale + P store + p_full arrive
       if (j + 1 < nt) {
         mbar_wait(&s_full[q * 2 + (buf ^ 1)], ((j + 1) >> 1) & 1, 37);
@@ -1232,31 +996,10 @@ struct AttnTcOp : esf_op {
   dim3 grid;
   int smem_bytes = 0;
   int v2 = 0;
-  int poly = 0;   // pairs of every 8 whose exponential runs on the FMA pipe (v2 only)
-  int pipe = 0;   // software-pipelined softmax loop (experiment, ESF_ATTN_PIPE=1)
   int launch(cudaStream_t stream) override {
     if (v2) {
-#define ESF_V2_LAUNCH(PL)                                                                                   \
-  if (params.f16) attn_tc_v2_kernel<true, PL, false><<<grid, kV2Threads, smem_bytes, stream>>>(params);      \
-  else attn_tc_v2_kernel<false, PL, false><<<grid, kV2Threads, smem_bytes, stream>>>(params);
-      if (pipe) {
-        if (params.f16) attn_tc_v2_kernel<true, 0, false, true><<<grid, kV2Threads, smem_bytes, stream>>>(params);
-        else attn_tc_v2_kernel<false, 0, false, true><<<grid, kV2Threads, smem_bytes, stream>>>(params);
-        return check_launch("attn_tc_v2_kernel");
-      }
-      if (params.pdbl || params.qk_async) {   // experiment build of the default (MUFU-only) loop
-        if (params.f16) attn_tc_v2_kernel<true, 0, true><<<grid, kV2Threads, smem_bytes, stream>>>(params);
-        else attn_tc_v2_kernel<false, 0, true><<<grid, kV2Threads, smem_bytes, stream>>>(params);
-        return check_launch("attn_tc_v2_kernel");
-      }
-      switch (poly) {
-        case 1: ESF_V2_LAUNCH(1) break;
-        case 2: ESF_V2_LAUNCH(2) break;
-        case 3: ESF_V2_LAUNCH(3) break;
-        case 4: ESF_V2_LAUNCH(4) break;
-        default: ESF_V2_LAUNCH(0) break;
-      }
-#undef ESF_V2_LAUNCH
+      if (params.f16) attn_tc_v2_kernel<true><<<grid, kV2Threads, smem_bytes, stream>>>(params);
+      else attn_tc_v2_kernel<false><<<grid, kV2Threads, smem_bytes, stream>>>(params);
       return check_launch("attn_tc_v2_kernel");
     }
     if (params.split) attn_tc_kernel<true><<<grid, kTcThreads, smem_bytes, stream>>>(params);
@@ -1447,8 +1190,6 @@ static int attn_tc_create_impl(const void* packed, const void* v_lo, int32_t B, 
     }
   }
   p.nsteps1 = n1, p.nsteps2 = n2;
-  if (const char* env = getenv("ESF_ATTN_QK_STEPS_DBG"))   // timing experiment only (drops logit correction terms)
-    if (atoi(env) > 0) p.nsteps2 = std::min(p.nsteps2, atoi(env));
   p.q_tile_bytes = 128 * g.KQ * 2;
   p.k_tile_bytes = kTcBN * g.KQ * 2;
   p.v_tile_bytes = g.DVp * 128;
@@ -1458,29 +1199,6 @@ static int attn_tc_create_impl(const void* packed, const void* v_lo, int32_t B, 
     p.v_half = p.v_tile_bytes;
     p.v_tile_bytes *= 2;
     op->v2 = 0;
-  }
-  {
-    // Measured (round 2, gpurun_out/r2_s4, profiles/r2_attention_experiments.md): a second P buffer (d < 32) and an
-    // independent Q.K^T issue of the two query tiles are both correct (kernel tests) and change nothing: d = 8
-    // 2.993 / 3.002 / 2.980 / 2.989 ms, d = 32 3.214 / 3.212 / 3.219 / 3.217 ms (16 clips, N = 25 088; off-off, P, QK,
-    // both).  The waits they remove (ncu: 4.7 % + 6 % of the softmax warps' samples) are not what bounds the loop.
-    // Both stay OFF by default; ESF_ATTN_PDBL=1 / ESF_ATTN_QKASYNC=1 enable them for A/B runs.
-    const char* e = getenv("ESF_ATTN_PDBL");
-    p.pdbl = (op->v2 && g.DVp <= 32 && e && atoi(e) == 1) ? 1 : 0;
-  }
-  {
-    const char* e = getenv("ESF_ATTN_QKASYNC");   // A/B knob: 1 = independent issue of the two query tiles
-    p.qk_async = (e && atoi(e) == 1) ? 1 : 0;
-  }
-  {
-    const char* e = getenv("ESF_ATTN_PIPE");
-    op->pipe = (op->v2 && e && atoi(e) == 1) ? 1 : 0;
-    if (op->pipe) p.pdbl = p.qk_async = 0;
-  }
-  {
-    const char* e = getenv("ESF_ATTN_POLY");   // experiment knob; default chosen from measurements (see header)
-    op->poly = e ? atoi(e) : kV2DefaultPoly;
-    if (op->poly < 0 || op->poly > 4) op->poly = 0;
   }
   // v1 streams P through 2 x 16 KB of shared memory; v2 keeps P in TMEM and needs 2 KB for the split-K maxima
   const int fixed = 1024 + 2 * (int)p.q_tile_bytes + 512 + (op->v2 ? 2048 : 2 * (p.split ? 32768 : 16384));
@@ -1509,20 +1227,9 @@ static int attn_tc_create_impl(const void* packed, const void* v_lo, int32_t B, 
       if (e == cudaSuccess)
         e = cudaFuncSetAttribute(attn_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
       if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(attn_tc_v2_kernel<true, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
+        e = cudaFuncSetAttribute(attn_tc_v2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
       if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(attn_tc_v2_kernel<false, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
-      if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(attn_tc_v2_kernel<true, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
-      if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(attn_tc_v2_kernel<false, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
-#define ESF_V2_ATTR(PL)                                                                                                  \
-  if (e == cudaSuccess)                                                                                                  \
-    e = cudaFuncSetAttribute(attn_tc_v2_kernel<true, PL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);    \
-  if (e == cudaSuccess)                                                                                                  \
-    e = cudaFuncSetAttribute(attn_tc_v2_kernel<false, PL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
-      ESF_V2_ATTR(0) ESF_V2_ATTR(1) ESF_V2_ATTR(2) ESF_V2_ATTR(3) ESF_V2_ATTR(4)
-#undef ESF_V2_ATTR
+        e = cudaFuncSetAttribute(attn_tc_v2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemLimit);
       if (e != cudaSuccess) rc = set_error(ESF_ERR_CUDA, "cudaFuncSetAttribute(attn_tc) failed: %s", cudaGetErrorString(e));
       else if (slot) *slot = 1;
     }

@@ -74,14 +74,6 @@ struct __align__(64) IgemmParams {
   // per-clip weights (Non-local block: the "weight" matrix of a clip is its own phi / g^T rows): the packed weight
   // matrices of all clips are stacked along n, b_clip_rows rows each, and an M tile never spans two clips (bb = 1)
   int b_clip_rows;
-  // T-halo mode (halo_g > 0): the taps of a group differ only by their T offset, stride 1.  The activation tile is
-  // loaded ONCE per (group, chunk) with halo_g - 1 extra T planes, and tap j of the group is the same smem tile read
-  // from row j * (bw * bh) on -- a descriptor offset of whole swizzle atoms because bw * bh is a multiple of 8 and
-  // bb = 1.  The A tiles then live in their own ring (a_stages, a_full / a_empty); rows >= `rows` of the M tile
-  // accumulate garbage that is never stored.  taps[g * halo_g] carries the group's map / W / H / first T offset.
-  int halo_g, halo_step16, a_stages;
-  uint32_t a_stride;   // bytes between A stages (kAStageBytes; more when a haloed tile has more than 128 rows)
-  int tap_k[kMaxTaps];   // K block (in the packed weights) of every tap in kernel order
   uint32_t dv_mul[5], dv_shr[5];   // magic numbers of the divisions by n_tiles, ncb, tw, th, tt (finish_op)
 };
 
@@ -283,7 +275,7 @@ __global__ void __launch_bounds__(kThreads, 1) igemm_kernel(const __grid_constan
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* smem_a = smem;
-  uint8_t* smem_b = smem_a + p.a_stages * p.a_stride;
+  uint8_t* smem_b = smem_a + p.stages * kAStageBytes;
   uint8_t* smem_out = smem_b + p.stages * p.b_stride;
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_out + p.obufs * kOutStageBytes);
   uint64_t* empty_bar = full_bar + kMaxStages;
@@ -291,9 +283,7 @@ __global__ void __launch_bounds__(kThreads, 1) igemm_kernel(const __grid_constan
   uint64_t* tmem_empty = tmem_full + 2;
   uint64_t* res_full = tmem_empty + 2;
   uint64_t* buf_free = res_full + kMaxOutBufs;
-  uint64_t* a_full = buf_free + kMaxOutBufs;
-  uint64_t* a_empty = a_full + kMaxStages;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(a_empty + kMaxStages);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(buf_free + kMaxOutBufs);
 
   const int warp = uniform_warp_idx();
   const int lane = threadIdx.x & 31;
@@ -311,11 +301,6 @@ __global__ void __launch_bounds__(kThreads, 1) igemm_kernel(const __grid_constan
       mbar_init(&res_full[a], 1);
       mbar_init(&buf_free[a], 1);
     }
-    if (p.halo_g)
-      for (int a = 0; a < p.a_stages; ++a) {
-        mbar_init(&a_full[a], 1);
-        mbar_init(&a_empty[a], 1);
-      }
     fence_barrier_init();
   }
   if (warp == kProducerWarp && lane == 0) {
@@ -335,63 +320,25 @@ __global__ void __launch_bounds__(kThreads, 1) igemm_kernel(const __grid_constan
   const int num_kb = p.num_taps * p.kchunks;
 
   if (warp == kProducerWarp) {
-    if (p.halo_g) {
-      int stage = 0, as = 0;
-      uint32_t phase = 0, aphase = 0;
-      const int groups = p.num_taps / p.halo_g;
-      for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-        const TileCoord tc = tile_coord(p, tile);
-        for (int g = 0; g < groups; ++g) {
-          const int4 tp = p.taps[g * p.halo_g];
-          for (int ch = 0; ch < p.kchunks; ++ch) {
-            mbar_wait(&a_empty[as], aphase ^ 1, 7);
-            if (elect_one()) {
-              mbar_arrive_expect_tx(&a_full[as], p.a_bytes);
-              tma_load_5d(smem_a + as * p.a_stride, &p.a_maps[tp.x], &a_full[as],
-                          p.a_c_base + tc.cb * p.a_cb_stride + ch * p.kc, tc.w0 + tp.y, tc.h0 + tp.z, tc.t0 + tp.w, tc.b0);
-            }
-            __syncwarp();
-            if (++as == p.a_stages) {
-              as = 0;
-              aphase ^= 1;
-            }
-            for (int j = 0; j < p.halo_g; ++j) {
-              mbar_wait(&empty_bar[stage], phase ^ 1, 1);
-              if (elect_one()) {
-                mbar_arrive_expect_tx(&full_bar[stage], p.b_bytes);
-                tma_load_2d(smem_b + stage * p.b_stride, &p.b_map, &full_bar[stage],
-                            (p.tap_k[g * p.halo_g + j] * p.kchunks + ch) * p.kc, tc.n_idx * p.n_tile);
-              }
-              __syncwarp();
-              if (++stage == p.stages) {
-                stage = 0;
-                phase ^= 1;
-              }
-            }
+    int stage = 0;
+    uint32_t phase = 0;
+    for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
+      const TileCoord tc = tile_coord(p, tile);
+      for (int tap = 0; tap < p.num_taps; ++tap) {
+        const int4 tp = p.taps[tap];
+        for (int ch = 0; ch < p.kchunks; ++ch) {
+          mbar_wait(&empty_bar[stage], phase ^ 1, 1);
+          if (elect_one()) {
+            mbar_arrive_expect_tx(&full_bar[stage], p.a_bytes + p.b_bytes);
+            tma_load_5d(smem_a + stage * kAStageBytes, &p.a_maps[tp.x], &full_bar[stage],
+                        p.a_c_base + tc.cb * p.a_cb_stride + ch * p.kc, tc.w0 + tp.y, tc.h0 + tp.z, tc.t0 + tp.w, tc.b0);
+            tma_load_2d(smem_b + stage * p.b_stride, &p.b_map, &full_bar[stage],
+                        (tap * p.kchunks + ch) * p.kc, tc.n_idx * p.n_tile + tc.b0 * p.b_clip_rows);
           }
-        }
-      }
-    } else {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-        const TileCoord tc = tile_coord(p, tile);
-        for (int tap = 0; tap < p.num_taps; ++tap) {
-          const int4 tp = p.taps[tap];
-          for (int ch = 0; ch < p.kchunks; ++ch) {
-            mbar_wait(&empty_bar[stage], phase ^ 1, 1);
-            if (elect_one()) {
-              mbar_arrive_expect_tx(&full_bar[stage], p.a_bytes + p.b_bytes);
-              tma_load_5d(smem_a + stage * p.a_stride, &p.a_maps[tp.x], &full_bar[stage],
-                            p.a_c_base + tc.cb * p.a_cb_stride + ch * p.kc, tc.w0 + tp.y, tc.h0 + tp.z, tc.t0 + tp.w, tc.b0);
-              tma_load_2d(smem_b + stage * p.b_stride, &p.b_map, &full_bar[stage],
-                          (p.tap_k[tap] * p.kchunks + ch) * p.kc, tc.n_idx * p.n_tile + tc.b0 * p.b_clip_rows);
-            }
-            __syncwarp();
-            if (++stage == p.stages) {
-              stage = 0;
-              phase ^= 1;
-            }
+          __syncwarp();
+          if (++stage == p.stages) {
+            stage = 0;
+            phase ^= 1;
           }
         }
       }
@@ -402,57 +349,12 @@ __global__ void __launch_bounds__(kThreads, 1) igemm_kernel(const __grid_constan
       const uint32_t idesc = make_idesc_16(128, p.n_tile, p.f16);
       const uint32_t desc_hi = kmajor_desc_hi(p.sbo, p.layout_type);
       const uint32_t a_lo0 = kmajor_desc_lo(smem_u32(smem_a)), b_lo0 = kmajor_desc_lo(smem_u32(smem_b));
-      const uint32_t a_step = p.a_stride >> 4, b_step = p.b_stride >> 4;
+      const uint32_t a_step = kAStageBytes >> 4, b_step = p.b_stride >> 4;
       const int ksteps = p.kc >> 4;
       int stage = 0;
       uint32_t phase = 0;
       uint32_t a_lo = a_lo0, b_lo = b_lo0;
       int iter = 0;
-      if (p.halo_g) {
-        int as = 0;
-        uint32_t aphase = 0;
-        const int groups = p.num_taps / p.halo_g;
-        const int nsteps = groups * p.kchunks;
-        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++iter) {
-          const int acc = iter & 1;
-          const uint32_t acc_phase = (iter >> 1) & 1;
-          mbar_wait(&tmem_empty[acc], acc_phase ^ 1, 2);
-          tc_fence_after();
-          const uint32_t d_tmem = tmem_base + acc * p.n_tile;
-          uint32_t accum = 0;
-          for (int st = 0; st < nsteps; ++st) {
-            mbar_wait(&a_full[as], aphase, 8);
-            tc_fence_after();
-            const uint32_t a_tile = a_lo0 + as * a_step;
-            for (int j = 0; j < p.halo_g; ++j) {
-              mbar_wait(&full_bar[stage], phase, 3);
-              tc_fence_after();
-              if (elect_one()) {
-                const uint32_t aj = a_tile + j * p.halo_step16;
-                for (int k = 0; k < ksteps; ++k)
-                  umma_bf16_lohi(d_tmem, aj + 2 * k, desc_hi, b_lo + 2 * k, desc_hi, idesc, k ? 1u : accum);
-                umma_commit(&empty_bar[stage]);
-                if (j == p.halo_g - 1) {
-                  umma_commit(&a_empty[as]);
-                  if (st == nsteps - 1) umma_commit(&tmem_full[acc]);
-                }
-              }
-              __syncwarp();
-              accum = 1;
-              b_lo += b_step;
-              if (++stage == p.stages) {
-                stage = 0;
-                phase ^= 1;
-                b_lo = b_lo0;
-              }
-            }
-            if (++as == p.a_stages) {
-              as = 0;
-              aphase ^= 1;
-            }
-          }
-        }
-      } else
       for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++iter) {
         const int acc = iter & 1;
         const uint32_t acc_phase = (iter >> 1) & 1;
@@ -561,19 +463,6 @@ EncodeTiledFn get_encode_fn() {
 // long K loop need the stages.
 static void plan_smem(IgemmParams& p, int* smem_bytes) {
   const int avail = kSmemLimit - 1024 - 512;
-  if (p.halo_g) {
-    // own A ring (one haloed tile per (group, chunk)), B ring as deep as two tap groups
-    p.a_stages = 3;
-    if (p.a_stride == 0) p.a_stride = kAStageBytes;
-    int R = p.has_res ? 4 : 3;
-    p.obufs = R;
-    const int left = avail - R * kOutStageBytes - p.a_stages * (int)p.a_stride;
-    p.stages = std::max(2, std::min({left / (int)p.b_stride, kMaxStages, 2 * p.halo_g + 2}));
-    *smem_bytes = 1024 + 512 + R * kOutStageBytes + p.a_stages * (int)p.a_stride + p.stages * (int)p.b_stride;
-    return;
-  }
-  p.a_stride = kAStageBytes;
-  for (int i = 0; i < kMaxTaps; ++i) p.tap_k[i] = i;
   const int stage_bytes = kAStageBytes + (int)p.b_stride;
   const int ksteps = p.num_taps * p.kchunks;
   const int want_stages = std::min(p.n_tile >= 256 ? 3 : 4, ksteps + 1);
@@ -582,7 +471,6 @@ static void plan_smem(IgemmParams& p, int* smem_bytes) {
   p.obufs = R;
   const int stages = (avail - R * kOutStageBytes) / stage_bytes;
   p.stages = std::max(2, std::min(stages, kMaxStages));
-  p.a_stages = p.stages;
   *smem_bytes = 1024 + 512 + R * kOutStageBytes + p.stages * stage_bytes;
 }
 
@@ -708,29 +596,6 @@ static void choose_box(int W, int H, int T, int B, int* obw, int* obh, int* obt,
   *obw = rb[0], *obh = rb[1], *obt = rb[2], *obb = rb[3];
 }
 
-// T-halo tile for a kT x 1 x 1, stride-1 conv: (bw, bh) with bw * bh a multiple of 8 and bt output planes such that
-// bw * bh * (bt + kT - 1) <= 128.  Picks the tile that loads the fewest rows; returns the loaded rows relative to the
-// ordinary one-box-per-tap scheme (< 1: fewer L2 -> smem bytes), or 0 when no such tile exists.
-static double choose_halo_box(int W, int H, int T, int kT, int* obw, int* obh, int* obt) {
-  long long best = -1;
-  int ordinary[4];
-  choose_box(W, H, T, 1, &ordinary[0], &ordinary[1], &ordinary[2], &ordinary[3]);
-  for (int bw = 1; bw <= std::min(W, 128); ++bw)
-    for (int bh = 1; bh <= std::min(H, 128 / bw); ++bh) {
-      const int r = bw * bh;
-      if (r % 8 != 0) continue;
-      const int bt = std::min(T, 128 / r - (kT - 1));
-      if (bt < 1) continue;
-      // rows actually fetched: planes outside [0, T) are TMA out-of-bounds fill, not traffic
-      const long long tiles_sp = (long long)cdiv(W, bw) * cdiv(H, bh);
-      long long planes = 0;
-      for (int t0 = 0; t0 < T; t0 += bt) planes += std::min(T, t0 + bt + kT / 2) - std::max(0, t0 - kT / 2);
-      const long long loaded = tiles_sp * r * planes;
-      if (best < 0 || loaded < best) best = loaded, *obw = bw, *obh = bh, *obt = bt;
-    }
-  if (best < 0) return 0.0;
-  return (double)best / ((double)W * H * T * kT);
-}
 
 
 static inline int floordiv(int a, int b) { return (a >= 0) ? a / b : -((-a + b - 1) / b); }
@@ -787,25 +652,11 @@ static int igemm_create_impl(const esf_conv_desc* d, int clip_weights, esf_op** 
   p.num_taps = num_taps;
   choose_box(Wo, Ho, To, clip_weights ? 1 : y.B, &p.bw, &p.bh, &p.bt, &p.bb);
   p.b_clip_rows = clip_weights ? n_pad : 0;
-  // T-halo mode for k x 1 x 1 layers: OFF by default (ESF_IGEMM_THALO=1: layers with n_tile <= 64 whose haloed tile
-  // loads < 0.7x the rows; =2: every k x 1 x 1 layer).  Measured on the fast pathway's thirteen 3x1x1 layers of the
-  // headline workload: correct, and the L2 -> smem bytes drop from 3x to 1.2x, but 1.25 ms -> 1.88 ms in total
-  // (64->16 @56^2: 0.42 -> 0.58 ms): with bw * bh = 8 only 112 of the 128 MMA rows are outputs and T = 32 splits into
-  // 14 + 14 + 4 planes, i.e. 1.5x the tiles -- these layers are bound by the per-tile hand-over (accumulator, epilogue,
-  // store), not by the activation loads.
-  {
-    const char* env = getenv("ESF_IGEMM_THALO");
-    const int mode = env ? atoi(env) : 0;
-    if (mode > 0 && !clip_weights && d->kT > 1 && d->kT <= 8 && d->kH == 1 && d->kW == 1 && d->sT == 1 && d->sH == 1 &&
-        d->sW == 1 && d->dT == 1 && d->pH == 0 && d->pW == 0 && (mode == 2 || n_tile <= 64)) {
-      int hw = 0, hh = 0, ht = 0;
-      const double rel = choose_halo_box(Wo, Ho, To, d->kT, &hw, &hh, &ht);
-      if (rel > 0.0 && (mode == 2 || rel < 0.7)) {
-        p.halo_g = d->kT;
-        p.bw = hw, p.bh = hh, p.bt = ht, p.bb = 1;
-      }
-    }
-  }
+  // A T-halo mode for k x 1 x 1 layers (one activation tile of bt + kT - 1 planes per chunk, shared by the kT taps)
+  // was measured on the fast pathway's thirteen 3x1x1 layers of the headline workload and removed: correct, and the
+  // L2 -> smem bytes drop from 3x to 1.2x, but 1.25 ms -> 1.88 ms in total (64->16 @56^2: 0.42 -> 0.58 ms): with
+  // bw * bh = 8 only 112 of the 128 MMA rows are outputs and T = 32 splits into 14 + 14 + 4 planes, i.e. 1.5x the
+  // tiles -- these layers are bound by the per-tile hand-over (accumulator, epilogue, store), not by the activation loads.
   p.tw = cdiv(Wo, p.bw);
   p.th = cdiv(Ho, p.bh);
   p.tt = cdiv(To, p.bt);
@@ -821,10 +672,6 @@ static int igemm_create_impl(const esf_conv_desc* d, int clip_weights, esf_op** 
   p.a_cb_stride = p.out_cb_w = 0;
   const int row_bytes = kc * 2;
   p.a_bytes = p.rows * row_bytes;
-  if (p.halo_g) {
-    p.a_bytes = p.bw * p.bh * (p.bt + p.halo_g - 1) * row_bytes;
-    p.halo_step16 = (p.bw * p.bh * row_bytes) >> 4;
-  }
   p.b_bytes = n_tile * row_bytes;
   p.b_stride = (p.b_bytes + 1023) & ~1023u;
   p.sbo = 8 * row_bytes;
@@ -876,11 +723,10 @@ static int igemm_create_impl(const esf_conv_desc* d, int clip_weights, esf_op** 
           }
           char* base = static_cast<char*>(x.ptr) + 2 * (ph.pt * x.sT + ph.ph * x.sH + ph.pw * x.sW);
           rc = encode_act_map(&p.a_maps[idx], dt16, 2, base, x.C, Wp, Hp, Tp, x.B,
-                              x.sW * d->sW, x.sH * d->sH, x.sT * d->sT, x.sB, kc, p.bw, p.bh,
-                              p.halo_g ? p.bt + p.halo_g - 1 : p.bt, p.bb, swizzle_for_row_bytes(row_bytes), "activation");
+                              x.sW * d->sW, x.sH * d->sH, x.sT * d->sT, x.sB, kc, p.bw, p.bh, p.bt, p.bb,
+                              swizzle_for_row_bytes(row_bytes), "activation");
         }
         p.taps[tap_i] = make_int4(idx, qw, qh, qt);
-        if (p.halo_g) p.tap_k[tap_i] = tap_i;   // kT x 1 x 1: one group, taps already ordered by kt
       }
   // unused map slots alias map 0 so that the kernel parameter block is fully initialised
   if (rc == ESF_OK)
@@ -986,21 +832,11 @@ extern "C" int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int
   esf_igemm_geometry(64, N, &kc, &kchunks, &n_tile, &n_pad);
   p.kc = 64, p.kchunks = 1, p.n_tile = n_tile, p.n_tiles = n_pad / n_tile, p.num_taps = num_taps;
   choose_box(1, Ho, To, B, &p.bw, &p.bh, &p.bt, &p.bb);
-  // T-halo mode (see IgemmParams::halo_g), opt-in with ESF_STEM_THALO=1: the kT taps of one kh share ONE activation
-  // tile of (bt + kT - 1) planes x 8 rows -- 7 tile loads per M tile instead of 35 for the 5x7x7 stem -- and the tile
-  // keeps all 128 MMA rows (16 output planes x 8 rows; the 160-row haloed tile gets a 20 KB stage).  Measured: bit-correct
-  // (kernel + model tests), 4x fewer L2 -> smem bytes, but 1.20 -> 1.36 ms: the stem is not bound by its 11.6 TB/s of
-  // smem fill either.  140 MMAs of 128 x 64 x 16 per tile take ~100 cycles each instead of 32 -- the serial
-  // wait / issue / commit loop of the MMA warp per 4-MMA k-block is the limit, and the halo adds a barrier to it.
-  {
-    const char* env = getenv("ESF_STEM_THALO");
-    if (env && atoi(env) != 0 && kT > 1 && kT <= 8 && Ho >= 8) {
-      p.halo_g = kT;
-      p.bw = 1, p.bh = 8, p.bt = std::min(To, 16), p.bb = 1;
-      p.a_stride = (uint32_t)((8 * (p.bt + kT - 1) * 128 + 1023) & ~1023);
-      p.halo_step16 = (8 * 128) >> 4;
-    }
-  }
+  // A T-halo mode (the kT taps of one kh sharing ONE activation tile of (bt + kT - 1) planes x 8 rows -- 7 tile loads
+  // per M tile instead of 35 for the 5x7x7 stem) was measured and removed: bit-correct, 4x fewer L2 -> smem bytes, but
+  // 1.20 -> 1.36 ms: the stem is not bound by its 11.6 TB/s of smem fill either.  140 MMAs of 128 x 64 x 16 per tile
+  // take ~100 cycles each instead of 32 -- the serial wait / issue / commit loop of the MMA warp per 4-MMA k-block is
+  // the limit, and the halo adds a barrier to it.
   p.tw = 1, p.th = cdiv(Ho, p.bh), p.tt = cdiv(To, p.bt), p.tb = cdiv(B, p.bb);
   p.rows = p.bw * p.bh * p.bt * p.bb;
   p.ncb = cdiv(Wo, kStemWB);
@@ -1013,7 +849,6 @@ extern "C" int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int
   }
   p.num_tiles = (int)ntiles;
   p.a_bytes = p.rows * 128, p.b_bytes = n_tile * 128, p.b_stride = (p.b_bytes + 1023) & ~1023u;
-  if (p.halo_g) p.a_bytes = 8 * (p.bt + kT - 1) * 128;
   p.sbo = 1024, p.layout_type = 2;
   p.bias = bias_tiled, p.act = act, p.has_res = 0, p.out_f32 = y->dtype == ESF_F32;
   p.f16 = y->dtype == ESF_F16 || y->dtype == ESF_F32;
@@ -1031,9 +866,7 @@ extern "C" int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int
   int nmaps = 0;
   for (int it = 0; it < kT && rc == ESF_OK; ++it)
     for (int ih = 0; ih < kH && rc == ESF_OK; ++ih) {
-      // kernel order of the taps: (kt, kh) as packed in the weights, or kh-major groups of kT taps in T-halo mode
-      const int tap_i = p.halo_g ? ih * kT + it : it * kH + ih;
-      p.tap_k[tap_i] = it * kH + ih;
+      const int tap_i = it * kH + ih;   // (kt, kh) as packed in the weights
       const int oh = ih - pH;
       const int qh = floordiv(oh, sH);
       const int ph = oh - qh * sH;
@@ -1050,7 +883,7 @@ extern "C" int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int
         char* base = static_cast<char*>(const_cast<void*>(xp)) + 2LL * ph * pitch;
         rc = encode_act_map(&p.a_maps[nmaps], dt16, 2, base, pitch, 1, Hp, T, B,
                             (int64_t)sH * pitch, (int64_t)sH * pitch, (int64_t)H * pitch, (int64_t)T * H * pitch, 64,
-                            1, p.bh, p.halo_g ? p.bt + kT - 1 : p.bt, p.bb, CU_TENSOR_MAP_SWIZZLE_128B, "stem activation");
+                            1, p.bh, p.bt, p.bb, CU_TENSOR_MAP_SWIZZLE_128B, "stem activation");
         phase_map[ph] = nmaps++;
       }
       p.taps[tap_i] = make_int4(phase_map[ph], 0, qh, it - pT);
@@ -1109,9 +942,9 @@ namespace esf {
 constexpr int kTbThreads = 6 * 32;   // TMA producer, MMA issuer, 4 epilogue warps (one per TMEM lane quarter)
 constexpr int kTbMaxKH = 8;
 constexpr int kTbMaxStages = 8;
-// Timing experiments are compile-time instantiations (template parameter DBG; bits: 1 no MMAs, 2 no tile loads, 4 no
-// epilogue work, 16 every MMA N = NB, 32 one k-step per tap (wrong results), 64 two MMA issuers), built only with ESF_NVCC_EXTRA=-DESF_TB_DBG_VARIANTS and
-// selected by ESF_STEM_TBAND_DBG.  Run-time switches in these loops are not free.
+// Where the time of this kernel goes was measured with timing variants that switched parts of the work off (no MMAs, no
+// tile loads, no epilogue, one k-step per tap, two alternating MMA issuers; profiles/r2_stem_tband.md).  They were
+// compile-time instantiations because run-time switches in these loops are not free, and they were removed afterwards.
 
 struct __align__(64) StemTbParams {
   CUtensorMap a_maps[kMaxAMaps];   // one per row phase of the H stride
@@ -1142,8 +975,8 @@ struct __align__(64) StemTbParams {
     if (c1 > 0) umma_bf16_lohi(tmem_base, a_lo + 2 * (ks), desc_hi, b1 + 2 * (ks), desc_hi, si1, 1);   \
   }
 
-template <int KSTEPS, bool F16, int ESF_TB_DBG = 0>
-__global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __grid_constant__ StemTbParams p) {
+template <int KSTEPS, bool F16>
+__global__ void __launch_bounds__(kTbThreads, 1) stem_tband_kernel(const __grid_constant__ StemTbParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* smem_b = smem;
@@ -1154,7 +987,7 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
   uint64_t* acc_full = a_empty + kTbMaxStages;   // [nslots <= 32]
   uint64_t* acc_free = acc_full + 32;
   uint64_t* b_full = acc_free + 32;
-  uint64_t* tok = b_full + 1;          // [2] (timing variant 64: two MMA issuers pass a token)
+  uint64_t* tok = b_full + 1;          // [2] unused since the two-issuer timing variant was removed (layout kept)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tok + 2);
   float* bias_sh = reinterpret_cast<float*>(bars) + 256;   // [NB <= 64], 1 KB into the 2 KB barrier / bias area
 
@@ -1209,12 +1042,9 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
         for (int kh = 0; kh < kH; ++kh) {
           mbar_wait(&a_empty[stage], phase ^ 1, 51);
           if (elect_one()) {
-            if (ESF_TB_DBG & 2) mbar_arrive(&a_full[stage]);
-            else {
-              mbar_arrive_expect_tx(&a_full[stage], a_bytes);
-              tma_load_5d(smem_a + stage * kAStageBytes, &p.a_maps[p.a_map_of_kh[kh]], &a_full[stage], c0, 0,
-                          h0 + p.qh_of_kh[kh], g, b0);
-            }
+            mbar_arrive_expect_tx(&a_full[stage], a_bytes);
+            tma_load_5d(smem_a + stage * kAStageBytes, &p.a_maps[p.a_map_of_kh[kh]], &a_full[stage], c0, 0,
+                        h0 + p.qh_of_kh[kh], g, b0);
           }
           __syncwarp();
           if (++stage == stages) {
@@ -1222,79 +1052,6 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
             phase ^= 1;
           }
         }
-    }
-  } else if ((ESF_TB_DBG & 64) && (warp == 1 || warp == 6)) {
-    // ------------------------------------------------------------------ timing variant: TWO MMA issuers, alternate taps
-    // The token fixes the global issue order (tap n before tap n + 1), so the accumulation order stays deterministic;
-    // the question is whether the ~50-cycle start-up of an MMA is hidden when consecutive taps come from two threads.
-    const int me = warp == 1 ? 0 : 1;
-    const uint32_t idesc0 = make_idesc_16(128, 0, F16);
-    const uint32_t desc_hi = kmajor_desc_hi(1024, 2);
-    const uint32_t a_lo0 = kmajor_desc_lo(smem_u32(smem_a)), b_lo0 = kmajor_desc_lo(smem_u32(smem_b));
-    const uint32_t b_kh_step = p.b_tile_bytes >> 4, b_u_step = (uint32_t)(p.NB * 128) >> 4;
-    const int kT = p.kT, kH = p.kH, pT = p.pT, T = p.T, To = p.To, NB = p.NB, nslots = p.nslots;
-    const int stages = p.stages, num_tiles = p.num_tiles, back = kT - 1 - pT;
-    mbar_wait(b_full, 0, 52);
-    tc_fence_after();
-    int stage = 0, n = 0;
-    uint32_t phase = 0, free_bits = 0, uses = 0, a_rel = 0;
-    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-      const uint32_t a_base = a_lo0 + (((tile % p.ncb) & p.odd_shift) ? 1u : 0u);
-      for (int g = 0; g < T; ++g) {
-        const int t_base = g + pT - kT + 1;
-        const int t_lo = max(t_base, 0), t_hi = min(g + pT, To - 1);
-        const int new_lo = g == 0 ? 0 : g + pT;
-        for (int t = max(new_lo, t_lo); t <= t_hi; ++t) {
-          const int s = t & smask;
-          mbar_wait(&acc_free[s], ((free_bits >> s) & 1) ^ 1, 53);
-          free_bits ^= 1u << s;
-        }
-        tc_fence_after();
-        auto seg_d = [&](int a) { return tmem_base + (uint32_t)((a & smask) * NB); };
-        auto seg_b = [&](int a) { return (uint32_t)(a - t_base) * b_u_step; };
-        auto seg_i = [&](int c) { return idesc0 | ((uint32_t)((c * NB) >> 3) << 17); };
-        const int cnt = t_hi - t_lo + 1;
-        const int c0 = min(cnt, nslots - (t_lo & smask)), c1 = cnt - c0;
-        const uint32_t sd0 = seg_d(t_lo), sb0 = seg_b(t_lo), si0 = seg_i(c0);
-        const uint32_t sb1 = seg_b(t_lo + c0), si1 = seg_i(c1);
-        const int old_cnt = max(min(new_lo - 1, t_hi) - t_lo + 1, 0);
-        const int o0 = min(old_cnt, c0), o1 = old_cnt - o0;
-        const int nw_lo = max(new_lo, t_lo), nw_cnt = t_hi - nw_lo + 1;
-        const uint32_t oi0 = seg_i(o0), oi1 = seg_i(o1);
-        const uint32_t nd = seg_d(nw_lo), nb = seg_b(nw_lo), ni = seg_i(nw_cnt);
-        const int done_lo = max(g == T - 1 ? t_lo : g - back, 0), done_hi = g == T - 1 ? t_hi : g - back;
-        for (int kh = 0; kh < kH; ++kh, ++n) {
-          if ((n & 1) == me) {
-            const uint32_t a_lo = a_base + a_rel;
-            const uint32_t b0 = b_lo0 + sb0 + kh * b_kh_step, b1 = b_lo0 + sb1 + kh * b_kh_step;
-            mbar_wait(&a_full[stage], phase, 54);
-            mbar_wait(&tok[me], (uses & 1) ^ (me ? 0u : 1u), 56);     // my turn: the other issuer has issued tap n - 1
-            ++uses;
-            tc_fence_after();
-            if (elect_one()) {
-              if (!(ESF_TB_DBG & 1)) {
-                if (kh == 0) {
-                  if (o0 > 0) umma_bf16_lohi(sd0, a_lo, desc_hi, b0, desc_hi, oi0, 1);
-                  if (o1 > 0) umma_bf16_lohi(tmem_base, a_lo, desc_hi, b1, desc_hi, oi1, 1);
-                  if (nw_cnt > 0) umma_bf16_lohi(nd, a_lo, desc_hi, b_lo0 + nb, desc_hi, ni, 0);
-                } else {
-                  ESF_TB_KSTEP(0)
-                }
-                if (KSTEPS > 1) ESF_TB_KSTEP(1)
-                if (KSTEPS > 2) ESF_TB_KSTEP(2)
-                if (KSTEPS > 3) ESF_TB_KSTEP(3)
-              }
-              mbar_arrive(&tok[me ^ 1]);
-              umma_commit(&a_empty[stage]);
-              if (kh == kH - 1)
-                for (int t = done_lo; t <= done_hi; ++t) umma_commit(&acc_full[t & smask]);
-            }
-            __syncwarp();
-          }
-          a_rel += kAStageBytes >> 4;
-          if (++stage == stages) stage = 0, phase ^= 1, a_rel = 0;
-        }
-      }
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
@@ -1330,7 +1087,7 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
         // segment = frames [a, a + n) in consecutive slots: (D address, weight-row offset in 16 B units, idesc)
         auto seg_d = [&](int a) { return tmem_base + (uint32_t)((a & smask) * NB); };
         auto seg_b = [&](int a) { return (uint32_t)(a - t_base) * b_u_step; };
-        auto seg_i = [&](int n) { return idesc0 | ((uint32_t)((((ESF_TB_DBG & 16) ? min(n, 1) : n) * NB) >> 3) << 17); };
+        auto seg_i = [&](int n) { return idesc0 | ((uint32_t)((n * NB) >> 3) << 17); };
         // steady k-steps: [t_lo, t_hi], split where the slot ring wraps
         const int cnt = t_hi - t_lo + 1;
         const int c0 = min(cnt, nslots - (t_lo & smask)), c1 = cnt - c0;
@@ -1351,14 +1108,12 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
         mbar_wait(&a_full[stage], phase, 54);
         tc_fence_after();
         if (elect_one()) {
-          if (!(ESF_TB_DBG & 1)) {
-            if (o0 > 0) umma_bf16_lohi(sd0, a_lo, desc_hi, b0, desc_hi, oi0, 1);
-            if (o1 > 0) umma_bf16_lohi(tmem_base, a_lo, desc_hi, b1, desc_hi, oi1, 1);
-            if (nw_cnt > 0) umma_bf16_lohi(nd, a_lo, desc_hi, b_lo0 + nb, desc_hi, ni, 0);
-            if (KSTEPS > 1 && !(ESF_TB_DBG & 32)) ESF_TB_KSTEP(1)
-            if (KSTEPS > 2 && !(ESF_TB_DBG & 32)) ESF_TB_KSTEP(2)
-            if (KSTEPS > 3 && !(ESF_TB_DBG & 32)) ESF_TB_KSTEP(3)
-          }
+          if (o0 > 0) umma_bf16_lohi(sd0, a_lo, desc_hi, b0, desc_hi, oi0, 1);
+          if (o1 > 0) umma_bf16_lohi(tmem_base, a_lo, desc_hi, b1, desc_hi, oi1, 1);
+          if (nw_cnt > 0) umma_bf16_lohi(nd, a_lo, desc_hi, b_lo0 + nb, desc_hi, ni, 0);
+          if (KSTEPS > 1) ESF_TB_KSTEP(1)
+          if (KSTEPS > 2) ESF_TB_KSTEP(2)
+          if (KSTEPS > 3) ESF_TB_KSTEP(3)
           umma_commit(&a_empty[stage]);
           if (kH == 1)
             for (int t = done_lo; t <= done_hi; ++t) umma_commit(&acc_full[t & smask]);
@@ -1373,12 +1128,10 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
           mbar_wait(&a_full[stage], phase, 54);
           tc_fence_after();
           if (elect_one()) {
-            if (!(ESF_TB_DBG & 1)) {
-              ESF_TB_KSTEP(0)
-              if (KSTEPS > 1 && !(ESF_TB_DBG & 32)) ESF_TB_KSTEP(1)
-              if (KSTEPS > 2 && !(ESF_TB_DBG & 32)) ESF_TB_KSTEP(2)
-              if (KSTEPS > 3 && !(ESF_TB_DBG & 32)) ESF_TB_KSTEP(3)
-            }
+            ESF_TB_KSTEP(0)
+            if (KSTEPS > 1) ESF_TB_KSTEP(1)
+            if (KSTEPS > 2) ESF_TB_KSTEP(2)
+            if (KSTEPS > 3) ESF_TB_KSTEP(3)
             umma_commit(&a_empty[stage]);
             if (kh == kH - 1)
               for (int t = done_lo; t <= done_hi; ++t) umma_commit(&acc_full[t & smask]);
@@ -1410,31 +1163,30 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
         mbar_wait(&acc_full[s], (full_bits >> s) & 1, 55);
         full_bits ^= 1u << s;
         tc_fence_after();
-        if (!(ESF_TB_DBG & 4))
-          for (int c0 = 0; c0 < NB; c0 += 16) {
-            float v[16];
-            tmem_ld16(lane_addr + s * NB + c0, v);
-            if (valid && out_f32) {
+        for (int c0 = 0; c0 < NB; c0 += 16) {
+          float v[16];
+          tmem_ld16(lane_addr + s * NB + c0, v);
+          if (valid && out_f32) {
 #pragma unroll
-              for (int i = 0; i < 4; ++i) {
-                const float4 bv = *reinterpret_cast<const float4*>(bias_sh + c0 + 4 * i);
-                *reinterpret_cast<float4*>(yrow32 + c0 + 4 * i) =
-                    make_float4(apply_act(v[4 * i] + bv.x, act), apply_act(v[4 * i + 1] + bv.y, act),
-                                apply_act(v[4 * i + 2] + bv.z, act), apply_act(v[4 * i + 3] + bv.w, act));
-              }
-            } else if (valid) {
-              uint32_t pk[8];
-#pragma unroll
-              for (int i = 0; i < 4; ++i) {       // the bias vector comes from shared memory, four columns per load
-                const float4 bv = *reinterpret_cast<const float4*>(bias_sh + c0 + 4 * i);
-                pk[2 * i] = pack16x2(apply_act(v[4 * i] + bv.x, act), apply_act(v[4 * i + 1] + bv.y, act), F16);
-                pk[2 * i + 1] = pack16x2(apply_act(v[4 * i + 2] + bv.z, act), apply_act(v[4 * i + 3] + bv.w, act), F16);
-              }
-              uint4* dst = reinterpret_cast<uint4*>(yrow + c0);
-              dst[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-              dst[1] = make_uint4(pk[4], pk[5], pk[6], pk[7]);
+            for (int i = 0; i < 4; ++i) {
+              const float4 bv = *reinterpret_cast<const float4*>(bias_sh + c0 + 4 * i);
+              *reinterpret_cast<float4*>(yrow32 + c0 + 4 * i) =
+                  make_float4(apply_act(v[4 * i] + bv.x, act), apply_act(v[4 * i + 1] + bv.y, act),
+                              apply_act(v[4 * i + 2] + bv.z, act), apply_act(v[4 * i + 3] + bv.w, act));
             }
+          } else if (valid) {
+            uint32_t pk[8];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {       // the bias vector comes from shared memory, four columns per load
+              const float4 bv = *reinterpret_cast<const float4*>(bias_sh + c0 + 4 * i);
+              pk[2 * i] = pack16x2(apply_act(v[4 * i] + bv.x, act), apply_act(v[4 * i + 1] + bv.y, act), F16);
+              pk[2 * i + 1] = pack16x2(apply_act(v[4 * i + 2] + bv.z, act), apply_act(v[4 * i + 3] + bv.w, act), F16);
+            }
+            uint4* dst = reinterpret_cast<uint4*>(yrow + c0);
+            dst[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+            dst[1] = make_uint4(pk[4], pk[5], pk[6], pk[7]);
           }
+        }
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&acc_free[s]);
@@ -1452,24 +1204,6 @@ __global__ void __launch_bounds__(kTbThreads + 32, 1) stem_tband_kernel(const __
 
 using StemTbKernel = void (*)(const StemTbParams);
 static StemTbKernel stem_tband_fn(int ksteps, bool f16) {
-#ifdef ESF_TB_DBG_VARIANTS
-  if (const char* env = getenv("ESF_STEM_TBAND_DBG")) {
-    switch (atoi(env)) {
-      case 1: return stem_tband_kernel<3, true, 1>;
-      case 2: return stem_tband_kernel<3, true, 2>;
-      case 3: return stem_tband_kernel<3, true, 3>;
-      case 4: return stem_tband_kernel<3, true, 4>;
-      case 5: return stem_tband_kernel<3, true, 5>;
-      case 6: return stem_tband_kernel<3, true, 6>;
-      case 7: return stem_tband_kernel<3, true, 7>;
-      case 22: return stem_tband_kernel<3, true, 22>;
-      case 38: return stem_tband_kernel<3, true, 38>;
-      case 64: return stem_tband_kernel<3, true, 64>;
-      case 70: return stem_tband_kernel<3, true, 70>;
-      default: break;
-    }
-  }
-#endif
   switch (ksteps * 2 + (f16 ? 1 : 0)) {
     case 2: return stem_tband_kernel<1, false>;
     case 3: return stem_tband_kernel<1, true>;
@@ -1489,12 +1223,7 @@ struct StemTbOp : esf_op {
   int grid = 0;
   int smem_bytes = 0;
   int launch(cudaStream_t stream) override {
-    int threads = kTbThreads;
-#ifdef ESF_TB_DBG_VARIANTS
-    if (const char* env = getenv("ESF_STEM_TBAND_DBG"))
-      if (atoi(env) & 64) threads += 32;     // the second MMA issuer of the timing variant
-#endif
-    stem_tband_fn(params.ksteps, params.f16 != 0)<<<grid, threads, smem_bytes, stream>>>(params);
+    stem_tband_fn(params.ksteps, params.f16 != 0)<<<grid, kTbThreads, smem_bytes, stream>>>(params);
     return check_launch("stem_tband_kernel");
   }
 };
@@ -1556,9 +1285,8 @@ extern "C" int esf_stem_tband_create(const void* xp, int32_t B, int32_t Cin, int
   p.ncb = Wo / WB, p.a_cb_stride = WB * sW * Cin;
   // TMA fetches rows that start in the middle of a 32 B sector at about 2/3 of the rate (measured: tile loads alone 0.59
   // -> 0.41 ms).  With Cin = 3 the blocks are 48 B apart, so every odd block is loaded 16 B early when the widened
-  // window still fits the same number of k-steps (ESF_STEM_TBAND_SHIFT=0: off, for A/B runs)
+  // window still fits the same number of k-steps
   p.odd_shift = ((p.a_cb_stride * 2) % 32 == 16 && win + 8 <= p.ksteps * 16) ? 1 : 0;
-  if (const char* env = getenv("ESF_STEM_TBAND_SHIFT")) p.odd_shift = p.odd_shift && atoi(env) != 0;
   int bw = 1, bt = 1;
   choose_box(1, Ho, 1, B, &bw, &p.bh, &bt, &p.bb);
   p.th = cdiv(Ho, p.bh), p.tb = cdiv(B, p.bb), p.rows = p.bh * p.bb;
@@ -1574,10 +1302,6 @@ extern "C" int esf_stem_tband_create(const void* xp, int32_t B, int32_t Cin, int
   p.y = static_cast<__nv_bfloat16*>(y->ptr), p.ysB = y->sB, p.ysT = y->sT, p.ysH = y->sH;
   p.stages = std::min(kTbMaxStages, (kSmemLimit - 1024 - 2048 - (int)(kH * p.b_tile_bytes)) / kAStageBytes);
   op->smem_bytes = 1024 + 2048 + kH * p.b_tile_bytes + p.stages * kAStageBytes;   // alignment slack, barriers + bias
-  {
-    const char* env = getenv("ESF_STEM_TBAND_STAGES");   // experiments: fewer activation stages
-    if (env && atoi(env) >= 2) p.stages = std::min(p.stages, atoi(env));
-  }
   const CUtensorMapDataType dt16 = p.f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
 
   int phase_map[8];

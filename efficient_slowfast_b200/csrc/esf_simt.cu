@@ -973,10 +973,6 @@ __global__ void __launch_bounds__(128) dwconv_march_kernel(const DirectParams p,
   }
 }
 
-static int dw_env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
 // Depthwise kT x 3 x 3 with SHARED-MEMORY HALO STAGING: the march above, fed by TMA instead of per-thread global loads.
 // A block of 128 threads owns a tile of cb channel groups (cb x 8 channels = one <= 128-byte row) x wbt column blocks of
 // 4 outputs x tt output planes and marches down `hs` output rows.  Per input row ONE 5-D TMA box
@@ -1201,23 +1197,6 @@ __global__ void __launch_bounds__(256, 2) dwconv_tma_kernel(const __grid_constan
     if constexpr (SW == 1) {
       // stride 1: input row hi feeds output rows hi+1 (kh 0), hi (kh 1), hi-1 (kh 2); row hi-1 is complete after it
       int hi = ho0 - 1;
-#ifdef ESF_DW_ROTATE_MOV
-      // one copy of the row body, the three accumulator sets rotated with register moves (32 MOVs per row, a third of
-      // the code size)
-      while (true) {
-        DW_ROW(2, 1, 0, hi, hi + 1 < ho1, hi >= ho0 && hi < ho1, hi - 1 >= ho0);
-        if (hi - 1 >= ho0) DW_STORE(0, hi - 1);
-        if (hi >= ho1) break;
-        ++hi;
-#pragma unroll
-        for (int o = 0; o < M::OW; ++o)
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const float fresh = m.acc[0][o][e];
-            m.acc[0][o][e] = m.acc[1][o][e], m.acc[1][o][e] = m.acc[2][o][e], m.acc[2][o][e] = fresh;
-          }
-      }
-#else
       while (true) {
         DW_ROW(2, 1, 0, hi, hi + 1 < ho1, hi >= ho0 && hi < ho1, hi - 1 >= ho0);
         if (hi - 1 >= ho0) DW_STORE(0, hi - 1);
@@ -1232,7 +1211,6 @@ __global__ void __launch_bounds__(256, 2) dwconv_tma_kernel(const __grid_constan
         if (hi >= ho1) break;
         ++hi;
       }
-#endif
     } else {
       // stride 2: output row ho reads input rows 2ho-1 (kh 0), 2ho (kh 1), 2ho+1 (kh 2); row 2ho+1 is also kh 0 of ho+1
       DW_ROW(0, -1, -1, 2 * ho0 - 1, true, false, false);
@@ -1260,9 +1238,6 @@ static bool launch_dwconv_tma(const DirectParams& p, cudaStream_t s) {
   if (p.has_res && !vec_ok(p.res, 2)) return false;
   EncodeTiledFn enc = get_encode_fn();
   if (!enc) return false;
-  static const int hs_env = dw_env_int("ESF_DW_HS", 0), tt_env = dw_env_int("ESF_DW_TT", 0),
-                   wbt_env = dw_env_int("ESF_DW_WBT", 0), st_env = dw_env_int("ESF_DW_STAGES", 0),
-                   ch8_env = dw_env_int("ESF_DW_CH8", 0);
   constexpr int OW = 8, kThreads = 256;
   DwTmaParams q;
   q.p = p;
@@ -1278,13 +1253,11 @@ static bool launch_dwconv_tma(const DirectParams& p, cudaStream_t s) {
   double best = -1;
   for (int ch8 = std::min(c8, 16); ch8 >= 1; --ch8) {
     const int cbc = ch8 * 4;
-    if (cbc > kThreads || (ch8_env > 0 && ch8 != std::min(ch8_env, c8))) continue;
-    if (ch8 == 1 && c8 > 1 && ch8_env == 0) continue;   // 16-byte rows: too many TMA rows / DRAM sectors per byte
+    if (cbc > kThreads) continue;
+    if (ch8 == 1 && c8 > 1) continue;   // 16-byte rows: too many TMA rows / DRAM sectors per byte
     const int lanes = kThreads / cbc, nct = cdiv(c8, ch8);
     for (int w = 1; w <= std::min(lanes, q.wblocks); ++w) {
-      if (wbt_env > 0 && w != std::min(wbt_env, q.wblocks)) continue;
       int t = std::min(p.y.T, lanes / w);
-      if (tt_env > 0) t = std::min(t, tt_env);
       t = cdiv(p.y.T, cdiv(p.y.T, t));
       const int ncols = (w * OW - 1) * SW + 3, planes = (t - 1) * p.sT + p.kT;
       const size_t bytes = (size_t)cbc * 4 * ncols * planes;
@@ -1307,7 +1280,6 @@ static bool launch_dwconv_tma(const DirectParams& p, cudaStream_t s) {
   q.stage_stride = (q.stage_bytes + 127u) & ~127u;
   if (q.ncols > 256 || q.planes > 256 || q.stage_bytes > 32 * 1024) return false;
   q.stages = std::max(2, std::min(kDwTmaMaxStages, (int)((100 * 1024 - kDwTmaHeader) / q.stage_stride)));
-  if (st_env > 0) q.stages = std::max(2, std::min(kDwTmaMaxStages, st_env));
   q.nwt = cdiv(q.wblocks, wbt), q.ntt = cdiv(p.y.T, tt);
   // rows per segment: long segments amortise the two halo rows (16 rows: 18 row steps, 32 rows: 34), short ones fill
   // the last wave of the persistent grid; pick by (useful rows / row steps) x (tiles / tiles rounded up to whole waves)
@@ -1315,7 +1287,6 @@ static bool launch_dwconv_tma(const DirectParams& p, cudaStream_t s) {
   const long long wave = (long long)std::max(num_sms(), 1) * 2;
   double best_hs = -1;
   for (int target : {16, 32, 56}) {
-    if (hs_env > 0) target = hs_env;
     const int nseg = cdiv(p.y.H, target), hs = cdiv(p.y.H, nseg);
     const long long tiles = per_seg * cdiv(p.y.H, hs);
     const double rows = (double)hs * SW / (hs * SW + (SW == 1 ? 2 : 1));
@@ -1356,14 +1327,6 @@ static bool launch_dwconv_tma(const DirectParams& p, cudaStream_t s) {
   return true;
 }
 
-static int dw_march_enabled() {
-  static const int on = [] {
-    const char* e = getenv("ESF_DW_MARCH");
-    return e ? atoi(e) : 2;
-  }();
-  return on;
-}
-
 template <int VEC>
 static bool launch_dwconv_march(const DirectParams& p, cudaStream_t s) {
   const int C = p.x.C, cgs = C / VEC;
@@ -1372,11 +1335,10 @@ static bool launch_dwconv_march(const DirectParams& p, cudaStream_t s) {
   if (smem > 96 * 1024) return false;
   constexpr int OW = 4;
   const int res_vec = p.has_res && vec_ok(p.res, VEC);
-  static const int hs_env = dw_env_int("ESF_DW_HS", 0), wbg_env = dw_env_int("ESF_DW_WBG", 0);
-  const int nseg = cdiv(p.y.H, hs_env > 0 ? hs_env : 16);
+  const int nseg = cdiv(p.y.H, 16);
   const int hs = cdiv(p.y.H, nseg);
   const int wblocks = cdiv(p.y.W, OW);
-  const int wbg = std::max(1, std::min(wblocks, wbg_env > 0 ? wbg_env : 32 / std::max(cgs, 1)));
+  const int wbg = std::max(1, std::min(wblocks, 32 / std::max(cgs, 1)));
   const long long items = (long long)p.y.B * cdiv(p.y.H, hs) * cdiv(wblocks, wbg) * p.y.T * wbg * cgs;
   const unsigned grid = (unsigned)std::min<long long>((items + 127) / 128, 148 * 16);
   auto launch = [&](auto kern) {
@@ -1396,13 +1358,14 @@ static bool launch_dwconv_march(const DirectParams& p, cudaStream_t s) {
 template <int VEC, int KW>
 static bool launch_dwconv(const DirectParams& p, cudaStream_t s) {
   if constexpr (KW == 3) {
-    if (p.kH == 3 && p.pH == 1 && p.pW == 1 && p.sH == p.sW && dw_march_enabled()) {
-      // 2 (default): TMA-staged march; 1: global-load march (kept for A/B); 0: tile kernel
+    if (p.kH == 3 && p.pH == 1 && p.pW == 1 && p.sH == p.sW) {
+      // the TMA-staged march; rows that TMA cannot address (C < 8: 4- or 8-byte pitch) take the global-load march
+      // (C = 4 @112^2: 0.286 -> 0.198 ms).  Either may decline a geometry: then the tile kernel below runs.
       if constexpr (VEC == 8) {
-        if (dw_march_enabled() >= 2 && launch_dwconv_tma(p, s)) return true;
+        if (launch_dwconv_tma(p, s)) return true;
+      } else {
+        if (launch_dwconv_march<VEC>(p, s)) return true;
       }
-      // rows that TMA cannot address (C < 8: 4- or 8-byte pitch): the global-load march (C = 4 @112^2: 0.286 -> 0.198 ms)
-      if ((dw_march_enabled() == 1 || (dw_march_enabled() >= 2 && VEC < 8)) && launch_dwconv_march<VEC>(p, s)) return true;
     }
   }
   const int cgs = p.x.C / VEC;
@@ -2268,8 +2231,7 @@ static int stem_pack_launch(const char* who, const float* x, int32_t B, int32_t 
   const long long nrows = (long long)B * T * H;
   // two buffers of clip rows [kPackRows][Cin][W] FP32 + (Cin = 3 static path) packed output rows [kPackRows][pitch] 16-bit
   const size_t tile_bytes = 2 * (size_t)kPackRows * Cin * W * sizeof(float) + (size_t)kPackRows * pitch * 2;
-  static const bool use_smem = []() { const char* e = getenv("ESF_STEM_PACK_SMEM"); return !(e && atoi(e) == 0); }();
-  if (use_smem && W % 4 == 0 && reinterpret_cast<uintptr_t>(x) % 16 == 0 && tile_bytes <= 48 * 1024 &&
+  if (W % 4 == 0 && reinterpret_cast<uintptr_t>(x) % 16 == 0 && tile_bytes <= 48 * 1024 &&
       nrows < (1LL << 31) - 148LL * 16 * kPackRows) {
     const unsigned g2 = (unsigned)std::max(1LL, std::min((nrows + kPackRows - 1) / kPackRows, 148LL * 16));
     if (Cin == 3)
@@ -2524,8 +2486,7 @@ extern "C" int esf_pool3d(const esf_view* x, const esf_view* y, int32_t kT, int3
   {
     const int cv = x->C / 8;
     const long long rows = (long long)y->B * To * Ho;
-    static const bool use_rows = []() { const char* e = getenv("ESF_POOL_ROWS"); return !(e && atoi(e) == 0); }();
-    if (use_rows && xv == 8 && yv == 8 && x->C % 8 == 0 && (cv & (cv - 1)) == 0 && !is_avg && act == 0 &&
+    if (xv == 8 && yv == 8 && x->C % 8 == 0 && (cv & (cv - 1)) == 0 && !is_avg && act == 0 &&
         rows < (1LL << 31) && x->sT < (1LL << 31) / std::max(1, x->T) && x->sB < (1LL << 40)) {
       int sh = 0;
       while ((1 << sh) < cv) ++sh;

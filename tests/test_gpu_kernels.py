@@ -66,21 +66,19 @@ CONV_CASES = [
     ("tiny_8to32", (2, 8, 14, 14), 8, 32, (1, 1, 1), (1, 1, 1), (0, 0, 0), (1, 1, 1), 0, True, False),
     ("b_1x3x3_s2_7x7", (3, 8, 14, 14), 512, 512, (1, 3, 3), (1, 2, 2), (0, 1, 1), (1, 1, 1), 1, False, False),
     ("many_tiles", (8, 8, 28, 28), 128, 128, (1, 3, 3), (1, 1, 1), (0, 1, 1), (1, 1, 1), 1, False, False),
-    # k x 1 x 1 layers in T-halo mode (one haloed activation tile per chunk, taps = descriptor offsets; opt-in)
-    ("halo_3x1x1_64to16", (2, 32, 28, 28), 64, 16, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 1, False, False),
-    ("halo_3x1x1_res_2chunks", (1, 16, 14, 14), 128, 32, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 1, True, False),
-    ("halo_5x1x1_partial_t", (1, 13, 8, 16), 64, 64, (5, 1, 1), (1, 1, 1), (2, 0, 0), (1, 1, 1), 0, False, False),
-    ("halo_3x1x1_kc32_odd", (2, 9, 7, 9), 32, 16, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 1, False, False),
-    ("halo_3x1x1_f32_out", (1, 8, 8, 8), 64, 32, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 0, False, True),
+    # k x 1 x 1, stride 1: residual over two K chunks, T not a multiple of the box, odd sizes, FP32 output
+    ("t3x1x1_64to16", (2, 32, 28, 28), 64, 16, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 1, False, False),
+    ("t3x1x1_res_2chunks", (1, 16, 14, 14), 128, 32, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 1, True, False),
+    ("t5x1x1_partial_t", (1, 13, 8, 16), 64, 64, (5, 1, 1), (1, 1, 1), (2, 0, 0), (1, 1, 1), 0, False, False),
+    ("t3x1x1_kc32_odd", (2, 9, 7, 9), 32, 16, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 1, False, False),
+    ("t3x1x1_f32_out", (1, 8, 8, 8), 64, 32, (3, 1, 1), (1, 1, 1), (1, 0, 0), (1, 1, 1), 0, False, True),
 ]
 
 
 @pytest.mark.parametrize("precision", ["bf16", "fp16"])
 @pytest.mark.parametrize("case", CONV_CASES, ids=[c[0] for c in CONV_CASES])
-def test_conv_igemm(esf_lib, case, precision, monkeypatch):
+def test_conv_igemm(esf_lib, case, precision):
     name, (B, T, H, W), cin, cout, k, s, p, d, act, use_res, out_f32 = case
-    if name.startswith("halo_"):        # the T-halo mode is an opt-in experiment (csrc/esf_igemm.cu): keep it tested
-        monkeypatch.setenv("ESF_IGEMM_THALO", "2")
     adt = rt.TORCH_DTYPE[precision]
     g = torch.Generator().manual_seed(sum(map(ord, name)) % 1000)
     # input and output live inside wider concat buffers (channel slices) to exercise strided views
@@ -365,15 +363,10 @@ def test_stem_conv(esf_lib, kt, cout):
     assert err <= 6e-3 * ref.abs().max().item()   # FP32 math, BF16 output rounding (2^-8 relative worst case)
 
 
-@pytest.mark.parametrize("thalo", [0, 1])
 @pytest.mark.parametrize("precision", ["bf16", "fp16"])
 @pytest.mark.parametrize("kt,cout,k,size", [(1, 64, 7, 64), (5, 8, 7, 64), (3, 24, 3, 48), (1, 64, 7, 224)])
-def test_stem_banded_gemm(esf_lib, kt, cout, k, size, precision, thalo, monkeypatch):
-    """Tensor-core stem (banded implicit GEMM) vs F.conv3d on the 16-bit-rounded clip and weights; also in the opt-in
-    T-halo mode (one haloed activation tile per kh, the kt taps as descriptor offsets)."""
-    if thalo and kt == 1:
-        pytest.skip("no temporal taps")
-    monkeypatch.setenv("ESF_STEM_THALO", str(thalo))
+def test_stem_banded_gemm(esf_lib, kt, cout, k, size, precision, monkeypatch):
+    """Tensor-core stem (banded implicit GEMM) vs F.conv3d on the 16-bit-rounded clip and weights."""
     monkeypatch.setenv("ESF_STEM_TBAND", "0")     # the temporal-band kernel has its own test below
     adt = rt.TORCH_DTYPE[precision]
     g = torch.Generator().manual_seed(kt + cout)
@@ -882,9 +875,9 @@ def test_global_mean(esf_lib, C, shape, dt):
 @pytest.mark.parametrize("cin,W,kw,pw", [(3, 224, 7, 3), (3, 64, 7, 3), (1, 112, 7, 3), (3, 48, 3, 1), (2, 40, 5, 2),
                                          (3, 50, 7, 3)])
 @pytest.mark.parametrize("precision", ["fp16", "bf16"])
-def test_stem_pack_variants(esf_lib, cin, W, kw, pw, precision, monkeypatch):
+def test_stem_pack_variants(esf_lib, cin, W, kw, pw, precision):
     """esf_stem_pack / _lo / _gather against a torch restatement of the packed row layout, for the shared-memory staged
-    kernel (W % 4 == 0; the static 24-element path when Cin = 3) and the scalar-load kernel (W = 50, or forced)."""
+    kernel (W % 4 == 0; the static 24-element path when Cin = 3) and the scalar-load kernel (W = 50)."""
     adt = rt.TORCH_DTYPE[precision]
     geo = rt.stem_geometry(W, cin, kw, 2, pw)
     if geo is None:
@@ -902,19 +895,17 @@ def test_stem_pack_variants(esf_lib, cin, W, kw, pw, precision, monkeypatch):
         out[..., lpad:lpad + W * cin] = v
         return out.to(adt)
 
-    for smem in ("1", "0"):
-        monkeypatch.setenv("ESF_STEM_PACK_SMEM", smem)   # read once per process: the second value only documents intent
-        a = torch.full((B, T, H, pitch), 7.0, dtype=adt, device=DEV)
-        rt.check(esf_lib.esf_stem_pack(x.data_ptr(), B, cin, T, H, W, pitch, lpad, rt.dtype_code(adt), a.data_ptr(), None))
-        lo = torch.full((B, T, H, pitch), 7.0, dtype=adt, device=DEV)
-        rt.check(esf_lib.esf_stem_pack_lo(x.data_ptr(), B, cin, T, H, W, pitch, lpad, rt.dtype_code(adt), lo.data_ptr(), None))
-        ga = torch.full((B, 3, H, pitch), 7.0, dtype=adt, device=DEV)
-        rt.check(esf_lib.esf_stem_pack_gather(x.data_ptr(), B, cin, T, H, W, idx.data_ptr(), 3, pitch, lpad,
-                                              rt.dtype_code(adt), ga.data_ptr(), None))
-        torch.cuda.synchronize()
-        assert torch.equal(a, expect(x, False))
-        assert torch.equal(lo, expect(x, True))
-        assert torch.equal(ga, expect(x.index_select(2, idx.long()), False))
+    a = torch.full((B, T, H, pitch), 7.0, dtype=adt, device=DEV)
+    rt.check(esf_lib.esf_stem_pack(x.data_ptr(), B, cin, T, H, W, pitch, lpad, rt.dtype_code(adt), a.data_ptr(), None))
+    lo = torch.full((B, T, H, pitch), 7.0, dtype=adt, device=DEV)
+    rt.check(esf_lib.esf_stem_pack_lo(x.data_ptr(), B, cin, T, H, W, pitch, lpad, rt.dtype_code(adt), lo.data_ptr(), None))
+    ga = torch.full((B, 3, H, pitch), 7.0, dtype=adt, device=DEV)
+    rt.check(esf_lib.esf_stem_pack_gather(x.data_ptr(), B, cin, T, H, W, idx.data_ptr(), 3, pitch, lpad,
+                                          rt.dtype_code(adt), ga.data_ptr(), None))
+    torch.cuda.synchronize()
+    assert torch.equal(a, expect(x, False))
+    assert torch.equal(lo, expect(x, True))
+    assert torch.equal(ga, expect(x.index_select(2, idx.long()), False))
 
 
 def test_pool3d_fp16_packed_max(esf_lib):

@@ -1,5 +1,5 @@
 """Time the depthwise layers of the efficient backbones alone (CUDA events, L2 flushed between launches):
-python tools/prof_dwconv.py [reps]      -- kernel knobs come from the environment (ESF_DW_MARCH, ESF_DW_VEC, ...)"""
+python tools/prof_dwconv.py [reps] [layer indices]"""
 import os
 import sys
 

@@ -1,28 +1,17 @@
 #!/bin/bash
-# round 2: temporal-band stem kernel -- kernel tests, time against the banded stem at the headline shape, and the
-# compile-time timing variants of profiles/r2_stem_tband.md:
+# round 2: temporal-band stem kernel -- kernel tests and time against the banded stem at the headline shape:
 #   gpurun -- 'bash tools/sessions/r2_s24_stem_tband.sh'                                  tests + A/B (+ BENCH=1: bench)
-#   gpurun -- 'EXTRA=-DESF_TB_DBG_VARIANTS VARIANTS="0 1 2 3 4 5 6 7 22 38 64 70" TESTS=0 bash tools/sessions/r2_s24_stem_tband.sh'
-# (build the library with the same ESF_NVCC_EXTRA before sending, or the box rebuilds it)
 set -u
 cd "$(dirname "$0")/../.."
 O=gpurun_out/r2_s24
 mkdir -p $O
-export ESF_NVCC_EXTRA="${EXTRA:-}"
 python -c "import __graft_entry__ as g; g.build()" > $O/build.log 2>&1 || { tail -5 $O/build.log; exit 1; }
 if [ "${TESTS:-1}" = 1 ]; then
   timeout 600 python -m pytest tests/test_gpu_kernels.py -x -q -m gpu -k "stem" > $O/pytest.log 2>&1; echo "pytest rc $?"; tail -3 $O/pytest.log
 fi
 {
-  if [ -z "${VARIANTS:-}" ]; then
-    ESF_STEM_TBAND=0 python tools/prof_stem.py 64 20
-    ESF_STEM_TBAND_SHIFT=0 python tools/prof_stem.py 64 20 | sed 's/$/  (odd blocks not sector aligned)/'
-    python tools/prof_stem.py 64 20
-  else
-    for v in $VARIANTS; do
-      echo -n "variant $v: "; ESF_STEM_TBAND_DBG=$v python tools/prof_stem.py 64 20
-    done
-  fi
+  ESF_STEM_TBAND=0 python tools/prof_stem.py 64 20
+  python tools/prof_stem.py 64 20
 } | tee $O/stem_ab.txt
 if [ "${BENCH:-0}" = 1 ]; then
   timeout 900 python bench.py --steps 10 --warmup 3 --no-extra-configs > $O/bench.json 2> $O/bench.err; echo "bench rc $?"
