@@ -4,7 +4,7 @@ Public surface mirrors SlowFast/slowfast/models/__init__.py of the reference:
     from efficient_slowfast_b200 import MODEL_REGISTRY, build_model, get_cfg
 """
 from .build import MODEL_REGISTRY, build_model  # noqa: F401
-from .config import (CfgNode, get_cfg, resnet_cfg, slowfast_4x16_r50_cfg, slowfast_dual_8x8_r50_cfg,  # noqa: F401
+from .config import (CfgNode, ava_slow_8x8_r50_cfg, ava_slowfast_32x2_r50_cfg, get_cfg, resnet_cfg, slowfast_4x16_r50_cfg, slowfast_dual_8x8_r50_cfg,  # noqa: F401
                      slowfast_ghostnet_cfg, slowfast_mobilenetv2_cfg, slowfast_shufflenet_cfg,
                      slowfast_shufflenetv2_cfg)
 from .pipeline import ClipStream  # noqa: F401

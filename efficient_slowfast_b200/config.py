@@ -72,7 +72,7 @@ def get_cfg():
     c.DATA = CfgNode(dict(NUM_FRAMES=8, CROP_SIZE=224, TRAIN_CROP_SIZE=224, TEST_CROP_SIZE=256,
                           INPUT_CHANNEL_NUM=[3, 3], MEAN=[0.45, 0.45, 0.45], STD=[0.225, 0.225, 0.225],
                           SAMPLING_RATE=8, REVERSE_INPUT_CHANNEL=False))
-    c.DETECTION = CfgNode(dict(ENABLE=False))
+    c.DETECTION = CfgNode(dict(ENABLE=False, ALIGNED=True, ROI_XFORM_RESOLUTION=7, SPATIAL_SCALE_FACTOR=16))
     c.MULTIGRID = CfgNode(dict(SHORT_CYCLE=False, LONG_CYCLE=False))
     c.TEST = CfgNode(dict(BATCH_SIZE=8, NUM_ENSEMBLE_VIEWS=10, NUM_SPATIAL_CROPS=3))
     c.NUM_GPUS = 1
@@ -127,6 +127,35 @@ def resnet_cfg(arch="i3d", num_frames=8, nln=False):
     c.DATA._merge(dict(NUM_FRAMES=num_frames, INPUT_CHANNEL_NUM=[3]))
     c.MODEL._merge(dict(NUM_CLASSES=400, ARCH=arch, MODEL_NAME="ResNet", DROPOUT_RATE=0.5))
     return c
+
+
+def _ava_cfg(c):
+    """What the AVA detection YAMLs of upstream SlowFast (configs/AVA/SLOWFAST_32x2_R50_SHORT.yaml,
+    SLOW_8x8_R50_SHORT.yaml) set on top of the Kinetics R50 models: the RoI head, 80 sigmoid classes and res5 at spatial
+    stride 1 with dilation 2 (feature stride 16, DETECTION.SPATIAL_SCALE_FACTOR).  The values are restated from the
+    upstream files; the fork's copies of these YAMLs could not be read when this was written, and
+    tests/test_detection.py::test_ava_yamls_match_reference compares them wherever the reference tree is available."""
+    npw = len(c.DATA.INPUT_CHANNEL_NUM)
+    c.RESNET._merge(dict(SPATIAL_STRIDES=[[1] * npw, [2] * npw, [2] * npw, [1] * npw],
+                         SPATIAL_DILATIONS=[[1] * npw, [1] * npw, [1] * npw, [2] * npw]))
+    c.DETECTION._merge(dict(ENABLE=True, ALIGNED=True, ROI_XFORM_RESOLUTION=7, SPATIAL_SCALE_FACTOR=16))
+    c.MODEL._merge(dict(NUM_CLASSES=80, HEAD_ACT="sigmoid"))
+    c.DATA._merge(dict(TRAIN_CROP_SIZE=224, TEST_CROP_SIZE=256))
+    return c
+
+
+def ava_slowfast_32x2_r50_cfg():
+    """configs/AVA/SLOWFAST_32x2_R50_SHORT.yaml: SlowFast R50, 32 fast / 8 slow frames (ALPHA 4), fusion kernel 7."""
+    c = slowfast_4x16_r50_cfg()
+    c.DATA._merge(dict(NUM_FRAMES=32, SAMPLING_RATE=2))
+    c.SLOWFAST._merge(dict(ALPHA=4, BETA_INV=8, FUSION_CONV_CHANNEL_RATIO=2, FUSION_KERNEL_SZ=7))
+    return _ava_cfg(c)
+
+
+def ava_slow_8x8_r50_cfg():
+    """configs/AVA/SLOW_8x8_R50_SHORT.yaml: single-pathway Slow R50, 8 frames."""
+    c = resnet_cfg("slow", num_frames=8)
+    return _ava_cfg(c)
 
 
 def _efficient_cfg(model_name, width_multi, groups=1, num_classes=400, num_frames=16, crop=112, dropout=0.5,

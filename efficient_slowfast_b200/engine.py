@@ -815,6 +815,48 @@ class Plan:
         self.out = out
         return out
 
+    def temporal_mean(self, x):
+        """ResNetRoIHead's temporal AvgPool3d([T, 1, 1]) where it leaves one frame: 16-bit (B, T, H, W, C) -> dense FP32
+        (B, H, W, C) map, the input of esf_roi_align_max.  A graph op: it reads plan-owned activations only."""
+        B, T, H, W, C = x.shape
+        y = torch.empty((B, H, W, C), dtype=torch.float32, device=self.device)
+        xv = rt.view(x)
+        self.keep += [y, xv]
+        L = rt.lib()
+        self._add(lambda s: rt.check(L.esf_temporal_mean(ctypes.byref(xv), y.data_ptr(), s), "esf_temporal_mean"),
+                  "roi_tpool", "T=%d C=%d @%s" % (T, C, (H, W)), nbytes=self._nbytes(x, y))
+        return y
+
+    def roi_head(self, maps, spatial_scales, resolutions, aligned, weight, bias, act):
+        """Box-dependent part of ResNetRoIHead over the FP32 `maps` (one per pathway, written by temporal_mean):
+        RoIAlign + MaxPool2d into one FP32 row per box, then Linear + activation.  Nothing is recorded into the plan's
+        launch list: the box count is only known per call, so run_boxes() issues these launches after the trunk."""
+        self.roi = dict(maps=maps, scales=[float(v) for v in spatial_scales], res=[int(v) for v in resolutions],
+                        aligned=int(bool(aligned)), w=self.tensor(weight), b=self.tensor(bias), act=act,
+                        cin=sum(m.shape[3] for m in maps), ncls=int(weight.shape[0]))
+        self.roi_feat = self.roi_out = None
+
+    def run_boxes(self, boxes):
+        """`boxes`: (K, 5) contiguous FP32 on this plan's device, K >= 1, rows [batch index, x1, y1, x2, y2].  Launches
+        esf_roi_align_max per pathway (both write slices of the same feature row) and esf_head_fc on the current
+        stream; the feat / out buffers grow to the largest K seen and are reused.  Returns a view of the first K rows."""
+        r = self.roi
+        K = boxes.shape[0]
+        if self.roi_out is None or self.roi_out.shape[0] < K:
+            self.roi_feat = torch.empty((K, r["cin"]), dtype=torch.float32, device=self.device)
+            self.roi_out = torch.empty((K, r["ncls"]), dtype=torch.float32, device=self.device)
+        L = rt.lib()
+        s = rt.current_stream_ptr()
+        off = 0
+        for m, scale, res in zip(r["maps"], r["scales"], r["res"]):
+            B, H, W, C = m.shape
+            rt.check(L.esf_roi_align_max(m.data_ptr(), B, H, W, C, boxes.data_ptr(), K, scale, res, r["aligned"],
+                                         self.roi_feat.data_ptr(), r["cin"], off, s), "esf_roi_align_max")
+            off += C
+        rt.check(L.esf_head_fc(self.roi_feat.data_ptr(), K, r["cin"], r["cin"], r["w"].data_ptr(), r["b"].data_ptr(),
+                               r["ncls"], r["act"], self.roi_out.data_ptr(), r["ncls"], s), "esf_head_fc")
+        return self.roi_out[:K]
+
     # ---------------------------------------------------------------- execution
     def launch_all(self):
         s = rt.current_stream_ptr()

@@ -242,6 +242,42 @@ class ResNetBasicHead(_Holder):
         self.act_func = act_func
 
 
+class ROIAlign(_Holder):
+    """detectron2.layers.ROIAlign (parameter-free): output_size, spatial_scale, sampling_ratio, aligned.  The sampling
+    itself is esf_roi_align_max (torchvision roi_align semantics, which detectron2's ROIAlign dispatches to)."""
+
+    def __init__(self, output_size, spatial_scale, sampling_ratio, aligned=True):
+        super().__init__()
+        self.output_size, self.spatial_scale = output_size, spatial_scale
+        self.sampling_ratio, self.aligned = sampling_ratio, aligned
+
+
+class ResNetRoIHead(_Holder):
+    """head_helper.py:12-130 (AVA detection): per pathway a temporal AvgPool3d, RoIAlign and a spatial MaxPool2d over the
+    RoIAlign output, then concat -> Linear -> softmax(dim=1) / sigmoid.  One row per box."""
+
+    def __init__(self, dim_in, num_classes, pool_size, resolution, scale_factor, dropout_rate=0.0, act_func="softmax",
+                 aligned=True):
+        super().__init__()
+        assert len({len(pool_size), len(dim_in)}) == 1, "pathway dimensions are not consistent."
+        self.num_pathways = len(pool_size)
+        for p in range(self.num_pathways):
+            self.add_module("s{}_tpool".format(p), nn.AvgPool3d([pool_size[p][0], 1, 1], stride=1))
+            self.add_module("s{}_roi".format(p), ROIAlign(resolution[p], spatial_scale=1.0 / scale_factor[p],
+                                                         sampling_ratio=0, aligned=aligned))
+            self.add_module("s{}_spool".format(p), nn.MaxPool2d(resolution[p], stride=1))
+        if dropout_rate > 0.0:
+            self.dropout = nn.Dropout(dropout_rate)
+        self.projection = nn.Linear(sum(dim_in), num_classes, bias=True)
+        if act_func == "softmax":
+            self.act = nn.Softmax(dim=1)
+        elif act_func == "sigmoid":
+            self.act = nn.Sigmoid()
+        else:
+            raise NotImplementedError("{} is not supported as an activation function.".format(act_func))
+        self.act_func = act_func
+
+
 def init_weights(model, fc_init_std=0.01, zero_init_final_bn=True):
     """utils/weight_init_helper.py:10-43: c2_msra_fill (kaiming normal, fan_out, relu; zero bias) on Conv3d, BN weight
     1 (0 for the last BN of a bottleneck when zero_init_final_bn), BN bias 0, Linear N(0, fc_init_std) / zero bias.
@@ -268,6 +304,7 @@ class _PlannedModel(nn.Module):
 
     num_pathways = 2
     supports_fp32 = False     # cfg.ESF.PRECISION = "fp32" (engine_fp32.PrecisePlan): the ResNet-50 family only
+    enable_detection = False  # cfg.DETECTION.ENABLE: ResNetRoIHead, forward(x, bboxes) returns one row per box
 
     def _init_runtime(self, cfg):
         self._cfg = cfg
@@ -306,11 +343,15 @@ class _PlannedModel(nn.Module):
         if ent is not None and ent[0] == stamp:
             self._plans.move_to_end(key)
             return ent[1]
+        self._check_roi_time_axis(shapes)            # before any cached plan is evicted for this shape
         if ent is not None or any(st != stamp for st, _ in self._plans.values()):
             self._plans.clear()                      # the weights changed: every compiled plan is stale
         prec = "fp16"
         if hasattr(self._cfg, "get") and self._cfg.get("ESF") is not None:
             prec = str(self._cfg.ESF.get("PRECISION", "fp16"))
+        if prec == "fp32" and self.enable_detection:
+            raise NotImplementedError("ESF.PRECISION = 'fp32' does not cover the detection head (DETECTION.ENABLE); run "
+                                      "detection models with 'fp16' / 'bf16'")
         while len(self._plans) >= self._max_plans:
             self._plans.popitem(last=False)          # frees the arena of the least recently used shape
         with torch.cuda.device(device):
@@ -341,14 +382,14 @@ class _PlannedModel(nn.Module):
         if self.training:
             raise NotImplementedError("efficient_slowfast_b200 implements the eval-mode forward path only; call "
                                       ".eval() (training / autograd is outside the accelerated hot path)")
-        if bboxes is not None:
-            raise NotImplementedError("detection (bboxes) is out of scope")
         dev = x[0].device
+        boxes = self._boxes(bboxes, x[0].shape[0], dev)
         if dev.type != "cuda":
             raise rt.EsfError("the forward path is CUDA-only (sm_100a); got tensors on %s -- there is no CPU fallback"
                               % dev)
-        if x[0].shape[0] == 0:        # an empty batch is an empty result (nn.Conv3d / nn.Linear of the reference agree)
-            return torch.empty((0, int(self._cfg.MODEL.NUM_CLASSES)), dtype=torch.float32, device=dev)
+        if x[0].shape[0] == 0 or (boxes is not None and boxes.shape[0] == 0):
+            # an empty batch is an empty result (nn.Conv3d / nn.Linear of the reference agree); so is an empty box list
+            return self._empty(dev)
         plan = self._get_plan([tuple(t.shape) for t in x], dev)
         # FP32 contiguous clips are read in place by the stem kernels (launched outside the CUDA graph); anything else
         # (other dtype / strides) is first converted into the plan-owned input buffers
@@ -359,7 +400,7 @@ class _PlannedModel(nn.Module):
                     if src.data_ptr() != dst.data_ptr():
                         dst.copy_(src, non_blocking=True)
             out = plan.run(list(x) if direct else None)
-            return out.clone()
+            return self._finish(plan, out, boxes)
 
     def forward_fast(self, fast, bboxes=None):
         """Same result as `forward(pack_pathway_output(cfg, fast))`: the loader's pack_pathway_output
@@ -372,17 +413,16 @@ class _PlannedModel(nn.Module):
             raise rt.EsfError("forward_fast is for the two-pathway models")
         if self.training:
             raise NotImplementedError("eval-mode forward path only")
-        if bboxes is not None:
-            raise NotImplementedError("detection (bboxes) is out of scope")
         dev = fast.device
+        boxes = self._boxes(bboxes, fast.shape[0], dev)
         if dev.type != "cuda":
             raise rt.EsfError("the forward path is CUDA-only (sm_100a); got tensors on %s -- there is no CPU fallback"
                               % dev)
         if fast.dtype != torch.float32 or fast.dim() != 5 or not fast.is_contiguous() or fast.data_ptr() % 16:
             raise rt.EsfError("forward_fast expects a contiguous FP32 clip (B, C, T, H, W)")
         B, C, T, H, W = fast.shape
-        if B == 0:
-            return torch.empty((0, int(self._cfg.MODEL.NUM_CLASSES)), dtype=torch.float32, device=dev)
+        if B == 0 or (boxes is not None and boxes.shape[0] == 0):
+            return self._empty(dev)
         alpha = self._cfg.SLOWFAST.ALPHA
         plan = self._get_plan([(B, C, T // alpha, H, W), (B, C, T, H, W)], dev)
         idx = getattr(plan, "slow_index", None)
@@ -394,7 +434,7 @@ class _PlannedModel(nn.Module):
             else:
                 torch.index_select(fast, 2, idx.long(), out=plan.inputs[0])
                 out = plan.run([None, fast])
-            return out.clone()
+            return self._finish(plan, out, boxes)
 
     def frame_shapes(self, frames_shape):
         """[slow, fast] (or [single]) clip shapes that pack_pathway_output (datasets/utils.py:73-112) makes of uint8
@@ -411,16 +451,15 @@ class _PlannedModel(nn.Module):
         from . import frames as esf_frames
         if self.training:
             raise NotImplementedError("eval-mode forward path only")
-        if bboxes is not None:
-            raise NotImplementedError("detection (bboxes) is out of scope")
+        boxes = self._boxes(bboxes, frames.shape[0] if frames.dim() else 0, frames.device)
         if frames.device.type != "cuda":
             raise rt.EsfError("the forward path is CUDA-only (sm_100a); got frames on %s -- there is no CPU fallback"
                               % frames.device)
         if frames.dtype != torch.uint8 or frames.dim() != 5 or not frames.is_contiguous():
             raise rt.EsfError("forward_frames expects contiguous uint8 frames (B, T, H, W, C)")
         dev = frames.device
-        if frames.shape[0] == 0:
-            return torch.empty((0, int(self._cfg.MODEL.NUM_CLASSES)), dtype=torch.float32, device=dev)
+        if frames.shape[0] == 0 or (boxes is not None and boxes.shape[0] == 0):
+            return self._empty(dev)
         shapes = self.frame_shapes(tuple(frames.shape))
         if frame_index is not None:     # explicit source frame of every pathway frame (frames may be a ring buffer)
             assert len(frame_index) == self.num_pathways
@@ -433,7 +472,68 @@ class _PlannedModel(nn.Module):
         alpha = self._cfg.SLOWFAST.ALPHA if self.num_pathways > 1 else 1
         with torch.cuda.device(dev):
             out = plan.run_frames(lambda: esf_frames.launch_frames(plan, fin, frames, alpha, frame_index))
-            return out.clone()
+            return self._finish(plan, out, boxes)
+
+    def _empty(self, dev):
+        return torch.empty((0, int(self._cfg.MODEL.NUM_CLASSES)), dtype=torch.float32, device=dev)
+
+    def _check_roi_time_axis(self, shapes):
+        """ResNetRoIHead's temporal AvgPool3d([t, 1, 1], stride 1) must leave one frame of every pathway's res5 output:
+        the reference asserts `out.shape[2] == 1` after it (head_helper.py) and AvgPool3d itself rejects t > T.  The
+        trunk keeps the time axis except for the max-pool after res2 (kernel = stride = pathway{p}_pool)."""
+        if not self.enable_detection:
+            return
+        for p, shape in enumerate(shapes):
+            k = int(getattr(self, "pathway%d_pool" % p).kernel_size[0])
+            T = (int(shape[2]) - k) // k + 1
+            kt = int(getattr(self.head, "s%d_tpool" % p).kernel_size[0])
+            if kt > T:
+                raise RuntimeError("head temporal AvgPool3d kernel %d is larger than the %d res5 frames of pathway %d"
+                                   % (kt, T, p))
+            if T - kt + 1 != 1:
+                raise AssertionError("pathway %d: the head's temporal pool (kernel %d) leaves %d frames of %d, the "
+                                     "reference's ResNetRoIHead asserts 1" % (p, kt, T - kt + 1, T))
+
+    def _boxes(self, bboxes, batch, dev):
+        """Detection models: `bboxes` (K, 5) rows [batch index, x1, y1, x2, y2] in input pixels, as one contiguous FP32
+        tensor on `dev` (a single copy).  Host boxes are checked before anything is launched: shape, and batch indices
+        in [0, batch).  Device boxes are only shape-checked (reading them would synchronise); there the kernel clamps the
+        batch index and writes NaN rows for non-finite boxes.  Classification models: None, and `bboxes` must be None."""
+        if not self.enable_detection:
+            if bboxes is not None:
+                raise NotImplementedError("bboxes given to a classification model; detection needs a model built with "
+                                          "cfg.DETECTION.ENABLE (ResNetRoIHead)")
+            return None
+        if bboxes is None:
+            raise ValueError("detection model (cfg.DETECTION.ENABLE): forward needs bboxes, a (K, 5) tensor of "
+                             "[batch index, x1, y1, x2, y2]")
+        if (not torch.is_tensor(bboxes) or not bboxes.is_floating_point() or bboxes.dim() != 2
+                or bboxes.shape[1] != 5):
+            raise ValueError("bboxes must be a floating-point (K, 5) tensor of [batch index, x1, y1, x2, y2]; got %s"
+                             % ((tuple(bboxes.shape), bboxes.dtype) if torch.is_tensor(bboxes) else type(bboxes).__name__,))
+        if bboxes.device.type == "cpu":
+            b = bboxes.detach().to(torch.float32).contiguous()
+            idx = b[:, 0]
+            bad = ~((idx >= 0) & (idx < batch))
+            if bool(bad.any()):
+                raise ValueError("bboxes[:, 0] must be batch indices in [0, %d); got %s"
+                                 % (batch, idx[bad][:4].tolist()))
+            if dev.type != "cuda":
+                return b
+            # staged through pinned memory: the copy is queued on the stream instead of waiting for earlier work.  The
+            # host caching allocator keeps the staging block until the copy has run, although the tensor dies here.
+            staged = torch.empty(b.shape, dtype=torch.float32, pin_memory=True)
+            staged.copy_(b)
+            with torch.cuda.device(dev):
+                return staged.to(dev, non_blocking=True)
+        return bboxes.detach().to(device=dev, dtype=torch.float32).contiguous()
+
+    @staticmethod
+    def _finish(plan, out, boxes):
+        """The caller's copy of the result; detection plans first run their box-dependent launches (Plan.run_boxes)."""
+        if boxes is not None:
+            out = plan.run_boxes(boxes)
+        return out.clone()
 
     def _emit_fuse(self, plan, fuse, cur):
         (sbuf, soff, cs), (fbuf, foff, cf) = cur
@@ -474,10 +574,11 @@ class _TwoStreamResNet(_PlannedModel):
         pool_size = _POOL1[cfg.MODEL.ARCH]
         assert len({len(pool_size), self.num_pathways}) == 1
         assert cfg.RESNET.DEPTH in _MODEL_STAGE_DEPTH.keys()
-        if cfg.DETECTION.ENABLE:
-            raise NotImplementedError("DETECTION.ENABLE (ResNetRoIHead) is out of scope")
+        if cfg.DETECTION.ENABLE and dual_attention:
+            raise NotImplementedError("DETECTION.ENABLE with SlowFastDualAttention: the fork's detection builder for this "
+                                      "model could not be checked; detection runs on SlowFast and ResNet")
         self.norm_module = get_norm(cfg)
-        self.enable_detection = False
+        self.enable_detection = bool(cfg.DETECTION.ENABLE)
         self.dual_attention = dual_attention
         depths = _MODEL_STAGE_DEPTH[cfg.RESNET.DEPTH]
         num_groups = cfg.RESNET.NUM_GROUPS
@@ -522,17 +623,26 @@ class _TwoStreamResNet(_PlannedModel):
                     self.add_module("pathway{}_pool".format(p),
                                     nn.MaxPool3d(kernel_size=pool_size[p], stride=pool_size[p], padding=[0, 0, 0]))
             c_prev = c_out
-        if cfg.MULTIGRID.SHORT_CYCLE:
-            head_pool = [None, None]
+        if self.enable_detection:      # video_model_builder.py: ResNetRoIHead branch of _construct_network
+            R = cfg.DETECTION.ROI_XFORM_RESOLUTION
+            self.head = ResNetRoIHead(
+                dim_in=[wpg * 32, wpg * 32 // beta], num_classes=cfg.MODEL.NUM_CLASSES,
+                pool_size=[[cfg.DATA.NUM_FRAMES // alpha // pool_size[0][0], 1, 1],
+                           [cfg.DATA.NUM_FRAMES // pool_size[1][0], 1, 1]],
+                resolution=[[R] * 2] * 2, scale_factor=[cfg.DETECTION.SPATIAL_SCALE_FACTOR] * 2,
+                dropout_rate=cfg.MODEL.DROPOUT_RATE, act_func=cfg.MODEL.HEAD_ACT, aligned=cfg.DETECTION.ALIGNED)
         else:
-            c = cfg.DATA.CROP_SIZE // 32
-            head_pool = [
-                [cfg.DATA.NUM_FRAMES // alpha // pool_size[0][0], c // pool_size[0][1], c // pool_size[0][2]],
-                [cfg.DATA.NUM_FRAMES // pool_size[1][0], c // pool_size[1][1], c // pool_size[1][2]],
-            ]
-        self.head = ResNetBasicHead(dim_in=[wpg * 32, wpg * 32 // beta], num_classes=cfg.MODEL.NUM_CLASSES,
-                                    pool_size=head_pool, dropout_rate=cfg.MODEL.DROPOUT_RATE,
-                                    act_func=cfg.MODEL.HEAD_ACT)
+            if cfg.MULTIGRID.SHORT_CYCLE:
+                head_pool = [None, None]
+            else:
+                c = cfg.DATA.CROP_SIZE // 32
+                head_pool = [
+                    [cfg.DATA.NUM_FRAMES // alpha // pool_size[0][0], c // pool_size[0][1], c // pool_size[0][2]],
+                    [cfg.DATA.NUM_FRAMES // pool_size[1][0], c // pool_size[1][1], c // pool_size[1][2]],
+                ]
+            self.head = ResNetBasicHead(dim_in=[wpg * 32, wpg * 32 // beta], num_classes=cfg.MODEL.NUM_CLASSES,
+                                        pool_size=head_pool, dropout_rate=cfg.MODEL.DROPOUT_RATE,
+                                        act_func=cfg.MODEL.HEAD_ACT)
         init_weights(self, cfg.MODEL.FC_INIT_STD, cfg.RESNET.ZERO_INIT_FINAL_BN)
         self._init_runtime(cfg)
 
@@ -612,6 +722,8 @@ class _TwoStreamResNet(_PlannedModel):
         # ---- head
         xs = [c[0] for c in cur]
         act = {"softmax": rt.HEAD_SOFTMAX, "sigmoid": rt.HEAD_SIGMOID}[self.head.act_func]
+        if self.enable_detection:
+            return self._emit_roi_head(plan, xs, act)
         self._emit_head(plan, xs, act)
 
     def _emit_head(self, plan, xs, act):
@@ -626,6 +738,23 @@ class _TwoStreamResNet(_PlannedModel):
                 raise NotImplementedError("head AvgPool3d kernel %s does not fit the feature map %s"
                                           % (ps, list(x.shape[1:4])))
         return plan.head_positions(xs, sizes, self.head.projection.weight, self.head.projection.bias, act)
+
+    def _emit_roi_head(self, plan, xs, act):
+        """ResNetRoIHead.forward (head_helper.py:100-130) in two parts.  In the plan (CUDA graph): the temporal
+        AvgPool3d of every pathway's res5 output into an FP32 map.  Per call, outside the graph (Plan.run_boxes):
+        RoIAlign + spatial max of every pathway into one FP32 row per box, then Linear + activation."""
+        maps, scales, res = [], [], []
+        for p, x in enumerate(xs):
+            roi = getattr(self.head, "s%d_roi" % p)
+            r = [int(v) for v in roi.output_size]
+            if r[0] != r[1] or roi.sampling_ratio != 0:
+                raise NotImplementedError("ROIAlign output %s / sampling_ratio %d: the kernel covers square outputs "
+                                          "with the adaptive grid (sampling_ratio 0) of ResNetRoIHead" % (r, roi.sampling_ratio))
+            maps.append(plan.temporal_mean(x))
+            scales.append(roi.spatial_scale)
+            res.append(r[0])
+        plan.roi_head(maps, scales, res, bool(self.head.s0_roi.aligned), self.head.projection.weight,
+                      self.head.projection.bias, act)
 
     def _emit_stage_pathway(self, plan, stage, pw, x, dst, stride, dil):
         """One pathway of ResStage.forward (resnet_helper.py:530-561): residual blocks, each optionally followed by
@@ -705,10 +834,8 @@ class ResNet(_TwoStreamResNet):
         pool_size = _POOL1[cfg.MODEL.ARCH]
         assert len({len(pool_size), self.num_pathways}) == 1
         assert cfg.RESNET.DEPTH in _MODEL_STAGE_DEPTH.keys()
-        if cfg.DETECTION.ENABLE:
-            raise NotImplementedError("DETECTION.ENABLE (ResNetRoIHead) is out of scope")
         self.norm_module = get_norm(cfg)
-        self.enable_detection = False
+        self.enable_detection = bool(cfg.DETECTION.ENABLE)
         depths = _MODEL_STAGE_DEPTH[cfg.RESNET.DEPTH]
         num_groups, wpg = cfg.RESNET.NUM_GROUPS, cfg.RESNET.WIDTH_PER_GROUP
         dim_inner = num_groups * wpg
@@ -729,13 +856,21 @@ class ResNet(_TwoStreamResNet):
                 self.add_module("pathway0_pool",
                                 nn.MaxPool3d(kernel_size=pool_size[0], stride=pool_size[0], padding=[0, 0, 0]))
             c_prev = c_out
-        if cfg.MULTIGRID.SHORT_CYCLE:
-            head_pool = [None, None]    # as in the reference (video_model_builder.py:584-586): the head then rejects it
+        if self.enable_detection:      # video_model_builder.py: ResNetRoIHead branch of ResNet._construct_network
+            R = cfg.DETECTION.ROI_XFORM_RESOLUTION
+            self.head = ResNetRoIHead(
+                dim_in=[wpg * 32], num_classes=cfg.MODEL.NUM_CLASSES,
+                pool_size=[[cfg.DATA.NUM_FRAMES // pool_size[0][0], 1, 1]], resolution=[[R] * 2],
+                scale_factor=[cfg.DETECTION.SPATIAL_SCALE_FACTOR], dropout_rate=cfg.MODEL.DROPOUT_RATE,
+                act_func=cfg.MODEL.HEAD_ACT, aligned=cfg.DETECTION.ALIGNED)
         else:
-            c = cfg.DATA.CROP_SIZE // 32
-            head_pool = [[cfg.DATA.NUM_FRAMES // pool_size[0][0], c // pool_size[0][1], c // pool_size[0][2]]]
-        self.head = ResNetBasicHead(dim_in=[wpg * 32], num_classes=cfg.MODEL.NUM_CLASSES, pool_size=head_pool,
-                                    dropout_rate=cfg.MODEL.DROPOUT_RATE, act_func=cfg.MODEL.HEAD_ACT)
+            if cfg.MULTIGRID.SHORT_CYCLE:
+                head_pool = [None, None]    # as in the reference (video_model_builder.py:584-586): the head then rejects it
+            else:
+                c = cfg.DATA.CROP_SIZE // 32
+                head_pool = [[cfg.DATA.NUM_FRAMES // pool_size[0][0], c // pool_size[0][1], c // pool_size[0][2]]]
+            self.head = ResNetBasicHead(dim_in=[wpg * 32], num_classes=cfg.MODEL.NUM_CLASSES, pool_size=head_pool,
+                                        dropout_rate=cfg.MODEL.DROPOUT_RATE, act_func=cfg.MODEL.HEAD_ACT)
         init_weights(self, cfg.MODEL.FC_INIT_STD, cfg.RESNET.ZERO_INIT_FINAL_BN)
         self._init_runtime(cfg)
 
@@ -774,4 +909,6 @@ class ResNet(_TwoStreamResNet):
                     plan.pool(cur, pooled, tuple(ks), tuple(ks), (0, 0, 0))
                     cur = pooled
         act = {"softmax": rt.HEAD_SOFTMAX, "sigmoid": rt.HEAD_SIGMOID}[self.head.act_func]
+        if self.enable_detection:
+            return self._emit_roi_head(plan, [cur], act)
         self._emit_head(plan, [cur], act)

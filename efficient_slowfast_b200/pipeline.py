@@ -28,6 +28,9 @@ class ClipStream:
         `[slow, fast] = pack_pathway_output(cfg, fast)` (datasets/utils.py:93-102: slow = the linspace frame subset of
         fast).  Only the fast clip is then copied to the device and the slow pathway's stem reads its frames out of it
         (`model.forward_fast`): 1/(1 + 1/ALPHA) of the H2D bytes.  The first batch is verified on the host."""
+        if getattr(model, "enable_detection", False):
+            raise NotImplementedError("ClipStream streams clip batches into classification models; call a detection "
+                                      "model (cfg.DETECTION.ENABLE) as model(inputs, bboxes)")
         device = torch.device(device) if device is not None else next(model.parameters()).device
         if device.type != "cuda":
             raise rt.EsfError("ClipStream needs a CUDA device; there is no CPU fallback")

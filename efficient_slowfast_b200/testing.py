@@ -9,7 +9,9 @@ Mirrors the interface of the reference's `TestMeter` (SlowFast/slowfast/utils/me
     labels / video indices are queued alongside);
   * multi-GPU: predictions are all-gathered on the device inside ClipStream, labels and clip indices with the same
     collective (`distributed.all_gather`), as `du.all_gather([preds, labels, video_idx])` does in the reference.
-Detection (AVAMeter) and multi-label mAP are out of scope (SURVEY.md section 8)."""
+Detection (cfg.DETECTION.ENABLE) follows the reference's branch: `model(inputs, meta["boxes"])` per batch, the caller's
+meter (the reference's AVAMeter) gets `update_stats(preds, ori_boxes, metadata)`; the AVA mAP evaluation is the meter's
+own business.  Multi-label mAP of TestMeter is out of scope (SURVEY.md section 8)."""
 import time
 
 import torch
@@ -99,7 +101,7 @@ def perform_test(test_loader, model, test_meter, cfg, depth=2, slow_from_fast=No
     batch may be shorter (the reference's test loader has drop_last=False).  `slow_from_fast`: upload only the fast
     clip and let the slow pathway read its frames out of it (ClipStream); None = decide from the first batch."""
     if cfg.DETECTION.ENABLE:
-        raise NotImplementedError("detection testing is out of scope")
+        return perform_detection_test(test_loader, model, test_meter, cfg)
     model.eval()
     multi = cfg.NUM_GPUS > 1 and esf_dist.dist.is_available() and esf_dist.dist.is_initialized()
     device = next(model.parameters()).device
@@ -135,3 +137,32 @@ def perform_test(test_loader, model, test_meter, cfg, depth=2, slow_from_fast=No
     stats = test_meter.finalize_metrics(ks=ks)
     test_meter.reset()
     return stats
+
+
+def _host(t):
+    return t.detach().cpu() if torch.is_tensor(t) else t
+
+
+@torch.no_grad()
+def perform_detection_test(test_loader, model, test_meter, cfg):
+    """Detection branch of tools/test_net.py:21-123 over `(inputs, labels, video_idx, meta)` batches: the clips go to the
+    model's device, `preds = model(inputs, meta["boxes"])` (boxes (K, 5) [batch index, x1, y1, x2, y2] in input pixels,
+    copied to the device once by the model), then `test_meter.update_stats(preds, meta["ori_boxes"], meta["metadata"])`
+    on the host and `log_iter_stats(None, cur_iter)`.  `test_meter` is duck-typed (the reference's AVAMeter);
+    returns what its finalize_metrics() returns.  One process: sharding boxes over GPUs is not implemented."""
+    if cfg.NUM_GPUS > 1:
+        raise NotImplementedError("multi-GPU detection testing (box sharding and all_gather_unaligned of the "
+                                  "predictions) is not implemented; run detection with NUM_GPUS = 1")
+    model.eval()
+    device = next(model.parameters()).device
+    test_meter.iter_tic()
+    for cur_iter, (inputs, _labels, _video_idx, meta) in enumerate(test_loader):
+        if not isinstance(inputs, (list, tuple)):
+            inputs = [inputs]
+        inputs = [t.to(device, non_blocking=True) for t in inputs]
+        preds = model(inputs, meta["boxes"])
+        test_meter.iter_toc()
+        test_meter.update_stats(_host(preds), _host(meta["ori_boxes"]), _host(meta["metadata"]))
+        test_meter.log_iter_stats(None, cur_iter)
+        test_meter.iter_tic()
+    return test_meter.finalize_metrics()

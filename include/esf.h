@@ -246,6 +246,19 @@ int esf_global_mean(const esf_view* x, float* scratch, float* feat, int32_t feat
  * out[b][k] = mean_p in[b][p][k]. */
 int esf_group_mean(const float* in, int32_t B, int32_t P, int32_t K, float* out, void* stream);
 
+/* ---- RoI head of the AVA detection models (ResNetRoIHead, head_helper.py:12-130; csrc/esf_roi.cu) ----------------
+ * esf_temporal_mean: y[b][h][w][c] = mean_t x[b, t, h, w, c] -- the head's AvgPool3d([T, 1, 1]) when it leaves one
+ *   frame; x: 16-bit view, y: dense FP32 (B, H, W, C).
+ * esf_roi_align_max: feat[k][c_off + c] = max over the R x R bins of RoIAlign(R, spatial_scale, sampling_ratio 0,
+ *   aligned) on map[b_k] (torchvision roi_align semantics, as detectron2's ROIAlign), i.e. RoIAlign + MaxPool2d(R).
+ *   map: dense FP32 (B, H, W, C); boxes: FP32 (K, 5) rows [batch index, x1, y1, x2, y2] in input pixels.  The batch
+ *   index is clamped to [0, B); a box with non-finite geometry gives a NaN row; the adaptive sampling grid of a bin is
+ *   capped at 64 x 64.  One row per box, deterministic (no atomics); both pathways write slices of one row. */
+int esf_temporal_mean(const esf_view* x, float* y, void* stream);
+int esf_roi_align_max(const float* map, int32_t B, int32_t H, int32_t W, int32_t C, const float* boxes, int32_t K,
+                      float spatial_scale, int32_t resolution, int32_t aligned, float* feat, int32_t feat_stride,
+                      int32_t c_off, void* stream);
+
 /* ---- FP32-accurate path (cfg.ESF.PRECISION = "fp32"; north star: rel err <= 1e-4 against the reference's FP32 forward) --
  * The reference is FP32 end to end (resnet_helper.py:182-240, wdf_attention_helper.py:42-53).  Here every tensor-core
  * operand is a pair of FP16 numbers x = hi + lo (22 mantissa bits) and x.w = x_hi.w_hi + x_lo.w_hi + x_hi.w_lo, evaluated
