@@ -7,9 +7,17 @@ crop, and `pack_pathway_output` (datasets/utils.py:73-112: optional channel reve
 PCIe.  `model.forward_frames(frames_u8)` takes the byte frames instead and the stem-pack kernel does the chain on the
 device: 1/5 of the H2D bytes, bit-identical stem input (the byte -> value table is computed here with the reference's
 own FP32 operations).
+
+Test-time spatial sampling (`forward_frames(frames, crop_size=S, spatial_idx=(0, 1, 2))`): the reference's Kinetics test
+branch resizes every normalised clip so that its short side is S (bilinear, on the CPU) and takes `uniform_crop`s of S x S
+(datasets/utils.py spatial_sampling, transform.py).  The byte frames at decode size go to the device instead and one
+kernel (csrc/esf_crop.cu) normalises, resizes, crops and packs; the resize follows the per-axis tables of `axis_table`,
+which reproduce torch's CPU weights bit for bit.
 """
 import ctypes
+import math
 
+import numpy as np
 import torch
 
 from . import runtime as rt
@@ -28,6 +36,103 @@ def normalization_table(mean, std, channels):
     t = t - torch.tensor(list(mean)[:channels], dtype=torch.float32)
     t = t / torch.tensor(list(std)[:channels], dtype=torch.float32)
     return t.t().contiguous()
+
+
+def resized_size(height, width, size):
+    """transform.random_short_side_scale_jitter in test mode (min_size = max_size = size): (height, width) after the
+    short-side resize; the frame is left alone when its short side already is `size`."""
+    if (width <= height and width == size) or (height <= width and height == size):
+        return height, width
+    if width < height:
+        return int(math.floor((float(height) / width) * size)), size
+    return size, int(math.floor((float(width) / height) * size))
+
+
+def crop_offset(height, width, size, spatial_idx):
+    """transform.uniform_crop: (y0, x0) of the size x size crop `spatial_idx` (0, 1, 2: start, centre, end of the long
+    axis) of a height x width frame."""
+    y0 = int(math.ceil((height - size) / 2))
+    x0 = int(math.ceil((width - size) / 2))
+    if height > width:
+        y0 = 0 if spatial_idx == 0 else (height - size if spatial_idx == 2 else y0)
+    else:
+        x0 = 0 if spatial_idx == 0 else (width - size if spatial_idx == 2 else x0)
+    return y0, x0
+
+
+MAX_VIEWS = 8   # csrc/esf_crop.cu kCropMaxViews
+
+
+def spatial_views(spatial_idx):
+    """`spatial_idx` (an int or a sequence of ints from {0, 1, 2}) as a tuple; ValueError otherwise."""
+    views = tuple(spatial_idx) if isinstance(spatial_idx, (list, tuple, range)) else (spatial_idx,)
+    if not 1 <= len(views) <= MAX_VIEWS:
+        raise ValueError("spatial_idx needs 1 to %d views, got %d" % (MAX_VIEWS, len(views)))
+    for v in views:
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or int(v) not in (0, 1, 2):
+            raise ValueError("spatial_idx values are 0, 1 or 2 (uniform_crop), got %r" % (v,))
+    return tuple(int(v) for v in views)
+
+
+def axis_table(n_in, n_out):
+    """Source indices (int32 [n_out][2]: i0, i1) and weights (FP32 [n_out][2]: l0, l1) of one axis of torch's CPU bilinear
+    interpolate (align_corners=False, output size given): ATen's compute_source_index_and_lambda with scale =
+    float(n_in) / n_out and the source index fma(scale, d + 0.5, -0.5) clamped at 0, as its kernels compile it with FMA
+    contraction (AVX2 / AVX512 CPU capability).  An axis that keeps its size is the identity (i0 = d, i1 = 0, 1, 0)."""
+    d = np.arange(n_out)
+    if n_in == n_out:
+        idx = np.stack([d, np.zeros_like(d)], 1)
+        wt = np.stack([np.ones(n_out, np.float32), np.zeros(n_out, np.float32)], 1)
+        return torch.from_numpy(idx.astype(np.int32)), torch.from_numpy(wt)
+    scale = np.float32(n_in) / np.float32(n_out)
+    # the product of two FP32 numbers and the sum with 0.5 are exact in FP64: one rounding to FP32, i.e. the FMA
+    real = (np.float64(scale) * (d.astype(np.float32) + np.float32(0.5)).astype(np.float64) - 0.5).astype(np.float32)
+    real = np.maximum(real, np.float32(0))
+    i0 = np.minimum(np.floor(real).astype(np.int64), n_in - 1)
+    l1 = np.minimum(np.maximum(real - i0.astype(np.float32), np.float32(0)), np.float32(1)).astype(np.float32)
+    i1 = i0 + (i0 < n_in - 1)
+    l0 = (np.float32(1) - l1).astype(np.float32)
+    return torch.from_numpy(np.stack([i0, i1], 1).astype(np.int32)), torch.from_numpy(np.stack([l0, l1], 1))
+
+
+def view_shapes(frames_shape, crop_size, spatial_idx, alpha=None):
+    """Clip shapes [slow, fast] (`alpha` given) or [single] that `forward_frames(frames, crop_size=, spatial_idx=)` runs
+    on for uint8 frames of `frames_shape` (B, T, H, W, C): B * V rows of crop_size x crop_size.  ValueError when a crop does
+    not fit the resized frame."""
+    B, T, H, W, C = (int(n) for n in frames_shape)
+    views = spatial_views(spatial_idx)
+    S = int(crop_size)
+    Hr, Wr = resized_size(H, W, S)
+    for v in views:
+        y0, x0 = crop_offset(Hr, Wr, S, v)
+        if S < 1 or y0 < 0 or x0 < 0 or y0 + S > Hr or x0 + S > Wr:
+            raise ValueError("a %d x %d crop does not fit frames of %d x %d resized to %d x %d" % (S, S, H, W, Hr, Wr))
+    n = B * len(views)
+    if alpha is None:
+        return [(n, C, T, S, S)]
+    return [(n, C, T // alpha, S, S), (n, C, T, S, S)]
+
+
+class CropTables:
+    """Device tables of one (H0, W0, crop size, views) geometry: the per-axis resize tables and the crop offsets."""
+
+    def __init__(self, H0, W0, size, views, device):
+        self.H0, self.W0, self.S, self.views = H0, W0, size, views
+        self.Hr, self.Wr = resized_size(H0, W0, size)
+        self.resize = (self.Hr, self.Wr) != (H0, W0)
+        self.tables = None
+        if self.resize:
+            yi, yw = axis_table(H0, self.Hr)
+            xi, xw = axis_table(W0, self.Wr)
+            self.tables = [t.to(device) for t in (yi, yw, xi, xw)]
+        offs = [crop_offset(self.Hr, self.Wr, size, v) for v in views]
+        self.crop_yx = (ctypes.c_int32 * (2 * len(views)))(*[o for yx in offs for o in yx])
+
+    def pointers(self):
+        if self.tables is None:
+            return None, None, self.Hr, None, None, self.Wr
+        yi, yw, xi, xw = self.tables
+        return yi.data_ptr(), yw.data_ptr(), self.Hr, xi.data_ptr(), xw.data_ptr(), self.Wr
 
 
 class FrameInput:
@@ -53,6 +158,14 @@ class FrameInput:
         self.chan_src = (ctypes.c_int32 * channels)(*src)
         self.device = device
         self._index = {}
+        self._crops = {}
+
+    def crop(self, H0, W0, size, views):
+        """CropTables of frames H0 x W0 cropped to size x size at `views` (cached per geometry)."""
+        key = (H0, W0, size, tuple(views))
+        if key not in self._crops:
+            self._crops[key] = CropTables(H0, W0, size, tuple(views), self.device)
+        return self._crops[key]
 
     def index(self, t_src, t_out, alpha):
         """device int32 frame gather for a pathway with t_out of t_src frames (None: identity)."""
@@ -66,16 +179,20 @@ class FrameInput:
         return self._index[key]
 
 
-def launch_frames(plan, fin, frames, alpha, frame_index=None):
+def launch_frames(plan, fin, frames, alpha, frame_index=None, crop=None):
     """Fill the stem inputs of `plan` from uint8 frames (B, T, H, W, C) on the current stream.  `frame_index`: optional
     list (one entry per pathway) of device int32 tensors, source frame of every pathway frame -- replaces the loader's
-    rule (slow = linspace gather of the fast frames) for callers that keep frames in a ring (demo.SlidingWindow)."""
+    rule (slow = linspace gather of the fast frames) for callers that keep frames in a ring (demo.SlidingWindow).
+    `crop`: CropTables (FrameInput.crop) -- the frames are at decode size and every clip becomes V rows of crops."""
     L = rt.lib()
     s = rt.current_stream_ptr()
     B, Tsrc, H, W, C = frames.shape
     for pw, own in enumerate(plan.inputs):
         b, c, T, h, w = own.shape
-        assert (b, c, h, w) == (B, C, H, W)
+        if crop is not None:
+            assert (b, c, h, w) == (B * len(crop.views), C, crop.S, crop.S) and (H, W) == (crop.H0, crop.W0)
+        else:
+            assert (b, c, h, w) == (B, C, H, W)
         if frame_index is not None:
             idx = frame_index[pw]
             assert idx.dtype == torch.int32 and idx.numel() == T and idx.device == frames.device
@@ -83,7 +200,18 @@ def launch_frames(plan, fin, frames, alpha, frame_index=None):
             idx = fin.index(Tsrc, T, alpha)
         iptr = idx.data_ptr() if idx is not None else None
         route = plan.stem_routes.get(own.data_ptr())
-        if route is not None:
+        if crop is not None:
+            geo = crop.pointers() + (crop.crop_yx, len(crop.views), crop.S)
+            if route is not None:
+                xp, pitch, lpad = route
+                rt.check(L.esf_stem_pack_u8_crop(frames.data_ptr(), B, Tsrc, H, W, C, iptr, T, fin.chan_src,
+                                                 fin.lut32.data_ptr(), *geo, rt.dtype_code(xp), pitch, lpad,
+                                                 xp.data_ptr(), s), "esf_stem_pack_u8_crop")
+            else:
+                rt.check(L.esf_frames_to_clip_crop(frames.data_ptr(), B, Tsrc, H, W, C, iptr, T, fin.chan_src,
+                                                   fin.lut32.data_ptr(), *geo, own.data_ptr(), s),
+                         "esf_frames_to_clip_crop")
+        elif route is not None:
             xp, pitch, lpad = route
             rt.check(L.esf_stem_pack_u8(frames.data_ptr(), B, Tsrc, H, W, C, iptr, T, fin.chan_src, fin.lut16.data_ptr(),
                                         pitch, lpad, xp.data_ptr(), s), "esf_stem_pack_u8")

@@ -444,13 +444,30 @@ class _PlannedModel(nn.Module):
             return [(B, C, T, H, W)]
         return [(B, C, T // self._cfg.SLOWFAST.ALPHA, H, W), (B, C, T, H, W)]
 
-    def forward_frames(self, frames, bboxes=None, frame_index=None):
+    def forward_frames(self, frames, bboxes=None, frame_index=None, crop_size=None, spatial_idx=None):
         """Same result as `forward(pack_pathway_output(cfg, tensor_normalize(frames, MEAN, STD).permute(...)))` of the
         reference's loader chain, from the decoder's uint8 frames (B, T, H, W, C) on the device: normalisation,
-        layout change and the slow-pathway frame gather run inside the stem-pack kernel (frames.py)."""
+        layout change and the slow-pathway frame gather run inside the stem-pack kernel (frames.py).
+
+        Test-time spatial sampling: with `spatial_idx` (an int or a sequence of V values from {0, 1, 2}) the frames are
+        at decode size and every clip also goes through the reference's test-mode `spatial_sampling` (short side
+        resized to `crop_size`, default cfg.DATA.TEST_CROP_SIZE, then `uniform_crop` at each index) on the device.  The
+        result has B * V rows, row b * V + v being clip b at view v (the order of the test loader's clip numbering).
+        `crop_size` alone means spatial_idx 1 (TEST.NUM_SPATIAL_CROPS = 1)."""
         from . import frames as esf_frames
         if self.training:
             raise NotImplementedError("eval-mode forward path only")
+        crop = crop_size is not None or spatial_idx is not None
+        if crop:
+            if bboxes is not None:
+                raise ValueError("forward_frames: bboxes together with spatial_idx is not supported (the boxes would "
+                                 "need the crop's transform)")
+            views = esf_frames.spatial_views(1 if spatial_idx is None else spatial_idx)
+            crop_size = int(self._cfg.DATA.TEST_CROP_SIZE if crop_size is None else crop_size)
+            if frames.dim() != 5:
+                raise rt.EsfError("forward_frames expects contiguous uint8 frames (B, T, H, W, C)")
+            shapes = esf_frames.view_shapes(tuple(frames.shape), crop_size, views,
+                                            self._cfg.SLOWFAST.ALPHA if self.num_pathways > 1 else None)
         boxes = self._boxes(bboxes, frames.shape[0] if frames.dim() else 0, frames.device)
         if frames.device.type != "cuda":
             raise rt.EsfError("the forward path is CUDA-only (sm_100a); got frames on %s -- there is no CPU fallback"
@@ -458,20 +475,21 @@ class _PlannedModel(nn.Module):
         if frames.dtype != torch.uint8 or frames.dim() != 5 or not frames.is_contiguous():
             raise rt.EsfError("forward_frames expects contiguous uint8 frames (B, T, H, W, C)")
         dev = frames.device
+        alpha = self._cfg.SLOWFAST.ALPHA if self.num_pathways > 1 else 1
+        if not crop:
+            shapes = self.frame_shapes(tuple(frames.shape))
         if frames.shape[0] == 0 or (boxes is not None and boxes.shape[0] == 0):
             return self._empty(dev)
-        shapes = self.frame_shapes(tuple(frames.shape))
         if frame_index is not None:     # explicit source frame of every pathway frame (frames may be a ring buffer)
             assert len(frame_index) == self.num_pathways
-            B, _, H, W, C = frames.shape
-            shapes = [(B, C, int(ix.numel()), H, W) for ix in frame_index]
+            shapes = [tuple(sh[:2]) + (int(ix.numel()),) + tuple(sh[3:]) for sh, ix in zip(shapes, frame_index)]
         plan = self._get_plan(shapes, dev)
         fin = getattr(plan, "frame_input", None)
         if fin is None:
             fin = plan.frame_input = esf_frames.FrameInput(self._cfg, dev, plan.adt, channels=frames.shape[4])
-        alpha = self._cfg.SLOWFAST.ALPHA if self.num_pathways > 1 else 1
+        tabs = fin.crop(frames.shape[2], frames.shape[3], crop_size, views) if crop else None
         with torch.cuda.device(dev):
-            out = plan.run_frames(lambda: esf_frames.launch_frames(plan, fin, frames, alpha, frame_index))
+            out = plan.run_frames(lambda: esf_frames.launch_frames(plan, fin, frames, alpha, frame_index, tabs))
             return self._finish(plan, out, boxes)
 
     def _empty(self, dev):

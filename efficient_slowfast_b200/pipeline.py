@@ -19,7 +19,8 @@ from . import runtime as rt
 
 
 class ClipStream:
-    def __init__(self, model, shapes, device=None, depth=2, gather=False, frames=False, slow_from_fast=False):
+    def __init__(self, model, shapes, device=None, depth=2, gather=False, frames=False, slow_from_fast=False,
+                 crop_size=None, spatial_idx=None):
         """`depth` staging slots (>= 2 overlaps copy and compute); `gather=True` all-gathers the predictions over the
         process group before the D2H copy, like the reference's test loop.  `frames=True`: every batch is ONE pinned
         uint8 tensor of decoded frames (B, T, H, W, C) (`shapes` = [that shape]) and goes through
@@ -39,6 +40,15 @@ class ClipStream:
         self.copy_stream = torch.cuda.Stream(device=device)
         self.frames = bool(frames)
         assert not self.frames or len(shapes) == 1
+        self.crop = None
+        if crop_size is not None or spatial_idx is not None:
+            if not self.frames:
+                raise ValueError("ClipStream: crop_size / spatial_idx need frames=True")
+            from . import frames as esf_frames
+            views = esf_frames.spatial_views(1 if spatial_idx is None else spatial_idx)
+            size = int(model._cfg.DATA.TEST_CROP_SIZE if crop_size is None else crop_size)
+            esf_frames.view_shapes(tuple(shapes[0]), size, views)    # ValueError now rather than at the first batch
+            self.crop = {"crop_size": size, "spatial_idx": views}
         self.slow_from_fast = bool(slow_from_fast) and not self.frames and len(shapes) == 2
         self._sff_checked = False
         if self.slow_from_fast:
@@ -87,7 +97,7 @@ class ClipStream:
             self.ready[slot].record(self.copy_stream)
         cur.wait_event(self.ready[slot])
         if self.frames:
-            out = self.model.forward_frames(views[0])
+            out = self.model.forward_frames(views[0], **(self.crop or {}))
         elif self.slow_from_fast:
             out = self.model.forward_fast(views[0])
         else:

@@ -142,6 +142,27 @@ int esf_stem_pack_u8(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H, 
 int esf_frames_to_clip(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H, int32_t W, int32_t C,
                        const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32, float* clip,
                        void* stream);
+/* ---- test-time spatial sampling of uint8 frames (csrc/esf_crop.cu) -------------------------------------------------
+ * The same chain with the reference's test-mode spatial_sampling in between (SlowFast/slowfast/datasets/utils.py
+ * spatial_sampling -> transform.random_short_side_scale_jitter with min = max = crop size S, bilinear
+ * F.interpolate(align_corners=False), then transform.uniform_crop at spatial_idx 0/1/2), from frames at decode size
+ * (B, Tsrc, H0, W0, C).  Output row b * V + v is source clip b cropped at view v.  The resize to Hr x Wr is given as
+ * per-axis tables built on the host (efficient_slowfast_b200/frames.py axis_table): y_index[2 * r + k] / y_weight[2 * r + k]
+ * are the source rows i0, i1 and weights l0, l1 of resized row r (x_* the same for columns); they may be null when
+ * Hr == H0 and Wr == W0 (a pure window).  crop_yx_host: host int32[2 * V], (y0, x0) of every view in the resized frame,
+ * V <= 8; each crop must lie inside it.  W0 * C <= 16384.  lut32 as esf_frames_to_clip.
+ * esf_stem_pack_u8_crop writes the packed stem rows of esf_stem_pack ([B * V][T][S][pitch], dtype ESF_BF16 / ESF_F16);
+ * esf_frames_to_clip_crop the FP32 (B * V, C, T, S, S) clip. */
+int esf_stem_pack_u8_crop(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0, int32_t W0, int32_t C,
+                          const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
+                          const int32_t* y_index, const float* y_weight, int32_t Hr, const int32_t* x_index,
+                          const float* x_weight, int32_t Wr, const int32_t* crop_yx_host, int32_t V, int32_t S,
+                          int32_t dtype, int32_t pitch, int32_t lpad, void* xp, void* stream);
+int esf_frames_to_clip_crop(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0, int32_t W0, int32_t C,
+                            const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
+                            const int32_t* y_index, const float* y_weight, int32_t Hr, const int32_t* x_index,
+                            const float* x_weight, int32_t Wr, const int32_t* crop_yx_host, int32_t V, int32_t S,
+                            float* clip, void* stream);
 int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int32_t T, int32_t H, int32_t W, int32_t pitch,
                           const void* w_band, const float* bias_tiled, int32_t Cout, int32_t kT, int32_t kH,
                           int32_t kW, int32_t sH, int32_t sW, int32_t pT, int32_t pH, int32_t pW, int32_t act,
