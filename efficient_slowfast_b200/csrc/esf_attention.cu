@@ -1,294 +1,17 @@
-// CMDA slow->fast position attention, fused: softmax_j(q_i . k_j) v_j over all N = T*H*W positions of a clip with an
-// online softmax (the N x N affinity matrix is never written), followed by gamma * O + x_d, the bn_s2f affine, ReLU,
-// the x alpha nearest temporal upsample and the store into the fast pathway's concat slice.
+// Generic CUDA-core fallback of the CMDA slow->fast position attention: softmax_j(q_i . k_j) v_j over all N = T*H*W
+// positions of a clip, then gamma * O + x_d, the bn_s2f affine, ReLU, the x alpha nearest temporal upsample and the
+// store into the fast pathway's concat slice.
 //
-// Roofline: one exp per (query, key) pair and only 2*d..4*d MACs per pair with d = 8..32 at the two N = 25 088
-// stages -> the kernel is bound by the MUFU (exp) pipe, not by the tensor pipe (SURVEY.md 8d).  The logits are not
-// scaled by 1/sqrt(d) in the reference and reach |s| ~ 1e2, so BF16 q/k would put ~|s| * 2^-9 of noise inside the exp;
-// q and k are therefore split into BF16 hi + lo parts and the tensor cores evaluate q_hi.k_hi + q_lo.k_hi + q_hi.k_lo
-// (one MMA chain over K = 3d), which keeps the logits at ~FP32 accuracy for the price of idle tensor-pipe cycles.
-//
-// Register-resident flash layout: warp-level mma.sync m16n8k16 (S and P never leave registers: the S accumulator
-// fragment is re-used directly as the A fragment of P.V), cp.async double-buffered K/V tiles.
+// Any head dim, FP32 math straight from the projection rows [x_d | q | k | v]: one warp per query, logits staged in
+// shared memory.  Used only where the tcgen05 kernel (csrc/esf_attn_tc.cu) does not apply: d > 128, which in the
+// reference's models only occurs with N <= 392 keys (SlowFastShuffleNet s4_fuse, d = 240).
 #include <math_constants.h>
-
-#include <algorithm>
 
 #include "esf_common.cuh"
 #include "esf_host.h"
 
 namespace esf {
 
-constexpr int kAttnThreads = 128;
-constexpr int kAttnBN = 64;  // keys per tile
-constexpr float kLog2e = 1.4426950408889634f;
-
-struct AttnParams {
-  const __nv_bfloat16* q;  // [B][N][DK]
-  const __nv_bfloat16* k;  // [B][N][DK]
-  const __nv_bfloat16* v;  // [B][N][DV]
-  const float* x;          // [B][N][DV]  (x_d, the residual input of SpatialAttention)
-  int B, N, T, H, W, d, alpha;
-  float gamma;
-  const float* bn_scale;
-  const float* bn_shift;
-  __nv_bfloat16* y;
-  long long ysB, ysT, ysH, ysW;
-};
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem, bool valid) {
-  const int sz = valid ? 16 : 0;
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(smem)), "l"(gmem), "r"(sz) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void ldsm_x4(uint32_t* r, const void* p) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(smem_u32(p)));
-}
-__device__ __forceinline__ void ldsm_x4_t(uint32_t* r, const void* p) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(smem_u32(p)));
-}
-__device__ __forceinline__ void ldsm_x2_t(uint32_t* r, const void* p) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x2.trans.shared.b16 {%0,%1}, [%2];"
-               : "=r"(r[0]), "=r"(r[1])
-               : "r"(smem_u32(p)));
-}
-__device__ __forceinline__ void mma_bf16(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-template <int DV, int DK, int MB>
-struct AttnCfg {
-  static constexpr int BM = 4 * 16 * MB;
-  static constexpr int KP = DK + 8;                  // smem row pitch (elements): odd number of 16 B chunks
-  static constexpr int VP = (DV == 8) ? 8 : DV + 8;
-  static constexpr int q_elems = BM * KP;
-  static constexpr int k_elems = kAttnBN * KP;
-  static constexpr int v_elems = kAttnBN * VP;
-  static constexpr int smem_bytes = 2 * (q_elems + 2 * k_elems + 2 * v_elems);
-  static constexpr int OP = DV + 1;                  // FP32 pitch of the output staging tile
-  static_assert(BM * OP * 4 <= smem_bytes, "output staging does not fit");
-};
-
-template <int ROWS, int DIM, int PITCH>
-__device__ __forceinline__ void load_tile_async(__nv_bfloat16* dst, const __nv_bfloat16* src, int row0, int nrows_total) {
-  constexpr int CH = DIM / 8;  // 16 B chunks per row
-  for (int i = threadIdx.x; i < ROWS * CH; i += kAttnThreads) {
-    const int r = i / CH, c = i % CH;
-    const bool valid = row0 + r < nrows_total;
-    const __nv_bfloat16* g = src + (long long)(valid ? row0 + r : 0) * DIM + c * 8;
-    cp_async16(dst + r * PITCH + c * 8, g, valid);
-  }
-}
-
-template <int DV, int DK, int MB>
-__global__ void __launch_bounds__(kAttnThreads) attn_kernel(const AttnParams p) {
-  using Cfg = AttnCfg<DV, DK, MB>;
-  constexpr int BM = Cfg::BM, KP = Cfg::KP, VP = Cfg::VP;
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  __nv_bfloat16* Qs = reinterpret_cast<__nv_bfloat16*>(smem_raw);
-  __nv_bfloat16* Ks = Qs + Cfg::q_elems;
-  __nv_bfloat16* Vs = Ks + 2 * Cfg::k_elems;
-
-  const int b = blockIdx.y;
-  const int q0 = blockIdx.x * BM;
-  const int N = p.N;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int g = lane >> 2, t4 = lane & 3;
-  const __nv_bfloat16* Qg = p.q + (long long)b * N * DK;
-  const __nv_bfloat16* Kg = p.k + (long long)b * N * DK;
-  const __nv_bfloat16* Vg = p.v + (long long)b * N * DV;
-
-  load_tile_async<BM, DK, KP>(Qs, Qg, q0, N);
-  load_tile_async<kAttnBN, DK, KP>(Ks, Kg, 0, N);
-  load_tile_async<kAttnBN, DV, VP>(Vs, Vg, 0, N);
-  cp_async_commit();
-
-  float O[MB][DV / 8][4];
-  float mrow[MB][2], lrow[MB][2];
-#pragma unroll
-  for (int mi = 0; mi < MB; ++mi) {
-    mrow[mi][0] = mrow[mi][1] = -CUDART_INF_F;
-    lrow[mi][0] = lrow[mi][1] = 0.f;
-#pragma unroll
-    for (int nb = 0; nb < DV / 8; ++nb) O[mi][nb][0] = O[mi][nb][1] = O[mi][nb][2] = O[mi][nb][3] = 0.f;
-  }
-
-  const int nt = (N + kAttnBN - 1) / kAttnBN;
-  for (int jt = 0; jt < nt; ++jt) {
-    const int buf = jt & 1;
-    if (jt + 1 < nt) {
-      load_tile_async<kAttnBN, DK, KP>(Ks + (buf ^ 1) * Cfg::k_elems, Kg, (jt + 1) * kAttnBN, N);
-      load_tile_async<kAttnBN, DV, VP>(Vs + (buf ^ 1) * Cfg::v_elems, Vg, (jt + 1) * kAttnBN, N);
-      cp_async_commit();
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncthreads();
-    const __nv_bfloat16* Kt = Ks + buf * Cfg::k_elems;
-    const __nv_bfloat16* Vt = Vs + buf * Cfg::v_elems;
-
-    // ---- S = Q K^T (16*MB x 64 per warp)
-    float S[MB][8][4];
-#pragma unroll
-    for (int mi = 0; mi < MB; ++mi)
-#pragma unroll
-      for (int nb = 0; nb < 8; ++nb) S[mi][nb][0] = S[mi][nb][1] = S[mi][nb][2] = S[mi][nb][3] = 0.f;
-#pragma unroll
-    for (int ks = 0; ks < DK / 16; ++ks) {
-      uint32_t a[MB][4];
-#pragma unroll
-      for (int mi = 0; mi < MB; ++mi)
-        ldsm_x4(a[mi], Qs + (warp * 16 * MB + mi * 16 + (lane & 7) + ((lane >> 3) & 1) * 8) * KP + ks * 16 +
-                           (lane >> 4) * 8);
-#pragma unroll
-      for (int nb2 = 0; nb2 < 4; ++nb2) {
-        uint32_t bf[4];
-        ldsm_x4(bf, Kt + (nb2 * 16 + (lane & 7) + (lane >> 4) * 8) * KP + ks * 16 + ((lane >> 3) & 1) * 8);
-#pragma unroll
-        for (int mi = 0; mi < MB; ++mi) {
-          mma_bf16(S[mi][2 * nb2], a[mi], bf[0], bf[1]);
-          mma_bf16(S[mi][2 * nb2 + 1], a[mi], bf[2], bf[3]);
-        }
-      }
-    }
-    if (jt == nt - 1 && (N % kAttnBN) != 0) {  // mask keys beyond N in the tail tile
-#pragma unroll
-      for (int nb = 0; nb < 8; ++nb) {
-        const int key = jt * kAttnBN + nb * 8 + 2 * t4;
-#pragma unroll
-        for (int mi = 0; mi < MB; ++mi) {
-          if (key >= N) S[mi][nb][0] = S[mi][nb][2] = -CUDART_INF_F;
-          if (key + 1 >= N) S[mi][nb][1] = S[mi][nb][3] = -CUDART_INF_F;
-        }
-      }
-    }
-
-    // ---- online softmax (FP32 statistics) and O += P V
-#pragma unroll
-    for (int mi = 0; mi < MB; ++mi) {
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        float mx = -CUDART_INF_F;
-#pragma unroll
-        for (int nb = 0; nb < 8; ++nb) mx = fmaxf(mx, fmaxf(S[mi][nb][2 * h], S[mi][nb][2 * h + 1]));
-        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
-        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
-        const float m_new = fmaxf(mrow[mi][h], mx);
-        const float corr = exp2f((mrow[mi][h] - m_new) * kLog2e);
-        mrow[mi][h] = m_new;
-        const float ms = m_new * kLog2e;
-        float sum = 0.f;
-#pragma unroll
-        for (int nb = 0; nb < 8; ++nb) {
-          const float p0 = exp2f(fmaf(S[mi][nb][2 * h], kLog2e, -ms));
-          const float p1 = exp2f(fmaf(S[mi][nb][2 * h + 1], kLog2e, -ms));
-          S[mi][nb][2 * h] = p0;
-          S[mi][nb][2 * h + 1] = p1;
-          sum += p0 + p1;
-        }
-        lrow[mi][h] = lrow[mi][h] * corr + sum;
-#pragma unroll
-        for (int nb = 0; nb < DV / 8; ++nb) {
-          O[mi][nb][2 * h] *= corr;
-          O[mi][nb][2 * h + 1] *= corr;
-        }
-      }
-    }
-#pragma unroll
-    for (int kk = 0; kk < 4; ++kk) {
-      uint32_t pa[MB][4];
-#pragma unroll
-      for (int mi = 0; mi < MB; ++mi) {
-        pa[mi][0] = pack_bf16x2(S[mi][2 * kk][0], S[mi][2 * kk][1]);
-        pa[mi][1] = pack_bf16x2(S[mi][2 * kk][2], S[mi][2 * kk][3]);
-        pa[mi][2] = pack_bf16x2(S[mi][2 * kk + 1][0], S[mi][2 * kk + 1][1]);
-        pa[mi][3] = pack_bf16x2(S[mi][2 * kk + 1][2], S[mi][2 * kk + 1][3]);
-      }
-      const int krow = kk * 16 + (lane & 7) + ((lane >> 3) & 1) * 8;
-      if constexpr (DV == 8) {
-        uint32_t bv[2];
-        ldsm_x2_t(bv, Vt + krow * VP);
-#pragma unroll
-        for (int mi = 0; mi < MB; ++mi) mma_bf16(O[mi][0], pa[mi], bv[0], bv[1]);
-      } else {
-#pragma unroll
-        for (int nb2 = 0; nb2 < DV / 16; ++nb2) {
-          uint32_t bv[4];
-          ldsm_x4_t(bv, Vt + krow * VP + nb2 * 16 + (lane >> 4) * 8);
-#pragma unroll
-          for (int mi = 0; mi < MB; ++mi) {
-            mma_bf16(O[mi][2 * nb2], pa[mi], bv[0], bv[1]);
-            mma_bf16(O[mi][2 * nb2 + 1], pa[mi], bv[2], bv[3]);
-          }
-        }
-      }
-    }
-    __syncthreads();  // every warp is done with this K/V buffer before it is refilled
-  }
-
-  // ---- epilogue: normalise, stage through smem, fused gamma*O + x -> BN -> ReLU -> x alpha upsample -> store
-  float* Os = reinterpret_cast<float*>(smem_raw);
-  constexpr int OP = Cfg::OP;
-#pragma unroll
-  for (int mi = 0; mi < MB; ++mi) {
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      float l = lrow[mi][h];
-      l += __shfl_xor_sync(0xffffffffu, l, 1);
-      l += __shfl_xor_sync(0xffffffffu, l, 2);
-      const float inv = 1.f / l;
-      const int row = warp * 16 * MB + mi * 16 + g + 8 * h;
-#pragma unroll
-      for (int nb = 0; nb < DV / 8; ++nb) {
-        Os[row * OP + nb * 8 + 2 * t4] = O[mi][nb][2 * h] * inv;
-        Os[row * OP + nb * 8 + 2 * t4 + 1] = O[mi][nb][2 * h + 1] * inv;
-      }
-    }
-  }
-  __syncthreads();
-  const int HW = p.H * p.W;
-  const int d8 = p.d / 8;
-  for (int i = threadIdx.x; i < BM * d8; i += kAttnThreads) {
-    const int row = i / d8, c0 = (i % d8) * 8;
-    const int n = q0 + row;
-    if (n >= N) continue;
-    const float* xr = p.x + ((long long)b * N + n) * DV + c0;
-    const float4 x0 = *reinterpret_cast<const float4*>(xr);
-    const float4 x1 = *reinterpret_cast<const float4*>(xr + 4);
-    const float xv[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
-    float o[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const float a = fmaf(p.gamma, Os[row * OP + c0 + j], xv[j]);
-      o[j] = fmaxf(fmaf(a, __ldg(p.bn_scale + c0 + j), __ldg(p.bn_shift + c0 + j)), 0.f);
-    }
-    uint4 pk;
-    pk.x = pack_bf16x2(o[0], o[1]);
-    pk.y = pack_bf16x2(o[2], o[3]);
-    pk.z = pack_bf16x2(o[4], o[5]);
-    pk.w = pack_bf16x2(o[6], o[7]);
-    const int t = n / HW, hw = n % HW, h = hw / p.W, w = hw % p.W;
-    __nv_bfloat16* yb = p.y + b * p.ysB + h * p.ysH + w * p.ysW + c0;
-    for (int r = 0; r < p.alpha; ++r) *reinterpret_cast<uint4*>(yb + (long long)(t * p.alpha + r) * p.ysT) = pk;
-  }
-}
-
-// ---------------------------------------------------------------------------------------------- generic fallback
-// Any head dim, FP32 math straight from the projection rows [x_d | q | k | v]: one warp per query, logits staged in
-// shared memory.  Used only where the tensor-core kernels do not apply (d > 128, which in the reference's models
-// only occurs with N <= 392 keys: SlowFastShuffleNet s4_fuse, d = 240).
 __global__ void __launch_bounds__(128) attn_generic_kernel(const float* __restrict__ proj, int N, int T, int H, int W,
                                                            int d, float gamma, const float* __restrict__ bn_scale,
                                                            const float* __restrict__ bn_shift, int alpha, int f16,
@@ -326,143 +49,9 @@ __global__ void __launch_bounds__(128) attn_generic_kernel(const float* __restri
   }
 }
 
-// ---------------------------------------------------------------------------------------------- packing
-struct PackGeom {
-  int DV, DK, split;
-};
-static bool attn_geom(int d, PackGeom* g) {
-  if (d <= 0 || d % 8 != 0) return false;
-  if (d <= 8) *g = {8, 32, 1};
-  else if (d <= 16) *g = {16, 48, 1};
-  else if (d <= 32) *g = {32, 96, 1};
-  else if (d <= 64) *g = {64, 192, 1};
-  else if (d <= 128) *g = {128, 128, 0};
-  else return false;
-  return true;
-}
-
-// proj rows are [x_d | q | k | v] (d each, FP32); one thread per (row, channel j < DV)
-__global__ void __launch_bounds__(256) attn_pack_kernel(const float* __restrict__ proj, long long rows, int d, int DV,
-                                                        int DK, int split, __nv_bfloat16* __restrict__ Q,
-                                                        __nv_bfloat16* __restrict__ K, __nv_bfloat16* __restrict__ V,
-                                                        float* __restrict__ X) {
-  const long long total = rows * DV;
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
-       i += (long long)gridDim.x * blockDim.x) {
-    const long long r = i / DV;
-    const int j = i % DV;
-    float xd = 0.f, q = 0.f, k = 0.f, v = 0.f;
-    if (j < d) {
-      const float* pr = proj + r * 4 * d;
-      xd = pr[j], q = pr[d + j], k = pr[2 * d + j], v = pr[3 * d + j];
-    }
-    const __nv_bfloat16 qh = __float2bfloat16(q), kh = __float2bfloat16(k);
-    __nv_bfloat16* qr = Q + r * DK;
-    __nv_bfloat16* kr = K + r * DK;
-    if (split) {
-      const __nv_bfloat16 ql = __float2bfloat16(q - __bfloat162float(qh));
-      const __nv_bfloat16 kl = __float2bfloat16(k - __bfloat162float(kh));
-      qr[j] = qh, qr[DV + j] = ql, qr[2 * DV + j] = qh;
-      kr[j] = kh, kr[DV + j] = kh, kr[2 * DV + j] = kl;
-      for (int c = 3 * DV + j; c < DK; c += DV) qr[c] = __float2bfloat16(0.f), kr[c] = __float2bfloat16(0.f);
-    } else {
-      qr[j] = qh, kr[j] = kh;
-    }
-    V[r * DV + j] = __float2bfloat16(v);
-    X[r * DV + j] = xd;
-  }
-}
-
-struct PackLayout {
-  long long q_off, k_off, v_off, x_off, total;
-};
-static PackLayout pack_layout(long long rows, const PackGeom& g) {
-  auto al = [](long long v) { return (v + 255) & ~255LL; };
-  PackLayout L;
-  L.q_off = 0;
-  L.k_off = al(L.q_off + rows * g.DK * 2);
-  L.v_off = al(L.k_off + rows * g.DK * 2);
-  L.x_off = al(L.v_off + rows * g.DV * 2);
-  L.total = al(L.x_off + rows * g.DV * 4);
-  return L;
-}
-
-template <int DV, int DK, int MB>
-static int launch_attn(const AttnParams& p, cudaStream_t s) {
-  using Cfg = AttnCfg<DV, DK, MB>;
-  static unsigned char attr_done[kMaxDevices] = {0};   // kernel attributes are per device
-  unsigned char* slot = device_slot(attr_done);
-  if (!slot || !*slot) {
-    ESF_CUDA(cudaFuncSetAttribute(attn_kernel<DV, DK, MB>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem_bytes));
-    if (slot) *slot = 1;
-  }
-  dim3 grid(cdiv(p.N, Cfg::BM), p.B);
-  attn_kernel<DV, DK, MB><<<grid, kAttnThreads, Cfg::smem_bytes, s>>>(p);
-  return check_launch("attn_kernel");
-}
-
 }  // namespace esf
 
 using namespace esf;
-
-extern "C" int64_t esf_attn_pack_bytes(int32_t B, int32_t N, int32_t d) {
-  PackGeom g;
-  if (!attn_geom(d, &g)) return set_error(ESF_ERR_UNSUPPORTED, "esf_attn: unsupported head dim %d", d);
-  return pack_layout((long long)B * N, g).total;
-}
-
-extern "C" int esf_attn_pack(const float* proj, int32_t B, int32_t N, int32_t d, void* packed, void* stream) {
-  ESF_CHECK_ARG(proj && packed && B > 0 && N > 0, "esf_attn_pack: null/bad argument");
-  PackGeom g;
-  if (!attn_geom(d, &g)) return set_error(ESF_ERR_UNSUPPORTED, "esf_attn_pack: unsupported head dim %d", d);
-  const long long rows = (long long)B * N;
-  const PackLayout L = pack_layout(rows, g);
-  char* base = static_cast<char*>(packed);
-  const long long total = rows * g.DV;
-  const int grid = (int)std::min<long long>((total + 255) / 256, 148LL * 32);
-  attn_pack_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      proj, rows, d, g.DV, g.DK, g.split, reinterpret_cast<__nv_bfloat16*>(base + L.q_off),
-      reinterpret_cast<__nv_bfloat16*>(base + L.k_off), reinterpret_cast<__nv_bfloat16*>(base + L.v_off),
-      reinterpret_cast<float*>(base + L.x_off));
-  return check_launch("attn_pack_kernel");
-}
-
-extern "C" int esf_attn_fused(const void* packed, int32_t B, int32_t T, int32_t H, int32_t W, int32_t d, float gamma,
-                              const float* bn_scale, const float* bn_shift, int32_t alpha,
-                              const esf_view* y_fast_slice, void* stream) {
-  ESF_CHECK_ARG(packed && bn_scale && bn_shift && view_ok(y_fast_slice), "esf_attn_fused: null/bad argument");
-  ESF_CHECK_ARG(y_fast_slice->dtype == ESF_BF16, "esf_attn_fused (mma.sync variant) is BF16-only; use esf_attn_tc_*");
-  PackGeom g;
-  if (!attn_geom(d, &g)) return set_error(ESF_ERR_UNSUPPORTED, "esf_attn_fused: unsupported head dim %d", d);
-  const esf_view* y = y_fast_slice;
-  ESF_CHECK_ARG(y->B == B && y->T == T * alpha && y->H == H && y->W == W && y->C == d,
-                "esf_attn_fused: output slice (%d,%d,%d,%d,%d) != (%d,%d,%d,%d,%d)", y->B, y->T, y->H, y->W, y->C, B,
-                T * alpha, H, W, d);
-  ESF_CHECK_ARG(reinterpret_cast<uintptr_t>(y->ptr) % 16 == 0 && y->sW % 8 == 0 && y->sH % 8 == 0 && y->sT % 8 == 0 &&
-                    y->sB % 8 == 0,
-                "esf_attn_fused: output slice must be 16-byte aligned");
-  const int N = T * H * W;
-  const PackLayout L = pack_layout((long long)B * N, g);
-  const char* base = static_cast<const char*>(packed);
-  AttnParams p;
-  p.q = reinterpret_cast<const __nv_bfloat16*>(base + L.q_off);
-  p.k = reinterpret_cast<const __nv_bfloat16*>(base + L.k_off);
-  p.v = reinterpret_cast<const __nv_bfloat16*>(base + L.v_off);
-  p.x = reinterpret_cast<const float*>(base + L.x_off);
-  p.B = B, p.N = N, p.T = T, p.H = H, p.W = W, p.d = d, p.alpha = alpha, p.gamma = gamma;
-  p.bn_scale = bn_scale, p.bn_shift = bn_shift;
-  p.y = static_cast<__nv_bfloat16*>(y->ptr);
-  p.ysB = y->sB, p.ysT = y->sT, p.ysH = y->sH, p.ysW = y->sW;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  switch (g.DV) {
-    case 8: return launch_attn<8, 32, 2>(p, s);
-    case 16: return launch_attn<16, 48, 2>(p, s);
-    case 32: return launch_attn<32, 96, 2>(p, s);
-    case 64: return launch_attn<64, 192, 2>(p, s);
-    case 128: return launch_attn<128, 128, 1>(p, s);
-  }
-  return set_error(ESF_ERR_UNSUPPORTED, "esf_attn_fused: no kernel for DV=%d", g.DV);
-}
 
 extern "C" int esf_attn_generic(const float* proj, int32_t B, int32_t T, int32_t H, int32_t W, int32_t d, float gamma,
                                 const float* bn_scale, const float* bn_shift, int32_t alpha,

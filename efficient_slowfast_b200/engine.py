@@ -9,7 +9,6 @@ Design (B200-first, not a module-by-module translation of the reference):
   * there is no PyTorch compute on the path -- torch only owns the memory and the stream.
 """
 import ctypes
-import os
 
 import torch
 
@@ -105,6 +104,20 @@ def pack_stem_tband(w, bias, WB, stride_w, device, dtype=torch.bfloat16):
     return to_device(band.reshape(kt * NB, kh * 64), device, dtype), to_device(bt, device, torch.float32)
 
 
+def stem_route(x_shape, w_shape, stride, padding):
+    """Stem kernel for a (B,Cin,T,H,W) clip and a (Cout,Cin,kT,kH,kW) weight: None for the CUDA-core stem
+    (esf_stem_conv), else (pitch, lpad, twb) -- the packed-row geometry of esf_stem_pack and the output-column block of
+    the temporal-band GEMM (esf_stem_tband_create: kT > 1, time taps folded into N), twb == 0 for the banded GEMM
+    (esf_stem_igemm_create)."""
+    _, cin, _, _, W = x_shape
+    cout, _, kt, kh, kw = w_shape
+    geo = rt.stem_geometry(W, cin, kw, stride[2], padding[2]) if stride[0] == 1 else None
+    if geo is None:
+        return None
+    pitch, lpad, _ = geo
+    return pitch, lpad, rt.stem_tband_wb(W, cin, cout, kt, kh, kw, stride[2], padding[2])
+
+
 def pack_wfold_band(w, bias, WB, stride_w, device, dtype=torch.bfloat16):
     """Folded (Cout,Cin,kT,kH,kW) weight of a thin layer -> band matrix [n_pad][kT*kH*kchunks*64] and tiled bias [n_pad]
     for esf_conv_wfold_create.  Row n = i*Cout + co (i = output column inside the WB-wide block); column
@@ -149,6 +162,29 @@ def wfold_block(x, y, res, w_shape, stride, padding, dilation):
     return best if best >= 2 else 0     # a block of one column is the plain implicit GEMM
 
 
+def attention_projection(w_down, att):
+    """The slow->fast fuse's 1x1x1 C->d conv composed with SpatialAttention's q/k/v 1x1x1 convs
+    (wdf_attention_helper.py:33-54): one FP64 (4d, C, 1, 1, 1) weight and (4d,) bias whose output rows are
+    [x_d | q | k | v], and the head dim d."""
+    wd = host64(w_down).reshape(w_down.shape[0], -1)                      # (d, C)
+    d, C = wd.shape
+    mats, biases = [wd], [torch.zeros(d, dtype=torch.float64)]
+    for conv in (att.query_conv, att.key_conv, att.value_conv):
+        wc = host64(conv.weight).reshape(conv.weight.shape[0], d)
+        bc = host64(conv.bias)
+        if wc.shape[0] < d:
+            # SpatialAttention(reduction > 1) (wdf_attention_helper.py:17-26): query / key have d / reduction
+            # channels.  Zero rows up to d leave every logit q.k unchanged and keep the kernels' one head dim.
+            # (No cfg key reaches this: every call site of the reference hard-codes reduction = 1.)
+            assert conv is not att.value_conv, "value_conv keeps all channels"
+            pad = d - wc.shape[0]
+            wc = torch.cat([wc, torch.zeros(pad, d, dtype=wc.dtype)], 0)
+            bc = torch.cat([bc, torch.zeros(pad, dtype=bc.dtype)], 0)
+        mats.append(wc @ wd)
+        biases.append(bc)
+    return torch.cat(mats, 0).reshape(4 * d, C, 1, 1, 1), torch.cat(biases, 0), d
+
+
 def head_fc_launches(B, cin, K, act):
     """Kernel launches of one esf_head_fc call: the tiled kernel (B >= 8, or rows too long for one block) applies the
     class softmax in a second, tiny kernel."""
@@ -159,6 +195,8 @@ def head_fc_launches(B, cin, K, act):
 class Plan:
     """Ordered kernel launches + every tensor they touch.  `eager` ops read the caller's input tensors and are
     launched on every forward; `graph` ops only touch plan-owned memory and are replayed from one CUDA graph."""
+
+    wfold = True     # thin layers (C_in <= 32) as W-folded banded GEMMs
 
     def __init__(self, device, precision="bf16"):
         self.device = device
@@ -179,8 +217,6 @@ class Plan:
         self.launches_per_run = 0
         self.buffers = {}     # name -> activation tensor (for tests / debugging)
         self.meta = []        # one dict per op: kind, label, algorithmic flops / bytes / exps, launches
-        self.wfold = True            # thin layers (C_in <= 32) as W-folded banded GEMMs
-        self.attn_impl = "tcgen05"   # "tcgen05" (TMEM, two-pass) or "mma_sync" (register-resident, online softmax)
 
     # ---------------------------------------------------------------- memory
     def act(self, B, T, H, W, C, name=None, dtype=None, role=None):
@@ -531,37 +567,49 @@ class Plan:
         return self.input_override.get(p, p)
 
     def stem(self, x_nc, y, w_folded, bias, stride, padding, act=rt.ACT_RELU):
-        """Stem conv + folded BN + ReLU.  Tensor-core banded GEMM when the geometry allows (temporal stride 1,
-        window <= 64 elements, dense output), else the generic CUDA-core stem kernel."""
-        B, Cin, T, H, W = x_nc.shape
+        """Stem conv + folded BN + ReLU on the kernel stem_route picks; an output that is not dense takes the CUDA-core
+        stem as well."""
+        route = stem_route(x_nc.shape, w_folded.shape, stride, padding)
+        if route is None or not y.is_contiguous():
+            return self.stem_conv(x_nc, y, w_folded, bias, stride, padding, act)
+        self.stem_gemm(x_nc, y, w_folded, bias, stride, padding, act, *route)
+
+    def _stem_gemm_op(self, xp, x_shape, y, w_folded, bias, stride, padding, act, pitch, twb, name=""):
+        """One tensor-core stem GEMM from the packed 16-bit rows `xp` into the dense `y`: the weight is band-packed for the
+        temporal-band kernel (twb > 0 output columns per block) or the banded kernel (twb == 0), the op is created and
+        its launch appended to the plan."""
+        B, Cin, T, H, W = x_shape
         cout = w_folded.shape[0]
         kt, kh, kw = w_folded.shape[2:]
-        geo = rt.stem_geometry(W, Cin, kw, stride[2], padding[2]) if stride[0] == 1 else None
-        if geo is None or not y.is_contiguous():
-            return self.stem_conv(x_nc, y, w_folded, bias, stride, padding, act)
-        pitch, lpad, _ = geo
         L = rt.lib()
-        xp = torch.empty((B, T, H, pitch), dtype=self.adt, device=self.device)
-        yv = rt.view(y)
-        h = ctypes.c_void_p()
-        # kT > 1: the time taps are folded into N and the input frames stream past a resident M tile (csrc/esf_igemm.cu,
-        # "temporal-band stem"); ESF_STEM_TBAND=0 keeps the banded stem for A/B runs
-        twb = rt.stem_tband_wb(W, Cin, cout, kt, kh, kw, stride[2], padding[2]) \
-            if os.environ.get("ESF_STEM_TBAND", "1") != "0" else 0
         if twb:
             wb, bt = pack_stem_tband(w_folded, bias, twb, stride[2], self.device, self.adt)
-            rt.check(L.esf_stem_tband_create(xp.data_ptr(), B, Cin, T, H, W, pitch, wb.data_ptr(), bt.data_ptr(), cout,
-                                             kt, kh, kw, stride[1], stride[2], padding[0], padding[1], padding[2], act,
-                                             ctypes.byref(yv), ctypes.byref(h)), "esf_stem_tband_create")
+            create, what = L.esf_stem_tband_create, "esf_stem_tband_create"
         else:
             wb, bt = pack_stem_band(w_folded, bias, stride[2], self.device, self.adt)
-            rt.check(L.esf_stem_igemm_create(xp.data_ptr(), B, Cin, T, H, W, pitch, wb.data_ptr(), bt.data_ptr(), cout,
-                                             kt, kh, kw, stride[1], stride[2], padding[0], padding[1], padding[2], act,
-                                             ctypes.byref(yv), ctypes.byref(h)), "esf_stem_igemm_create")
-        self.keep += [xp, wb, bt]
+            create, what = L.esf_stem_igemm_create, "esf_stem_igemm_create"
+        yv = rt.view(y)
+        h = ctypes.c_void_p()
+        rt.check(create(xp.data_ptr(), B, Cin, T, H, W, pitch, wb.data_ptr(), bt.data_ptr(), cout, kt, kh, kw,
+                        stride[1], stride[2], padding[0], padding[1], padding[2], act, ctypes.byref(yv),
+                        ctypes.byref(h)), what)
+        self.keep += [wb, bt]
         self.handles.append(h)
+        label = "%dx%dx%d %d->%d %s" % (kt, kh, kw, Cin, cout, "t-band" if twb else "banded")
         m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
+        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "stem_igemm",
+                  label + (" " + name if name else ""), flops=2.0 * m * cout * Cin * kt * kh * kw,
+                  nbytes=self._nbytes(xp, y) + wb.numel() * 2)
+
+    def stem_gemm(self, x_nc, y, w_folded, bias, stride, padding, act, pitch, lpad, twb):
+        """Stem on the tensor cores: the clip is packed into 16-bit rows (`pitch`, `lpad`: esf_stem_geometry), then one
+        GEMM -- temporal-band for twb > 0, banded for twb == 0 (see stem_route)."""
+        B, Cin, T, H, W = x_nc.shape
+        L = rt.lib()
+        xp = torch.empty((B, T, H, pitch), dtype=self.adt, device=self.device)
+        self.keep.append(xp)
         self.stem_routes[x_nc.data_ptr()] = (xp, pitch, lpad)   # the uint8 frame route writes xp itself (frames.py)
+
         def pack(s):
             g = self.gather.get(x_nc.data_ptr())
             if g is not None:       # frames of this pathway are read out of another pathway's clip (slow from fast)
@@ -574,9 +622,7 @@ class Plan:
 
         self._add(pack, "stem_pack", "", nbytes=self._nbytes(x_nc, xp), eager=True)
         self.meta[-1]["is_pack"] = True
-        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "stem_igemm",
-                  "%dx%dx%d %d->%d %s" % (kt, kh, kw, Cin, cout, "t-band" if twb else "banded"), flops=2.0 * m * cout * Cin * kt * kh * kw,
-                  nbytes=self._nbytes(xp, y) + wb.numel() * 2)
+        self._stem_gemm_op(xp, x_nc.shape, y, w_folded, bias, stride, padding, act, pitch, twb)
 
     def pool(self, x, y, kernel, stride, padding, is_avg=False, act=rt.ACT_NONE):
         xv, yv = rt.view(x), rt.view(y)
@@ -659,81 +705,41 @@ class Plan:
             nbytes=2 * self._nbytes(x_fast) + self._nbytes(y_slice), launches=2)
 
     def position_attention(self, x_slow, y_slice, alpha, w_down, att, bn):
-        """1x1x1 C->d conv composed with the q/k/v 1x1x1 convs into one GEMM (FP32 out), hi/lo packing, fused
-        flash-style attention + gamma*O + x + BN + ReLU + x alpha upsample + concat
-        (custom_video_model_builder.py:141-146, wdf_attention_helper.py:33-54)."""
+        """attention_projection as one GEMM (FP32 out), hi/lo packing, fused flash-style attention + gamma*O + x + BN +
+        ReLU + x alpha upsample + concat (custom_video_model_builder.py:141-146, wdf_attention_helper.py:33-54): the
+        tcgen05 kernel up to d = 128, the CUDA-core fallback above."""
         B, T, H, W, C = x_slow.shape
-        wd = host64(w_down).reshape(w_down.shape[0], C)                      # (d, C)
-        d = wd.shape[0]
-        mats, biases = [wd], [torch.zeros(d, dtype=torch.float64)]
-        for conv in (att.query_conv, att.key_conv, att.value_conv):
-            wc = host64(conv.weight).reshape(conv.weight.shape[0], d)
-            bc = host64(conv.bias)
-            if wc.shape[0] < d:
-                # SpatialAttention(reduction > 1) (wdf_attention_helper.py:17-26): query / key have d / reduction
-                # channels.  Zero rows up to d leave every logit q.k unchanged and keep the kernels' one head dim.
-                # (No cfg key reaches this: every call site of the reference hard-codes reduction = 1.)
-                assert conv is not att.value_conv, "value_conv keeps all channels"
-                pad = d - wc.shape[0]
-                wc = torch.cat([wc, torch.zeros(pad, d, dtype=wc.dtype)], 0)
-                bc = torch.cat([bc, torch.zeros(pad, dtype=bc.dtype)], 0)
-            mats.append(wc @ wd)
-            biases.append(bc)
-        w_all = torch.cat(mats, 0).reshape(4 * d, C, 1, 1, 1)
-        b_all = torch.cat(biases, 0)
+        w_all, b_all, d = attention_projection(w_down, att)
         proj = self.act(B, T, H, W, 4 * d, dtype=torch.float32)
         self.conv(x_slow, proj, w_all, b_all)
         L = rt.lib()
         N = T * H * W
-        if d > 128:
-            scale, shift = bn_affine(bn)
-            sc, sh = self.tensor(scale), self.tensor(shift)
-            gamma = float(att.gamma.detach().float().item())
-            yv = rt.view(y_slice)
-            self.keep.append(yv)
-            self._add(lambda s: rt.check(
-                L.esf_attn_generic(proj.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                                   ctypes.byref(yv), s), "esf_attn_generic"), "attention", "N=%d d=%d generic" % (N, d),
-                flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj, y_slice))
-            return
-        if self.attn_impl == "tcgen05":
-            nbytes = int(L.esf_attn_tc_pack_bytes(B, N, d))
-            if nbytes < 0:
-                rt.check(nbytes, "esf_attn_tc_pack_bytes")
-            packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-            self.keep.append(packed)
-            scale, shift = bn_affine(bn)
-            sc, sh = self.tensor(scale), self.tensor(shift)
-            gamma = float(att.gamma.detach().float().item())
-            yv = rt.view(y_slice)
-            h = ctypes.c_void_p()
-            rt.check(L.esf_attn_tc_create(packed.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                                          ctypes.byref(yv), ctypes.byref(h)), "esf_attn_tc_create")
-            self.handles.append(h)
-            self._add(lambda s: rt.check(L.esf_attn_tc_pack(proj.data_ptr(), B, N, d, self.a16, packed.data_ptr(), s),
-                                         "esf_attn_tc_pack"), "attn_pack", "N=%d d=%d" % (N, d),
-                      nbytes=self._nbytes(proj) + nbytes)
-            self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "attention",
-                      "N=%d d=%d" % (N, d), flops=4.0 * B * N * N * d, exps=float(B) * N * N,
-                      nbytes=nbytes + self._nbytes(y_slice))
-            return
-        nbytes = int(L.esf_attn_pack_bytes(B, N, d))
-        if nbytes < 0:
-            rt.check(nbytes, "esf_attn_pack_bytes")
-        packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-        self.keep.append(packed)
         scale, shift = bn_affine(bn)
         sc, sh = self.tensor(scale), self.tensor(shift)
         gamma = float(att.gamma.detach().float().item())
         yv = rt.view(y_slice)
         self.keep.append(yv)
-        self._add(lambda s: rt.check(L.esf_attn_pack(proj.data_ptr(), B, N, d, packed.data_ptr(), s),
-                                     "esf_attn_pack"), "attn_pack", "N=%d d=%d" % (N, d),
+        if d > 128:
+            self._add(lambda s: rt.check(
+                L.esf_attn_generic(proj.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
+                                   ctypes.byref(yv), s), "esf_attn_generic"), "attention", "N=%d d=%d generic" % (N, d),
+                flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj, y_slice))
+            return
+        nbytes = int(L.esf_attn_tc_pack_bytes(B, N, d))
+        if nbytes < 0:
+            rt.check(nbytes, "esf_attn_tc_pack_bytes")
+        packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        self.keep.append(packed)
+        h = ctypes.c_void_p()
+        rt.check(L.esf_attn_tc_create(packed.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
+                                      ctypes.byref(yv), ctypes.byref(h)), "esf_attn_tc_create")
+        self.handles.append(h)
+        self._add(lambda s: rt.check(L.esf_attn_tc_pack(proj.data_ptr(), B, N, d, self.a16, packed.data_ptr(), s),
+                                     "esf_attn_tc_pack"), "attn_pack", "N=%d d=%d" % (N, d),
                   nbytes=self._nbytes(proj) + nbytes)
-        self._add(lambda s: rt.check(
-            L.esf_attn_fused(packed.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                             ctypes.byref(yv), s), "esf_attn_fused"), "attention", "N=%d d=%d" % (N, d),
-            flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=nbytes + self._nbytes(y_slice))
+        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "attention",
+                  "N=%d d=%d" % (N, d), flops=4.0 * B * N * N * d, exps=float(B) * N * N,
+                  nbytes=nbytes + self._nbytes(y_slice))
 
     def head(self, xs, weight, bias, act):
         B = xs[0].shape[0]
@@ -924,7 +930,7 @@ class Plan:
         """`inputs`: optional caller tensors to read INSTEAD of the plan-owned input buffers (same shape, FP32,
         contiguous, same device; None entries keep the plan's buffer) -- saves the device-to-device staging copy.
         `gather`: {pathway: (source clip tensor, device int32 frame index)} -- that pathway's banded stem packs its rows
-        out of the source clip's frames (Plan.stem / esf_stem_pack_gather)."""
+        out of the source clip's frames (Plan.stem_gemm / esf_stem_pack_gather)."""
         self.input_override = {}
         if inputs is not None:
             self.input_override = {own.data_ptr(): src.data_ptr() for own, src in zip(self.inputs, inputs)

@@ -19,12 +19,11 @@ Scope: the two ResNet-50 two-stream models and the single-pathway ResNet (C2D / 
 tensor-core work and ~5x the activation bytes of the FP16 plan: an accuracy mode, benchmarked beside it.
 """
 import ctypes
-import os
 
 import torch
 
 from . import runtime as rt
-from .engine import Plan, bn_affine, fold_conv_bn, host64
+from .engine import Plan, attention_projection, bn_affine, fold_conv_bn, host64, stem_route
 
 
 class Act32:
@@ -79,9 +78,10 @@ def split_weight_rows(w):
 
 
 class PrecisePlan(Plan):
+    wfold = False    # the banded thin-layer GEMM has no FP32 output; every conv is the plain igemm
+
     def __init__(self, device, precision="fp32"):
         super().__init__(device, precision="fp32")
-        self.wfold = False           # the banded thin-layer GEMM has no FP32 output; every conv is the plain igemm
         self.precise = True
 
     # ---------------------------------------------------------------- memory
@@ -150,19 +150,18 @@ class PrecisePlan(Plan):
         self._post(acc, y, self.tensor(inv_scale), self.tensor(bias), res, act)
 
     def stem(self, x_nc, y, w_folded, bias, stride, padding, act=rt.ACT_RELU):
-        """Stem conv + folded BN + ReLU at FP32 accuracy.  Banded tensor-core GEMM (Plan.stem) when the geometry
-        allows: the clip is packed twice (hi and lo halves), the band weight is split like any other weight, and the
-        three products hi.hi, lo.hi, hi.lo are three launches of the same GEMM with FP32 outputs (its tap table cannot
-        hold 3 x kT x kH taps), summed, un-scaled, biased and activated by esf_p32_post3.  Else the FP32 CUDA-core stem."""
-        from .engine import pack_stem_band, pack_stem_tband
-        B, Cin, T, H, W = x_nc.shape
-        cout = w_folded.shape[0]
-        kt, kh, kw = w_folded.shape[2:]
-        geo = rt.stem_geometry(W, Cin, kw, stride[2], padding[2]) if stride[0] == 1 else None
-        if geo is None or not y.f32.is_contiguous():
+        """Stem conv + folded BN + ReLU at FP32 accuracy.  Tensor-core GEMM (the kernel stem_route picks) when the
+        geometry allows: the clip is packed twice (hi and lo halves), the band weight is split like any other weight, and
+        the three products hi.hi, lo.hi, hi.lo are three launches of the same GEMM with FP32 outputs (its tap table
+        cannot hold 3 x kT x kH taps), summed, un-scaled, biased and activated by esf_p32_post3.  Else the FP32
+        CUDA-core stem."""
+        route = stem_route(x_nc.shape, w_folded.shape, stride, padding)
+        if route is None or not y.f32.is_contiguous():
             self.stem_conv(x_nc, y.f32, w_folded, bias, stride, padding, act)
             return self._post(y.f32, y, label="split")
-        pitch, lpad, _ = geo
+        pitch, lpad, twb = route
+        B, Cin, T, H, W = x_nc.shape
+        cout = w_folded.shape[0]
         L = rt.lib()
         hi, lo, inv_scale = split_weight_rows(w_folded.to(torch.float64))
         zero = torch.zeros(cout, dtype=torch.float64)
@@ -175,27 +174,10 @@ class PrecisePlan(Plan):
                                                           xp.data_ptr(), s), "esf_stem_pack"),
                       "stem_pack", "lo" if part else "hi", nbytes=self._nbytes(x_nc, xp), eager=True)
             xps.append(xp)
-        m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
-        # kT > 1: the temporal-band kernel (Plan.stem), one launch per split product as well
-        twb = rt.stem_tband_wb(W, Cin, cout, kt, kh, kw, stride[2], padding[2]) \
-            if os.environ.get("ESF_STEM_TBAND", "1") != "0" else 0
         for name, xp, wpart in (("hi.hi", xps[0], hi), ("lo.hi", xps[1], hi), ("hi.lo", xps[0], lo)):
-            if twb:
-                wb, bt = pack_stem_tband(wpart, zero, twb, stride[2], self.device, torch.float16)
-            else:
-                wb, bt = pack_stem_band(wpart, zero, stride[2], self.device, torch.float16)
-            create = L.esf_stem_tband_create if twb else L.esf_stem_igemm_create
             acc = torch.empty(tuple(y.shape), dtype=torch.float32, device=self.device)
-            self.keep += [wb, bt, acc]
-            yv = rt.view(acc)
-            h = ctypes.c_void_p()
-            rt.check(create(xp.data_ptr(), B, Cin, T, H, W, pitch, wb.data_ptr(), bt.data_ptr(), cout,
-                            kt, kh, kw, stride[1], stride[2], padding[0], padding[1], padding[2],
-                            rt.ACT_NONE, ctypes.byref(yv), ctypes.byref(h)), "stem GEMM create")
-            self.handles.append(h)
-            self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "stem_igemm",
-                      "%dx%dx%d %d->%d %s %s" % (kt, kh, kw, Cin, cout, "t-band" if twb else "banded", name),
-                      flops=2.0 * m * cout * Cin * kt * kh * kw, nbytes=self._nbytes(xp, acc) + wb.numel() * 2)
+            self.keep.append(acc)
+            self._stem_gemm_op(xp, x_nc.shape, acc, wpart, zero, stride, padding, rt.ACT_NONE, pitch, twb, name)
             accs.append(acc)
         sc, bs = self.tensor(inv_scale), self.tensor(bias)
         avs = [rt.view(a) for a in accs]
@@ -236,26 +218,9 @@ class PrecisePlan(Plan):
         """Same composition as Plan.position_attention; the projection GEMM runs on the split operands, the fused
         attention kernel writes FP32 into the concat slice, which is then split into planes."""
         B, T, H, W, C = x_slow.shape
-        wd = host64(w_down).reshape(w_down.shape[0], C)
-        d = wd.shape[0]
+        w_all, b_all, d = attention_projection(w_down, att)
         if d not in (8, 16, 32, 64, 128):
             raise NotImplementedError("head dim %d is not part of the FP32-accurate plan (8, 16, 32, 64, 128)" % d)
-        mats, biases = [wd], [torch.zeros(d, dtype=torch.float64)]
-        for conv in (att.query_conv, att.key_conv, att.value_conv):
-            wc = host64(conv.weight).reshape(conv.weight.shape[0], d)
-            bc = host64(conv.bias)
-            if wc.shape[0] < d:
-                # SpatialAttention(reduction > 1) (wdf_attention_helper.py:17-26): query / key have d / reduction
-                # channels.  Zero rows up to d leave every logit q.k unchanged and keep the kernels' one head dim.
-                # (No cfg key reaches this: every call site of the reference hard-codes reduction = 1.)
-                assert conv is not att.value_conv, "value_conv keeps all channels"
-                pad = d - wc.shape[0]
-                wc = torch.cat([wc, torch.zeros(pad, d, dtype=wc.dtype)], 0)
-                bc = torch.cat([bc, torch.zeros(pad, dtype=bc.dtype)], 0)
-            mats.append(wc @ wd)
-            biases.append(bc)
-        w_all = torch.cat(mats, 0).reshape(4 * d, C, 1, 1, 1)
-        b_all = torch.cat(biases, 0)
         proj = super().act(B, T, H, W, 4 * d, dtype=torch.float32)
         self.conv(x_slow, proj, w_all, b_all)
         L = rt.lib()
@@ -265,7 +230,7 @@ class PrecisePlan(Plan):
         gamma = float(att.gamma.detach().float().item())
         yv = rt.view(y_slice.f32)
         self.keep.append(yv)
-        if d <= 64 and self.attn_impl == "tcgen05":
+        if d <= 64:
             # tensor cores at FP32 accuracy: the logits are hi/lo split already; P and V become FP16 pairs too
             # (esf_attn_tc_create_split: O += P_hi V_hi + P_lo V_hi + P_hi V_lo, row sums in FP32 registers)
             nbytes = int(L.esf_attn_tc_pack_bytes(B, N, d))

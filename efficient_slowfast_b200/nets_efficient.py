@@ -11,7 +11,6 @@ arithmetic is a launch plan of libesf_b200 kernels.  These backbones have channe
 automatically (engine.Plan.conv).
 """
 import math
-import os
 
 import torch
 import torch.nn as nn
@@ -402,13 +401,10 @@ class SlowFastShuffleNet(_EfficientBase):
         init_weights(self, cfg.MODEL.FC_INIT_STD, cfg.RESNET.ZERO_INIT_FINAL_BN)
         self._init_runtime(cfg)
 
-    # fold the channel shuffle behind conv1 into its weight rows (A/B knob: ESF_FOLD_SHUFFLE=0 keeps the shuffle kernel)
-    _fold_shuffle = os.environ.get("ESF_FOLD_SHUFFLE", "1") != "0"
-
     def _emit_unit(self, plan, blk, x, y):
         """Bottleneck.forward (shufflenet_helper.py:75-84)."""
         conv1 = blk.conv1
-        if (blk.groups > 1 and self._fold_shuffle and tuple(conv1.kernel_size) == (1, 1, 1) and x.shape[4] >= 8
+        if (blk.groups > 1 and tuple(conv1.kernel_size) == (1, 1, 1) and x.shape[4] >= 8
                 and conv1.out_channels % blk.groups == 0):
             # channel_shuffle(relu(bn(conv1(x)))) is a permutation of conv1's output channels: fold it into the ORDER of
             # the weight rows.  A permuted grouped conv is no longer grouped, so the layer runs as one dense implicit

@@ -207,18 +207,11 @@ int esf_eca_fuse(const esf_view* x_fast, int32_t alpha, const float* eca_w, int3
  * replaces SpatialAttention.forward (wdf_attention_helper.py:33-54) + bn_s2f + ReLU + nearest upsample +
  * concat (custom_video_model_builder.py:142-146).
  *   proj: FP32 (B*N, 4*d) rows [x_d | q | k | v] produced by the composed 1x1x1 GEMM (out_dtype F32);
- *   esf_attn_pack splits q,k into BF16 hi/lo parts so QK^T keeps ~FP32 logits on BF16 tensor cores;
- *   esf_attn_fused computes softmax_j(q_i.k_j) v_j with an online softmax, then
- *   y[b, alpha*t + r, h, w, 0:d] = relu(bn_scale * (gamma * O + x_d) + bn_shift), r = 0..alpha-1. */
-int64_t esf_attn_pack_bytes(int32_t B, int32_t N, int32_t d);
-int esf_attn_pack(const float* proj, int32_t B, int32_t N, int32_t d, void* packed, void* stream);
-int esf_attn_fused(const void* packed, int32_t B, int32_t T, int32_t H, int32_t W, int32_t d, float gamma,
-                   const float* bn_scale, const float* bn_shift, int32_t alpha, const esf_view* y_fast_slice,
-                   void* stream);
-
-/* ---- the same attention on the tcgen05 tensor cores (TMEM accumulators, two-pass softmax) -------------------
- * Preferred path; any head dim d <= 128.  esf_attn_tc_pack writes Q~/K~ (BF16 hi/lo split rows), V^T and x_d into
- * `packed` (esf_attn_tc_pack_bytes bytes); esf_attn_tc_create plans the fused kernel (launch: esf_op_launch). */
+ *   y[b, alpha*t + r, h, w, 0:d] = relu(bn_scale * (gamma * O + x_d) + bn_shift), r = 0..alpha-1, where
+ *   O = softmax_j(q_i.k_j) v_j runs on the tcgen05 tensor cores (TMEM accumulators, two-pass softmax), any head dim
+ *   d <= 128.  esf_attn_tc_pack writes Q~/K~ (hi/lo split rows, so QK^T keeps ~FP32 logits on 16-bit tensor cores),
+ *   V^T and x_d into `packed` (esf_attn_tc_pack_bytes bytes); esf_attn_tc_create plans the fused kernel (launch:
+ *   esf_op_launch). */
 int64_t esf_attn_tc_pack_bytes(int32_t B, int32_t N, int32_t d);
 int esf_attn_tc_pack(const float* proj, int32_t B, int32_t N, int32_t d, int32_t dtype, void* packed, void* stream);
 int esf_attn_tc_create(const void* packed, int32_t B, int32_t T, int32_t H, int32_t W, int32_t d, float gamma,

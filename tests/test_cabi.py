@@ -34,13 +34,14 @@ def test_geometry_rule(esf_lib):
     assert rt.igemm_geometry(1152, 2048) == (64, 18, 256, 2048)
 
 
-def test_bad_arguments_give_error_codes(esf_lib):
+def test_bad_sizes_and_null_descriptors_give_error_codes(esf_lib):
     from efficient_slowfast_b200 import runtime as rt
 
     assert esf_lib.esf_igemm_geometry(0, 4, None, None, None, None) < 0
     assert b"positive" in esf_lib.esf_last_error()
-    assert esf_lib.esf_attn_pack_bytes(2, 100, 7) < 0      # head dim must be a multiple of 8 (R50 models)
-    assert esf_lib.esf_attn_pack_bytes(2, 100, 8) > 0
+    assert esf_lib.esf_attn_tc_pack_bytes(2, 100, 0) < 0
+    assert esf_lib.esf_attn_tc_pack_bytes(2, 100, 129) < 0    # d > 128 is the CUDA-core fallback's (esf_attn_generic)
+    assert esf_lib.esf_attn_tc_pack_bytes(2, 100, 8) > 0
     h = ctypes.c_void_p()
     assert esf_lib.esf_conv_igemm_create(None, ctypes.byref(h)) < 0
 
@@ -105,5 +106,19 @@ def test_library_reads_no_environment():
         if f.endswith((".cu", ".cuh", ".h", ".cpp")):
             for i, line in enumerate(open(os.path.join(csrc, f)), 1):
                 if re.search(r"\bgetenv\s*\(", line):
+                    hits.append("%s:%d: %s" % (f, i, line.strip()))
+    assert not hits, hits
+
+
+def test_package_reads_no_environment():
+    """The same rule one layer up: the plan builder picks kernels from shapes and parameters only.  The two exceptions
+    read no switch: _build.py takes the compiler and its extra flags (NVCC, ESF_NVCC_EXTRA; the flags are part of the
+    library's digest), workloads.py the directory test fixtures are read from (ESF_GOLDEN_DIR)."""
+    pkg = os.path.join(ROOT, "efficient_slowfast_b200")
+    hits = []
+    for f in sorted(os.listdir(pkg)):
+        if f.endswith(".py") and f not in ("_build.py", "workloads.py"):
+            for i, line in enumerate(open(os.path.join(pkg, f)), 1):
+                if re.search(r"\b(environ|getenv)\b", line):
                     hits.append("%s:%d: %s" % (f, i, line.strip()))
     assert not hits, hits

@@ -7,7 +7,7 @@ import torch
 import torch.nn.functional as F
 
 from efficient_slowfast_b200 import runtime as rt
-from efficient_slowfast_b200.engine import Plan
+from efficient_slowfast_b200.engine import Plan, stem_route
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -365,9 +365,9 @@ def test_stem_conv(esf_lib, kt, cout):
 
 @pytest.mark.parametrize("precision", ["bf16", "fp16"])
 @pytest.mark.parametrize("kt,cout,k,size", [(1, 64, 7, 64), (5, 8, 7, 64), (3, 24, 3, 48), (1, 64, 7, 224)])
-def test_stem_banded_gemm(esf_lib, kt, cout, k, size, precision, monkeypatch):
-    """Tensor-core stem (banded implicit GEMM) vs F.conv3d on the 16-bit-rounded clip and weights."""
-    monkeypatch.setenv("ESF_STEM_TBAND", "0")     # the temporal-band kernel has its own test below
+def test_stem_banded_gemm(esf_lib, kt, cout, k, size, precision):
+    """Tensor-core stem (banded implicit GEMM; the temporal-band kernel has its own test below) vs F.conv3d on the
+    16-bit-rounded clip and weights."""
     adt = rt.TORCH_DTYPE[precision]
     g = torch.Generator().manual_seed(kt + cout)
     B, T = (2, 8) if size < 200 else (1, 2)
@@ -380,8 +380,9 @@ def test_stem_banded_gemm(esf_lib, kt, cout, k, size, precision, monkeypatch):
     y = torch.full(_to_ndhwc(ref).shape, 7.0, dtype=adt, device=DEV)
     plan = Plan(DEV, precision)
     xd = x.to(DEV)
-    plan.stem(xd, y, w.double(), bias.double(), (1, 2, 2), pad)
-    assert plan.meta[-1]["kind"] == "stem_igemm"
+    pitch, lpad, _ = stem_route(xd.shape, w.shape, (1, 2, 2), pad)
+    plan.stem_gemm(xd, y, w.double(), bias.double(), (1, 2, 2), pad, rt.ACT_RELU, pitch, lpad, 0)
+    assert plan.meta[-1]["kind"] == "stem_igemm" and plan.meta[-1]["label"].endswith("banded")
     plan.launch_all()
     torch.cuda.synchronize()
     got = _to_ncdhw(y.cpu())
@@ -402,11 +403,10 @@ def test_stem_banded_gemm(esf_lib, kt, cout, k, size, precision, monkeypatch):
     (2, 3, 5, 64, 5, 4),       # 16-column slots (32 slots)
     (8, 3, 4, 224, 5, 8),      # 196 tiles on 148 SMs: slots and stages carried from one tile into the next
 ])
-def test_stem_temporal_band(esf_lib, B, cin, T, size, kt, cout, precision, monkeypatch):
+def test_stem_temporal_band(esf_lib, B, cin, T, size, kt, cout, precision):
     """stem_tband_kernel (time taps folded into N, input frames streaming past a resident M tile, output frames in a ring
     of TMEM slots) vs F.conv3d on the 16-bit-rounded clip and weights, and bit-identical to nothing less than itself on a
     second launch (the barriers' phases must survive re-launching the same op)."""
-    monkeypatch.setenv("ESF_STEM_TBAND", "1")
     adt = rt.TORCH_DTYPE[precision]
     g = torch.Generator().manual_seed(B + T + cout)
     x = torch.randn(B, cin, T, size, size, generator=g)
@@ -435,11 +435,10 @@ def test_stem_temporal_band(esf_lib, B, cin, T, size, kt, cout, precision, monke
     assert torch.equal(_to_ncdhw(y.cpu()), got)
 
 
-def test_stem_temporal_band_random_geometries(esf_lib, monkeypatch):
+def test_stem_temporal_band_random_geometries(esf_lib):
     """Seeded sweep over clip sizes the fixed cases do not hit: odd frame counts around the slot ring (15 .. 18, 33),
     batches that do not fill the 8-clip box, heights that leave a ragged last row tile, padded / unpadded time."""
     import random
-    monkeypatch.setenv("ESF_STEM_TBAND", "1")
     rnd = random.Random(7)
     done = 0
     for _ in range(40):
@@ -468,19 +467,21 @@ def test_stem_temporal_band_random_geometries(esf_lib, monkeypatch):
     assert done >= 10
 
 
-def test_stem_temporal_band_matches_banded_stem(esf_lib, monkeypatch):
+def test_stem_temporal_band_matches_banded_stem(esf_lib):
     """Both tensor-core stems accumulate the same FP16 products in FP32: their outputs may differ only by the order of
     the additions (one 16-bit ulp at most after rounding)."""
     g = torch.Generator().manual_seed(5)
     x = torch.randn(2, 3, 8, 64, 64, generator=g)
     w = torch.randn(8, 3, 5, 7, 7, generator=g) * 0.1
     bias = torch.randn(8, generator=g) * 0.1
+    pitch, lpad, twb = stem_route(x.shape, w.shape, (1, 2, 2), (2, 3, 3))
+    assert twb > 0
     outs = []
-    for tband in ("1", "0"):
-        monkeypatch.setenv("ESF_STEM_TBAND", tband)
+    for wb, label in ((twb, "t-band"), (0, "banded")):
         y = torch.empty(2, 8, 32, 32, 8, dtype=torch.float16, device=DEV)
         plan = Plan(DEV, "fp16")
-        plan.stem(x.to(DEV), y, w.double(), bias.double(), (1, 2, 2), (2, 3, 3))
+        plan.stem_gemm(x.to(DEV), y, w.double(), bias.double(), (1, 2, 2), (2, 3, 3), rt.ACT_RELU, pitch, lpad, wb)
+        assert plan.meta[-1]["label"].endswith(label)
         plan.launch_all()
         torch.cuda.synchronize()
         outs.append(y.float().cpu())
@@ -607,43 +608,11 @@ def _attention_reference(proj, B, T, H, W, d, gamma, scale, shift, alpha):
     return o.repeat_interleave(alpha, dim=1)
 
 
-@pytest.mark.parametrize("d,T,H,W,qk_scale", [(8, 2, 9, 8, 1.0), (8, 2, 9, 8, 4.0), (32, 2, 12, 11, 1.0),
-                                              (32, 4, 8, 8, 2.0), (64, 2, 7, 7, 1.0), (128, 2, 7, 7, 0.5),
-                                              (16, 1, 9, 9, 1.0)])
-def test_attention_fused(esf_lib, d, T, H, W, qk_scale):
-    g = torch.Generator().manual_seed(d + T)
-    B, alpha = 2, 4
-    N = T * H * W
-    proj = torch.randn(B * N, 4 * d, generator=g)
-    proj[:, d:3 * d] *= qk_scale / d ** 0.25      # logits ~ N(0, qk_scale^2 ...) up to |s| ~ 4*qk_scale^2
-    gamma = 0.7
-    scale = torch.rand(d, generator=g) + 0.5
-    shift = torch.rand(d, generator=g) - 0.5
-    ref = _attention_reference(proj, B, T, H, W, d, gamma, scale, shift, alpha)
-    L = esf_lib
-    nbytes = L.esf_attn_pack_bytes(B, N, d)
-    assert nbytes > 0
-    packed = torch.empty(nbytes, dtype=torch.uint8, device=DEV)
-    pj = proj.to(DEV)
-    ybuf = torch.zeros(B, T * alpha, H, W, 2 * d, dtype=torch.bfloat16, device=DEV)
-    yv = rt.view(ybuf[..., :d])
-    sc, sh = scale.to(DEV), shift.to(DEV)
-    s = rt.current_stream_ptr()
-    rt.check(L.esf_attn_pack(pj.data_ptr(), B, N, d, packed.data_ptr(), s))
-    rt.check(L.esf_attn_fused(packed.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                              ctypes.byref(yv), s))
-    torch.cuda.synchronize()
-    got = ybuf[..., :d].cpu().double()
-    err = (got - ref).abs().max().item()
-    # BF16 P and V (2^-9 each) + BF16 output rounding; logits themselves are ~FP32 thanks to the hi/lo split
-    assert err <= 1.5e-2 * ref.abs().max().item(), "d=%d err %.4g scale %.4g" % (d, err, ref.abs().max().item())
-    assert (ybuf[..., d:] == 0).all()
-
-
-@pytest.mark.parametrize("d,T,H,W,qk_scale", [(8, 2, 9, 8, 1.0), (8, 2, 16, 16, 4.0), (32, 2, 12, 11, 1.0),
-                                              (32, 4, 16, 8, 2.0), (64, 2, 7, 7, 1.0), (128, 2, 7, 7, 0.5),
-                                              (16, 1, 9, 9, 1.0), (3, 2, 8, 8, 1.0), (12, 1, 20, 20, 1.0),
-                                              (24, 2, 14, 14, 1.0), (32, 8, 14, 14, 1.0)])
+@pytest.mark.parametrize("d,T,H,W,qk_scale", [(8, 2, 9, 8, 1.0), (8, 2, 9, 8, 4.0), (8, 2, 16, 16, 4.0),
+                                              (32, 2, 12, 11, 1.0), (32, 4, 8, 8, 2.0), (32, 4, 16, 8, 2.0),
+                                              (64, 2, 7, 7, 1.0), (128, 2, 7, 7, 0.5), (16, 1, 9, 9, 1.0),
+                                              (3, 2, 8, 8, 1.0), (12, 1, 20, 20, 1.0), (24, 2, 14, 14, 1.0),
+                                              (32, 8, 14, 14, 1.0)])
 @pytest.mark.parametrize("precision", ["bf16", "fp16"])
 def test_attention_tcgen05(esf_lib, d, T, H, W, qk_scale, precision):
     """tcgen05/TMEM fused attention vs FP64 softmax attention on the same FP32 projections."""

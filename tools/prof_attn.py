@@ -1,4 +1,4 @@
-"""Launch the fused attention kernels alone (for ncu): python tools/prof_attn.py [d] [T] [HW] [B] [impl]"""
+"""Launch the fused attention kernel alone (for ncu): python tools/prof_attn.py [d] [T] [HW] [B] [reps]"""
 import ctypes
 import os
 import sys
@@ -13,8 +13,7 @@ d = int(sys.argv[1]) if len(sys.argv) > 1 else 32
 T = int(sys.argv[2]) if len(sys.argv) > 2 else 8
 HW = int(sys.argv[3]) if len(sys.argv) > 3 else 56
 B = int(sys.argv[4]) if len(sys.argv) > 4 else 2
-impl = sys.argv[5] if len(sys.argv) > 5 else "tc"
-reps = int(sys.argv[6]) if len(sys.argv) > 6 else 3
+reps = int(sys.argv[5]) if len(sys.argv) > 5 else 3
 DEV = "cuda:0"
 L = rt.lib()
 N = T * HW * HW
@@ -27,18 +26,12 @@ yv = rt.view(ybuf[..., :d])
 sc = torch.ones(d, device=DEV)
 sh = torch.zeros(d, device=DEV)
 s = rt.current_stream_ptr()
-if impl == "tc":
-    packed = torch.empty(L.esf_attn_tc_pack_bytes(B, N, d), dtype=torch.uint8, device=DEV)
-    rt.check(L.esf_attn_tc_pack(proj.data_ptr(), B, N, d, rt.F16, packed.data_ptr(), s))
-    h = ctypes.c_void_p()
-    rt.check(L.esf_attn_tc_create(packed.data_ptr(), B, T, HW, HW, d, 0.5, sc.data_ptr(), sh.data_ptr(), alpha,
-                                  ctypes.byref(yv), ctypes.byref(h)))
-    launch = lambda: rt.check(L.esf_op_launch(h, s))
-else:
-    packed = torch.empty(L.esf_attn_pack_bytes(B, N, d), dtype=torch.uint8, device=DEV)
-    rt.check(L.esf_attn_pack(proj.data_ptr(), B, N, d, packed.data_ptr(), s))
-    launch = lambda: rt.check(L.esf_attn_fused(packed.data_ptr(), B, T, HW, HW, d, 0.5, sc.data_ptr(), sh.data_ptr(),
-                                               alpha, ctypes.byref(yv), s))
+packed = torch.empty(L.esf_attn_tc_pack_bytes(B, N, d), dtype=torch.uint8, device=DEV)
+rt.check(L.esf_attn_tc_pack(proj.data_ptr(), B, N, d, rt.F16, packed.data_ptr(), s))
+h = ctypes.c_void_p()
+rt.check(L.esf_attn_tc_create(packed.data_ptr(), B, T, HW, HW, d, 0.5, sc.data_ptr(), sh.data_ptr(), alpha,
+                              ctypes.byref(yv), ctypes.byref(h)))
+launch = lambda: rt.check(L.esf_op_launch(h, s))
 launch()
 torch.cuda.synchronize()
 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -48,5 +41,5 @@ for _ in range(reps):
 e1.record()
 torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / reps
-print("attn %s d=%d N=%d B=%d: %.3f ms  %.2f Texp/s  %.1f TFLOP/s" % (impl, d, N, B, ms, B * N * N / ms / 1e9,
+print("attn tc d=%d N=%d B=%d: %.3f ms  %.2f Texp/s  %.1f TFLOP/s" % (d, N, B, ms, B * N * N / ms / 1e9,
                                                                      4.0 * B * N * N * d / ms / 1e9))

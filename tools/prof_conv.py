@@ -1,5 +1,6 @@
 """Launch one conv layer alone (for ncu / timing):
-python tools/prof_conv.py B T H W Cin Cout kT kH kW sT sH sW res(0|1) [reps] [precision] [wfold(0|1)]"""
+python tools/prof_conv.py B T H W Cin Cout kT kH kW sT sH sW res(0|1) [reps] [precision] [wfold(0|1)]
+wfold=0 runs the dense layer on the plain implicit GEMM where Plan.conv would pick the W-folded one."""
 import os
 import sys
 
@@ -27,9 +28,11 @@ x.copy_(torch.randn(B, T, H, W, cin, generator=g).to(DEV, adt))
 y = plan.act(B, To, Ho, Wo, cout)
 res = torch.randn(B, To, Ho, Wo, cout, generator=g).to(DEV, adt) if use_res else None
 w = torch.randn(cout, cin // groups, kt, kh, kw, generator=g).double() * (2.0 * groups / (cin * kt * kh * kw)) ** 0.5
-plan.wfold = bool(wfold)
-plan.conv(x, y, w, torch.zeros(cout, dtype=torch.float64), stride=(st, sh, sw), padding=pad, groups=groups, act=rt.ACT_RELU,
-          res=res)
+zero = torch.zeros(cout, dtype=torch.float64)
+if wfold:
+    plan.conv(x, y, w, zero, stride=(st, sh, sw), padding=pad, groups=groups, act=rt.ACT_RELU, res=res)
+else:
+    plan.conv_igemm(x, y, w, zero, stride=(st, sh, sw), padding=pad, act=rt.ACT_RELU, res=res)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device=DEV)
 plan.launch_all()
 torch.cuda.synchronize()

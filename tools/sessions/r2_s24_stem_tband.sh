@@ -10,7 +10,7 @@ if [ "${TESTS:-1}" = 1 ]; then
   timeout 600 python -m pytest tests/test_gpu_kernels.py -x -q -m gpu -k "stem" > $O/pytest.log 2>&1; echo "pytest rc $?"; tail -3 $O/pytest.log
 fi
 {
-  ESF_STEM_TBAND=0 python tools/prof_stem.py 64 20
+  python tools/prof_stem.py 64 20 1
   python tools/prof_stem.py 64 20
 } | tee $O/stem_ab.txt
 if [ "${BENCH:-0}" = 1 ]; then

@@ -7,5 +7,5 @@ mkdir -p $O
 export ESF_NVCC_EXTRA=-DESF_ATTN_TIMING
 python -c "import __graft_entry__ as g; g.build()" > $O/build.log 2>&1 || { tail -5 $O/build.log; exit 1; }
 for d in 8 32; do
-  echo "== d = $d"; python tools/prof_attn.py $d 8 56 4 tc 1 2>&1 | grep -E "^warp|attn tc" | sort | head -20
+  echo "== d = $d"; python tools/prof_attn.py $d 8 56 4 1 2>&1 | grep -E "^warp|attn tc" | sort | head -20
 done | tee $O/timing.txt
