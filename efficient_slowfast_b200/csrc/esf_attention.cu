@@ -3,8 +3,9 @@
 // store into the fast pathway's concat slice.
 //
 // Any head dim, FP32 math straight from the projection rows [x_d | q | k | v]: one warp per query, logits staged in
-// shared memory.  Used only where the tcgen05 kernel (csrc/esf_attn_tc.cu) does not apply: d > 128, which in the
-// reference's models only occurs with N <= 392 keys (SlowFastShuffleNet s4_fuse, d = 240).
+// shared memory.  Used only where the tcgen05 kernel (csrc/esf_attn_tc.cu) and the FP32 flash kernel
+// (csrc/esf_precise.cu) do not apply: d > 128, which in the reference's models only occurs with N <= 392 keys
+// (SlowFastShuffleNet s4_fuse, d = 240).  The output is 16-bit, or FP32 for the FP32-accurate plan.
 #include <math_constants.h>
 
 #include "esf_common.cuh"
@@ -15,7 +16,7 @@ namespace esf {
 __global__ void __launch_bounds__(128) attn_generic_kernel(const float* __restrict__ proj, int N, int T, int H, int W,
                                                            int d, float gamma, const float* __restrict__ bn_scale,
                                                            const float* __restrict__ bn_shift, int alpha, int f16,
-                                                           __nv_bfloat16* __restrict__ y, long long ysB, long long ysT,
+                                                           int out_f32, void* __restrict__ y, long long ysB, long long ysT,
                                                            long long ysH, long long ysW) {
   extern __shared__ float srow[];  // [4 warps][N]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -44,8 +45,12 @@ __global__ void __launch_bounds__(128) attn_generic_kernel(const float* __restri
     float o = 0.f;
     for (int j = 0; j < N; ++j) o = fmaf(expf(s[j] - m), base[(long long)j * 4 * d + 3 * d + c], o);
     const float a = fmaf(gamma, o / l, base[(long long)i * 4 * d + c]);
-    const __nv_bfloat16 v = f2h16(fmaxf(fmaf(a, bn_scale[c], bn_shift[c]), 0.f), f16);
-    for (int r = 0; r < alpha; ++r) y[b * ysB + (long long)(t * alpha + r) * ysT + hh * ysH + ww * ysW + c] = v;
+    const float v = fmaxf(fmaf(a, bn_scale[c], bn_shift[c]), 0.f);
+    for (int r = 0; r < alpha; ++r) {
+      const long long at = b * ysB + (long long)(t * alpha + r) * ysT + hh * ysH + ww * ysW + c;
+      if (out_f32) static_cast<float*>(y)[at] = v;
+      else static_cast<__nv_bfloat16*>(y)[at] = f2h16(v, f16);
+    }
   }
 }
 
@@ -70,7 +75,7 @@ extern "C" int esf_attn_generic(const float* proj, int32_t B, int32_t T, int32_t
     if (slot) *slot = 1;
   }
   attn_generic_kernel<<<dim3(cdiv(N, 4), B), 128, smem, static_cast<cudaStream_t>(stream)>>>(
-      proj, N, T, H, W, d, gamma, bn_scale, bn_shift, alpha, y->dtype == ESF_F16, static_cast<__nv_bfloat16*>(y->ptr),
-      y->sB, y->sT, y->sH, y->sW);
+      proj, N, T, H, W, d, gamma, bn_scale, bn_shift, alpha, y->dtype == ESF_F16, y->dtype == ESF_F32, y->ptr, y->sB,
+      y->sT, y->sH, y->sW);
   return check_launch("attn_generic_kernel");
 }

@@ -310,9 +310,10 @@ __global__ void __launch_bounds__(256) p32_head_pool_kernel(const V32 x, float* 
 // [x_d | q | k | v] (D FP32 each).  A block owns 128 / G query rows, G = D / DT threads per row (DT = min(D, 32) channels
 // of q and O per thread); key tiles of 32 rows of K and V go through shared memory, every thread computes the 32 logits
 // of its row (partial dot over its channels, summed across the G lanes), one online-softmax update per tile, then
-// O += P V on its channels.  The N x N matrix is never formed.
+// O += P V on its channels.  The N x N matrix is never formed.  The head dim d may be below D (the smallest of 8, 16,
+// 32, 64, 128 that holds it): channels [d, D) are zeros in registers and shared memory and are not stored.
 template <int D>
-__global__ void __launch_bounds__(128) p32_attn_kernel(const float* __restrict__ proj, int N, int T, int H, int W,
+__global__ void __launch_bounds__(128) p32_attn_kernel(const float* __restrict__ proj, int d, int N, int T, int H, int W,
                                                        float gamma, const float* __restrict__ bn_scale,
                                                        const float* __restrict__ bn_shift, int alpha,
                                                        float* __restrict__ y, long long ysB, long long ysT, long long ysH,
@@ -328,26 +329,34 @@ __global__ void __launch_bounds__(128) p32_attn_kernel(const float* __restrict__
   const int g = threadIdx.x % G;
   const int row = blockIdx.x * R + threadIdx.x / G;
   const bool valid = row < N;
-  const float* base = proj + (long long)b * N * 4 * D;
+  const float* base = proj + (long long)b * N * 4 * d;
   float q[DT], o[DT];
   {
-    const float* qr = base + (long long)(valid ? row : 0) * 4 * D + D + g * DT;
+    const float* qr = base + (long long)(valid ? row : 0) * 4 * d + d + g * DT;
 #pragma unroll
-    for (int c = 0; c < DT; ++c) q[c] = valid ? qr[c] : 0.f, o[c] = 0.f;
+    for (int c = 0; c < DT; ++c) q[c] = (valid && g * DT + c < d) ? qr[c] : 0.f, o[c] = 0.f;
   }
   float m = -CUDART_INF_F, l = 0.f;
   const float kLog2e = 1.4426950408889634f;
   for (int j0 = 0; j0 < N; j0 += KT) {
     __syncthreads();
-    // cooperative tile load: KT rows x D floats of K and of V (float4, coalesced within a row)
+    // cooperative tile load: KT rows x D floats of K and of V (float4 when d % 4 == 0, coalesced within a row)
     for (int i = threadIdx.x; i < KT * (D / 4); i += 128) {
       const int j = i / (D / 4), c4 = i % (D / 4);
       const int c = c4 * 4, sub = c / DT, cc = c % DT;
       float4 kv = make_float4(0.f, 0.f, 0.f, 0.f), vv = kv;
-      if (j0 + j < N) {
-        const float* r = base + (long long)(j0 + j) * 4 * D;
-        kv = *reinterpret_cast<const float4*>(r + 2 * D + c);
-        vv = *reinterpret_cast<const float4*>(r + 3 * D + c);
+      if (j0 + j < N && c < d) {
+        const float* r = base + (long long)(j0 + j) * 4 * d;
+        if (d % 4 == 0) {
+          kv = *reinterpret_cast<const float4*>(r + 2 * d + c);
+          vv = *reinterpret_cast<const float4*>(r + 3 * d + c);
+        } else {
+          float kk[4], vk[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e) kk[e] = c + e < d ? r[2 * d + c + e] : 0.f, vk[e] = c + e < d ? r[3 * d + c + e] : 0.f;
+          kv = make_float4(kk[0], kk[1], kk[2], kk[3]);
+          vv = make_float4(vk[0], vk[1], vk[2], vk[3]);
+        }
       }
       *reinterpret_cast<float4*>(&Ks[j * PITCH + sub * (DT + 4) + cc]) = kv;
       *reinterpret_cast<float4*>(&Vs[j * PITCH + sub * (DT + 4) + cc]) = vv;
@@ -399,18 +408,21 @@ __global__ void __launch_bounds__(128) p32_attn_kernel(const float* __restrict__
   const float inv = 1.f / l;
   const int HW = H * W;
   const int t = row / HW, hw = row % HW, hh = hw / W, ww = hw % W;
-  const float* xr = base + (long long)row * 4 * D + g * DT;
+  const float* xr = base + (long long)row * 4 * d + g * DT;
   float* yb = y + b * ysB + hh * ysH + ww * ysW + g * DT;
 #pragma unroll
   for (int c = 0; c < DT; ++c) {
     const int ch = g * DT + c;
-    const float a = fmaf(gamma, o[c] * inv, xr[c]);
-    o[c] = fmaxf(fmaf(a, __ldg(bn_scale + ch), __ldg(bn_shift + ch)), 0.f);
+    if (ch < d) {
+      const float a = fmaf(gamma, o[c] * inv, xr[c]);
+      o[c] = fmaxf(fmaf(a, __ldg(bn_scale + ch), __ldg(bn_shift + ch)), 0.f);
+    }
   }
   for (int r = 0; r < alpha; ++r) {
     float* yp = yb + (long long)(t * alpha + r) * ysT;
 #pragma unroll
-    for (int c = 0; c < DT; ++c) yp[c] = o[c];
+    for (int c = 0; c < DT; ++c)
+      if (g * DT + c < d) yp[c] = o[c];
   }
 }
 
@@ -587,15 +599,13 @@ extern "C" int esf_p32_attention(const float* proj, int32_t B, int32_t T, int32_
   float* yp = static_cast<float*>(y->ptr);
 #define ESF_P32_ATTN(DD)                                                                                              \
   p32_attn_kernel<DD><<<dim3(cdiv(N, 128 / (DD / (DD < 32 ? DD : 32))), B), 128, 0, s>>>(                             \
-      proj, N, T, H, W, gamma, bn_scale, bn_shift, alpha, yp, y->sB, y->sT, y->sH, y->sW)
-  switch (d) {
-    case 8: ESF_P32_ATTN(8); break;
-    case 16: ESF_P32_ATTN(16); break;
-    case 32: ESF_P32_ATTN(32); break;
-    case 64: ESF_P32_ATTN(64); break;
-    case 128: ESF_P32_ATTN(128); break;
-    default: return set_error(ESF_ERR_UNSUPPORTED, "esf_p32_attention: head dim %d (8, 16, 32, 64 or 128)", d);
-  }
+      proj, d, N, T, H, W, gamma, bn_scale, bn_shift, alpha, yp, y->sB, y->sT, y->sH, y->sW)
+  if (d <= 0 || d > 128) return set_error(ESF_ERR_UNSUPPORTED, "esf_p32_attention: head dim %d (1 ... 128)", d);
+  if (d <= 8) ESF_P32_ATTN(8);
+  else if (d <= 16) ESF_P32_ATTN(16);
+  else if (d <= 32) ESF_P32_ATTN(32);
+  else if (d <= 64) ESF_P32_ATTN(64);
+  else ESF_P32_ATTN(128);
 #undef ESF_P32_ATTN
   return check_launch("p32_attn_kernel");
 }

@@ -185,6 +185,26 @@ def attention_projection(w_down, att):
     return torch.cat(mats, 0).reshape(4 * d, C, 1, 1, 1), torch.cat(biases, 0), d
 
 
+def block_diagonal(w, groups):
+    """Grouped (Cout, Cin/groups, kT, kH, kW) weight -> the dense (Cout, Cin, kT, kH, kW) weight of the same convolution:
+    group g's block at output rows g*Cout/groups and input channels g*Cin/groups, zeros elsewhere."""
+    cout, cin_g = w.shape[:2]
+    cout_g = cout // groups
+    wd = torch.zeros((cout, cin_g * groups) + tuple(w.shape[2:]), dtype=w.dtype, device=w.device)
+    for g in range(groups):
+        wd[g * cout_g:(g + 1) * cout_g, g * cin_g:(g + 1) * cin_g] = w[g * cout_g:(g + 1) * cout_g]
+    return wd
+
+
+def fold_time_groups(t, group):
+    """(B, T, H, W, C) view -> (B * group, T / group, H, W, C): the temporal group folding of ResStage.forward
+    (resnet_helper.py:541-560) for the Non-local blocks, a pure view in channels-last memory."""
+    B, T, H, W, C = t.shape
+    assert T % group == 0 and t.stride(0) == T * t.stride(1)
+    return t.as_strided((B * group, T // group, H, W, C),
+                        (t.stride(1) * (T // group), t.stride(1), t.stride(2), t.stride(3), 1), t.storage_offset())
+
+
 def head_fc_launches(B, cin, K, act):
     """Kernel launches of one esf_head_fc call: the tiled kernel (B >= 8, or rows too long for one block) applies the
     class softmax in a second, tiny kernel."""
@@ -329,14 +349,8 @@ class Plan:
         esf_row_softmax (softmax with d^-0.5, or the 1/N_keys of "dot_product") into the 16-bit A operand of the
         second product."""
         L = rt.lib()
-        if group > 1:   # (b, t) -> (b * group, t / group): a pure view in channels-last memory
-            def fold(t):
-                B, T, H, W, C = t.shape
-                assert T % group == 0 and t.stride(0) == T * t.stride(1)
-                return t.as_strided((B * group, T // group, H, W, C),
-                                    (t.stride(1) * (T // group), t.stride(1), t.stride(2), t.stride(3), 1),
-                                    t.storage_offset())
-            x, y = fold(x), fold(y)
+        if group > 1:
+            x, y = fold_time_groups(x, group), fold_time_groups(y, group)
         B, T, H, W, C = x.shape
         d = nln.dim_inner
         f64 = torch.float64
@@ -494,12 +508,8 @@ class Plan:
             # grouped conv whose group slices are not 16-byte addressable (ShuffleNet g3: 180 / 18 / 5 channels per
             # group): one dense GEMM over all input channels with a block-diagonal weight.  The layer is HBM bound, the
             # `groups`-fold MACs on structural zeros cost nothing next to the CUDA-core fallback.
-            cout_g = cout // groups
-            wd = torch.zeros((cout, cin_g * groups) + tuple(w_folded.shape[2:]), dtype=w_folded.dtype,
-                             device=w_folded.device)
-            for g in range(groups):
-                wd[g * cout_g:(g + 1) * cout_g, g * cin_g:(g + 1) * cin_g] = w_folded[g * cout_g:(g + 1) * cout_g]
-            return self.conv_igemm(x, y, wd, bias, stride, padding, dilation, act, res, out_dtype)
+            return self.conv_igemm(x, y, block_diagonal(w_folded, groups), bias, stride, padding, dilation, act, res,
+                                   out_dtype)
         self.conv_direct(x, y, w_folded, bias, stride, padding, dilation, groups, act, res, out_dtype)
         why = [n for n, t in (("x", x), ("y", y), ("res", res)) if not self._aligned(t)]
         self.meta[-1]["why_direct"] = ("groups=%d " % groups if groups != 1 else "") + \
@@ -772,6 +782,12 @@ class Plan:
             y = self.act(B, T - kt + 1, H - kh + 1, W - kw + 1, C)
             self.pool(x, y, (kt, kh, kw), (1, 1, 1), (0, 0, 0), is_avg=True)
             pooled.append(y)
+        return self.positions_head(pooled, weight, bias, act)
+
+    def positions_head(self, pooled, weight, bias, act):
+        """Second half of head_positions: Linear + activation at every position of the pooled maps (B, T', H', W', C)
+        of all pathways, then the mean over the positions."""
+        B = pooled[0].shape[0]
         pos = tuple(pooled[0].shape[1:4])
         assert all(tuple(y.shape[1:4]) == pos for y in pooled), "pathway dimensions are not consistent."
         P = pos[0] * pos[1] * pos[2]

@@ -15,15 +15,18 @@ Concat stays free: a producer writes its channel slice of the FP32 buffer and of
 runs in FP32 on the CUDA cores (esf_p32_attention, flash style): the tcgen05 attention kernel rounds P and V to FP16,
 which alone costs 5e-4 on the probabilities (measured).
 
-Scope: the two ResNet-50 two-stream models and the single-pathway ResNet (C2D / I3D / Slow), Non-local blocks included.  About 3x the
-tensor-core work and ~5x the activation bytes of the FP16 plan: an accuracy mode, benchmarked beside it.
+Scope: every classification model of nets_resnet.py -- the two-stream models and the single-pathway ResNet (C2D / I3D /
+Slow), grouped bottlenecks, Non-local blocks (also with temporal groups), any attention head dim and the
+fully-convolutional test head.  Depthwise convolutions (the efficient backbones) and the detection head are not covered.
+About 3x the tensor-core work and ~5x the activation bytes of the FP16 plan: an accuracy mode, benchmarked beside it.
 """
 import ctypes
 
 import torch
 
 from . import runtime as rt
-from .engine import Plan, attention_projection, bn_affine, fold_conv_bn, host64, stem_route
+from .engine import (Plan, attention_projection, block_diagonal, bn_affine, fold_conv_bn, fold_time_groups, host64,
+                     stem_route)
 
 
 class Act32:
@@ -127,11 +130,18 @@ class PrecisePlan(Plan):
     def conv(self, x, y, w_folded, bias, stride=(1, 1, 1), padding=(0, 0, 0), dilation=(1, 1, 1), groups=1,
              act=rt.ACT_NONE, res=None, out_dtype=None):
         """Conv3d + folded BN (+ residual) + activation at ~FP32 accuracy: igemm over the [hi|lo|hi] planes with the
-        [w_hi|w_hi|w_lo] weight (raw FP32 accumulators), then the FP32 post-pass."""
-        if groups != 1:
-            raise NotImplementedError("grouped convolutions are not part of the FP32-accurate plan (R50 models only)")
+        [w_hi|w_hi|w_lo] weight (raw FP32 accumulators), then the FP32 post-pass.
+
+        groups > 1 (RESNET.NUM_GROUPS, resnet_helper.py:196-205) runs as ONE dense split GEMM over a block-diagonal
+        weight: `groups` times the MACs of the layer, spent on structural zeros, for a single launch on the same kernel.
+        Depthwise convolutions (one input channel per group: the efficient backbones) are not covered."""
         assert isinstance(x, Act32) and not x.weight_order
         assert x.has_planes, "a convolution reads the planes of an activation that was planned without them"
+        if groups != 1:
+            if w_folded.shape[1] == 1:
+                raise NotImplementedError("depthwise convolutions are not part of the FP32-accurate plan (efficient "
+                                          "backbones); run them with 'fp16' / 'bf16'")
+            w_folded = block_diagonal(w_folded, groups)
         w = w_folded.to(torch.float64)
         cout, cin = w.shape[:2]
         assert cin == x.shape[4]
@@ -190,13 +200,17 @@ class PrecisePlan(Plan):
 
     def pool(self, x, y, kernel, stride, padding, is_avg=False, act=rt.ACT_NONE):
         assert act == rt.ACT_NONE
-        xv, yv = rt.view(x.f32), rt.view(y.f32)
+        self._pool32(x.f32, y.f32, kernel, stride, padding, is_avg)
+        self._post(y.f32, y, label="split")
+
+    def _pool32(self, x, y, kernel, stride, padding, is_avg):
+        """esf_p32_pool3d between two FP32 tensors."""
+        xv, yv = rt.view(x), rt.view(y)
         self.keep += [xv, yv]
         L = rt.lib()
         self._add(lambda s: rt.check(L.esf_p32_pool3d(ctypes.byref(xv), ctypes.byref(yv), *kernel, *stride, *padding,
                                                       int(is_avg), s), "esf_p32_pool3d"),
-                  "p32_pool", "%s C=%d" % (tuple(kernel), x.shape[4]), nbytes=self._nbytes(x.f32, y.f32))
-        self._post(y.f32, y, label="split")
+                  "p32_pool", "%s C=%d" % (tuple(kernel), x.shape[4]), nbytes=self._nbytes(x, y))
 
     def eca_fuse(self, x_fast, y_slice, alpha, eca_weight, bn):
         scale, shift = bn_affine(bn)
@@ -216,11 +230,11 @@ class PrecisePlan(Plan):
 
     def position_attention(self, x_slow, y_slice, alpha, w_down, att, bn):
         """Same composition as Plan.position_attention; the projection GEMM runs on the split operands, the fused
-        attention kernel writes FP32 into the concat slice, which is then split into planes."""
+        attention kernel writes FP32 into the concat slice, which is then split into planes.  Any head dim: the split
+        tensor-core kernel up to d = 64 (its geometry pads d like the 16-bit kernel's), FP32 flash attention on the CUDA
+        cores up to 128, the generic FP32 CUDA-core kernel of the 16-bit plan above."""
         B, T, H, W, C = x_slow.shape
         w_all, b_all, d = attention_projection(w_down, att)
-        if d not in (8, 16, 32, 64, 128):
-            raise NotImplementedError("head dim %d is not part of the FP32-accurate plan (8, 16, 32, 64, 128)" % d)
         proj = super().act(B, T, H, W, 4 * d, dtype=torch.float32)
         self.conv(x_slow, proj, w_all, b_all)
         L = rt.lib()
@@ -254,16 +268,23 @@ class PrecisePlan(Plan):
             self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "attention",
                       "N=%d d=%d split" % (N, d), flops=8.0 * B * N * N * d, exps=float(B) * N * N,
                       nbytes=nbytes + nlo + self._nbytes(y_slice.f32))
-        else:
-            # d = 128 has no hi/lo logit split on the tensor cores (the split Q tile does not fit in shared memory):
-            # FP32 flash attention on the CUDA cores (N = 1 568 there)
+        elif d <= 128:
+            # d in (64, 128] has no hi/lo logit split on the tensor cores (the split Q tile does not fit in shared
+            # memory): FP32 flash attention on the CUDA cores (d = 128: N = 1 568 there)
             self._add(lambda s: rt.check(
                 L.esf_p32_attention(proj.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
                                     ctypes.byref(yv), s), "esf_p32_attention"), "p32_attention", "N=%d d=%d" % (N, d),
                 flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj) + self._nbytes(y_slice.f32))
+        else:
+            self._add(lambda s: rt.check(
+                L.esf_attn_generic(proj.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
+                                   ctypes.byref(yv), s), "esf_attn_generic"), "attention", "N=%d d=%d generic" % (N, d),
+                flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj) + self._nbytes(y_slice.f32))
         self._post(y_slice.f32, y_slice, label="split")
 
     def head(self, xs, weight, bias, act):
+        """xs: Act32 activations, or plain FP32 tensors (the pooled rows of positions_head)."""
+        xs = [x.f32 if isinstance(x, Act32) else x for x in xs]
         B = xs[0].shape[0]
         cin = sum(x.shape[4] for x in xs)
         K = weight.shape[0]
@@ -274,11 +295,11 @@ class PrecisePlan(Plan):
         L = rt.lib()
         off = 0
         for x in xs:
-            xv = rt.view(x.f32)
+            xv = rt.view(x)
             self.keep.append(xv)
             self._add(lambda s, xv=xv, off=off: rt.check(L.esf_p32_head_pool(ctypes.byref(xv), feat.data_ptr(), cin, off, s),
                                                          "esf_p32_head_pool"), "p32_head_pool", "",
-                      nbytes=self._nbytes(x.f32))
+                      nbytes=self._nbytes(x))
             off += x.shape[4]
         from .engine import head_fc_launches
         self._add(lambda s: rt.check(
@@ -289,16 +310,29 @@ class PrecisePlan(Plan):
         return out
 
     def head_positions(self, xs, pool_sizes, weight, bias, act):
-        raise NotImplementedError("fully-convolutional testing is not part of the FP32-accurate plan")
+        """Plan.head_positions on the FP32 tensors: AvgPool3d(kernel, stride 1) of every pathway into a plain FP32
+        buffer (nothing multiplies it on the tensor cores, so it gets no planes), then the shared positions_head --
+        Linear + activation at every position (esf_p32_head_pool of a one-position row is a copy) and their mean."""
+        pooled = []
+        for x, ps in zip(xs, pool_sizes):
+            B, T, H, W, C = x.shape
+            kt, kh, kw = [int(v) for v in ps]
+            y = torch.empty((B, T - kt + 1, H - kh + 1, W - kw + 1, C), dtype=torch.float32, device=self.device)
+            self.keep.append(y)
+            self._pool32(x.need_f32("the head"), y, (kt, kh, kw), (1, 1, 1), (0, 0, 0), is_avg=True)
+            pooled.append(y)
+        return self.positions_head(pooled, weight, bias, act)
 
     def nonlocal_block(self, x, y, nln, group=1):
         """Nonlocal.forward (nonlocal_helper.py:105-148) at FP32 accuracy: theta / phi / g / out are split-operand convs;
         the two matrix products are per-clip-weight GEMMs on split operands as well -- theta and the normalised affinity
         are A operands ([hi | lo | hi] planes), the clip's phi rows and transposed g rows are the weight operands
         ([hi | hi | lo]); the affinity is materialised in FP32 and normalised by esf_p32_row_softmax.  (Not fused: an
-        accuracy mode.)"""
+        accuracy mode.)  NONLOCAL.GROUP > 1: the (b, t) -> (b * group, t / group) view of Plan.nonlocal_block, applied to
+        the FP32 tensor and to the planes of x and y."""
         if group > 1:
-            raise NotImplementedError("NONLOCAL.GROUP > 1 is not part of the FP32-accurate plan")
+            x, y = (Act32(fold_time_groups(a.f32, group), fold_time_groups(a.x3, group) if a.has_planes else None,
+                          a.plane, a.c0, a.c_total, a.weight_order, a.has_f32, a.has_planes) for a in (x, y))
         L = rt.lib()
         B, T, H, W, C = x.shape
         d = nln.dim_inner

@@ -303,7 +303,7 @@ class _PlannedModel(nn.Module):
     """Shared forward machinery: shape-keyed launch plans, weight-version tracking, CUDA-graph replay."""
 
     num_pathways = 2
-    supports_fp32 = False     # cfg.ESF.PRECISION = "fp32" (engine_fp32.PrecisePlan): the ResNet-50 family only
+    supports_fp32 = False     # cfg.ESF.PRECISION = "fp32" (engine_fp32.PrecisePlan): every classification model here
     enable_detection = False  # cfg.DETECTION.ENABLE: ResNetRoIHead, forward(x, bboxes) returns one row per box
 
     def _init_runtime(self, cfg):
@@ -357,7 +357,7 @@ class _PlannedModel(nn.Module):
         with torch.cuda.device(device):
             if prec == "fp32":
                 if not self.supports_fp32:
-                    raise NotImplementedError("ESF.PRECISION = 'fp32' (FP32-accurate plan) covers the ResNet-50 based "
+                    raise NotImplementedError("ESF.PRECISION = 'fp32' (FP32-accurate plan) covers the ResNet based "
                                               "models; %s runs with 'fp16' / 'bf16'" % type(self).__name__)
                 from .engine_fp32 import PrecisePlan
                 plan = PrecisePlan(device)
@@ -813,7 +813,8 @@ class _TwoStreamResNet(_PlannedModel):
         w, b = fold_conv_bn(t.a.weight, None, t.a_bn)
         plan.conv(x, ta, w, b, stride=tuple(t.a.stride), padding=tuple(t.a.padding), act=rt.ACT_RELU)
         # RESNET.NUM_GROUPS > 1 (ResNeXt, resnet_helper.py:196-205): Plan.conv runs one implicit GEMM per group on
-        # channel slices, or one dense GEMM over a block-diagonal weight when the slices are thinner than a TMA row
+        # channel slices, or one dense GEMM over a block-diagonal weight when the slices are thinner than a TMA row;
+        # PrecisePlan.conv always takes the block-diagonal weight
         w, b = fold_conv_bn(t.b.weight, None, t.b_bn)
         plan.conv(ta, tb, w, b, stride=tuple(t.b.stride), padding=tuple(t.b.padding),
                   dilation=tuple(t.b.dilation), groups=t.b.groups, act=rt.ACT_RELU)

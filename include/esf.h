@@ -221,7 +221,8 @@ int esf_attn_tc_create(const void* packed, int32_t B, int32_t T, int32_t H, int3
 /* (esf_attn_tc_create also accepts an FP32 output view: the FP32-accurate path below; operands are then FP16.) */
 
 /* ---- generic CUDA-core fallback of the same attention for head dims the tensor-core kernels do not cover (d > 128;
- * in the reference's models that only happens with N <= 392 keys).  Reads the FP32 projection rows directly. */
+ * in the reference's models that only happens with N <= 392 keys).  Reads the FP32 projection rows directly; the
+ * output view is BF16, F16 or F32 (FP32 math throughout: the FP32-accurate plan uses it above d = 128 too). */
 int esf_attn_generic(const float* proj, int32_t B, int32_t T, int32_t H, int32_t W, int32_t d, float gamma,
                      const float* bn_scale, const float* bn_shift, int32_t alpha, const esf_view* y_fast_slice,
                      void* stream);
@@ -289,7 +290,7 @@ int esf_roi_align_max(const float* map, int32_t B, int32_t H, int32_t W, int32_t
  *   esf_p32_head_pool: feat[b][feat_off + c] = mean_{t,h,w} x (head_helper.py:198-210) on an FP32 view.
  *   esf_p32_attention: SpatialAttention.forward (wdf_attention_helper.py:33-54) + bn_s2f + ReLU + x alpha upsample in
  *                      FP32 on the CUDA cores (flash style, no N x N matrix); proj: FP32 rows [x_d | q | k | v];
- *                      d in {8, 16, 32, 64, 128}.  (The tcgen05 attention rounds P and V to FP16.)
+ *                      any d <= 128.  (The tcgen05 attention rounds P and V to FP16.)
  * esf_stem_conv accepts an FP32 output view (FP32 CUDA-core stem) and esf_attn_tc_create an FP32 output slice. */
 int esf_p32_post(const esf_view* acc, const float* scale, const float* bias, const esf_view* res, int32_t act,
                  const esf_view* y32, const esf_view* y3, int32_t plane, int32_t weight_order, void* stream);
