@@ -15,6 +15,7 @@ import torch
 from . import runtime as rt
 
 BN_EPS_DEFAULT = 1e-5
+_VIEW_P = ctypes.POINTER(rt.EsfView)
 
 
 def host64(t):
@@ -237,6 +238,7 @@ class Plan:
         self.launches_per_run = 0
         self.buffers = {}     # name -> activation tensor (for tests / debugging)
         self.meta = []        # one dict per op: kind, label, algorithmic flops / bytes / exps, launches
+        self._scratch = {}    # (shape, dtype, zero) -> tensor shared by the ops of this plan (scratch())
 
     # ---------------------------------------------------------------- memory
     def act(self, B, T, H, W, C, name=None, dtype=None, role=None):
@@ -284,6 +286,64 @@ class Plan:
                               launches=launches))
         self.launches_per_run += launches
 
+    def _bind(self, fn_name, *args):
+        """The library function `fn_name` with every argument but the last (the stream, or the esf_op** of a create
+        call) converted now, by the function's argtypes: a tensor for an esf_view* becomes a pointer to its view (None:
+        the null view), a tensor for a void* its data pointer.  A launch replays these pointers for the plan's lifetime,
+        so every converted tensor and view is kept.  Returns the checked call taking that last argument."""
+        f = getattr(rt.lib(), fn_name)
+        assert len(args) == len(f.argtypes) - 1, fn_name
+        frozen = []
+        for a, t in zip(args, f.argtypes):
+            if t is _VIEW_P:
+                v = rt.view(a) if a is not None else rt.null_view()
+                self.keep += [a, v]
+                a = ctypes.byref(v)
+            elif t is ctypes.c_void_p and isinstance(a, torch.Tensor):
+                self.keep.append(a)
+                a = a.data_ptr()
+            frozen.append(a)
+        return lambda s: rt.check(f(*frozen, s), fn_name)
+
+    def _launch(self, fn_name, *args, kind, label="", flops=0, nbytes=0, exps=0, launches=1, eager=False):
+        """Record one launch of `fn_name` (arguments as _bind converts them) as an op of the plan."""
+        self._add(self._bind(fn_name, *args), kind, label, flops, nbytes, exps, launches, eager)
+
+    def _create(self, fn_name, *args):
+        """Plan an esf_op with the create function `fn_name` (arguments as _bind converts them); returns its handle, which
+        the plan destroys."""
+        h = ctypes.c_void_p()
+        self._bind(fn_name, *args)(ctypes.byref(h))
+        self.handles.append(h)
+        return h
+
+    @staticmethod
+    def _call(fn_name, *args):
+        """Checked call of `fn_name` with arguments read at launch time (the ops that read the caller's clip)."""
+        rt.check(getattr(rt.lib(), fn_name)(*args), fn_name)
+
+    @staticmethod
+    def _size(fn_name, *args):
+        """A host-side size query of the library (esf_*_bytes, esf_*_scratch_floats); a negative result is its error."""
+        n = int(getattr(rt.lib(), fn_name)(*args))
+        rt.check(min(n, 0), fn_name)
+        return n
+
+    def _conv_desc(self, x, y, res, w, bias, ksize, stride=(1, 1, 1), padding=(0, 0, 0), dilation=(1, 1, 1), groups=1,
+                   act=rt.ACT_NONE):
+        """esf_conv_desc* of a convolution into `y` (output format: y's dtype); the descriptor and its tensors are kept."""
+        d = rt.EsfConvDesc(rt.view(x), rt.view(y), rt.view(res) if res is not None else rt.null_view(), w.data_ptr(),
+                           bias.data_ptr(), *ksize, *stride, *padding, *dilation, groups, act, rt.dtype_code(y))
+        self.keep += [d, x, y, res, w, bias]
+        return ctypes.byref(d)
+
+    def _head_fc(self, feat, w, b, act, out, out_stride=None, kind="head_fc", **meta):
+        """esf_head_fc: out = act(feat @ w^T + b) on FP32 rows (feat (B, Cin), w (K, Cin), out rows of stride
+        out_stride, default K)."""
+        (B, cin), K = feat.shape, w.shape[0]
+        self._launch("esf_head_fc", feat, B, cin, cin, w, b, K, act, out, out_stride or K, kind=kind,
+                     launches=head_fc_launches(B, cin, K, act), **meta)
+
     @staticmethod
     def _nbytes(*tensors):
         return sum(t.numel() * t.element_size() for t in tensors if t is not None)
@@ -291,21 +351,16 @@ class Plan:
     # ---------------------------------------------------------------- ops
     def conv_igemm(self, x, y, w_folded, bias, stride=(1, 1, 1), padding=(0, 0, 0), dilation=(1, 1, 1), act=rt.ACT_NONE,
                    res=None, out_dtype=None):
-        out_dtype = rt.dtype_code(y)
         wp, bp = pack_igemm_weight(w_folded, bias, self.device, self.adt)
-        self.keep += [wp, bp]
         kt, kh, kw = w_folded.shape[2:]
-        d = rt.EsfConvDesc(rt.view(x), rt.view(y), rt.view(res) if res is not None else rt.null_view(),
-                           wp.data_ptr(), bp.data_ptr(), kt, kh, kw, *stride, *padding, *dilation, 1, act, out_dtype)
-        h = ctypes.c_void_p()
-        rt.check(rt.lib().esf_conv_igemm_create(ctypes.byref(d), ctypes.byref(h)), "esf_conv_igemm_create")
-        self.handles.append(h)
-        L = rt.lib()
+        h = self._create("esf_conv_igemm_create",
+                         self._conv_desc(x, y, res, wp, bp, (kt, kh, kw), stride, padding, dilation, 1, act))
         cout, cin = w_folded.shape[:2]
         m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
-        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "conv_igemm",
-                  "%dx%dx%d s%s %d->%d @%s" % (kt, kh, kw, "".join(map(str, stride)), cin, cout, tuple(y.shape[1:4])),
-                  flops=2.0 * m * cout * cin * kt * kh * kw, nbytes=self._nbytes(x, y, res) + wp.numel() * 2)
+        self._launch("esf_op_launch", h, kind="conv_igemm",
+                     label="%dx%dx%d s%s %d->%d @%s" % (kt, kh, kw, "".join(map(str, stride)), cin, cout,
+                                                        tuple(y.shape[1:4])),
+                     flops=2.0 * m * cout * cin * kt * kh * kw, nbytes=self._nbytes(x, y, res) + wp.numel() * 2)
 
     def gemm_rows(self, x, y, w_rows, bias, kind, label):
         """y[b, pos, n] = sum_c x[b, pos, c] * w_rows[b, n, c] + bias[n] on the implicit-GEMM kernel with one
@@ -315,27 +370,38 @@ class Plan:
         kc, kchunks, _, n_pad = rt.igemm_geometry(cin, cout)
         assert tuple(w_rows.shape) == (x.shape[0], n_pad, kc * kchunks) and w_rows.is_contiguous()
         assert w_rows.dtype == self.adt and bias.numel() == n_pad and bias.dtype == torch.float32
-        d = rt.EsfConvDesc(rt.view(x), rt.view(y), rt.null_view(), w_rows.data_ptr(), bias.data_ptr(), 1, 1, 1,
-                           1, 1, 1, 0, 0, 0, 1, 1, 1, 1, rt.ACT_NONE, rt.dtype_code(y))
-        h = ctypes.c_void_p()
-        L = rt.lib()
-        rt.check(L.esf_gemm_clip_weights_create(ctypes.byref(d), ctypes.byref(h)), "esf_gemm_clip_weights_create")
-        self.handles.append(h)
+        h = self._create("esf_gemm_clip_weights_create", self._conv_desc(x, y, None, w_rows, bias, (1, 1, 1)))
         m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
-        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), kind, label,
-                  flops=2.0 * m * cout * cin, nbytes=self._nbytes(x, y) + x.shape[0] * cout * cin * 2)
+        self._launch("esf_op_launch", h, kind=kind, label=label, flops=2.0 * m * cout * cin,
+                     nbytes=self._nbytes(x, y) + x.shape[0] * cout * cin * 2)
 
     def scratch(self, shape, dtype, zero=False):
         """Plan-lifetime scratch tensor shared by every op that asks for the same (shape, dtype): the launches of a
         plan are serialised on one stream, so the Non-local blocks of a model reuse one affinity matrix."""
         key = (tuple(shape), dtype, bool(zero))
-        if not hasattr(self, "_scratch"):
-            self._scratch = {}
         if key not in self._scratch:
             t = (torch.zeros if zero else torch.empty)(tuple(shape), dtype=dtype, device=self.device)
             self.keep.append(t)
             self._scratch[key] = t
         return self._scratch[key]
+
+    @staticmethod
+    def _weight_bias(conv):
+        return host64(conv.weight), host64(conv.bias)
+
+    def _nonlocal_keys(self, x, nln):
+        """Key side of a Non-local block on the (group-folded) input x: x max-pooled by nln.pool_size when nln.use_pool,
+        else x itself, and whether the instantiation is "softmax" (else "dot_product")."""
+        softmax = nln.instantiation == "softmax"
+        if not softmax and nln.instantiation != "dot_product":
+            raise NotImplementedError("Unknown norm type {}".format(nln.instantiation))
+        if not nln.use_pool:
+            return x, softmax
+        B, T, H, W, C = x.shape
+        ps = tuple(int(v) for v in nln.pool_size)
+        xp = self.act(B, (T - ps[0]) // ps[0] + 1, (H - ps[1]) // ps[1] + 1, (W - ps[2]) // ps[2] + 1, C)
+        self.pool(x, xp, ps, ps, (0, 0, 0))
+        return xp, softmax
 
     def nonlocal_block(self, x, y, nln, group=1):
         """Nonlocal.forward (nonlocal_helper.py:105-148) + the temporal group folding of ResStage.forward
@@ -348,27 +414,15 @@ class Plan:
         ([d][N_keys], written by esf_transpose16); the affinity matrix is materialised once in FP32, normalised by
         esf_row_softmax (softmax with d^-0.5, or the 1/N_keys of "dot_product") into the 16-bit A operand of the
         second product."""
-        L = rt.lib()
         if group > 1:
             x, y = fold_time_groups(x, group), fold_time_groups(y, group)
         B, T, H, W, C = x.shape
         d = nln.dim_inner
         f64 = torch.float64
-
-        def wb(conv):
-            return host64(conv.weight), host64(conv.bias)
-
-        if nln.use_pool:
-            ps = [int(v) for v in nln.pool_size]
-            Tp, Hp, Wp = (T - ps[0]) // ps[0] + 1, (H - ps[1]) // ps[1] + 1, (W - ps[2]) // ps[2] + 1
-            xp = self.act(B, Tp, Hp, Wp, C)
-            self.pool(x, xp, tuple(ps), tuple(ps), (0, 0, 0))
-        else:
-            Tp, Hp, Wp, xp = T, H, W, x
+        xp, softmax = self._nonlocal_keys(x, nln)
+        Tp, Hp, Wp = xp.shape[1:4]
         Nq, Nk = T * H * W, Tp * Hp * Wp
-        softmax = nln.instantiation == "softmax"
-        if not softmax and nln.instantiation != "dot_product":
-            raise NotImplementedError("Unknown norm type {}".format(nln.instantiation))
+        wb = self._weight_bias
         # Precision: with near-uniform attention the block output is a large per-channel constant plus a small
         # variation, and the BN behind conv_out removes the constant -- 16-bit rounding of `att` would then be
         # amplified by |mean| / std.  conv_out is linear, so a per-channel offset mu can be subtracted in the FP32
@@ -390,10 +444,8 @@ class Plan:
             kc, kch, _, npad = rt.igemm_geometry(Nk, d)
             kpad = kc * kch
             tT = torch.zeros((B, npad, kpad), dtype=self.adt, device=self.device)
-            self.keep.append(tT)
-            self._add(lambda s: rt.check(L.esf_transpose16(t.data_ptr(), B, Nk, d, t.stride(0), t.stride(3), tT.data_ptr(),
-                                                           npad * kpad, kpad, s), "esf_transpose16"),
-                      "nl_transpose", name, nbytes=2 * self._nbytes(t))
+            self._launch("esf_transpose16", t, B, Nk, d, t.stride(0), t.stride(3), tT, npad * kpad, kpad,
+                         kind="nl_transpose", label=name, nbytes=2 * self._nbytes(t))
             return tT
 
         if softmax:
@@ -415,9 +467,9 @@ class Plan:
             P = Pbuf[..., :Nk]
             zero1 = self.scratch((npad1,), torch.float32, zero=True)
             self.gemm_rows(theta, S, phi_rows, zero1, "nl_gemm", "theta.phi N=%dx%d d=%d" % (Nq, Nk, d))
-            self._add(lambda s: rt.check(L.esf_row_softmax(Sbuf.data_ptr(), B * Nq, Nk, Sbuf.shape[4], float(d) ** -0.5, 0,
-                                                           self.a16, Pbuf.data_ptr(), Pbuf.shape[4], s), "esf_row_softmax"),
-                      "nl_softmax", nln.instantiation, nbytes=self._nbytes(S, P), exps=float(B * Nq * Nk))
+            self._launch("esf_row_softmax", Sbuf, B * Nq, Nk, Sbuf.shape[4], float(d) ** -0.5, 0, self.a16, Pbuf,
+                         Pbuf.shape[4], kind="nl_softmax", label=nln.instantiation, nbytes=self._nbytes(S, P),
+                         exps=float(B * Nq * Nk))
             self.gemm_rows(P, att, gT, bias2, "nl_gemm", "p.g N=%dx%d d=%d" % (Nq, Nk, d))
         else:
             # "dot_product" has no non-linearity between the two products:  (theta^T phi / Nk) g^T = theta^T (phi g^T / Nk),
@@ -448,21 +500,15 @@ class Plan:
     def conv_wfold(self, x, y, w_folded, bias, WB, stride=(1, 1, 1), padding=(0, 0, 0), act=rt.ACT_NONE, res=None):
         """Thin-layer (C_in <= 32) conv as a W-folded banded GEMM: see esf_conv_wfold_create."""
         wp, bp = pack_wfold_band(w_folded, bias, WB, stride[2], self.device, self.adt)
-        self.keep += [wp, bp]
         kt, kh, kw = w_folded.shape[2:]
-        d = rt.EsfConvDesc(rt.view(x), rt.view(y), rt.view(res) if res is not None else rt.null_view(),
-                           wp.data_ptr(), bp.data_ptr(), kt, kh, kw, *stride, *padding, 1, 1, 1, 1, act,
-                           rt.dtype_code(y))
-        h = ctypes.c_void_p()
-        L = rt.lib()
-        rt.check(L.esf_conv_wfold_create(ctypes.byref(d), WB, ctypes.byref(h)), "esf_conv_wfold_create")
-        self.handles.append(h)
+        h = self._create("esf_conv_wfold_create",
+                         self._conv_desc(x, y, res, wp, bp, (kt, kh, kw), stride, padding, act=act), WB)
         cout, cin = w_folded.shape[:2]
         m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
-        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "conv_wfold",
-                  "%dx%dx%d s%s %d->%d @%s wb%d" % (kt, kh, kw, "".join(map(str, stride)), cin, cout,
-                                                   tuple(y.shape[1:4]), WB),
-                  flops=2.0 * m * cout * cin * kt * kh * kw, nbytes=self._nbytes(x, y, res) + wp.numel() * 2)
+        self._launch("esf_op_launch", h, kind="conv_wfold",
+                     label="%dx%dx%d s%s %d->%d @%s wb%d" % (kt, kh, kw, "".join(map(str, stride)), cin, cout,
+                                                             tuple(y.shape[1:4]), WB),
+                     flops=2.0 * m * cout * cin * kt * kh * kw, nbytes=self._nbytes(x, y, res) + wp.numel() * 2)
 
     @staticmethod
     def _aligned(t):
@@ -519,15 +565,10 @@ class Plan:
 
     def conv_direct(self, x, y, w_folded, bias, stride=(1, 1, 1), padding=(0, 0, 0), dilation=(1, 1, 1), groups=1,
                     act=rt.ACT_NONE, res=None, out_dtype=None):
-        out_dtype = rt.dtype_code(y)
         wd = self.tensor(w_folded.permute(0, 2, 3, 4, 1))  # [Cout][kT][kH][kW][Cin/g]
         bd = self.tensor(bias)
         kt, kh, kw = w_folded.shape[2:]
-        d = rt.EsfConvDesc(rt.view(x), rt.view(y), rt.view(res) if res is not None else rt.null_view(),
-                           wd.data_ptr(), bd.data_ptr(), kt, kh, kw, *stride, *padding, *dilation, groups, act,
-                           out_dtype)
-        self.keep.append(d)
-        L = rt.lib()
+        d = self._conv_desc(x, y, res, wd, bd, (kt, kh, kw), stride, padding, dilation, groups, act)
         m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
         depthwise = groups == x.shape[4] == y.shape[4] and kw in (3, 5)
         C = x.shape[4]
@@ -536,24 +577,22 @@ class Plan:
                 and all(pad_of(t) == (C, (C + 7) // 8 * 8) for t in (x, y, res)) and y.dtype == x.dtype == self.adt):
             # rows padded to a multiple of 8 channels by act(): 16-byte vectors over the padded width (zero weights)
             cp = (C + 7) // 8 * 8
-            self._add(lambda s, d=d: rt.check(L.esf_dwconv_padded(ctypes.byref(d), cp, s), "esf_dwconv_padded"),
-                      "dwconv", "%dx%dx%d s%d%d%d g%d %d->%d pad%d @%s" % (kt, kh, kw, *stride, groups, C, C, cp,
-                                                                              tuple(x.shape[1:4])),
-                      flops=2.0 * m * C * kt * kh * kw, nbytes=self._nbytes(x, y, res) + wd.numel() * 4)
+            self._launch("esf_dwconv_padded", d, cp, kind="dwconv",
+                         label="%dx%dx%d s%d%d%d g%d %d->%d pad%d @%s" % (kt, kh, kw, *stride, groups, C, C, cp,
+                                                                          tuple(x.shape[1:4])),
+                         flops=2.0 * m * C * kt * kh * kw, nbytes=self._nbytes(x, y, res) + wd.numel() * 4)
             return
         cout = y.shape[4]
-        call = lambda s, d=d: rt.check(L.esf_conv_direct(ctypes.byref(d), s), "esf_conv_direct")
+        call = ("esf_conv_direct", d)
         if (groups == 1 and (kt, kh, kw) == (1, 1, 1) and cout >= 8 and cout % 8 != 0 and y.dtype == self.adt
                 and self.padded.get(y.data_ptr()) == (cout, (cout + 7) // 8 * 8)):
             # y is a whole padded allocation (not a concat slice): the kernel may write the row padding too
-            cp = (cout + 7) // 8 * 8
-            call = lambda s, d=d, cp=cp: rt.check(L.esf_pointwise_padded(ctypes.byref(d), cp, s), "esf_pointwise_padded")
-        self._add(call,
-                  "dwconv" if depthwise else "conv_direct",
-                  "%dx%dx%d s%d%d%d g%d %d->%d @%s" % (kt, kh, kw, *stride, groups, x.shape[4], y.shape[4],
-                                                       tuple(x.shape[1:4])),
-                  flops=2.0 * m * y.shape[4] * (x.shape[4] // groups) * kt * kh * kw,
-                  nbytes=self._nbytes(x, y, res) + wd.numel() * 4)
+            call = ("esf_pointwise_padded", d, (cout + 7) // 8 * 8)
+        self._launch(*call, kind="dwconv" if depthwise else "conv_direct",
+                     label="%dx%dx%d s%d%d%d g%d %d->%d @%s" % (kt, kh, kw, *stride, groups, x.shape[4], y.shape[4],
+                                                                tuple(x.shape[1:4])),
+                     flops=2.0 * m * y.shape[4] * (x.shape[4] // groups) * kt * kh * kw,
+                     nbytes=self._nbytes(x, y, res) + wd.numel() * 4)
 
     def stem_conv(self, x_nc, y, w_folded, bias, stride, padding, act=rt.ACT_RELU):
         """x_nc: FP32 (B,Cin,T,H,W) contiguous plan-owned input buffer."""
@@ -563,12 +602,11 @@ class Plan:
         cout = w_folded.shape[0]
         kt, kh, kw = w_folded.shape[2:]
         yv = rt.view(y)
-        self.keep.append(yv)
-        L = rt.lib()
+        self.keep += [y, yv]
         m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
-        self._add(lambda s: rt.check(
-            L.esf_stem_conv(self._in_ptr(x_nc), B, Cin, T, H, W, ws.data_ptr(), bs.data_ptr(), cout, kt, kh, kw, *stride,
-                            *padding, act, ctypes.byref(yv), s), "esf_stem_conv"), "stem_conv",
+        self._add(lambda s: self._call(
+            "esf_stem_conv", self._in_ptr(x_nc), B, Cin, T, H, W, ws.data_ptr(), bs.data_ptr(), cout, kt, kh, kw, *stride,
+            *padding, act, ctypes.byref(yv), s), "stem_conv",
             "%dx%dx%d %d->%d" % (kt, kh, kw, Cin, cout), flops=2.0 * m * cout * Cin * kt * kh * kw,
             nbytes=self._nbytes(x_nc, y), eager=True)
 
@@ -591,31 +629,21 @@ class Plan:
         B, Cin, T, H, W = x_shape
         cout = w_folded.shape[0]
         kt, kh, kw = w_folded.shape[2:]
-        L = rt.lib()
         if twb:
             wb, bt = pack_stem_tband(w_folded, bias, twb, stride[2], self.device, self.adt)
-            create, what = L.esf_stem_tband_create, "esf_stem_tband_create"
         else:
             wb, bt = pack_stem_band(w_folded, bias, stride[2], self.device, self.adt)
-            create, what = L.esf_stem_igemm_create, "esf_stem_igemm_create"
-        yv = rt.view(y)
-        h = ctypes.c_void_p()
-        rt.check(create(xp.data_ptr(), B, Cin, T, H, W, pitch, wb.data_ptr(), bt.data_ptr(), cout, kt, kh, kw,
-                        stride[1], stride[2], padding[0], padding[1], padding[2], act, ctypes.byref(yv),
-                        ctypes.byref(h)), what)
-        self.keep += [wb, bt]
-        self.handles.append(h)
+        h = self._create("esf_stem_tband_create" if twb else "esf_stem_igemm_create", xp, B, Cin, T, H, W, pitch, wb, bt,
+                         cout, kt, kh, kw, stride[1], stride[2], padding[0], padding[1], padding[2], act, y)
         label = "%dx%dx%d %d->%d %s" % (kt, kh, kw, Cin, cout, "t-band" if twb else "banded")
         m = y.shape[0] * y.shape[1] * y.shape[2] * y.shape[3]
-        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "stem_igemm",
-                  label + (" " + name if name else ""), flops=2.0 * m * cout * Cin * kt * kh * kw,
-                  nbytes=self._nbytes(xp, y) + wb.numel() * 2)
+        self._launch("esf_op_launch", h, kind="stem_igemm", label=label + (" " + name if name else ""),
+                     flops=2.0 * m * cout * Cin * kt * kh * kw, nbytes=self._nbytes(xp, y) + wb.numel() * 2)
 
     def stem_gemm(self, x_nc, y, w_folded, bias, stride, padding, act, pitch, lpad, twb):
         """Stem on the tensor cores: the clip is packed into 16-bit rows (`pitch`, `lpad`: esf_stem_geometry), then one
         GEMM -- temporal-band for twb > 0, banded for twb == 0 (see stem_route)."""
         B, Cin, T, H, W = x_nc.shape
-        L = rt.lib()
         xp = torch.empty((B, T, H, pitch), dtype=self.adt, device=self.device)
         self.keep.append(xp)
         self.stem_routes[x_nc.data_ptr()] = (xp, pitch, lpad)   # the uint8 frame route writes xp itself (frames.py)
@@ -624,38 +652,24 @@ class Plan:
             g = self.gather.get(x_nc.data_ptr())
             if g is not None:       # frames of this pathway are read out of another pathway's clip (slow from fast)
                 src, tsrc, idx = g
-                rt.check(L.esf_stem_pack_gather(src, B, Cin, tsrc, H, W, idx, T, pitch, lpad, self.a16, xp.data_ptr(), s),
-                         "esf_stem_pack_gather")
+                self._call("esf_stem_pack_gather", src, B, Cin, tsrc, H, W, idx, T, pitch, lpad, self.a16, xp.data_ptr(), s)
             else:
-                rt.check(L.esf_stem_pack(self._in_ptr(x_nc), B, Cin, T, H, W, pitch, lpad, self.a16, xp.data_ptr(), s),
-                         "esf_stem_pack")
+                self._call("esf_stem_pack", self._in_ptr(x_nc), B, Cin, T, H, W, pitch, lpad, self.a16, xp.data_ptr(), s)
 
         self._add(pack, "stem_pack", "", nbytes=self._nbytes(x_nc, xp), eager=True)
         self.meta[-1]["is_pack"] = True
         self._stem_gemm_op(xp, x_nc.shape, y, w_folded, bias, stride, padding, act, pitch, twb)
 
     def pool(self, x, y, kernel, stride, padding, is_avg=False, act=rt.ACT_NONE):
-        xv, yv = rt.view(x), rt.view(y)
-        self.keep += [xv, yv]
-        L = rt.lib()
-        self._add(lambda s: rt.check(
-            L.esf_pool3d(ctypes.byref(xv), ctypes.byref(yv), *kernel, *stride, *padding, int(is_avg), act, s),
-            "esf_pool3d"), "pool", "%s C=%d" % (tuple(kernel), x.shape[4]), nbytes=self._nbytes(x, y))
+        self._launch("esf_pool3d", x, y, *kernel, *stride, *padding, int(is_avg), act, kind="pool",
+                     label="%s C=%d" % (tuple(kernel), x.shape[4]), nbytes=self._nbytes(x, y))
 
     def shuffle_concat(self, a, b, groups, y):
-        av, yv = rt.view(a), rt.view(y)
-        bv = rt.view(b) if b is not None else rt.null_view()
-        self.keep += [av, bv, yv]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_shuffle_concat(ctypes.byref(av), ctypes.byref(bv), groups, ctypes.byref(yv), s),
-                                     "esf_shuffle_concat"), "shuffle", "g%d" % groups, nbytes=2 * self._nbytes(y))
+        self._launch("esf_shuffle_concat", a, b, groups, y, kind="shuffle", label="g%d" % groups,
+                     nbytes=2 * self._nbytes(y))
 
     def eltwise_add(self, a, b, y, act=rt.ACT_NONE):
-        av, bv, yv = rt.view(a), rt.view(b), rt.view(y)
-        self.keep += [av, bv, yv]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_eltwise_add(ctypes.byref(av), ctypes.byref(bv), ctypes.byref(yv), act, s),
-                                     "esf_eltwise_add"), "add", "", nbytes=3 * self._nbytes(y))
+        self._launch("esf_eltwise_add", a, b, y, act, kind="add", nbytes=3 * self._nbytes(y))
 
     def squeeze_excite(self, x, y, se):
         """SqueezeExcite (ghostnet_helper.py:34-52): global mean -> 1x1x1(+bias) -> ReLU -> 1x1x1(+bias) -> hard-sigmoid
@@ -667,89 +681,73 @@ class Plan:
         gate = torch.empty((B, C), dtype=torch.float32, device=self.device)
         w1, b1 = self.tensor(se.conv_reduce.weight.reshape(R, C)), self.tensor(se.conv_reduce.bias)
         w2, b2 = self.tensor(se.conv_expand.weight.reshape(C, R)), self.tensor(se.conv_expand.bias)
-        xv, yv, nv = rt.view(x), rt.view(y), rt.null_view()
-        self.keep += [feat, hid, gate, xv, yv, nv]
-        L = rt.lib()
         self.global_mean(x, feat, C, 0, "se_pool")
-        self._add(lambda s: rt.check(L.esf_head_fc(feat.data_ptr(), B, C, C, w1.data_ptr(), b1.data_ptr(), R, rt.HEAD_RELU,
-                                                   hid.data_ptr(), R, s), "esf_head_fc"), "se_fc", "")
-        self._add(lambda s: rt.check(L.esf_head_fc(hid.data_ptr(), B, R, R, w2.data_ptr(), b2.data_ptr(), C,
-                                                   rt.HEAD_HARD_SIGMOID, gate.data_ptr(), C, s), "esf_head_fc"), "se_fc", "")
-        self._add(lambda s: rt.check(L.esf_channel_scale(ctypes.byref(xv), gate.data_ptr(), ctypes.byref(yv), s),
-                                     "esf_channel_scale"), "se_scale", "", nbytes=2 * self._nbytes(x))
+        self._head_fc(feat, w1, b1, rt.HEAD_RELU, hid, kind="se_fc")
+        self._head_fc(hid, w2, b2, rt.HEAD_HARD_SIGMOID, gate, kind="se_fc")
+        self._launch("esf_channel_scale", x, gate, y, kind="se_scale", nbytes=2 * self._nbytes(x))
 
     def global_mean(self, x, feat, feat_stride, feat_off, kind="head_pool"):
         """feat[:, feat_off : feat_off + C] = mean over (T, H, W) of x: the two-pass esf_global_mean for large maps, the
         single-block head kernel for the small ones."""
-        L = rt.lib()
-        xv = rt.view(x)
-        self.keep.append(xv)
         B, T, H, W, C = x.shape
         if T * H * W >= 1024 and (C % 8 == 0 or C <= 256):
-            scratch = self.scratch((int(L.esf_global_mean_scratch_floats(B, C)),), torch.float32)
-            self._add(lambda s: rt.check(L.esf_global_mean(ctypes.byref(xv), scratch.data_ptr(), feat.data_ptr(),
-                                                           feat_stride, feat_off, s), "esf_global_mean"),
-                      kind, "two-pass", nbytes=self._nbytes(x), launches=2)
+            scratch = self.scratch((self._size("esf_global_mean_scratch_floats", B, C),), torch.float32)
+            self._launch("esf_global_mean", x, scratch, feat, feat_stride, feat_off, kind=kind, label="two-pass",
+                         nbytes=self._nbytes(x), launches=2)
         else:
             assert feat_off == 0
-            nv = rt.null_view()
-            self.keep.append(nv)
-            self._add(lambda s: rt.check(L.esf_head_pool(ctypes.byref(xv), ctypes.byref(nv), feat.data_ptr(), s),
-                                         "esf_head_pool"), kind, "", nbytes=self._nbytes(x))
+            self._launch("esf_head_pool", x, None, feat, kind=kind, nbytes=self._nbytes(x))
 
     def eca_fuse(self, x_fast, y_slice, alpha, eca_weight, bn):
         """MaxPool(alpha,1,1) -> ECA -> BN -> ReLU -> concat slice (custom_video_model_builder.py:131-135)."""
+        self._eca_fuse("esf_eca_fuse", "esf_eca_scratch_floats", "eca_fuse", x_fast, y_slice, alpha, eca_weight, bn)
+
+    def _eca_fuse(self, fn_name, scratch_fn_name, kind, x_fast, y_slice, alpha, eca_weight, bn):
+        """eca_fuse on the entry point `fn_name` (the 16-bit one or its FP32 form) and its partial-sum scratch."""
         scale, shift = bn_affine(bn)
         w = self.tensor(eca_weight.reshape(-1))
         sc, sh = self.tensor(scale), self.tensor(shift)
         B, C = x_fast.shape[0], x_fast.shape[4]
-        L = rt.lib()
-        scratch = torch.empty(int(L.esf_eca_scratch_floats(B, C)), dtype=torch.float32, device=self.device)
-        self.keep.append(scratch)
-        xv, yv = rt.view(x_fast), rt.view(y_slice)
-        self.keep += [xv, yv]
-        k = int(w.numel())
-        self._add(lambda s: rt.check(
-            L.esf_eca_fuse(ctypes.byref(xv), alpha, w.data_ptr(), k, sc.data_ptr(), sh.data_ptr(), scratch.data_ptr(),
-                           ctypes.byref(yv), s), "esf_eca_fuse"), "eca_fuse", "C=%d" % C,
-            nbytes=2 * self._nbytes(x_fast) + self._nbytes(y_slice), launches=2)
+        scratch = torch.empty(self._size(scratch_fn_name, B, C), dtype=torch.float32, device=self.device)
+        self._launch(fn_name, x_fast, alpha, w, int(w.numel()), sc, sh, scratch, y_slice, kind=kind, label="C=%d" % C,
+                     nbytes=2 * self._nbytes(x_fast) + self._nbytes(y_slice), launches=2)
+
+    def _attention_operands(self, x_slow, alpha, w_down, att, bn):
+        """Common part of position_attention: attention_projection as one conv into the FP32 rows `proj`
+        [x_d | q | k | v], and the (B, T, H, W, d, gamma, bn scale, bn shift, alpha) arguments that every attention entry
+        point takes after its operand."""
+        B, T, H, W, C = x_slow.shape
+        w_all, b_all, d = attention_projection(w_down, att)
+        proj = self.act(B, T, H, W, 4 * d, dtype=torch.float32)
+        self.conv(x_slow, proj, w_all, b_all)
+        scale, shift = bn_affine(bn)
+        sc, sh = self.tensor(scale), self.tensor(shift)
+        gamma = float(att.gamma.detach().float().item())
+        return proj, (B, T, H, W, d, gamma, sc, sh, alpha)
+
+    def _attention_generic(self, proj, geo, y):
+        """esf_attn_generic: the CUDA-core attention for head dims above the tensor-core kernels' (d > 128)."""
+        B, T, H, W, d = geo[:5]
+        N = T * H * W
+        self._launch("esf_attn_generic", proj, *geo, y, kind="attention", label="N=%d d=%d generic" % (N, d),
+                     flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj, y))
 
     def position_attention(self, x_slow, y_slice, alpha, w_down, att, bn):
         """attention_projection as one GEMM (FP32 out), hi/lo packing, fused flash-style attention + gamma*O + x + BN +
         ReLU + x alpha upsample + concat (custom_video_model_builder.py:141-146, wdf_attention_helper.py:33-54): the
         tcgen05 kernel up to d = 128, the CUDA-core fallback above."""
-        B, T, H, W, C = x_slow.shape
-        w_all, b_all, d = attention_projection(w_down, att)
-        proj = self.act(B, T, H, W, 4 * d, dtype=torch.float32)
-        self.conv(x_slow, proj, w_all, b_all)
-        L = rt.lib()
+        proj, geo = self._attention_operands(x_slow, alpha, w_down, att, bn)
+        B, T, H, W, d = geo[:5]
         N = T * H * W
-        scale, shift = bn_affine(bn)
-        sc, sh = self.tensor(scale), self.tensor(shift)
-        gamma = float(att.gamma.detach().float().item())
-        yv = rt.view(y_slice)
-        self.keep.append(yv)
         if d > 128:
-            self._add(lambda s: rt.check(
-                L.esf_attn_generic(proj.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                                   ctypes.byref(yv), s), "esf_attn_generic"), "attention", "N=%d d=%d generic" % (N, d),
-                flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj, y_slice))
-            return
-        nbytes = int(L.esf_attn_tc_pack_bytes(B, N, d))
-        if nbytes < 0:
-            rt.check(nbytes, "esf_attn_tc_pack_bytes")
+            return self._attention_generic(proj, geo, y_slice)
+        nbytes = self._size("esf_attn_tc_pack_bytes", B, N, d)
         packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-        self.keep.append(packed)
-        h = ctypes.c_void_p()
-        rt.check(L.esf_attn_tc_create(packed.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                                      ctypes.byref(yv), ctypes.byref(h)), "esf_attn_tc_create")
-        self.handles.append(h)
-        self._add(lambda s: rt.check(L.esf_attn_tc_pack(proj.data_ptr(), B, N, d, self.a16, packed.data_ptr(), s),
-                                     "esf_attn_tc_pack"), "attn_pack", "N=%d d=%d" % (N, d),
-                  nbytes=self._nbytes(proj) + nbytes)
-        self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "attention",
-                  "N=%d d=%d" % (N, d), flops=4.0 * B * N * N * d, exps=float(B) * N * N,
-                  nbytes=nbytes + self._nbytes(y_slice))
+        h = self._create("esf_attn_tc_create", packed, *geo, y_slice)
+        self._launch("esf_attn_tc_pack", proj, B, N, d, self.a16, packed, kind="attn_pack", label="N=%d d=%d" % (N, d),
+                     nbytes=self._nbytes(proj) + nbytes)
+        self._launch("esf_op_launch", h, kind="attention", label="N=%d d=%d" % (N, d), flops=4.0 * B * N * N * d,
+                     exps=float(B) * N * N, nbytes=nbytes + self._nbytes(y_slice))
 
     def head(self, xs, weight, bias, act):
         B = xs[0].shape[0]
@@ -758,31 +756,31 @@ class Plan:
         feat = torch.empty((B, cin), dtype=torch.float32, device=self.device)
         out = torch.empty((B, K), dtype=torch.float32, device=self.device)
         w, b = self.tensor(weight), self.tensor(bias)
-        v0 = rt.view(xs[0])
-        v1 = rt.view(xs[1]) if len(xs) > 1 else rt.null_view()
-        self.keep += [feat, out, v0, v1]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_head_pool(ctypes.byref(v0), ctypes.byref(v1), feat.data_ptr(), s),
-                                     "esf_head_pool"), "head_pool", "", nbytes=self._nbytes(*xs), launches=len(xs))
-        self._add(lambda s: rt.check(
-            L.esf_head_fc(feat.data_ptr(), B, cin, cin, w.data_ptr(), b.data_ptr(), K, act, out.data_ptr(), K, s),
-            "esf_head_fc"), "head_fc", "", flops=2.0 * B * cin * K, nbytes=self._nbytes(feat, w, out),
-            launches=head_fc_launches(B, cin, K, act))
+        self._head_pool(xs, feat)
+        self._head_fc(feat, w, b, act, out, flops=2.0 * B * cin * K, nbytes=self._nbytes(feat, w, out))
         self.out = out
         return out
+
+    def _head_pool(self, xs, feat):
+        """feat = the global means of the one or two pathways `xs`, concatenated."""
+        self._launch("esf_head_pool", xs[0], xs[1] if len(xs) > 1 else None, feat, kind="head_pool",
+                     nbytes=self._nbytes(*xs), launches=len(xs))
 
     def head_positions(self, xs, pool_sizes, weight, bias, act):
         """ResNetBasicHead.forward, eval branch, general case (head_helper.py:198-223): per-pathway AvgPool3d(kernel,
         stride 1) leaves P = T' * H' * W' positions; Linear + activation at every position, mean over the positions."""
-        B = xs[0].shape[0]
         pooled = []
         for x, ps in zip(xs, pool_sizes):
-            _, T, H, W, C = x.shape
+            B, T, H, W, C = x.shape
             kt, kh, kw = [int(v) for v in ps]
-            y = self.act(B, T - kt + 1, H - kh + 1, W - kw + 1, C)
-            self.pool(x, y, (kt, kh, kw), (1, 1, 1), (0, 0, 0), is_avg=True)
-            pooled.append(y)
+            pooled.append(self._head_avg_pool(x, (kt, kh, kw), (B, T - kt + 1, H - kh + 1, W - kw + 1, C)))
         return self.positions_head(pooled, weight, bias, act)
+
+    def _head_avg_pool(self, x, kernel, shape):
+        """AvgPool3d(kernel, stride 1) of head_positions into a new activation of `shape`."""
+        y = self.act(*shape)
+        self.pool(x, y, kernel, (1, 1, 1), (0, 0, 0), is_avg=True)
+        return y
 
     def positions_head(self, pooled, weight, bias, act):
         """Second half of head_positions: Linear + activation at every position of the pooled maps (B, T', H', W', C)
@@ -800,10 +798,8 @@ class Plan:
         per_pos = self.head(rows, weight, bias, act)
         K = weight.shape[0]
         out = torch.empty((B, K), dtype=torch.float32, device=self.device)
-        self.keep += [out]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_group_mean(per_pos.data_ptr(), B, P, K, out.data_ptr(), s), "esf_group_mean"),
-                  "head_mean", "P=%d" % P, nbytes=self._nbytes(per_pos, out))
+        self._launch("esf_group_mean", per_pos, B, P, K, out, kind="head_mean", label="P=%d" % P,
+                     nbytes=self._nbytes(per_pos, out))
         self.out = out
         return out
 
@@ -814,26 +810,13 @@ class Plan:
         K = weight.shape[0]
         feat = torch.empty((B, C), dtype=torch.float32, device=self.device)
         w, b = self.tensor(weight.reshape(K, C)), self.tensor(bias)
-        xv, nv = rt.view(x), rt.null_view()
-        self.keep += [feat, xv, nv, out]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_head_pool(ctypes.byref(xv), ctypes.byref(nv), feat.data_ptr(), s),
-                                     "esf_head_pool"), "head_pool", "", nbytes=self._nbytes(x))
-        self._add(lambda s: rt.check(L.esf_head_fc(feat.data_ptr(), B, C, C, w.data_ptr(), b.data_ptr(), K, act,
-                                                   out.data_ptr(), out_stride, s), "esf_head_fc"), "head_fc", "",
-                  launches=head_fc_launches(B, C, K, act))
+        self._head_pool([x], feat)
+        self._head_fc(feat, w, b, act, out, out_stride)
 
     def fc(self, feat, weight, bias, act):
         """out = act(feat @ weight^T + bias) on FP32 rows (final classifier of the GhostNet head)."""
-        B, cin = feat.shape
-        K = weight.shape[0]
-        out = torch.empty((B, K), dtype=torch.float32, device=self.device)
-        w, b = self.tensor(weight), self.tensor(bias)
-        self.keep += [out, feat]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_head_fc(feat.data_ptr(), B, cin, cin, w.data_ptr(), b.data_ptr(), K, act,
-                                                   out.data_ptr(), K, s), "esf_head_fc"), "head_fc", "",
-                  launches=head_fc_launches(B, cin, K, act))
+        out = torch.empty((feat.shape[0], weight.shape[0]), dtype=torch.float32, device=self.device)
+        self._head_fc(feat, self.tensor(weight), self.tensor(bias), act, out)
         self.out = out
         return out
 
@@ -842,11 +825,8 @@ class Plan:
         (B, H, W, C) map, the input of esf_roi_align_max.  A graph op: it reads plan-owned activations only."""
         B, T, H, W, C = x.shape
         y = torch.empty((B, H, W, C), dtype=torch.float32, device=self.device)
-        xv = rt.view(x)
-        self.keep += [y, xv]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_temporal_mean(ctypes.byref(xv), y.data_ptr(), s), "esf_temporal_mean"),
-                  "roi_tpool", "T=%d C=%d @%s" % (T, C, (H, W)), nbytes=self._nbytes(x, y))
+        self._launch("esf_temporal_mean", x, y, kind="roi_tpool", label="T=%d C=%d @%s" % (T, C, (H, W)),
+                     nbytes=self._nbytes(x, y))
         return y
 
     def roi_head(self, maps, spatial_scales, resolutions, aligned, weight, bias, act):

@@ -20,13 +20,10 @@ Slow), grouped bottlenecks, Non-local blocks (also with temporal groups), any at
 fully-convolutional test head.  Depthwise convolutions (the efficient backbones) and the detection head are not covered.
 About 3x the tensor-core work and ~5x the activation bytes of the FP16 plan: an accuracy mode, benchmarked beside it.
 """
-import ctypes
-
 import torch
 
 from . import runtime as rt
-from .engine import (Plan, attention_projection, block_diagonal, bn_affine, fold_conv_bn, fold_time_groups, host64,
-                     stem_route)
+from .engine import Plan, block_diagonal, fold_conv_bn, fold_time_groups, stem_route
 
 
 class Act32:
@@ -64,6 +61,11 @@ class Act32:
     def need_f32(self, who):
         assert self.has_f32, "%s reads the FP32 copy of an activation that was planned without one" % who
         return self.f32
+
+    def fold_time_groups(self, group):
+        """engine.fold_time_groups of the FP32 tensor and of the planes."""
+        return Act32(fold_time_groups(self.f32, group), fold_time_groups(self.x3, group) if self.has_planes else None,
+                     self.plane, self.c0, self.c_total, self.weight_order, self.has_f32, self.has_planes)
 
 
 def split_weight_rows(w):
@@ -106,25 +108,18 @@ class PrecisePlan(Plan):
 
     def _post(self, acc, y, scale=None, bias=None, res=None, act=rt.ACT_NONE, label=""):
         """esf_p32_post: y.f32 = act(acc * scale + bias + res) and its three FP16 planes (y: Act32 or FP32 tensor)."""
-        L = rt.lib()
-        av = rt.view(acc)
-        rv = rt.view(res.need_f32("a residual add") if isinstance(res, Act32) else res) if res is not None else rt.null_view()
+        if isinstance(res, Act32):
+            res = res.need_f32("a residual add")
         if isinstance(y, Act32):
             in_place = y.has_f32 and y.f32.data_ptr() == acc.data_ptr() and scale is None and bias is None and \
                 res is None and act == rt.ACT_NONE
-            y32 = rt.null_view() if (in_place or not y.has_f32) else rt.view(y.f32)
-            y3, plane = (rt.view(y.hi) if y.has_planes else rt.null_view()), y.plane
-            worder = int(y.weight_order)
+            y32 = None if (in_place or not y.has_f32) else y.f32
+            y3, plane, worder = (y.hi if y.has_planes else None), y.plane, int(y.weight_order)
         else:
-            y32, y3, plane, worder = rt.view(y), rt.null_view(), 0, 0
-        sc = scale.data_ptr() if scale is not None else None
-        bs = bias.data_ptr() if bias is not None else None
-        self.keep += [av, rv, y32, y3, scale, bias]
-        n = acc.numel()
-        self._add(lambda s: rt.check(L.esf_p32_post(ctypes.byref(av), sc, bs, ctypes.byref(rv), act, ctypes.byref(y32),
-                                                    ctypes.byref(y3), plane, worder, s), "esf_p32_post"),
-                  "p32_post", label, nbytes=n * (4 + (4 if res is not None else 0) + (4 if y32.ptr else 0) +
-                                                  (6 if y3.ptr else 0)))
+            y32, y3, plane, worder = y, None, 0, 0
+        self._launch("esf_p32_post", acc, scale, bias, res, act, y32, y3, plane, worder, kind="p32_post", label=label,
+                     nbytes=acc.numel() * (4 + (4 if res is not None else 0) + (4 if y32 is not None else 0) +
+                                           (6 if y3 is not None else 0)))
 
     # ---------------------------------------------------------------- ops
     def conv(self, x, y, w_folded, bias, stride=(1, 1, 1), padding=(0, 0, 0), dilation=(1, 1, 1), groups=1,
@@ -172,31 +167,25 @@ class PrecisePlan(Plan):
         pitch, lpad, twb = route
         B, Cin, T, H, W = x_nc.shape
         cout = w_folded.shape[0]
-        L = rt.lib()
         hi, lo, inv_scale = split_weight_rows(w_folded.to(torch.float64))
         zero = torch.zeros(cout, dtype=torch.float64)
+
+        def pack(fn_name, xp):      # reads the caller's clip: its pointer is looked up at launch time
+            return lambda s: self._call(fn_name, self._in_ptr(x_nc), B, Cin, T, H, W, pitch, lpad, rt.F16, xp.data_ptr(), s)
+
         xps, accs = [], []
-        for part in range(2):
+        for fn_name, part in (("esf_stem_pack", "hi"), ("esf_stem_pack_lo", "lo")):
             xp = torch.empty((B, T, H, pitch), dtype=torch.float16, device=self.device)
             self.keep.append(xp)
-            fn = L.esf_stem_pack_lo if part else L.esf_stem_pack
-            self._add(lambda s, xp=xp, fn=fn: rt.check(fn(self._in_ptr(x_nc), B, Cin, T, H, W, pitch, lpad, rt.F16,
-                                                          xp.data_ptr(), s), "esf_stem_pack"),
-                      "stem_pack", "lo" if part else "hi", nbytes=self._nbytes(x_nc, xp), eager=True)
+            self._add(pack(fn_name, xp), "stem_pack", part, nbytes=self._nbytes(x_nc, xp), eager=True)
             xps.append(xp)
         for name, xp, wpart in (("hi.hi", xps[0], hi), ("lo.hi", xps[1], hi), ("hi.lo", xps[0], lo)):
             acc = torch.empty(tuple(y.shape), dtype=torch.float32, device=self.device)
             self.keep.append(acc)
             self._stem_gemm_op(xp, x_nc.shape, acc, wpart, zero, stride, padding, rt.ACT_NONE, pitch, twb, name)
             accs.append(acc)
-        sc, bs = self.tensor(inv_scale), self.tensor(bias)
-        avs = [rt.view(a) for a in accs]
-        y32, y3 = rt.view(y.f32), rt.view(y.hi)
-        self.keep += avs + [y32, y3]
-        self._add(lambda s: rt.check(L.esf_p32_post3(ctypes.byref(avs[0]), ctypes.byref(avs[1]), ctypes.byref(avs[2]),
-                                                     sc.data_ptr(), bs.data_ptr(), act, ctypes.byref(y32),
-                                                     ctypes.byref(y3), y.plane, s), "esf_p32_post3"),
-                  "p32_post", "stem sum", nbytes=accs[0].numel() * (12 + 4 + 6))
+        self._launch("esf_p32_post3", *accs, self.tensor(inv_scale), self.tensor(bias), act, y.f32, y.hi, y.plane,
+                     kind="p32_post", label="stem sum", nbytes=accs[0].numel() * (12 + 4 + 6))
 
     def pool(self, x, y, kernel, stride, padding, is_avg=False, act=rt.ACT_NONE):
         assert act == rt.ACT_NONE
@@ -205,27 +194,12 @@ class PrecisePlan(Plan):
 
     def _pool32(self, x, y, kernel, stride, padding, is_avg):
         """esf_p32_pool3d between two FP32 tensors."""
-        xv, yv = rt.view(x), rt.view(y)
-        self.keep += [xv, yv]
-        L = rt.lib()
-        self._add(lambda s: rt.check(L.esf_p32_pool3d(ctypes.byref(xv), ctypes.byref(yv), *kernel, *stride, *padding,
-                                                      int(is_avg), s), "esf_p32_pool3d"),
-                  "p32_pool", "%s C=%d" % (tuple(kernel), x.shape[4]), nbytes=self._nbytes(x, y))
+        self._launch("esf_p32_pool3d", x, y, *kernel, *stride, *padding, int(is_avg), kind="p32_pool",
+                     label="%s C=%d" % (tuple(kernel), x.shape[4]), nbytes=self._nbytes(x, y))
 
     def eca_fuse(self, x_fast, y_slice, alpha, eca_weight, bn):
-        scale, shift = bn_affine(bn)
-        w = self.tensor(host64(eca_weight).reshape(-1))
-        sc, sh = self.tensor(scale), self.tensor(shift)
-        B, C = x_fast.shape[0], x_fast.shape[4]
-        L = rt.lib()
-        scratch = torch.empty(int(L.esf_p32_eca_scratch_floats(B, C)), dtype=torch.float32, device=self.device)
-        xv, yv = rt.view(x_fast.f32), rt.view(y_slice.f32)
-        self.keep += [scratch, xv, yv]
-        k = int(w.numel())
-        self._add(lambda s: rt.check(
-            L.esf_p32_eca_fuse(ctypes.byref(xv), alpha, w.data_ptr(), k, sc.data_ptr(), sh.data_ptr(),
-                               scratch.data_ptr(), ctypes.byref(yv), s), "esf_p32_eca_fuse"), "p32_eca_fuse",
-            "C=%d" % C, nbytes=2 * self._nbytes(x_fast.f32) + self._nbytes(y_slice.f32), launches=2)
+        self._eca_fuse("esf_p32_eca_fuse", "esf_p32_eca_scratch_floats", "p32_eca_fuse", x_fast.f32, y_slice.f32, alpha,
+                       eca_weight, bn)
         self._post(y_slice.f32, y_slice, label="split")
 
     def position_attention(self, x_slow, y_slice, alpha, w_down, att, bn):
@@ -233,95 +207,48 @@ class PrecisePlan(Plan):
         attention kernel writes FP32 into the concat slice, which is then split into planes.  Any head dim: the split
         tensor-core kernel up to d = 64 (its geometry pads d like the 16-bit kernel's), FP32 flash attention on the CUDA
         cores up to 128, the generic FP32 CUDA-core kernel of the 16-bit plan above."""
-        B, T, H, W, C = x_slow.shape
-        w_all, b_all, d = attention_projection(w_down, att)
-        proj = super().act(B, T, H, W, 4 * d, dtype=torch.float32)
-        self.conv(x_slow, proj, w_all, b_all)
-        L = rt.lib()
+        proj, geo = self._attention_operands(x_slow, alpha, w_down, att, bn)
+        B, T, H, W, d = geo[:5]
         N = T * H * W
-        scale, shift = bn_affine(bn)
-        sc, sh = self.tensor(scale), self.tensor(shift)
-        gamma = float(att.gamma.detach().float().item())
-        yv = rt.view(y_slice.f32)
-        self.keep.append(yv)
+        y = y_slice.f32
         if d <= 64:
             # tensor cores at FP32 accuracy: the logits are hi/lo split already; P and V become FP16 pairs too
             # (esf_attn_tc_create_split: O += P_hi V_hi + P_lo V_hi + P_hi V_lo, row sums in FP32 registers)
-            nbytes = int(L.esf_attn_tc_pack_bytes(B, N, d))
-            nlo = int(L.esf_attn_tc_vlo_bytes(B, N, d))
-            if nbytes < 0 or nlo < 0:
-                rt.check(min(nbytes, nlo), "esf_attn_tc_pack_bytes")
+            nbytes = self._size("esf_attn_tc_pack_bytes", B, N, d)
+            nlo = self._size("esf_attn_tc_vlo_bytes", B, N, d)
             packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
             vlo = torch.empty(nlo, dtype=torch.uint8, device=self.device)
-            self.keep += [packed, vlo]
-            h = ctypes.c_void_p()
-            rt.check(L.esf_attn_tc_create_split(packed.data_ptr(), vlo.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(),
-                                                sh.data_ptr(), alpha, ctypes.byref(yv), ctypes.byref(h)),
-                     "esf_attn_tc_create_split")
-            self.handles.append(h)
-
-            def pack(s):
-                rt.check(L.esf_attn_tc_pack(proj.data_ptr(), B, N, d, rt.F16, packed.data_ptr(), s), "esf_attn_tc_pack")
-                rt.check(L.esf_attn_tc_pack_vlo(proj.data_ptr(), B, N, d, vlo.data_ptr(), s), "esf_attn_tc_pack_vlo")
-
-            self._add(pack, "attn_pack", "N=%d d=%d split" % (N, d), nbytes=self._nbytes(proj) + nbytes + nlo, launches=2)
-            self._add(lambda s, h=h: rt.check(L.esf_op_launch(h, s), "esf_op_launch"), "attention",
-                      "N=%d d=%d split" % (N, d), flops=8.0 * B * N * N * d, exps=float(B) * N * N,
-                      nbytes=nbytes + nlo + self._nbytes(y_slice.f32))
+            h = self._create("esf_attn_tc_create_split", packed, vlo, *geo, y)
+            pack = self._bind("esf_attn_tc_pack", proj, B, N, d, rt.F16, packed)
+            pack_vlo = self._bind("esf_attn_tc_pack_vlo", proj, B, N, d, vlo)
+            self._add(lambda s: (pack(s), pack_vlo(s)), "attn_pack", "N=%d d=%d split" % (N, d),
+                      nbytes=self._nbytes(proj) + nbytes + nlo, launches=2)
+            self._launch("esf_op_launch", h, kind="attention", label="N=%d d=%d split" % (N, d),
+                         flops=8.0 * B * N * N * d, exps=float(B) * N * N, nbytes=nbytes + nlo + self._nbytes(y))
         elif d <= 128:
             # d in (64, 128] has no hi/lo logit split on the tensor cores (the split Q tile does not fit in shared
             # memory): FP32 flash attention on the CUDA cores (d = 128: N = 1 568 there)
-            self._add(lambda s: rt.check(
-                L.esf_p32_attention(proj.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                                    ctypes.byref(yv), s), "esf_p32_attention"), "p32_attention", "N=%d d=%d" % (N, d),
-                flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj) + self._nbytes(y_slice.f32))
+            self._launch("esf_p32_attention", proj, *geo, y, kind="p32_attention", label="N=%d d=%d" % (N, d),
+                         flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj, y))
         else:
-            self._add(lambda s: rt.check(
-                L.esf_attn_generic(proj.data_ptr(), B, T, H, W, d, gamma, sc.data_ptr(), sh.data_ptr(), alpha,
-                                   ctypes.byref(yv), s), "esf_attn_generic"), "attention", "N=%d d=%d generic" % (N, d),
-                flops=4.0 * B * N * N * d, exps=float(B) * N * N, nbytes=self._nbytes(proj) + self._nbytes(y_slice.f32))
-        self._post(y_slice.f32, y_slice, label="split")
+            self._attention_generic(proj, geo, y)
+        self._post(y, y_slice, label="split")
 
-    def head(self, xs, weight, bias, act):
-        """xs: Act32 activations, or plain FP32 tensors (the pooled rows of positions_head)."""
-        xs = [x.f32 if isinstance(x, Act32) else x for x in xs]
-        B = xs[0].shape[0]
-        cin = sum(x.shape[4] for x in xs)
-        K = weight.shape[0]
-        feat = torch.empty((B, cin), dtype=torch.float32, device=self.device)
-        out = torch.empty((B, K), dtype=torch.float32, device=self.device)
-        w, b = self.tensor(weight), self.tensor(bias)
-        self.keep += [feat, out]
-        L = rt.lib()
+    def _head_pool(self, xs, feat):
+        """xs: Act32 activations, or plain FP32 tensors (the pooled rows of positions_head): one esf_p32_head_pool per
+        pathway into its slice of feat."""
         off = 0
         for x in xs:
-            xv = rt.view(x)
-            self.keep.append(xv)
-            self._add(lambda s, xv=xv, off=off: rt.check(L.esf_p32_head_pool(ctypes.byref(xv), feat.data_ptr(), cin, off, s),
-                                                         "esf_p32_head_pool"), "p32_head_pool", "",
-                      nbytes=self._nbytes(x))
+            x = x.f32 if isinstance(x, Act32) else x
+            self._launch("esf_p32_head_pool", x, feat, feat.shape[1], off, kind="p32_head_pool", nbytes=self._nbytes(x))
             off += x.shape[4]
-        from .engine import head_fc_launches
-        self._add(lambda s: rt.check(
-            L.esf_head_fc(feat.data_ptr(), B, cin, cin, w.data_ptr(), b.data_ptr(), K, act, out.data_ptr(), K, s),
-            "esf_head_fc"), "head_fc", "", flops=2.0 * B * cin * K, nbytes=self._nbytes(feat, w, out),
-            launches=head_fc_launches(B, cin, K, act))
-        self.out = out
-        return out
 
-    def head_positions(self, xs, pool_sizes, weight, bias, act):
-        """Plan.head_positions on the FP32 tensors: AvgPool3d(kernel, stride 1) of every pathway into a plain FP32
-        buffer (nothing multiplies it on the tensor cores, so it gets no planes), then the shared positions_head --
-        Linear + activation at every position (esf_p32_head_pool of a one-position row is a copy) and their mean."""
-        pooled = []
-        for x, ps in zip(xs, pool_sizes):
-            B, T, H, W, C = x.shape
-            kt, kh, kw = [int(v) for v in ps]
-            y = torch.empty((B, T - kt + 1, H - kh + 1, W - kw + 1, C), dtype=torch.float32, device=self.device)
-            self.keep.append(y)
-            self._pool32(x.need_f32("the head"), y, (kt, kh, kw), (1, 1, 1), (0, 0, 0), is_avg=True)
-            pooled.append(y)
-        return self.positions_head(pooled, weight, bias, act)
+    def _head_avg_pool(self, x, kernel, shape):
+        """The head's AvgPool3d into a plain FP32 buffer: nothing multiplies it on the tensor cores, so it gets no
+        planes (esf_p32_head_pool of its one-position rows in positions_head is a copy)."""
+        y = super().act(*shape, dtype=torch.float32)
+        self._pool32(x.need_f32("the head"), y, kernel, (1, 1, 1), (0, 0, 0), is_avg=True)
+        return y
 
     def nonlocal_block(self, x, y, nln, group=1):
         """Nonlocal.forward (nonlocal_helper.py:105-148) at FP32 accuracy: theta / phi / g / out are split-operand convs;
@@ -331,27 +258,14 @@ class PrecisePlan(Plan):
         accuracy mode.)  NONLOCAL.GROUP > 1: the (b, t) -> (b * group, t / group) view of Plan.nonlocal_block, applied to
         the FP32 tensor and to the planes of x and y."""
         if group > 1:
-            x, y = (Act32(fold_time_groups(a.f32, group), fold_time_groups(a.x3, group) if a.has_planes else None,
-                          a.plane, a.c0, a.c_total, a.weight_order, a.has_f32, a.has_planes) for a in (x, y))
-        L = rt.lib()
+            x, y = x.fold_time_groups(group), y.fold_time_groups(group)
         B, T, H, W, C = x.shape
         d = nln.dim_inner
         dp = (d + 7) // 8 * 8
-
-        def wb(conv):
-            return host64(conv.weight), host64(conv.bias)
-
-        if nln.use_pool:
-            ps = [int(v) for v in nln.pool_size]
-            Tp, Hp, Wp = (T - ps[0]) // ps[0] + 1, (H - ps[1]) // ps[1] + 1, (W - ps[2]) // ps[2] + 1
-            xp = self.act(B, Tp, Hp, Wp, C)
-            self.pool(x, xp, tuple(ps), tuple(ps), (0, 0, 0))
-        else:
-            Tp, Hp, Wp, xp = T, H, W, x
+        xp, softmax = self._nonlocal_keys(x, nln)
+        Tp, Hp, Wp = xp.shape[1:4]
         Nq, Nk = T * H * W, Tp * Hp * Wp
-        softmax = nln.instantiation == "softmax"
-        if not softmax and nln.instantiation != "dot_product":
-            raise NotImplementedError("Unknown norm type {}".format(nln.instantiation))
+        wb = self._weight_bias
         theta = self.act(B, T, H, W, d)
         self.conv(x, theta, *wb(nln.conv_theta))
         # phi rows of a clip ARE the [n][k] weight matrix of theta^T phi (k = the 3 d plane channels): allocate them
@@ -376,20 +290,17 @@ class PrecisePlan(Plan):
         nkp = (Nk + 7) // 8 * 8
         P3 = self.scratch((B, T, H, W, 3 * nkp), torch.float16, zero=True)
         scale, mode = (float(d) ** -0.5, 0) if softmax else (1.0 / Nk, 1)
-        self._add(lambda s: rt.check(L.esf_p32_row_softmax(S.data_ptr(), B * Nq, Nk, S.shape[4], scale, mode, P3.data_ptr(),
-                                                           3 * nkp, nkp, s), "esf_p32_row_softmax"),
-                  "p32_nl_softmax", nln.instantiation, nbytes=B * Nq * Nk * 10.0, exps=float(B * Nq * Nk))
+        self._launch("esf_p32_row_softmax", S, B * Nq, Nk, S.shape[4], scale, mode, P3, 3 * nkp, nkp,
+                     kind="p32_nl_softmax", label=nln.instantiation, nbytes=B * Nq * Nk * 10.0, exps=float(B * Nq * Nk))
         # g^T in weight order: gT3[b][c][plane * nkp + k] = plane(g)[b, k, c], planes (hi, hi, lo)
         kc2, kch2, _, npad2 = rt.igemm_geometry(3 * nkp, d)
         kpad = kc2 * kch2
         gT3 = torch.zeros((B, npad2, kpad), dtype=torch.float16, device=self.device)
         self.keep.append(gT3)
         for pl in range(3):
-            src = g_x3.data_ptr() + 2 * pl * dp
-            dst = gT3.data_ptr() + 2 * pl * nkp
-            self._add(lambda s, src=src, dst=dst: rt.check(
-                L.esf_transpose16(src, B, Nk, d, Nk * 3 * dp, 3 * dp, dst, npad2 * kpad, kpad, s), "esf_transpose16"),
-                "nl_transpose", "g plane %d" % pl, nbytes=4.0 * B * Nk * d)
+            self._launch("esf_transpose16", g_x3.data_ptr() + 2 * pl * dp, B, Nk, d, Nk * 3 * dp, 3 * dp,
+                         gT3.data_ptr() + 2 * pl * nkp, npad2 * kpad, kpad, kind="nl_transpose", label="g plane %d" % pl,
+                         nbytes=4.0 * B * Nk * d)
         att = self.act(B, T, H, W, d)
         acc = self.scratch((B, T, H, W, d), torch.float32)
         zero2 = self.scratch((npad2,), torch.float32, zero=True)

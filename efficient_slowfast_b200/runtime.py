@@ -61,7 +61,6 @@ def lib():
     P = ctypes.POINTER
     L.esf_last_error.restype = ctypes.c_char_p
     L.esf_last_error.argtypes = []
-    L.esf_version.restype = ctypes.c_int
     L.esf_launch_count.restype = i64
     L.esf_igemm_geometry.argtypes = [i32, i32, P(i32), P(i32), P(i32), P(i32)]
     L.esf_conv_igemm_create.argtypes = [P(EsfConvDesc), P(vp)]
@@ -76,7 +75,6 @@ def lib():
     L.esf_stem_geometry.argtypes = [i32, i32, i32, i32, i32, P(i32), P(i32), P(i32)]
     L.esf_stem_pack.argtypes = [vp, i32, i32, i32, i32, i32, i32, i32, i32, vp, vp]
     L.esf_stem_pack_gather.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, i32, i32, i32, vp, vp]
-    i64 = ctypes.c_int64
     L.esf_row_softmax.argtypes = [vp, i64, i32, i64, f32, i32, i32, vp, i64, vp]
     L.esf_transpose16.argtypes = [vp, i32, i32, i32, i64, i64, vp, i64, i64, vp]
     L.esf_global_mean_scratch_floats.argtypes = [i32, i32]
@@ -125,10 +123,6 @@ def lib():
     L.esf_p32_eca_fuse.argtypes = [P(EsfView), i32, vp, i32, vp, vp, vp, P(EsfView), vp]
     L.esf_p32_head_pool.argtypes = [P(EsfView), vp, i32, i32, vp]
     L.esf_p32_attention.argtypes = [vp, i32, i32, i32, i32, i32, f32, vp, vp, i32, P(EsfView), vp]
-    for name in ("esf_stem_pack_u8_crop", "esf_frames_to_clip_crop", "esf_temporal_mean", "esf_roi_align_max", "esf_stem_tband_create", "esf_stem_tband_wb", "esf_p32_post3", "esf_stem_pack_lo", "esf_attn_tc_pack_vlo", "esf_attn_tc_create_split", "esf_p32_row_softmax", "esf_p32_attention", "esf_p32_post", "esf_p32_pool3d", "esf_p32_eca_fuse", "esf_p32_head_pool", "esf_stem_pack_gather", "esf_dwconv_padded", "esf_pointwise_padded", "esf_global_mean", "esf_gemm_clip_weights_create", "esf_group_mean", "esf_row_softmax", "esf_transpose16", "esf_stem_pack_u8", "esf_frames_to_clip", "esf_attn_generic", "esf_shuffle_concat", "esf_eltwise_add", "esf_channel_scale", "esf_attn_tc_pack", "esf_attn_tc_create", "esf_stem_geometry", "esf_stem_pack", "esf_stem_igemm_create", "esf_igemm_geometry",
-                 "esf_conv_igemm_create", "esf_conv_wfold_create", "esf_op_launch", "esf_conv_direct", "esf_stem_conv",
-                 "esf_pool3d", "esf_eca_fuse", "esf_head_pool", "esf_head_fc"):
-        getattr(L, name).restype = ctypes.c_int
     _LIB = L
     return L
 

@@ -10,10 +10,46 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _declared_symbols():
+def _header():
     src = open(os.path.join(ROOT, "include", "esf.h")).read()
-    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
-    return sorted(set(re.findall(r"\b(esf_[a-z0-9_]+)\s*\(", src)))
+    return re.sub(r"/\*.*?\*/", "", src, flags=re.S)
+
+
+def _declared_symbols():
+    return sorted(set(re.findall(r"\b(esf_[a-z0-9_]+)\s*\(", _header())))
+
+
+def _declarations():
+    """{name: (return type, [(parameter type, parameter name)])} of every function include/esf.h declares."""
+    decls = {}
+    for ret, name, params in re.findall(r"((?:const\s+)?\w+\s*\**)\s*\b(esf_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", _header()):
+        args = []
+        for p in params.split(","):
+            p = " ".join(p.split())
+            if p and p != "void":
+                ctype, pname = re.match(r"(.*?)\s*(\w+)$", p).groups()
+                args.append((ctype, pname))
+        decls[name] = (ret.replace(" ", ""), args)
+    return decls
+
+
+def _ctypes_of(ctype, pname):
+    """The ctypes type the binding must give a parameter of C type `ctype`."""
+    from efficient_slowfast_b200 import runtime as rt
+
+    base = ctype.replace("const", "").replace(" ", "")
+    if base == "esf_view*":
+        return ctypes.POINTER(rt.EsfView)
+    if base == "esf_conv_desc*":
+        return ctypes.POINTER(rt.EsfConvDesc)
+    if base == "esf_op**":
+        return ctypes.POINTER(ctypes.c_void_p)
+    # int32_t* out-parameters and the host int32 tables (esf.h: a name ending in _host, and chan_src "host int32[C]")
+    if base == "int32_t*" and ("const" not in ctype or pname.endswith("_host") or pname == "chan_src"):
+        return ctypes.POINTER(ctypes.c_int32)
+    if base.endswith("*"):
+        return ctypes.c_void_p       # device pointers, esf_op*, the stream
+    return {"int32_t": ctypes.c_int32, "int64_t": ctypes.c_int64, "float": ctypes.c_float}[base]
 
 
 def test_header_symbols_exported(esf_lib):
@@ -22,6 +58,24 @@ def test_header_symbols_exported(esf_lib):
     for s in syms:
         assert hasattr(esf_lib, s), "libesf_b200.so does not export %s" % s
     assert esf_lib.esf_version() >= 100
+
+
+def test_binding_signatures_match_header(esf_lib):
+    """runtime.lib()'s argtypes / restype are the Python side's only description of the C ABI, and Plan._bind converts
+    arguments by them: every function include/esf.h declares has its parameters' kinds, in order."""
+    decls = _declarations()
+    assert set(decls) == set(_declared_symbols())
+    restypes = {"int": ctypes.c_int, "int64_t": ctypes.c_int64, "constchar*": ctypes.c_char_p, "void": None}
+    for name, (ret, params) in sorted(decls.items()):
+        f = getattr(esf_lib, name)
+        assert f.restype is restypes[ret], "%s returns %s, bound as %s" % (name, ret, f.restype)
+        if not params and f.argtypes is None:
+            continue
+        assert f.argtypes is not None, "%s has no argtypes" % name
+        assert len(f.argtypes) == len(params), "%s: %d argtypes for %d parameters" % (name, len(f.argtypes), len(params))
+        for i, ((ctype, pname), got) in enumerate(zip(params, f.argtypes)):
+            want = _ctypes_of(ctype, pname)
+            assert got is want, "%s parameter %d (%s %s): bound as %s, expected %s" % (name, i, ctype, pname, got, want)
 
 
 def test_geometry_rule(esf_lib):
