@@ -15,6 +15,14 @@
 // Work split.  One block per (clip, output frame, output row y); it loops over the V views.  Views along the long axis of a
 // landscape clip share the resized row, hence the two source rows: those are read once (16-byte loads into shared memory)
 // and all V crops of the row are emitted from them.  Portrait clips crop along y, so each view reloads its own rows.
+//
+// Mixed decode sizes (esf_*_crop_ragged).  A test split mixes resolutions and aspect ratios, but every clip's output is
+// the same V x (C, T, S, S); only the source geometry differs.  Each clip brings its own source address, (H0, W0),
+// resized size, axis tables and crop offsets (CropClip), and the geometry of up to kCropChunk clips travels by value in
+// the kernel parameters of one launch (CropChunk, inside the classic 4 KB parameter block): a call uploads nothing,
+// allocates nothing and keeps no host array past its return.  The work split is the uniform kernel's; a block reads
+// its clip's entry and takes the resize or the pure-window path for that clip (a block-uniform branch).  Both kernels
+// run the same row loads and emission loop (crop_rows).
 #include <algorithm>
 
 #include "esf_common.cuh"
@@ -25,20 +33,40 @@ namespace esf {
 constexpr int kCropThreads = 256;
 constexpr int kCropMaxViews = 8;
 constexpr int kCropMaxRowBytes = 16384;  // W0 * C of one source row (two rows live in shared memory)
+constexpr int kCropChunk = 32;           // clips of one ragged launch (their geometry is in the parameter block)
 
-struct CropParams {
-  const uint8_t* frames;  // (B, Tsrc, H0, W0, C)
-  const int32_t* t_index;
-  int B, Tsrc, T, H0, W0, C;
-  int chan_src[4];
-  const float* lut;       // [C][256] normalised value of byte u in OUTPUT channel c
+// Source geometry of one clip.
+struct CropClip {
+  const uint8_t* frames;  // (Tsrc, H0, W0, C); in a uniform batch that of clip 0, clip b following at b * Tsrc * H0 * W0 * C
   const int32_t* y_idx;   // [Hr][2] source rows (i0, i1) of every resized row
   const float* y_wt;      // [Hr][2] (l0, l1)
   const int32_t* x_idx;   // [Wr][2]
   const float* x_wt;      // [Wr][2]
-  int Hr, Wr, S, V;
+  int H0, W0, Hr, Wr;
   int y0[kCropMaxViews], x0[kCropMaxViews];
 };
+
+// What every clip of a call shares.
+struct CropShared {
+  const int32_t* t_index;
+  const float* lut;       // [C][256] normalised value of byte u in OUTPUT channel c
+  int Tsrc, T, C, S, V;
+  int chan_src[4];
+};
+
+struct CropParams {       // B clips of one geometry
+  CropShared s;
+  CropClip g;
+  int B;
+};
+
+struct CropChunk {        // up to kCropChunk clips of their own geometry; g[i] is output clip clip0 + i
+  CropShared s;
+  int clip0;
+  CropClip g[kCropChunk];
+};
+// + the kernel's other parameters (pitch, lpad, f16, out)
+static_assert(sizeof(CropChunk) + 3 * sizeof(int) + sizeof(void*) + 8 <= 4096, "CropChunk must fit the 4 KB parameters");
 
 // copy bytes [src, src + n) into shared memory at dst + (src & 15), i.e. with the source's 16-byte phase, so that the
 // aligned body moves as 16-byte loads and stores and only the ragged ends go byte by byte; returns the row's start
@@ -57,44 +85,45 @@ __device__ __forceinline__ const uint8_t* load_row_bytes(uint8_t* dst, const uin
 
 // One output value of the view at resized column xr, output channel c (source channel cs), rows r0 / r1 in shared memory.
 template <bool RESIZE>
-__device__ __forceinline__ float crop_value(const CropParams& p, const uint8_t* r0, const uint8_t* r1, const float* lut_s,
-                                            int xr, int c, int cs, float l0, float l1) {
+__device__ __forceinline__ float crop_value(const CropClip& g, int C, const uint8_t* r0, const uint8_t* r1,
+                                            const float* lut_s, int xr, int c, int cs, float l0, float l1) {
   const float* lc = lut_s + c * 256;
-  if (!RESIZE) return lc[r0[xr * p.C + cs]];
-  const int2 xi = __ldg(reinterpret_cast<const int2*>(p.x_idx) + xr);
-  const float2 xw = __ldg(reinterpret_cast<const float2*>(p.x_wt) + xr);
-  const int a = min(max(xi.x, 0), p.W0 - 1) * p.C + cs, b = min(max(xi.y, 0), p.W0 - 1) * p.C + cs;
+  if (!RESIZE) return lc[r0[xr * C + cs]];
+  const int2 xi = __ldg(reinterpret_cast<const int2*>(g.x_idx) + xr);
+  const float2 xw = __ldg(reinterpret_cast<const float2*>(g.x_wt) + xr);
+  const int a = min(max(xi.x, 0), g.W0 - 1) * C + cs, b = min(max(xi.y, 0), g.W0 - 1) * C + cs;
   const float t0 = __fmaf_rn(lc[r0[a]], xw.x, __fmul_rn(lc[r0[b]], xw.y));
   const float t1 = __fmaf_rn(lc[r1[a]], xw.x, __fmul_rn(lc[r1[b]], xw.y));
   return __fmaf_rn(t0, l0, __fmul_rn(t1, l1));
 }
 
+// The block's (clip, output frame, output row) and the source frame of that output frame.
+__device__ __forceinline__ void crop_block(const CropShared& s, int& b, int& t, int& y, int& ts) {
+  y = blockIdx.x % s.S;
+  t = (blockIdx.x / s.S) % s.T;
+  b = blockIdx.x / (s.S * s.T);
+  ts = s.t_index ? min(max(__ldg(s.t_index + t), 0), s.Tsrc - 1) : t;
+}
+
+// All V crops of output row y of frame t of output clip oc, from the source frame `frame` of geometry g.
 // PACKED: rows [B*V][T][S][pitch] of 16-bit stem input (layout of esf_stem_pack), else FP32 NCDHW (B*V, C, T, S, S)
 template <bool RESIZE, bool PACKED>
-__global__ void __launch_bounds__(kCropThreads) crop_frames_kernel(const CropParams p, int pitch, int lpad, int f16,
-                                                                   void* __restrict__ out) {
-  __shared__ float lut_s[4 * 256];
-  extern __shared__ __align__(16) uint8_t rows_s[];
-  const int row_bytes = p.W0 * p.C;
+__device__ __forceinline__ void crop_rows(const CropShared& s, const CropClip& g, const uint8_t* frame, int oc, int t,
+                                          int y, const float* lut_s, uint8_t* rows_s, int pitch, int lpad, int f16,
+                                          void* __restrict__ out) {
+  const int row_bytes = g.W0 * s.C;
   const int row_pitch = ((row_bytes + 15) & ~15) + 16;   // + 16: room for the source's 16-byte phase
   const uint8_t* r0 = rows_s;
   const uint8_t* r1 = rows_s + row_pitch;
-  for (int i = threadIdx.x; i < p.C * 256; i += blockDim.x) lut_s[i] = p.lut[i];
-
-  const int y = blockIdx.x % p.S;
-  const int t = (blockIdx.x / p.S) % p.T;
-  const int b = blockIdx.x / (p.S * p.T);
-  const int ts = p.t_index ? min(max(__ldg(p.t_index + t), 0), p.Tsrc - 1) : t;
-  const uint8_t* frame = p.frames + ((long long)b * p.Tsrc + ts) * p.H0 * row_bytes;
   int loaded = -1;   // resized row whose source rows are in shared memory
-  for (int v = 0; v < p.V; ++v) {
-    const int yr = p.y0[v] + y;
+  for (int v = 0; v < s.V; ++v) {
+    const int yr = g.y0[v] + y;
     float l0 = 1.f, l1 = 0.f;
     if (yr != loaded) {
       int s0 = yr, s1 = yr;
       if (RESIZE) {
-        const int2 yi = __ldg(reinterpret_cast<const int2*>(p.y_idx) + yr);
-        s0 = min(max(yi.x, 0), p.H0 - 1), s1 = min(max(yi.y, 0), p.H0 - 1);
+        const int2 yi = __ldg(reinterpret_cast<const int2*>(g.y_idx) + yr);
+        s0 = min(max(yi.x, 0), g.H0 - 1), s1 = min(max(yi.y, 0), g.H0 - 1);
       }
       __syncthreads();   // the previous view's reads of the rows are done
       r0 = load_row_bytes(rows_s, frame + (long long)s0 * row_bytes, row_bytes);
@@ -103,24 +132,24 @@ __global__ void __launch_bounds__(kCropThreads) crop_frames_kernel(const CropPar
       loaded = yr;
     }
     if (RESIZE) {
-      const float2 yw = __ldg(reinterpret_cast<const float2*>(p.y_wt) + yr);
+      const float2 yw = __ldg(reinterpret_cast<const float2*>(g.y_wt) + yr);
       l0 = yw.x, l1 = yw.y;
     }
-    const long long orow = ((long long)(b * p.V + v) * p.T + t) * p.S + y;   // (clip row, t, y) of the output
-    const int x0 = p.x0[v];
+    const long long orow = ((long long)(oc * s.V + v) * s.T + t) * s.S + y;   // (clip row, t, y) of the output
+    const int x0 = g.x0[v];
     if (PACKED) {
       uint16_t* dst = static_cast<uint16_t*>(out) + orow * pitch;
-      const int SC = p.S * p.C;
+      const int SC = s.S * s.C;
       for (int ck = threadIdx.x; ck < pitch / 8; ck += blockDim.x) {
         const int j0 = ck * 8 - lpad;
-        int x = j0 >= 0 ? j0 / p.C : -1 - ((-1 - j0) / p.C);   // floor division: lpad need not be a multiple of C
-        int c = j0 - x * p.C;
+        int x = j0 >= 0 ? j0 / s.C : -1 - ((-1 - j0) / s.C);   // floor division: lpad need not be a multiple of C
+        int c = j0 - x * s.C;
         float f[8];
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
           const int j = j0 + e;
-          f[e] = (j >= 0 && j < SC) ? crop_value<RESIZE>(p, r0, r1, lut_s, x0 + x, c, p.chan_src[c], l0, l1) : 0.f;
-          if (++c == p.C) c = 0, ++x;
+          f[e] = (j >= 0 && j < SC) ? crop_value<RESIZE>(g, s.C, r0, r1, lut_s, x0 + x, c, s.chan_src[c], l0, l1) : 0.f;
+          if (++c == s.C) c = 0, ++x;
         }
         uint4 o;
         o.x = pack16x2(f[0], f[1], f16);
@@ -130,69 +159,179 @@ __global__ void __launch_bounds__(kCropThreads) crop_frames_kernel(const CropPar
         *reinterpret_cast<uint4*>(dst + ck * 8) = o;
       }
     } else {
-      // out[(b*V + v), c, t, y, :]: one thread = 4 consecutive x of one channel (16-byte store when S % 4 == 0)
-      const int S4 = (p.S + 3) / 4;
-      const bool vec = (p.S & 3) == 0;
-      for (int i = threadIdx.x; i < p.C * S4; i += blockDim.x) {
+      // out[(oc*V + v), c, t, y, :]: one thread = 4 consecutive x of one channel (16-byte store when S % 4 == 0)
+      const int S4 = (s.S + 3) / 4;
+      const bool vec = (s.S & 3) == 0;
+      for (int i = threadIdx.x; i < s.C * S4; i += blockDim.x) {
         const int c = i / S4, xs = (i - c * S4) * 4;
         float f[4];
 #pragma unroll
         for (int e = 0; e < 4; ++e)
-          f[e] = xs + e < p.S ? crop_value<RESIZE>(p, r0, r1, lut_s, x0 + xs + e, c, p.chan_src[c], l0, l1) : 0.f;
-        float* dst = static_cast<float*>(out) + ((((long long)(b * p.V + v) * p.C + c) * p.T + t) * p.S + y) * p.S + xs;
+          f[e] = xs + e < s.S ? crop_value<RESIZE>(g, s.C, r0, r1, lut_s, x0 + xs + e, c, s.chan_src[c], l0, l1) : 0.f;
+        float* dst = static_cast<float*>(out) + ((((long long)(oc * s.V + v) * s.C + c) * s.T + t) * s.S + y) * s.S + xs;
         if (vec) {
           *reinterpret_cast<float4*>(dst) = make_float4(f[0], f[1], f[2], f[3]);
         } else {
 #pragma unroll
           for (int e = 0; e < 4; ++e)
-            if (xs + e < p.S) dst[e] = f[e];
+            if (xs + e < s.S) dst[e] = f[e];
         }
       }
     }
   }
 }
 
+// B clips of one geometry: clip b's frames follow clip b - 1's.
+template <bool RESIZE, bool PACKED>
+__global__ void __launch_bounds__(kCropThreads) crop_frames_kernel(const CropParams p, int pitch, int lpad, int f16,
+                                                                   void* __restrict__ out) {
+  __shared__ float lut_s[4 * 256];
+  extern __shared__ __align__(16) uint8_t rows_s[];
+  for (int i = threadIdx.x; i < p.s.C * 256; i += blockDim.x) lut_s[i] = p.s.lut[i];
+  int b, t, y, ts;
+  crop_block(p.s, b, t, y, ts);
+  const uint8_t* frame = p.g.frames + ((long long)b * p.s.Tsrc + ts) * p.g.H0 * (p.g.W0 * p.s.C);
+  crop_rows<RESIZE, PACKED>(p.s, p.g, frame, b, t, y, lut_s, rows_s, pitch, lpad, f16, out);
+}
+
+// A chunk of clips, each of its own geometry; resized and pure-window clips may be mixed.  Both paths live in one
+// kernel, and the clip's entry is addressed by register: at the default budget of 32 registers the packed variant
+// spills, at 6 blocks per SM (<= 40 registers) neither does.
+template <bool PACKED>
+__global__ void __launch_bounds__(kCropThreads, 6) crop_frames_ragged_kernel(const __grid_constant__ CropChunk p, int pitch,
+                                                                          int lpad, int f16, void* __restrict__ out) {
+  __shared__ float lut_s[4 * 256];
+  extern __shared__ __align__(16) uint8_t rows_s[];
+  for (int i = threadIdx.x; i < p.s.C * 256; i += blockDim.x) lut_s[i] = p.s.lut[i];
+  int b, t, y, ts;
+  crop_block(p.s, b, t, y, ts);
+  const CropClip& g = p.g[b];
+  const uint8_t* frame = g.frames + (long long)ts * g.H0 * (g.W0 * p.s.C);
+  if (g.Hr != g.H0 || g.Wr != g.W0)
+    crop_rows<true, PACKED>(p.s, g, frame, p.clip0 + b, t, y, lut_s, rows_s, pitch, lpad, f16, out);
+  else
+    crop_rows<false, PACKED>(p.s, g, frame, p.clip0 + b, t, y, lut_s, rows_s, pitch, lpad, f16, out);
+}
+
+static int crop_shared(CropShared* s, const char* who, int32_t B, int32_t Tsrc, int32_t C, const int32_t* t_index,
+                       int32_t T, const int32_t* chan_src, const float* lut32, int32_t V, int32_t S) {
+  ESF_CHECK_ARG(lut32 && B > 0 && Tsrc > 0 && T > 0 && C >= 1 && C <= 4, "%s: null/bad argument", who);
+  ESF_CHECK_ARG(t_index || T == Tsrc, "%s: T (%d) != Tsrc (%d) needs a frame index", who, T, Tsrc);
+  ESF_CHECK_ARG(V >= 1 && V <= kCropMaxViews && S > 0, "%s: bad views (%d) / crop size (%d)", who, V, S);
+  s->t_index = t_index, s->lut = lut32;
+  s->Tsrc = Tsrc, s->T = T, s->C = C, s->S = S, s->V = V;
+  for (int c = 0; c < 4; ++c) {
+    s->chan_src[c] = (chan_src && c < C) ? chan_src[c] : c;
+    ESF_CHECK_ARG(c >= C || (s->chan_src[c] >= 0 && s->chan_src[c] < C), "%s: chan_src[%d] out of range", who, c);
+  }
+  return ESF_OK;
+}
+
+// Geometry of clip `clip` (-1: the one geometry of a uniform batch); needs the checked CropShared s.
+static int crop_clip(CropClip* g, const char* who, int clip, const CropShared& s, const void* frames, int32_t H0,
+                     int32_t W0, const void* y_index, const void* y_weight, int32_t Hr, const void* x_index,
+                     const void* x_weight, int32_t Wr, const int32_t* crop_yx) {
+  ESF_CHECK_ARG(frames && crop_yx && H0 > 0 && W0 > 0, "%s: clip %d: null/bad argument", who, clip);
+  ESF_CHECK_ARG((long long)W0 * s.C <= kCropMaxRowBytes, "%s: clip %d: source rows of %lld bytes exceed %d", who, clip,
+                (long long)W0 * s.C, kCropMaxRowBytes);
+  ESF_CHECK_ARG(Hr > 0 && Wr > 0, "%s: clip %d: bad resized size %d x %d", who, clip, Hr, Wr);
+  const bool resize = Hr != H0 || Wr != W0;
+  ESF_CHECK_ARG(!resize || (y_index && y_weight && x_index && x_weight), "%s: clip %d: resize tables missing", who, clip);
+  g->frames = static_cast<const uint8_t*>(frames);
+  g->y_idx = static_cast<const int32_t*>(y_index), g->y_wt = static_cast<const float*>(y_weight);
+  g->x_idx = static_cast<const int32_t*>(x_index), g->x_wt = static_cast<const float*>(x_weight);
+  g->H0 = H0, g->W0 = W0, g->Hr = Hr, g->Wr = Wr;
+  const int V = s.V, S = s.S;
+  for (int v = 0; v < kCropMaxViews; ++v) {
+    g->y0[v] = v < V ? crop_yx[2 * v] : 0;
+    g->x0[v] = v < V ? crop_yx[2 * v + 1] : 0;
+    ESF_CHECK_ARG(v >= V || (g->y0[v] >= 0 && g->y0[v] + S <= Hr && g->x0[v] >= 0 && g->x0[v] + S <= Wr),
+                  "%s: clip %d: crop %d at (%d, %d) of size %d leaves the %d x %d frame", who, clip, v, g->y0[v],
+                  g->x0[v], S, Hr, Wr);
+  }
+  return ESF_OK;
+}
+
+static size_t crop_smem(int W0, int C) { return 2 * (size_t)(((W0 * C + 15) & ~15) + 16); }
+
 static int crop_params(CropParams* p, const char* who, const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0,
                        int32_t W0, int32_t C, const int32_t* t_index, int32_t T, const int32_t* chan_src,
                        const float* lut32, const int32_t* y_index, const float* y_weight, int32_t Hr,
                        const int32_t* x_index, const float* x_weight, int32_t Wr, const int32_t* crop_yx_host,
                        int32_t V, int32_t S) {
-  ESF_CHECK_ARG(frames && lut32 && crop_yx_host && B > 0 && Tsrc > 0 && T > 0 && H0 > 0 && W0 > 0 && C >= 1 && C <= 4,
-                "%s: null/bad argument", who);
-  ESF_CHECK_ARG(t_index || T == Tsrc, "%s: T (%d) != Tsrc (%d) needs a frame index", who, T, Tsrc);
-  ESF_CHECK_ARG(W0 * C <= kCropMaxRowBytes, "%s: source rows of %d bytes exceed %d", who, W0 * C, kCropMaxRowBytes);
-  ESF_CHECK_ARG(V >= 1 && V <= kCropMaxViews && S > 0 && Hr > 0 && Wr > 0, "%s: bad views (%d) / crop size (%d)", who, V, S);
-  const bool resize = Hr != H0 || Wr != W0;
-  ESF_CHECK_ARG(!resize || (y_index && y_weight && x_index && x_weight), "%s: resize tables missing", who);
+  int rc = crop_shared(&p->s, who, B, Tsrc, C, t_index, T, chan_src, lut32, V, S);
+  if (rc != ESF_OK) return rc;
+  rc = crop_clip(&p->g, who, -1, p->s, frames, H0, W0, y_index, y_weight, Hr, x_index, x_weight, Wr, crop_yx_host);
+  if (rc != ESF_OK) return rc;
   ESF_CHECK_ARG((long long)B * T * S < (1LL << 31), "%s: grid too large", who);
-  p->frames = frames, p->t_index = t_index, p->lut = lut32;
-  p->B = B, p->Tsrc = Tsrc, p->T = T, p->H0 = H0, p->W0 = W0, p->C = C;
-  for (int c = 0; c < 4; ++c) {
-    p->chan_src[c] = (chan_src && c < C) ? chan_src[c] : c;
-    ESF_CHECK_ARG(c >= C || (p->chan_src[c] >= 0 && p->chan_src[c] < C), "%s: chan_src[%d] out of range", who, c);
-  }
-  p->y_idx = y_index, p->y_wt = y_weight, p->x_idx = x_index, p->x_wt = x_weight;
-  p->Hr = Hr, p->Wr = Wr, p->S = S, p->V = V;
-  for (int v = 0; v < kCropMaxViews; ++v) {
-    p->y0[v] = v < V ? crop_yx_host[2 * v] : 0;
-    p->x0[v] = v < V ? crop_yx_host[2 * v + 1] : 0;
-    ESF_CHECK_ARG(v >= V || (p->y0[v] >= 0 && p->y0[v] + S <= Hr && p->x0[v] >= 0 && p->x0[v] + S <= Wr),
-                  "%s: crop %d at (%d, %d) of size %d leaves the %d x %d frame", who, v, p->y0[v], p->x0[v], S, Hr, Wr);
-  }
+  p->B = B;
   return ESF_OK;
 }
 
 template <bool PACKED>
 static int crop_launch(const char* who, const CropParams& p, int pitch, int lpad, int f16, void* out, void* stream) {
-  const bool resize = p.Hr != p.H0 || p.Wr != p.W0;
-  const size_t smem = 2 * (size_t)(((p.W0 * p.C + 15) & ~15) + 16);
-  const unsigned grid = (unsigned)((long long)p.B * p.T * p.S);
+  const bool resize = p.g.Hr != p.g.H0 || p.g.Wr != p.g.W0;
+  const size_t smem = crop_smem(p.g.W0, p.s.C);
+  const unsigned grid = (unsigned)((long long)p.B * p.s.T * p.s.S);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (resize)
     crop_frames_kernel<true, PACKED><<<grid, kCropThreads, smem, s>>>(p, pitch, lpad, f16, out);
   else
     crop_frames_kernel<false, PACKED><<<grid, kCropThreads, smem, s>>>(p, pitch, lpad, f16, out);
   return check_launch(who);
+}
+
+// frames_host: B device addresses; geom_host [B][4]: H0, W0, Hr, Wr; tables_host [B][4]: device addresses of y_index,
+// y_weight, x_index, x_weight; crop_yx_host [B][V][2].  Every clip is checked before the first launch.
+template <bool PACKED>
+static int crop_ragged(const char* who, const char* kernel, const void* frames_host, int32_t B, int32_t Tsrc, int32_t C,
+                       const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
+                       const int32_t* geom_host, const void* tables_host, const int32_t* crop_yx_host, int32_t V,
+                       int32_t S, int pitch, int lpad, int f16, void* out, void* stream) {
+  CropChunk p{};
+  int rc = crop_shared(&p.s, who, B, Tsrc, C, t_index, T, chan_src, lut32, V, S);
+  if (rc != ESF_OK) return rc;
+  ESF_CHECK_ARG(frames_host && geom_host && tables_host && crop_yx_host, "%s: null host array", who);
+  ESF_CHECK_ARG((long long)kCropChunk * T * S < (1LL << 31), "%s: grid too large", who);
+  const void* const* fr = static_cast<const void* const*>(frames_host);
+  const void* const* tb = static_cast<const void* const*>(tables_host);
+  auto clip = [&](CropClip* g, int b) {
+    const int32_t* gm = geom_host + 4 * b;
+    return crop_clip(g, who, b, p.s, fr[b], gm[0], gm[1], tb[4 * b], tb[4 * b + 1], gm[2], tb[4 * b + 2],
+                     tb[4 * b + 3], gm[3], crop_yx_host + 2 * V * b);
+  };
+  for (int b = 0; b < B; ++b) {   // a bad clip anywhere: nothing is written
+    CropClip g;
+    if ((rc = clip(&g, b)) != ESF_OK) return rc;
+  }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  for (int b0 = 0; b0 < B; b0 += kCropChunk) {
+    const int n = std::min(B - b0, kCropChunk);
+    p.clip0 = b0;
+    int w0 = 0;
+    for (int i = 0; i < n; ++i) {
+      clip(&p.g[i], b0 + i);
+      w0 = std::max(w0, p.g[i].W0);
+    }
+    const unsigned grid = (unsigned)(n * T * S);
+    crop_frames_ragged_kernel<PACKED><<<grid, kCropThreads, crop_smem(w0, C), s>>>(p, pitch, lpad, f16, out);
+    if ((rc = check_launch(kernel)) != ESF_OK) return rc;
+  }
+  return ESF_OK;
+}
+
+static int check_packed_out(const char* who, int32_t dtype, int32_t pitch, int32_t lpad, int32_t S, int32_t C,
+                            const void* xp) {
+  ESF_CHECK_ARG(xp && is16(dtype), "%s: null output / bad dtype", who);
+  ESF_CHECK_ARG(pitch % 8 == 0 && lpad >= 0 && pitch >= lpad + S * C && (reinterpret_cast<uintptr_t>(xp) & 15) == 0,
+                "%s: bad pitch %d / lpad %d", who, pitch, lpad);
+  return ESF_OK;
+}
+
+static int check_clip_out(const char* who, int32_t S, const float* clip) {
+  ESF_CHECK_ARG(clip && ((S & 3) != 0 || (reinterpret_cast<uintptr_t>(clip) & 15) == 0), "%s: null / misaligned clip",
+                who);
+  return ESF_OK;
 }
 
 }  // namespace esf
@@ -205,12 +344,10 @@ extern "C" int esf_stem_pack_u8_crop(const uint8_t* frames, int32_t B, int32_t T
                                      const float* x_weight, int32_t Wr, const int32_t* crop_yx_host, int32_t V, int32_t S,
                                      int32_t dtype, int32_t pitch, int32_t lpad, void* xp, void* stream) {
   CropParams p;
-  const int rc = crop_params(&p, "esf_stem_pack_u8_crop", frames, B, Tsrc, H0, W0, C, t_index, T, chan_src, lut32,
-                             y_index, y_weight, Hr, x_index, x_weight, Wr, crop_yx_host, V, S);
+  int rc = crop_params(&p, "esf_stem_pack_u8_crop", frames, B, Tsrc, H0, W0, C, t_index, T, chan_src, lut32, y_index,
+                       y_weight, Hr, x_index, x_weight, Wr, crop_yx_host, V, S);
   if (rc != ESF_OK) return rc;
-  ESF_CHECK_ARG(xp && is16(dtype), "esf_stem_pack_u8_crop: null output / bad dtype");
-  ESF_CHECK_ARG(pitch % 8 == 0 && lpad >= 0 && pitch >= lpad + S * C && (reinterpret_cast<uintptr_t>(xp) & 15) == 0,
-                "esf_stem_pack_u8_crop: bad pitch %d / lpad %d", pitch, lpad);
+  if ((rc = check_packed_out("esf_stem_pack_u8_crop", dtype, pitch, lpad, S, C, xp)) != ESF_OK) return rc;
   return crop_launch<true>("crop_frames_kernel (packed)", p, pitch, lpad, dtype == ESF_F16, xp, stream);
 }
 
@@ -220,10 +357,33 @@ extern "C" int esf_frames_to_clip_crop(const uint8_t* frames, int32_t B, int32_t
                                        const float* x_weight, int32_t Wr, const int32_t* crop_yx_host, int32_t V,
                                        int32_t S, float* clip, void* stream) {
   CropParams p;
-  const int rc = crop_params(&p, "esf_frames_to_clip_crop", frames, B, Tsrc, H0, W0, C, t_index, T, chan_src, lut32,
-                             y_index, y_weight, Hr, x_index, x_weight, Wr, crop_yx_host, V, S);
+  int rc = crop_params(&p, "esf_frames_to_clip_crop", frames, B, Tsrc, H0, W0, C, t_index, T, chan_src, lut32, y_index,
+                       y_weight, Hr, x_index, x_weight, Wr, crop_yx_host, V, S);
   if (rc != ESF_OK) return rc;
-  ESF_CHECK_ARG(clip && ((S & 3) != 0 || (reinterpret_cast<uintptr_t>(clip) & 15) == 0),
-                "esf_frames_to_clip_crop: null / misaligned clip");
+  if ((rc = check_clip_out("esf_frames_to_clip_crop", S, clip)) != ESF_OK) return rc;
   return crop_launch<false>("crop_frames_kernel (clip)", p, 0, 0, 0, clip, stream);
+}
+
+extern "C" int esf_stem_pack_u8_crop_ragged(const void* frames_host, int32_t B, int32_t Tsrc, int32_t C,
+                                            const int32_t* t_index, int32_t T, const int32_t* chan_src,
+                                            const float* lut32, const int32_t* geom_host, const void* tables_host,
+                                            const int32_t* crop_yx_host, int32_t V, int32_t S, int32_t dtype,
+                                            int32_t pitch, int32_t lpad, void* xp, void* stream) {
+  const int rc = check_packed_out("esf_stem_pack_u8_crop_ragged", dtype, pitch, lpad, S, C, xp);
+  if (rc != ESF_OK) return rc;
+  return crop_ragged<true>("esf_stem_pack_u8_crop_ragged", "crop_frames_ragged_kernel (packed)", frames_host, B, Tsrc,
+                           C, t_index, T, chan_src, lut32, geom_host, tables_host, crop_yx_host, V, S, pitch, lpad,
+                           dtype == ESF_F16, xp, stream);
+}
+
+extern "C" int esf_frames_to_clip_crop_ragged(const void* frames_host, int32_t B, int32_t Tsrc, int32_t C,
+                                              const int32_t* t_index, int32_t T, const int32_t* chan_src,
+                                              const float* lut32, const int32_t* geom_host, const void* tables_host,
+                                              const int32_t* crop_yx_host, int32_t V, int32_t S, float* clip,
+                                              void* stream) {
+  const int rc = check_clip_out("esf_frames_to_clip_crop_ragged", S, clip);
+  if (rc != ESF_OK) return rc;
+  return crop_ragged<false>("esf_frames_to_clip_crop_ragged", "crop_frames_ragged_kernel (clip)", frames_host, B, Tsrc,
+                            C, t_index, T, chan_src, lut32, geom_host, tables_host, crop_yx_host, V, S, 0, 0, 0, clip,
+                            stream);
 }

@@ -13,6 +13,11 @@ branch resizes every normalised clip so that its short side is S (bilinear, on t
 (datasets/utils.py spatial_sampling, transform.py).  The byte frames at decode size go to the device instead and one
 kernel (csrc/esf_crop.cu) normalises, resizes, crops and packs; the resize follows the per-axis tables of `axis_table`,
 which reproduce torch's CPU weights bit for bit.
+
+Mixed decode sizes (`forward_frames([clip, ...], crop_size=S, spatial_idx=...)`): a test split mixes resolutions and
+aspect ratios, and the reference's loader resizes and crops every clip on its own before collating the S x S crops.  A
+list of B uint8 clips (T, H_b, W_b, C) of one T and C runs the same crops through one launch per 32 clips
+(esf_*_crop_ragged); the output shapes, hence the plan, are those of a stacked batch of B clips.
 """
 import ctypes
 import math
@@ -61,6 +66,7 @@ def crop_offset(height, width, size, spatial_idx):
 
 
 MAX_VIEWS = 8   # csrc/esf_crop.cu kCropMaxViews
+MAX_ROW_BYTES = 16384   # csrc/esf_crop.cu kCropMaxRowBytes: W * C of one source row
 
 
 def spatial_views(spatial_idx):
@@ -95,22 +101,80 @@ def axis_table(n_in, n_out):
     return torch.from_numpy(np.stack([i0, i1], 1).astype(np.int32)), torch.from_numpy(np.stack([l0, l1], 1))
 
 
+def _is_shape(x):
+    return all(isinstance(n, (int, np.integer)) and not isinstance(n, bool) for n in x)
+
+
+def clip_shapes(shapes):
+    """`shapes` of a list of clips as (T, H, W, C) int tuples; ValueError unless every clip has 4 dimensions, they share
+    T and C, and a source row (W * C bytes) fits the crop kernel."""
+    out = []
+    for sh in shapes:
+        if len(sh) != 4 or not _is_shape(sh):
+            raise ValueError("a list of clips holds uint8 clips (T, H, W, C), got shape %s" % (tuple(sh),))
+        out.append(tuple(int(n) for n in sh))
+    if not out:
+        raise ValueError("an empty list of clips has no clip shapes")
+    T, C = out[0][0], out[0][3]
+    for T_b, H_b, W_b, C_b in out:
+        if (T_b, C_b) != (T, C):
+            raise ValueError("the clips of a list share T and C: (T, C) = (%d, %d) next to (%d, %d)" % (T, C, T_b, C_b))
+        if min(T_b, H_b, W_b, C_b) < 1:
+            raise ValueError("empty clip of shape %s" % ((T_b, H_b, W_b, C_b),))
+        if W_b * C_b > MAX_ROW_BYTES:
+            raise ValueError("clip rows of %d x %d bytes exceed the crop kernel's %d" % (W_b, C_b, MAX_ROW_BYTES))
+    return out
+
+
 def view_shapes(frames_shape, crop_size, spatial_idx, alpha=None):
     """Clip shapes [slow, fast] (`alpha` given) or [single] that `forward_frames(frames, crop_size=, spatial_idx=)` runs
-    on for uint8 frames of `frames_shape` (B, T, H, W, C): B * V rows of crop_size x crop_size.  ValueError when a crop does
-    not fit the resized frame."""
-    B, T, H, W, C = (int(n) for n in frames_shape)
+    on for uint8 frames of `frames_shape` (B, T, H, W, C), or for a list of B clips of the shapes (T, H_b, W_b, C)
+    (`frames_shape` a list of such shapes, see clip_shapes): B * V rows of crop_size x crop_size.  ValueError when a crop
+    does not fit a resized frame."""
     views = spatial_views(spatial_idx)
     S = int(crop_size)
-    Hr, Wr = resized_size(H, W, S)
-    for v in views:
-        y0, x0 = crop_offset(Hr, Wr, S, v)
-        if S < 1 or y0 < 0 or x0 < 0 or y0 + S > Hr or x0 + S > Wr:
-            raise ValueError("a %d x %d crop does not fit frames of %d x %d resized to %d x %d" % (S, S, H, W, Hr, Wr))
+    if len(frames_shape) == 0 or not _is_shape(frames_shape):
+        clips = clip_shapes(frames_shape)
+        B, (T, _, _, C) = len(clips), clips[0]
+        sizes = sorted({(H, W) for _, H, W, _ in clips})
+    else:
+        B, T, H, W, C = (int(n) for n in frames_shape)
+        sizes = [(H, W)]
+    for H, W in sizes:
+        Hr, Wr = resized_size(H, W, S)
+        for v in views:
+            y0, x0 = crop_offset(Hr, Wr, S, v)
+            if S < 1 or y0 < 0 or x0 < 0 or y0 + S > Hr or x0 + S > Wr:
+                raise ValueError("a %d x %d crop does not fit frames of %d x %d resized to %d x %d" % (S, S, H, W, Hr, Wr))
     n = B * len(views)
     if alpha is None:
         return [(n, C, T, S, S)]
     return [(n, C, T // alpha, S, S), (n, C, T, S, S)]
+
+
+def check_clips(clips):
+    """Shapes (T, H, W, C) of a list of clip tensors; ValueError unless they are contiguous uint8 clips of 4 dimensions
+    on one device that share T and C (clip_shapes)."""
+    for c in clips:
+        if not isinstance(c, torch.Tensor) or c.dtype != torch.uint8 or c.dim() != 4 or not c.is_contiguous():
+            raise ValueError("a list of clips holds contiguous uint8 tensors (T, H, W, C), got %s"
+                             % (("%s %s" % (c.dtype, tuple(c.shape))) if isinstance(c, torch.Tensor) else type(c)))
+    if len({c.device for c in clips}) > 1:
+        raise ValueError("the clips of a list are on one device, got %s" % sorted({str(c.device) for c in clips}))
+    return clip_shapes([tuple(c.shape) for c in clips])
+
+
+def arena_layout(shapes, capacity=None, align=16):
+    """Byte offsets of uint8 clips of `shapes` (T, H, W, C) placed one after another in one buffer, each at a multiple of
+    `align` bytes, and the bytes they span.  EsfError when `capacity` (bytes) is given and they need more."""
+    offsets, end = [], 0
+    for sh in shapes:
+        start = -(-end // align) * align
+        offsets.append(start)
+        end = start + math.prod(int(n) for n in sh)
+    if capacity is not None and end > capacity:
+        raise rt.EsfError("clips of %d bytes (%d-byte aligned) exceed the %d-byte staging buffer" % (end, align, capacity))
+    return offsets, end
 
 
 class CropTables:
@@ -133,6 +197,25 @@ class CropTables:
             return None, None, self.Hr, None, None, self.Wr
         yi, yw, xi, xw = self.tables
         return yi.data_ptr(), yw.data_ptr(), self.Hr, xi.data_ptr(), xw.data_ptr(), self.Wr
+
+    def addresses(self):
+        """Device addresses of (y_index, y_weight, x_index, x_weight); None where the frames are not resized."""
+        return (None,) * 4 if self.tables is None else tuple(t.data_ptr() for t in self.tables)
+
+
+class ClipList:
+    """The host arrays of esf_*_crop_ragged for B clips (T, H_b, W_b, C) of mixed decode sizes: every clip's device
+    address and the geometry of its CropTables (FrameInput.crop, cached per geometry).  Built per call; the library
+    reads them before the call returns."""
+
+    def __init__(self, clips, tables):
+        self.B = len(clips)
+        self.T, _, _, self.C = clips[0].shape
+        self.S, self.V = tables[0].S, len(tables[0].views)
+        self.frames = (ctypes.c_void_p * self.B)(*[c.data_ptr() for c in clips])
+        self.geom = (ctypes.c_int32 * (4 * self.B))(*[n for t in tables for n in (t.H0, t.W0, t.Hr, t.Wr)])
+        self.tables = (ctypes.c_void_p * (4 * self.B))(*[a for t in tables for a in t.addresses()])
+        self.crop_yx = (ctypes.c_int32 * (2 * self.V * self.B))(*[o for t in tables for o in t.crop_yx])
 
 
 class FrameInput:
@@ -218,3 +301,22 @@ def launch_frames(plan, fin, frames, alpha, frame_index=None, crop=None):
         else:
             rt.check(L.esf_frames_to_clip(frames.data_ptr(), B, Tsrc, H, W, C, iptr, T, fin.chan_src,
                                           fin.lut32.data_ptr(), own.data_ptr(), s), "esf_frames_to_clip")
+
+
+def launch_clip_list(plan, fin, clips, alpha):
+    """Fill the stem inputs of `plan` from a ClipList on the current stream: row b * V + v is clip b at view v."""
+    L = rt.lib()
+    s = rt.current_stream_ptr()
+    for own in plan.inputs:
+        b, c, T, h, w = own.shape
+        assert (b, c, h, w) == (clips.B * clips.V, clips.C, clips.S, clips.S)
+        idx = fin.index(clips.T, T, alpha)
+        args = (clips.frames, clips.B, clips.T, clips.C, idx.data_ptr() if idx is not None else None, T, fin.chan_src,
+                fin.lut32.data_ptr(), clips.geom, clips.tables, clips.crop_yx, clips.V, clips.S)
+        route = plan.stem_routes.get(own.data_ptr())
+        if route is not None:
+            xp, pitch, lpad = route
+            rt.check(L.esf_stem_pack_u8_crop_ragged(*args, rt.dtype_code(xp), pitch, lpad, xp.data_ptr(), s),
+                     "esf_stem_pack_u8_crop_ragged")
+        else:
+            rt.check(L.esf_frames_to_clip_crop_ragged(*args, own.data_ptr(), s), "esf_frames_to_clip_crop_ragged")

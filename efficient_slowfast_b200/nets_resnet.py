@@ -453,10 +453,18 @@ class _PlannedModel(nn.Module):
         at decode size and every clip also goes through the reference's test-mode `spatial_sampling` (short side
         resized to `crop_size`, default cfg.DATA.TEST_CROP_SIZE, then `uniform_crop` at each index) on the device.  The
         result has B * V rows, row b * V + v being clip b at view v (the order of the test loader's clip numbering).
-        `crop_size` alone means spatial_idx 1 (TEST.NUM_SPATIAL_CROPS = 1)."""
+        `crop_size` alone means spatial_idx 1 (TEST.NUM_SPATIAL_CROPS = 1).
+
+        Mixed decode sizes: `frames` may also be a list or tuple of B contiguous uint8 clips (T, H_b, W_b, C) on one
+        device, of one T and C.  A list always means test-time spatial sampling (same defaults); every clip is resized
+        and cropped on its own, as the reference's loader does before collating.  The plan is that of a stacked batch
+        of B clips, so batches of any mix of sizes share it, and a list of clips of one size gives the stacked result
+        bit for bit."""
         from . import frames as esf_frames
         if self.training:
             raise NotImplementedError("eval-mode forward path only")
+        if isinstance(frames, (list, tuple)):
+            return self._forward_clip_list(list(frames), bboxes, frame_index, crop_size, spatial_idx)
         crop = crop_size is not None or spatial_idx is not None
         if crop:
             if bboxes is not None:
@@ -483,14 +491,44 @@ class _PlannedModel(nn.Module):
         if frame_index is not None:     # explicit source frame of every pathway frame (frames may be a ring buffer)
             assert len(frame_index) == self.num_pathways
             shapes = [tuple(sh[:2]) + (int(ix.numel()),) + tuple(sh[3:]) for sh, ix in zip(shapes, frame_index)]
-        plan = self._get_plan(shapes, dev)
-        fin = getattr(plan, "frame_input", None)
-        if fin is None:
-            fin = plan.frame_input = esf_frames.FrameInput(self._cfg, dev, plan.adt, channels=frames.shape[4])
+        plan, fin = self._frame_plan(shapes, dev, frames.shape[4])
         tabs = fin.crop(frames.shape[2], frames.shape[3], crop_size, views) if crop else None
         with torch.cuda.device(dev):
             out = plan.run_frames(lambda: esf_frames.launch_frames(plan, fin, frames, alpha, frame_index, tabs))
             return self._finish(plan, out, boxes)
+
+    def _frame_plan(self, shapes, dev, channels):
+        """The plan for `shapes` and its FrameInput (frames.py) for frames of `channels` channels."""
+        from . import frames as esf_frames
+        plan = self._get_plan(shapes, dev)
+        fin = getattr(plan, "frame_input", None)
+        if fin is None:
+            fin = plan.frame_input = esf_frames.FrameInput(self._cfg, dev, plan.adt, channels=channels)
+        return plan, fin
+
+    def _forward_clip_list(self, clips, bboxes, frame_index, crop_size, spatial_idx):
+        """forward_frames on a list of clips of mixed decode sizes: every argument is checked before anything runs."""
+        from . import frames as esf_frames
+        if bboxes is not None or frame_index is not None:
+            raise ValueError("forward_frames: a list of clips takes neither bboxes nor frame_index (the boxes would need "
+                             "each crop's transform)")
+        views = esf_frames.spatial_views(1 if spatial_idx is None else spatial_idx)
+        crop_size = int(self._cfg.DATA.TEST_CROP_SIZE if crop_size is None else crop_size)
+        if not clips:
+            return self._empty(next(self.parameters()).device)
+        sizes = esf_frames.check_clips(clips)
+        shapes = esf_frames.view_shapes(sizes, crop_size, views,
+                                        self._cfg.SLOWFAST.ALPHA if self.num_pathways > 1 else None)
+        dev = clips[0].device
+        if dev.type != "cuda":
+            raise rt.EsfError("the forward path is CUDA-only (sm_100a); got frames on %s -- there is no CPU fallback"
+                              % dev)
+        alpha = self._cfg.SLOWFAST.ALPHA if self.num_pathways > 1 else 1
+        plan, fin = self._frame_plan(shapes, dev, sizes[0][3])
+        batch = esf_frames.ClipList(clips, [fin.crop(H, W, crop_size, views) for _, H, W, _ in sizes])
+        with torch.cuda.device(dev):
+            out = plan.run_frames(lambda: esf_frames.launch_clip_list(plan, fin, batch, alpha))
+            return self._finish(plan, out, None)
 
     def _empty(self, dev):
         return torch.empty((0, int(self._cfg.MODEL.NUM_CLASSES)), dtype=torch.float32, device=dev)

@@ -12,6 +12,8 @@ computes.  Results are returned in submission order.
         done = stream.submit(host_inputs)         # -> (index, preds) of an EARLIER batch, or None while filling
     for index, preds in stream.flush(): ...
 """
+import math
+
 import torch
 
 from . import distributed as esf_dist
@@ -25,6 +27,10 @@ class ClipStream:
         process group before the D2H copy, like the reference's test loop.  `frames=True`: every batch is ONE pinned
         uint8 tensor of decoded frames (B, T, H, W, C) (`shapes` = [that shape]) and goes through
         `model.forward_frames` -- normalisation and pathway packing on the device, 1/5 of the H2D bytes.
+        With `crop_size` / `spatial_idx` (test-time crops of frames at decode size) a batch may also be a list of at
+        most B pinned uint8 clips (T, H_b, W_b, C) of mixed decode sizes: they are copied to 16-byte aligned offsets
+        of the same staging slot (frames.arena_layout; its B * T * H * W * C bytes are the capacity) and run as
+        `model.forward_frames(list)`.
         `slow_from_fast=True`: the caller vouches that every batch is what the reference's loader produces,
         `[slow, fast] = pack_pathway_output(cfg, fast)` (datasets/utils.py:93-102: slow = the linspace frame subset of
         fast).  Only the fast clip is then copied to the device and the slow pathway's stem reads its frames out of it
@@ -84,15 +90,20 @@ class ClipStream:
                                           "subset of the fast clip (pack_pathway_output)")
                     self._sff_checked = True
                 host_inputs = host_inputs[1:]
-        views = []
-        for h, d in zip(host_inputs, self.stage[slot]):
-            if tuple(h.shape[1:]) != tuple(d.shape[1:]) or h.shape[0] > d.shape[0] or h.shape[0] == 0:
-                raise rt.EsfError("ClipStream was built for batches of shape <= %s, got %s"
-                                  % (tuple(d.shape), tuple(h.shape)))
-            views.append(d if h.shape[0] == d.shape[0] else d[:h.shape[0]])
+        if self.crop is not None and host_inputs and all(h.dim() == 4 for h in host_inputs):
+            clips = self._clip_views(host_inputs, self.stage[slot][0])   # clips of mixed decode sizes
+            copies, views = list(zip(host_inputs, clips)), [clips]
+        else:
+            views = []
+            for h, d in zip(host_inputs, self.stage[slot]):
+                if tuple(h.shape[1:]) != tuple(d.shape[1:]) or h.shape[0] > d.shape[0] or h.shape[0] == 0:
+                    raise rt.EsfError("ClipStream was built for batches of shape <= %s, got %s"
+                                      % (tuple(d.shape), tuple(h.shape)))
+                views.append(d if h.shape[0] == d.shape[0] else d[:h.shape[0]])
+            copies = list(zip(host_inputs, views))
         with torch.cuda.stream(self.copy_stream):
             self.copy_stream.wait_event(self.consumed[slot])
-            for h, d in zip(host_inputs, views):
+            for h, d in copies:
                 d.copy_(h, non_blocking=True)
             self.ready[slot].record(self.copy_stream)
         cur.wait_event(self.ready[slot])
@@ -113,6 +124,19 @@ class ClipStream:
         self.pending.append((self.n, slot, out.shape[0]))
         self.n += 1
         return finished
+
+    def _clip_views(self, clips, stage):
+        """Views of the staging slot `stage` (B, T, H, W, C) that a list of clips (T, H_b, W_b, C) is copied to, at the
+        offsets of frames.arena_layout.  ValueError / EsfError before any copy when the clips are not a valid list
+        (frames.check_clips, crops that do not fit) or exceed the slot's B clips or its bytes."""
+        from . import frames as esf_frames
+        if len(clips) > stage.shape[0]:
+            raise rt.EsfError("ClipStream was built for batches of at most %d clips, got %d" % (stage.shape[0], len(clips)))
+        sizes = esf_frames.check_clips(clips)
+        esf_frames.view_shapes(sizes, self.crop["crop_size"], self.crop["spatial_idx"])
+        flat = stage.view(-1)
+        offsets, _ = esf_frames.arena_layout(sizes, flat.numel())
+        return [flat[o:o + math.prod(sh)].view(sh) for o, sh in zip(offsets, sizes)]
 
     def _pop(self):
         index, slot, rows = self.pending.pop(0)

@@ -163,6 +163,19 @@ int esf_frames_to_clip_crop(const uint8_t* frames, int32_t B, int32_t Tsrc, int3
                             const int32_t* y_index, const float* y_weight, int32_t Hr, const int32_t* x_index,
                             const float* x_weight, int32_t Wr, const int32_t* crop_yx_host, int32_t V, int32_t S,
                             float* clip, void* stream);
+/* The same for a batch of B clips of mixed decode sizes (one Tsrc, C for all): clip b is (Tsrc, H0_b, W0_b, C) uint8 at
+ * the device address frames_host[b] (a host array of B addresses).  geom_host: host int32[B][4], (H0, W0, Hr, Wr) of
+ * every clip; tables_host: host array [B][4] of the device addresses of its y_index, y_weight, x_index, x_weight (null
+ * allowed where the clip is not resized); crop_yx_host: host int32[B][V][2].  Output row b * V + v is clip b at view v,
+ * as above.  Every clip is checked before anything is launched; the host arrays are read before the call returns. */
+int esf_stem_pack_u8_crop_ragged(const void* frames_host, int32_t B, int32_t Tsrc, int32_t C, const int32_t* t_index,
+                                 int32_t T, const int32_t* chan_src, const float* lut32, const int32_t* geom_host,
+                                 const void* tables_host, const int32_t* crop_yx_host, int32_t V, int32_t S,
+                                 int32_t dtype, int32_t pitch, int32_t lpad, void* xp, void* stream);
+int esf_frames_to_clip_crop_ragged(const void* frames_host, int32_t B, int32_t Tsrc, int32_t C, const int32_t* t_index,
+                                   int32_t T, const int32_t* chan_src, const float* lut32, const int32_t* geom_host,
+                                   const void* tables_host, const int32_t* crop_yx_host, int32_t V, int32_t S,
+                                   float* clip, void* stream);
 int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int32_t T, int32_t H, int32_t W, int32_t pitch,
                           const void* w_band, const float* bias_tiled, int32_t Cout, int32_t kT, int32_t kH,
                           int32_t kW, int32_t sH, int32_t sW, int32_t pT, int32_t pH, int32_t pW, int32_t act,
