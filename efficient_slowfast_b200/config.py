@@ -71,7 +71,7 @@ def get_cfg():
                               WIDTH_MULTI=2.0, GROUPS=1))
     c.DATA = CfgNode(dict(NUM_FRAMES=8, CROP_SIZE=224, TRAIN_CROP_SIZE=224, TEST_CROP_SIZE=256,
                           INPUT_CHANNEL_NUM=[3, 3], MEAN=[0.45, 0.45, 0.45], STD=[0.225, 0.225, 0.225],
-                          SAMPLING_RATE=8, REVERSE_INPUT_CHANNEL=False))
+                          SAMPLING_RATE=8, TARGET_FPS=30, REVERSE_INPUT_CHANNEL=False))
     c.DETECTION = CfgNode(dict(ENABLE=False, ALIGNED=True, ROI_XFORM_RESOLUTION=7, SPATIAL_SCALE_FACTOR=16))
     c.MULTIGRID = CfgNode(dict(SHORT_CYCLE=False, LONG_CYCLE=False))
     c.TEST = CfgNode(dict(BATCH_SIZE=8, NUM_ENSEMBLE_VIEWS=10, NUM_SPATIAL_CROPS=3))

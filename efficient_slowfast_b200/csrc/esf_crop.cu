@@ -23,7 +23,14 @@
 // allocates nothing and keeps no host array past its return.  The work split is the uniform kernel's; a block reads
 // its clip's entry and takes the resize or the pure-window path for that clip (a block-uniform branch).  Both kernels
 // run the same row loads and emission loop (crop_rows).
+//
+// Temporal views of whole videos (esf_*_crop_videos).  The reference's test loader samples NUM_ENSEMBLE_VIEWS clips out of
+// every decoded video (decoder.get_start_end_idx + temporal_sampling).  There a "clip" is one (video, temporal view)
+// pair: its source is the whole video (Tsrc_b, H0, W0, C), shared by the video's views, and its frames are row b of a
+// device frame table t_index[B][T], each entry clamped to the clip's own Tsrc_b.  The chunk (CropVideoChunk) is the
+// ragged one plus the per-clip Tsrc; the kernel body is the ragged kernel's, instantiated for that chunk.
 #include <algorithm>
+#include <type_traits>
 
 #include "esf_common.cuh"
 #include "esf_host.h"
@@ -68,6 +75,21 @@ struct CropChunk {        // up to kCropChunk clips of their own geometry; g[i] 
 // + the kernel's other parameters (pitch, lpad, f16, out)
 static_assert(sizeof(CropChunk) + 3 * sizeof(int) + sizeof(void*) + 8 <= 4096, "CropChunk must fit the 4 KB parameters");
 
+struct CropVideoChunk {   // up to kCropChunk (video, temporal view) clips; clip clip0 + i reads row clip0 + i of t_index
+  CropShared s;
+  int clip0;
+  int Tsrc[kCropChunk];   // frames of clip i's video
+  CropClip g[kCropChunk];
+};
+static_assert(sizeof(CropVideoChunk) + 3 * sizeof(int) + sizeof(void*) + 8 <= 4096,
+              "CropVideoChunk must fit the 4 KB parameters");
+
+// Frame-table row and source length of clip b of a chunk: one shared row for a ragged chunk, one row per clip of videos.
+__device__ __forceinline__ int chunk_row(const CropChunk&, int) { return 0; }
+__device__ __forceinline__ int chunk_tsrc(const CropChunk& p, int) { return p.s.Tsrc; }
+__device__ __forceinline__ int chunk_row(const CropVideoChunk& p, int b) { return p.clip0 + b; }
+__device__ __forceinline__ int chunk_tsrc(const CropVideoChunk& p, int b) { return p.Tsrc[b]; }
+
 // copy bytes [src, src + n) into shared memory at dst + (src & 15), i.e. with the source's 16-byte phase, so that the
 // aligned body moves as 16-byte loads and stores and only the ragged ends go byte by byte; returns the row's start
 __device__ __forceinline__ const uint8_t* load_row_bytes(uint8_t* dst, const uint8_t* __restrict__ src, int n) {
@@ -97,12 +119,16 @@ __device__ __forceinline__ float crop_value(const CropClip& g, int C, const uint
   return __fmaf_rn(t0, l0, __fmul_rn(t1, l1));
 }
 
-// The block's (clip, output frame, output row) and the source frame of that output frame.
-__device__ __forceinline__ void crop_block(const CropShared& s, int& b, int& t, int& y, int& ts) {
+// The block's (clip, output frame, output row) and the source frame of that output frame: entry t of row `row` of the
+// frame table, clamped to the clip's Tsrc frames.
+__device__ __forceinline__ void crop_block(const CropShared& s, int& b, int& t, int& y) {
   y = blockIdx.x % s.S;
   t = (blockIdx.x / s.S) % s.T;
   b = blockIdx.x / (s.S * s.T);
-  ts = s.t_index ? min(max(__ldg(s.t_index + t), 0), s.Tsrc - 1) : t;
+}
+
+__device__ __forceinline__ int source_frame(const CropShared& s, int row, int t, int Tsrc) {
+  return s.t_index ? min(max(__ldg(s.t_index + row * s.T + t), 0), Tsrc - 1) : t;
 }
 
 // All V crops of output row y of frame t of output clip oc, from the source frame `frame` of geometry g.
@@ -188,23 +214,26 @@ __global__ void __launch_bounds__(kCropThreads) crop_frames_kernel(const CropPar
   __shared__ float lut_s[4 * 256];
   extern __shared__ __align__(16) uint8_t rows_s[];
   for (int i = threadIdx.x; i < p.s.C * 256; i += blockDim.x) lut_s[i] = p.s.lut[i];
-  int b, t, y, ts;
-  crop_block(p.s, b, t, y, ts);
+  int b, t, y;
+  crop_block(p.s, b, t, y);
+  const int ts = source_frame(p.s, 0, t, p.s.Tsrc);
   const uint8_t* frame = p.g.frames + ((long long)b * p.s.Tsrc + ts) * p.g.H0 * (p.g.W0 * p.s.C);
   crop_rows<RESIZE, PACKED>(p.s, p.g, frame, b, t, y, lut_s, rows_s, pitch, lpad, f16, out);
 }
 
 // A chunk of clips, each of its own geometry; resized and pure-window clips may be mixed.  Both paths live in one
 // kernel, and the clip's entry is addressed by register: at the default budget of 32 registers the packed variant
-// spills, at 6 blocks per SM (<= 40 registers) neither does.
-template <bool PACKED>
-__global__ void __launch_bounds__(kCropThreads, 6) crop_frames_ragged_kernel(const __grid_constant__ CropChunk p, int pitch,
+// spills, at 6 blocks per SM (<= 40 registers) neither does.  Chunk: CropChunk (clips of one frame count and one frame
+// index) or CropVideoChunk (temporal views of videos: a frame-table row and a source length per clip).
+template <bool PACKED, class Chunk>
+__global__ void __launch_bounds__(kCropThreads, 6) crop_frames_ragged_kernel(const __grid_constant__ Chunk p, int pitch,
                                                                           int lpad, int f16, void* __restrict__ out) {
   __shared__ float lut_s[4 * 256];
   extern __shared__ __align__(16) uint8_t rows_s[];
   for (int i = threadIdx.x; i < p.s.C * 256; i += blockDim.x) lut_s[i] = p.s.lut[i];
-  int b, t, y, ts;
-  crop_block(p.s, b, t, y, ts);
+  int b, t, y;
+  crop_block(p.s, b, t, y);
+  const int ts = source_frame(p.s, chunk_row(p, b), t, chunk_tsrc(p, b));
   const CropClip& g = p.g[b];
   const uint8_t* frame = g.frames + (long long)ts * g.H0 * (g.W0 * p.s.C);
   if (g.Hr != g.H0 || g.Wr != g.W0)
@@ -281,22 +310,27 @@ static int crop_launch(const char* who, const CropParams& p, int pitch, int lpad
   return check_launch(who);
 }
 
-// frames_host: B device addresses; geom_host [B][4]: H0, W0, Hr, Wr; tables_host [B][4]: device addresses of y_index,
-// y_weight, x_index, x_weight; crop_yx_host [B][V][2].  Every clip is checked before the first launch.
-template <bool PACKED>
+// frames_host: B device addresses; geom_host [B][4]: H0, W0, Hr, Wr (CropChunk) or [B][5]: Tsrc, H0, W0, Hr, Wr
+// (CropVideoChunk, whose t_index is a [B][T] table); tables_host [B][4]: device addresses of y_index, y_weight, x_index,
+// x_weight; crop_yx_host [B][V][2].  Every clip is checked before the first launch.
+template <bool PACKED, class Chunk>
 static int crop_ragged(const char* who, const char* kernel, const void* frames_host, int32_t B, int32_t Tsrc, int32_t C,
                        const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
                        const int32_t* geom_host, const void* tables_host, const int32_t* crop_yx_host, int32_t V,
                        int32_t S, int pitch, int lpad, int f16, void* out, void* stream) {
-  CropChunk p{};
+  constexpr bool kVideos = std::is_same<Chunk, CropVideoChunk>::value;
+  constexpr int kGeom = kVideos ? 5 : 4;   // int32 entries of a clip's geom_host row
+  Chunk p{};
   int rc = crop_shared(&p.s, who, B, Tsrc, C, t_index, T, chan_src, lut32, V, S);
   if (rc != ESF_OK) return rc;
   ESF_CHECK_ARG(frames_host && geom_host && tables_host && crop_yx_host, "%s: null host array", who);
   ESF_CHECK_ARG((long long)kCropChunk * T * S < (1LL << 31), "%s: grid too large", who);
+  ESF_CHECK_ARG((long long)B * T < (1LL << 31), "%s: frame table too large", who);
   const void* const* fr = static_cast<const void* const*>(frames_host);
   const void* const* tb = static_cast<const void* const*>(tables_host);
   auto clip = [&](CropClip* g, int b) {
-    const int32_t* gm = geom_host + 4 * b;
+    const int32_t* gm = geom_host + kGeom * b + (kVideos ? 1 : 0);
+    if constexpr (kVideos) ESF_CHECK_ARG(gm[-1] >= 1, "%s: clip %d: a video of %d frames", who, b, gm[-1]);
     return crop_clip(g, who, b, p.s, fr[b], gm[0], gm[1], tb[4 * b], tb[4 * b + 1], gm[2], tb[4 * b + 2],
                      tb[4 * b + 3], gm[3], crop_yx_host + 2 * V * b);
   };
@@ -312,9 +346,10 @@ static int crop_ragged(const char* who, const char* kernel, const void* frames_h
     for (int i = 0; i < n; ++i) {
       clip(&p.g[i], b0 + i);
       w0 = std::max(w0, p.g[i].W0);
+      if constexpr (kVideos) p.Tsrc[i] = geom_host[kGeom * (b0 + i)];
     }
     const unsigned grid = (unsigned)(n * T * S);
-    crop_frames_ragged_kernel<PACKED><<<grid, kCropThreads, crop_smem(w0, C), s>>>(p, pitch, lpad, f16, out);
+    crop_frames_ragged_kernel<PACKED, Chunk><<<grid, kCropThreads, crop_smem(w0, C), s>>>(p, pitch, lpad, f16, out);
     if ((rc = check_launch(kernel)) != ESF_OK) return rc;
   }
   return ESF_OK;
@@ -331,6 +366,12 @@ static int check_packed_out(const char* who, int32_t dtype, int32_t pitch, int32
 static int check_clip_out(const char* who, int32_t S, const float* clip) {
   ESF_CHECK_ARG(clip && ((S & 3) != 0 || (reinterpret_cast<uintptr_t>(clip) & 15) == 0), "%s: null / misaligned clip",
                 who);
+  return ESF_OK;
+}
+
+// The video entry points read every clip's frames through its row of the table: there is no identity default.
+static int check_frame_table(const char* who, const int32_t* t_index) {
+  ESF_CHECK_ARG(t_index, "%s: null frame table (t_index [B][T])", who);
   return ESF_OK;
 }
 
@@ -371,7 +412,7 @@ extern "C" int esf_stem_pack_u8_crop_ragged(const void* frames_host, int32_t B, 
                                             int32_t pitch, int32_t lpad, void* xp, void* stream) {
   const int rc = check_packed_out("esf_stem_pack_u8_crop_ragged", dtype, pitch, lpad, S, C, xp);
   if (rc != ESF_OK) return rc;
-  return crop_ragged<true>("esf_stem_pack_u8_crop_ragged", "crop_frames_ragged_kernel (packed)", frames_host, B, Tsrc,
+  return crop_ragged<true, CropChunk>("esf_stem_pack_u8_crop_ragged", "crop_frames_ragged_kernel (packed)", frames_host, B, Tsrc,
                            C, t_index, T, chan_src, lut32, geom_host, tables_host, crop_yx_host, V, S, pitch, lpad,
                            dtype == ESF_F16, xp, stream);
 }
@@ -383,7 +424,33 @@ extern "C" int esf_frames_to_clip_crop_ragged(const void* frames_host, int32_t B
                                               void* stream) {
   const int rc = check_clip_out("esf_frames_to_clip_crop_ragged", S, clip);
   if (rc != ESF_OK) return rc;
-  return crop_ragged<false>("esf_frames_to_clip_crop_ragged", "crop_frames_ragged_kernel (clip)", frames_host, B, Tsrc,
+  return crop_ragged<false, CropChunk>("esf_frames_to_clip_crop_ragged", "crop_frames_ragged_kernel (clip)", frames_host, B, Tsrc,
                             C, t_index, T, chan_src, lut32, geom_host, tables_host, crop_yx_host, V, S, 0, 0, 0, clip,
                             stream);
+}
+
+extern "C" int esf_stem_pack_u8_crop_videos(const void* frames_host, int32_t B, int32_t C, const int32_t* t_index,
+                                            int32_t T, const int32_t* chan_src, const float* lut32,
+                                            const int32_t* geom_host, const void* tables_host,
+                                            const int32_t* crop_yx_host, int32_t V, int32_t S, int32_t dtype,
+                                            int32_t pitch, int32_t lpad, void* xp, void* stream) {
+  int rc = check_packed_out("esf_stem_pack_u8_crop_videos", dtype, pitch, lpad, S, C, xp);
+  if (rc != ESF_OK) return rc;
+  if ((rc = check_frame_table("esf_stem_pack_u8_crop_videos", t_index)) != ESF_OK) return rc;
+  return crop_ragged<true, CropVideoChunk>("esf_stem_pack_u8_crop_videos", "crop_frames_ragged_kernel (videos, packed)",
+                                           frames_host, B, T, C, t_index, T, chan_src, lut32, geom_host, tables_host,
+                                           crop_yx_host, V, S, pitch, lpad, dtype == ESF_F16, xp, stream);
+}
+
+extern "C" int esf_frames_to_clip_crop_videos(const void* frames_host, int32_t B, int32_t C, const int32_t* t_index,
+                                              int32_t T, const int32_t* chan_src, const float* lut32,
+                                              const int32_t* geom_host, const void* tables_host,
+                                              const int32_t* crop_yx_host, int32_t V, int32_t S, float* clip,
+                                              void* stream) {
+  int rc = check_clip_out("esf_frames_to_clip_crop_videos", S, clip);
+  if (rc != ESF_OK) return rc;
+  if ((rc = check_frame_table("esf_frames_to_clip_crop_videos", t_index)) != ESF_OK) return rc;
+  return crop_ragged<false, CropVideoChunk>("esf_frames_to_clip_crop_videos", "crop_frames_ragged_kernel (videos, clip)",
+                                            frames_host, B, T, C, t_index, T, chan_src, lut32, geom_host, tables_host,
+                                            crop_yx_host, V, S, 0, 0, 0, clip, stream);
 }

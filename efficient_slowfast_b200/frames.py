@@ -18,6 +18,12 @@ Mixed decode sizes (`forward_frames([clip, ...], crop_size=S, spatial_idx=...)`)
 aspect ratios, and the reference's loader resizes and crops every clip on its own before collating the S x S crops.  A
 list of B uint8 clips (T, H_b, W_b, C) of one T and C runs the same crops through one launch per 32 clips
 (esf_*_crop_ragged); the output shapes, hence the plan, are those of a stacked batch of B clips.
+
+Temporal views (`forward_videos([video, ...], fps=...)`): the reference tests every video as TEST.NUM_ENSEMBLE_VIEWS
+temporal clips x TEST.NUM_SPATIAL_CROPS crops.  Its decoder samples temporal clip j out of all decoded frames
+(datasets/decoder.py decode with the whole video decoded: get_start_end_idx + temporal_sampling).  `temporal_index`
+evaluates those expressions here, and the whole video (N, H, W, C) uint8 goes to the device once; the kernel reads
+every view's frames through a per-clip frame table (esf_*_crop_videos).
 """
 import ctypes
 import math
@@ -31,6 +37,40 @@ from . import runtime as rt
 def slow_frame_index(num_frames, alpha):
     """datasets/utils.py:93-102 -- the reference's own expression, so that float rounding of linspace matches."""
     return torch.linspace(0, num_frames - 1, num_frames // alpha).long()
+
+
+def temporal_index(video_size, fps, num_frames, sampling_rate, target_fps, clip_idx, num_clips):
+    """Source frames (int64 [num_frames]) of temporal clip `clip_idx` of `num_clips` out of a video of `video_size`
+    decoded frames at `fps`: datasets/decoder.py decode's clip size, get_start_end_idx at clip_idx / num_clips (the
+    branch of a fully decoded video; the uniform split, which later upstream versions keep as the default of
+    DATA.USE_OFFSET_SAMPLING = False) and temporal_sampling -- the reference's own Python float and torch expressions,
+    so that every rounding matches."""
+    clip_size = sampling_rate * num_frames / target_fps * fps
+    delta = max(video_size - clip_size, 0)
+    start_idx = delta * clip_idx / num_clips
+    end_idx = start_idx + clip_size - 1
+    index = torch.linspace(start_idx, end_idx, num_frames)
+    return torch.clamp(index, 0, video_size - 1).long()
+
+
+def video_frame_tables(video_size, fps, num_frames, sampling_rate, target_fps, num_clips, alpha=None):
+    """int32 tables [num_clips][T_p] of the source frames of every pathway frame of the `num_clips` temporal clips of
+    one video: [slow, fast] (`alpha` given) or [single].  The slow table is pack_pathway_output's linspace gather of the
+    sampled clip, i.e. fast[:, slow_frame_index(num_frames, alpha)]."""
+    fast = torch.stack([temporal_index(video_size, fps, num_frames, sampling_rate, target_fps, j, num_clips)
+                        for j in range(num_clips)]).to(torch.int32)
+    if alpha is None:
+        return [fast]
+    return [fast[:, slow_frame_index(num_frames, alpha)].contiguous(), fast]
+
+
+def ensemble_spatial_views(num_spatial_crops):
+    """The test loader's spatial indices for TEST.NUM_SPATIAL_CROPS (datasets/kinetics.py): idx % n for n > 1, else
+    the centre crop 1."""
+    n = int(num_spatial_crops)
+    if n < 1:
+        raise ValueError("TEST.NUM_SPATIAL_CROPS must be >= 1, got %d" % n)
+    return (1,) if n == 1 else tuple(range(n))
 
 
 def normalization_table(mean, std, channels):
@@ -164,6 +204,38 @@ def check_clips(clips):
     return clip_shapes([tuple(c.shape) for c in clips])
 
 
+def check_videos(videos, fps, num_clips):
+    """Shapes (N, H, W, C) of a list of whole videos and their fps as a list of floats; ValueError unless the videos are
+    contiguous uint8 tensors (N, H, W, C) on one device with N >= 1, one C and rows that fit the crop kernel, every fps
+    is > 0 and num_clips >= 1."""
+    if isinstance(num_clips, bool) or not isinstance(num_clips, (int, np.integer)) or num_clips < 1:
+        raise ValueError("num_clips (temporal views per video) must be an int >= 1, got %r" % (num_clips,))
+    for v in videos:
+        if not isinstance(v, torch.Tensor) or v.dtype != torch.uint8 or v.dim() != 4 or not v.is_contiguous():
+            raise ValueError("forward_videos takes contiguous uint8 videos (N, H, W, C), got %s"
+                             % (("%s %s" % (v.dtype, tuple(v.shape))) if isinstance(v, torch.Tensor) else type(v)))
+    if len({v.device for v in videos}) > 1:
+        raise ValueError("the videos of a list are on one device, got %s" % sorted({str(v.device) for v in videos}))
+    shapes = [tuple(int(n) for n in v.shape) for v in videos]
+    for N, H, W, C in shapes:
+        if min(N, H, W, C) < 1:
+            raise ValueError("empty video of shape %s" % ((N, H, W, C),))
+        if C != shapes[0][3]:
+            raise ValueError("the videos of a list share C: %d next to %d" % (shapes[0][3], C))
+        if W * C > MAX_ROW_BYTES:
+            raise ValueError("video rows of %d x %d bytes exceed the crop kernel's %d" % (W, C, MAX_ROW_BYTES))
+    rates = list(fps) if isinstance(fps, (list, tuple)) else [fps] * len(videos)
+    if len(rates) != len(videos):
+        raise ValueError("%d fps values for %d videos" % (len(rates), len(videos)))
+    out = []
+    for f in rates:
+        if isinstance(f, bool) or not isinstance(f, (int, float, np.integer, np.floating)) or not f > 0 \
+                or not math.isfinite(f):
+            raise ValueError("fps must be a finite number > 0, got %r" % (f,))
+        out.append(float(f))
+    return shapes, out
+
+
 def arena_layout(shapes, capacity=None, align=16):
     """Byte offsets of uint8 clips of `shapes` (T, H, W, C) placed one after another in one buffer, each at a multiple of
     `align` bytes, and the bytes they span.  EsfError when `capacity` (bytes) is given and they need more."""
@@ -218,6 +290,31 @@ class ClipList:
         self.crop_yx = (ctypes.c_int32 * (2 * self.V * self.B))(*[o for t in tables for o in t.crop_yx])
 
 
+class VideoList:
+    """The host arrays of esf_*_crop_videos for the temporal views of whole videos (N_v, H_v, W_v, C): clip
+    v * num_clips + j is temporal clip j of video v, with the video's device address, its geometry (N_v, H0, W0, Hr,
+    Wr), its CropTables and row v * num_clips + j of every pathway's frame table (`tables[v]`, video_frame_tables).
+    `index` is one pinned int32 array, the tables of all pathways one after another, copied to the plan's device
+    buffer by launch_video_list.  Built per call."""
+
+    def __init__(self, videos, crops, tables, num_clips):
+        self.n, self.num_clips = len(videos), num_clips
+        self.B = self.n * num_clips
+        self.C = videos[0].shape[3]
+        self.S, self.V = crops[0].S, len(crops[0].views)
+        rep = [i for i in range(self.n) for _ in range(num_clips)]
+        self.frames = (ctypes.c_void_p * self.B)(*[videos[i].data_ptr() for i in rep])
+        self.geom = (ctypes.c_int32 * (5 * self.B))(*[n for i in rep for n in (videos[i].shape[0], crops[i].H0,
+                                                                                crops[i].W0, crops[i].Hr, crops[i].Wr)])
+        self.tables = (ctypes.c_void_p * (4 * self.B))(*[a for i in rep for a in crops[i].addresses()])
+        self.crop_yx = (ctypes.c_int32 * (2 * self.V * self.B))(*[o for i in rep for o in crops[i].crop_yx])
+        self.T = [int(t.shape[1]) for t in tables[0]]    # frames of every pathway
+        parts = [torch.cat([tab[p] for tab in tables]).reshape(-1) for p in range(len(self.T))]
+        self.index = torch.empty(sum(int(t.numel()) for t in parts), dtype=torch.int32,
+                                 pin_memory=torch.cuda.is_available())
+        torch.cat(parts, out=self.index)
+
+
 class FrameInput:
     """Per-(model, device) state of the frame route: look-up tables and frame indices on the device."""
 
@@ -242,6 +339,7 @@ class FrameInput:
         self.device = device
         self._index = {}
         self._crops = {}
+        self._videos = {}
 
     def crop(self, H0, W0, size, views):
         """CropTables of frames H0 x W0 cropped to size x size at `views` (cached per geometry)."""
@@ -249,6 +347,15 @@ class FrameInput:
         if key not in self._crops:
             self._crops[key] = CropTables(H0, W0, size, tuple(views), self.device)
         return self._crops[key]
+
+    def video_tables(self, video_size, fps, num_frames, sampling_rate, target_fps, num_clips, alpha=None):
+        """video_frame_tables, cached per (video length, fps, ...): a test split repeats few lengths and rates."""
+        key = (video_size, fps, num_frames, sampling_rate, target_fps, num_clips, alpha)
+        if key not in self._videos:
+            if len(self._videos) >= 4096:
+                self._videos.clear()
+            self._videos[key] = video_frame_tables(*key)
+        return self._videos[key]
 
     def index(self, t_src, t_out, alpha):
         """device int32 frame gather for a pathway with t_out of t_src frames (None: identity)."""
@@ -320,3 +427,31 @@ def launch_clip_list(plan, fin, clips, alpha):
                      "esf_stem_pack_u8_crop_ragged")
         else:
             rt.check(L.esf_frames_to_clip_crop_ragged(*args, own.data_ptr(), s), "esf_frames_to_clip_crop_ragged")
+
+
+def launch_video_list(plan, fin, videos):
+    """Fill the stem inputs of `plan` from a VideoList on the current stream: row (v * num_clips + j) * V + s is video
+    v, temporal clip j, crop s.  The frame tables go to a plan-owned device buffer with one copy from pinned memory."""
+    L = rt.lib()
+    s = rt.current_stream_ptr()
+    need = sum(own.shape[0] * own.shape[2] for own in plan.inputs)   # >= B * T_p of every pathway
+    dev = getattr(plan, "video_index", None)
+    if dev is None or dev.numel() < need:
+        dev = plan.video_index = torch.empty(need, dtype=torch.int32, device=plan.inputs[0].device)
+    n = videos.index.numel()
+    assert n <= dev.numel()
+    dev[:n].copy_(videos.index, non_blocking=True)
+    off = 0
+    for own, T in zip(plan.inputs, videos.T):
+        b, c, t, h, w = own.shape
+        assert (b, c, t, h, w) == (videos.B * videos.V, videos.C, T, videos.S, videos.S)
+        args = (videos.frames, videos.B, videos.C, dev[off:].data_ptr(), T, fin.chan_src, fin.lut32.data_ptr(),
+                videos.geom, videos.tables, videos.crop_yx, videos.V, videos.S)
+        off += videos.B * T
+        route = plan.stem_routes.get(own.data_ptr())
+        if route is not None:
+            xp, pitch, lpad = route
+            rt.check(L.esf_stem_pack_u8_crop_videos(*args, rt.dtype_code(xp), pitch, lpad, xp.data_ptr(), s),
+                     "esf_stem_pack_u8_crop_videos")
+        else:
+            rt.check(L.esf_frames_to_clip_crop_videos(*args, own.data_ptr(), s), "esf_frames_to_clip_crop_videos")

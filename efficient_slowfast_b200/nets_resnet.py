@@ -530,6 +530,55 @@ class _PlannedModel(nn.Module):
             out = plan.run_frames(lambda: esf_frames.launch_clip_list(plan, fin, batch, alpha))
             return self._finish(plan, out, None)
 
+    def forward_videos(self, videos, fps=None, num_clips=None, spatial_idx=None, crop_size=None, bboxes=None):
+        """The reference's whole test protocol from decoded videos: every video is tested as `num_clips` temporal clips
+        (default cfg.TEST.NUM_ENSEMBLE_VIEWS) x V crops (default the test loader's views for cfg.TEST.NUM_SPATIAL_CROPS:
+        (0, 1, 2) for 3, (1,) for 1).  Temporal clip j of a video is what the reference's decoder samples when it has
+        decoded the whole video (datasets/decoder.py: get_start_end_idx(N, clip_size, j, num_clips) and
+        temporal_sampling, clip_size = SAMPLING_RATE * NUM_FRAMES / TARGET_FPS * fps); each clip then goes through the
+        loader's normalisation, short-side resize to `crop_size` (default cfg.DATA.TEST_CROP_SIZE), uniform crops and
+        pack_pathway_output, as in forward_frames.  The pyav branch that seeks to a per-clip timestamp window (whose
+        frames depend on the container's keyframes) is not covered.
+
+        `videos`: list of contiguous uint8 videos (N_v, H_v, W_v, C) on one CUDA device, of any length and size, one
+        C.  `fps`: a number or one per video (default cfg.DATA.TARGET_FPS).  Each video is read in place; only the
+        frame tables (a few KB) are uploaded.  The result has len(videos) * num_clips * V rows, row
+        (v * num_clips + j) * V + s being video v, temporal clip j, crop s: the order of the test loader's clip
+        numbering, so TestMeter.update_stats takes the rows with clip ids video_idx * num_clips * V + row.  The plan
+        is that of forward_frames on a stacked batch of len(videos) * num_clips clips, so both routes share it."""
+        from . import frames as esf_frames
+        if self.training:
+            raise NotImplementedError("eval-mode forward path only")
+        if bboxes is not None:
+            raise ValueError("forward_videos takes no bboxes (the boxes would need each view's transform)")
+        if not isinstance(videos, (list, tuple)):
+            raise ValueError("forward_videos takes a list of videos (N, H, W, C), got %s" % type(videos).__name__)
+        cfg = self._cfg
+        target_fps = cfg.DATA.get("TARGET_FPS", 30) if hasattr(cfg.DATA, "get") else cfg.DATA.TARGET_FPS
+        num_clips = cfg.TEST.NUM_ENSEMBLE_VIEWS if num_clips is None else num_clips
+        views = esf_frames.spatial_views(esf_frames.ensemble_spatial_views(cfg.TEST.NUM_SPATIAL_CROPS)
+                                         if spatial_idx is None else spatial_idx)
+        crop_size = int(cfg.DATA.TEST_CROP_SIZE if crop_size is None else crop_size)
+        sizes, rates = esf_frames.check_videos(list(videos), target_fps if fps is None else fps, num_clips)
+        if not sizes:
+            return self._empty(next(self.parameters()).device)
+        two = self.num_pathways > 1
+        T = int(cfg.DATA.NUM_FRAMES)
+        shapes = esf_frames.view_shapes([(T, H, W, C) for _, H, W, C in sizes for _ in range(num_clips)], crop_size,
+                                        views, cfg.SLOWFAST.ALPHA if two else None)
+        dev = videos[0].device
+        if dev.type != "cuda":
+            raise rt.EsfError("the forward path is CUDA-only (sm_100a); got videos on %s -- there is no CPU fallback"
+                              % dev)
+        plan, fin = self._frame_plan(shapes, dev, sizes[0][3])
+        crops = [fin.crop(H, W, crop_size, views) for _, H, W, _ in sizes]
+        tables = [fin.video_tables(N, f, T, int(cfg.DATA.SAMPLING_RATE), target_fps, int(num_clips),
+                                   cfg.SLOWFAST.ALPHA if two else None) for (N, _, _, _), f in zip(sizes, rates)]
+        batch = esf_frames.VideoList(list(videos), crops, tables, int(num_clips))
+        with torch.cuda.device(dev):
+            out = plan.run_frames(lambda: esf_frames.launch_video_list(plan, fin, batch))
+            return self._finish(plan, out, None)
+
     def _empty(self, dev):
         return torch.empty((0, int(self._cfg.MODEL.NUM_CLASSES)), dtype=torch.float32, device=dev)
 

@@ -22,7 +22,7 @@ from . import runtime as rt
 
 class ClipStream:
     def __init__(self, model, shapes, device=None, depth=2, gather=False, frames=False, slow_from_fast=False,
-                 crop_size=None, spatial_idx=None):
+                 crop_size=None, spatial_idx=None, num_clips=None):
         """`depth` staging slots (>= 2 overlaps copy and compute); `gather=True` all-gathers the predictions over the
         process group before the D2H copy, like the reference's test loop.  `frames=True`: every batch is ONE pinned
         uint8 tensor of decoded frames (B, T, H, W, C) (`shapes` = [that shape]) and goes through
@@ -31,6 +31,11 @@ class ClipStream:
         most B pinned uint8 clips (T, H_b, W_b, C) of mixed decode sizes: they are copied to 16-byte aligned offsets
         of the same staging slot (frames.arena_layout; its B * T * H * W * C bytes are the capacity) and run as
         `model.forward_frames(list)`.
+        Video mode, `num_clips` given (frames=True, `shapes` = [(n_max, N_max, H, W, C)]): every batch is a list of at
+        most n_max pinned uint8 videos (N_v, H_v, W_v, C), copied one `copy_` each to 16-byte aligned offsets of a
+        staging slot of n_max * N_max * H * W * C bytes (frames.arena_layout), and run as `model.forward_videos` with
+        `num_clips` temporal views (e.g. TEST.NUM_ENSEMBLE_VIEWS) and the crops of `crop_size` / `spatial_idx`
+        (defaults as there); `submit(videos, fps=...)` gives the frame rates.
         `slow_from_fast=True`: the caller vouches that every batch is what the reference's loader produces,
         `[slow, fast] = pack_pathway_output(cfg, fast)` (datasets/utils.py:93-102: slow = the linspace frame subset of
         fast).  Only the fast clip is then copied to the device and the slow pathway's stem reads its frames out of it
@@ -47,7 +52,19 @@ class ClipStream:
         self.frames = bool(frames)
         assert not self.frames or len(shapes) == 1
         self.crop = None
-        if crop_size is not None or spatial_idx is not None:
+        self.videos = None
+        if num_clips is not None:
+            if not self.frames:
+                raise ValueError("ClipStream: num_clips (video mode) needs frames=True")
+            from . import frames as esf_frames
+            cfg = model._cfg
+            esf_frames.check_videos([], 1.0, num_clips)
+            views = esf_frames.spatial_views(esf_frames.ensemble_spatial_views(cfg.TEST.NUM_SPATIAL_CROPS)
+                                             if spatial_idx is None else spatial_idx)
+            size = int(cfg.DATA.TEST_CROP_SIZE if crop_size is None else crop_size)
+            esf_frames.view_shapes(tuple(shapes[0]), size, views)    # ValueError now rather than at the first batch
+            self.videos = {"num_clips": int(num_clips), "spatial_idx": views, "crop_size": size}
+        elif crop_size is not None or spatial_idx is not None:
             if not self.frames:
                 raise ValueError("ClipStream: crop_size / spatial_idx need frames=True")
             from . import frames as esf_frames
@@ -69,9 +86,14 @@ class ClipStream:
         self.n = 0
         self.h2d_bytes = sum(t.numel() * t.element_size() for t in self.stage[0])
 
-    def submit(self, host_inputs):
-        """Queue one batch (list of pinned host tensors, reference order [slow, fast]).  Never blocks on the batch just
-        queued; when all staging slots are busy it first waits for the oldest batch and returns its (index, preds)."""
+    def submit(self, host_inputs, fps=None):
+        """Queue one batch (list of pinned host tensors, reference order [slow, fast]; in video mode a list of videos
+        and their `fps`).  Never blocks on the batch just queued; when all staging slots are busy it first waits for
+        the oldest batch and returns its (index, preds)."""
+        if fps is not None and self.videos is None:
+            raise ValueError("ClipStream.submit: fps is for video mode (ClipStream(..., num_clips=...))")
+        if self.videos is not None:     # every check before a slot is waited for or a copy is queued
+            video_views = self._video_views(host_inputs, fps)
         finished = None
         if len(self.pending) == self.depth:
             finished = self._pop()
@@ -90,7 +112,10 @@ class ClipStream:
                                           "subset of the fast clip (pack_pathway_output)")
                     self._sff_checked = True
                 host_inputs = host_inputs[1:]
-        if self.crop is not None and host_inputs and all(h.dim() == 4 for h in host_inputs):
+        if self.videos is not None:
+            clips = video_views(self.stage[slot][0])
+            copies, views = list(zip(host_inputs, clips)), [clips]
+        elif self.crop is not None and host_inputs and all(h.dim() == 4 for h in host_inputs):
             clips = self._clip_views(host_inputs, self.stage[slot][0])   # clips of mixed decode sizes
             copies, views = list(zip(host_inputs, clips)), [clips]
         else:
@@ -107,7 +132,9 @@ class ClipStream:
                 d.copy_(h, non_blocking=True)
             self.ready[slot].record(self.copy_stream)
         cur.wait_event(self.ready[slot])
-        if self.frames:
+        if self.videos is not None:
+            out = self.model.forward_videos(views[0], fps=fps, **self.videos)
+        elif self.frames:
             out = self.model.forward_frames(views[0], **(self.crop or {}))
         elif self.slow_from_fast:
             out = self.model.forward_fast(views[0])
@@ -137,6 +164,24 @@ class ClipStream:
         flat = stage.view(-1)
         offsets, _ = esf_frames.arena_layout(sizes, flat.numel())
         return [flat[o:o + math.prod(sh)].view(sh) for o, sh in zip(offsets, sizes)]
+
+    def _video_views(self, videos, fps):
+        """Checks a list of videos (N, H, W, C) for video mode and returns the function that gives, for a staging
+        slot, the views they are copied to at the offsets of frames.arena_layout.  ValueError / EsfError before any
+        copy when the list is not valid for forward_videos or exceeds the slot's n_max videos or its bytes."""
+        from . import frames as esf_frames
+        stage = self.stage[0][0]
+        videos = list(videos)
+        if len(videos) > stage.shape[0]:
+            raise rt.EsfError("ClipStream was built for batches of at most %d videos, got %d"
+                              % (stage.shape[0], len(videos)))
+        cfg = self.model._cfg
+        sizes, _ = esf_frames.check_videos(videos, 1.0 if fps is None else fps, self.videos["num_clips"])
+        if sizes:
+            esf_frames.view_shapes([(cfg.DATA.NUM_FRAMES,) + sh[1:] for sh in sizes], self.videos["crop_size"],
+                                   self.videos["spatial_idx"])
+        offsets, _ = esf_frames.arena_layout(sizes, stage.numel())
+        return lambda slot_stage: [slot_stage.view(-1)[o:o + math.prod(sh)].view(sh) for o, sh in zip(offsets, sizes)]
 
     def _pop(self):
         index, slot, rows = self.pending.pop(0)

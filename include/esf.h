@@ -176,6 +176,21 @@ int esf_frames_to_clip_crop_ragged(const void* frames_host, int32_t B, int32_t T
                                    int32_t T, const int32_t* chan_src, const float* lut32, const int32_t* geom_host,
                                    const void* tables_host, const int32_t* crop_yx_host, int32_t V, int32_t S,
                                    float* clip, void* stream);
+/* Temporal views of whole videos (the reference's test loader: NUM_ENSEMBLE_VIEWS temporal clips per video, each then
+ * resized and cropped as above).  Clip b is one (video, temporal view) pair: frames_host[b] is the device address of
+ * its video (Tsrc_b, H0_b, W0_b, C) uint8, and views of one video share that address.  geom_host: host int32[B][5],
+ * (Tsrc, H0, W0, Hr, Wr) of every clip; t_index: DEVICE int32[B][T], row b the source frames of clip b (required;
+ * every entry is clamped to [0, Tsrc_b - 1]); tables_host and crop_yx_host as for the ragged entry points.  Output row
+ * b * V + v is clip b at view v.  Every clip is checked before anything is launched; the host arrays are read before
+ * the call returns. */
+int esf_stem_pack_u8_crop_videos(const void* frames_host, int32_t B, int32_t C, const int32_t* t_index, int32_t T,
+                                 const int32_t* chan_src, const float* lut32, const int32_t* geom_host,
+                                 const void* tables_host, const int32_t* crop_yx_host, int32_t V, int32_t S,
+                                 int32_t dtype, int32_t pitch, int32_t lpad, void* xp, void* stream);
+int esf_frames_to_clip_crop_videos(const void* frames_host, int32_t B, int32_t C, const int32_t* t_index, int32_t T,
+                                   const int32_t* chan_src, const float* lut32, const int32_t* geom_host,
+                                   const void* tables_host, const int32_t* crop_yx_host, int32_t V, int32_t S,
+                                   float* clip, void* stream);
 int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int32_t T, int32_t H, int32_t W, int32_t pitch,
                           const void* w_band, const float* bias_tiled, int32_t Cout, int32_t kT, int32_t kH,
                           int32_t kW, int32_t sH, int32_t sW, int32_t pT, int32_t pH, int32_t pW, int32_t act,
