@@ -206,6 +206,48 @@ def fold_time_groups(t, group):
                         (t.stride(1) * (T // group), t.stride(1), t.stride(2), t.stride(3), 1), t.storage_offset())
 
 
+def conv_weight_bias(conv):
+    """A conv's weight and bias as FP64 host tensors."""
+    return host64(conv.weight), host64(conv.bias)
+
+
+def nonlocal_offset(nln, d, npad_d):
+    """The per-channel offset mu of Plan.nonlocal_block's last product: least-squares solution of
+    conv_out.weight mu = bn.running_mean - conv_out.bias.  Returns mu as FP64 (the FP32-rounded value actually
+    subtracted) and the FP32 bias [npad_d] of that product, -mu padded with zeros."""
+    C = nln.conv_out.weight.shape[0]
+    w_out = host64(nln.conv_out.weight).reshape(C, d)
+    rhs = (host64(nln.bn.running_mean) - host64(nln.conv_out.bias)).reshape(C, 1)
+    mu = torch.linalg.lstsq(w_out, rhs).solution.reshape(d)
+    bias2 = torch.zeros(npad_d, dtype=torch.float32)
+    bias2[:d] = (-mu).to(torch.float32)
+    return -bias2[:d].to(torch.float64), bias2
+
+
+def _shape_only(x):
+    """Host tensors of a weight-preparation result as meta tensors of the same shape and dtype (device tensors and
+    other values as they are)."""
+    if isinstance(x, tuple):
+        return tuple(_shape_only(v) for v in x)
+    if isinstance(x, torch.Tensor) and x.device.type == "cpu":
+        return torch.empty_like(x, device="meta")
+    return x
+
+
+class Family:
+    """What the plans of one per-clip input shape share when cfg.ESF.MAX_BATCH is set.  The CAPACITY plan, compiled at
+    the largest batch, records every device tensor it allocates (Plan.alloc) and every result of its host weight
+    preparation (Plan.once), in call order.  A VARIANT, compiled later at a smaller batch, replays both lists: it
+    allocates no activation arena and folds no weights.  It keeps its own op handles, metadata and CUDA graph.  The
+    family also holds the run-time state of its plans (Plan.shared): frame-route tables and the detection rows."""
+
+    def __init__(self):
+        self.allocs = []      # (tensor, zero, flat) of every Plan.alloc of the capacity plan
+        self.memo = []        # (function name, result) of every Plan.once of the capacity plan
+        self.built = False    # the capacity plan is compiled: every later plan of the family is a variant
+        self.roi_feat = self.roi_out = None
+
+
 def head_fc_launches(B, cin, K, act):
     """Kernel launches of one esf_head_fc call: the tiled kernel (B >= 8, or rows too long for one block) applies the
     class softmax in a second, tiny kernel."""
@@ -219,8 +261,12 @@ class Plan:
 
     wfold = True     # thin layers (C_in <= 32) as W-folded banded GEMMs
 
-    def __init__(self, device, precision="bf16"):
+    def __init__(self, device, precision="bf16", family=None):
         self.device = device
+        self.family = family
+        self.variant = family is not None and family.built
+        self.variants = {}    # capacity plan of a family: batch rows -> variant plan
+        self._n_alloc = self._n_memo = 0     # variant: position in the family's lists
         self.precision = precision
         self.adt = rt.TORCH_DTYPE[precision]      # 16-bit storage format of activations / tensor-core operands
         self.a16 = rt.dtype_code(self.adt)
@@ -241,6 +287,64 @@ class Plan:
         self._scratch = {}    # (shape, dtype, zero) -> tensor shared by the ops of this plan (scratch())
 
     # ---------------------------------------------------------------- memory
+    @property
+    def shared(self):
+        """Holder of the run-time state (frame tables, detection rows) of this plan: its family, else the plan."""
+        return self.family if self.family is not None else self
+
+    def alloc(self, shape, dtype, zero=False, flat=False):
+        """Every device tensor a plan allocates while it is compiled comes from here (zero-filled with `zero`).  A
+        variant of a Family allocates nothing: its i-th call resolves to the capacity plan's i-th tensor -- that tensor
+        itself when the shape does not depend on the batch, its first rows when only dim 0 does (zero-filled state thus
+        keeps its per-clip layout), and a prefix of it for `flat` scratch: 1-D, written before it is read, of a size
+        that grows with the batch.  Any other mismatch is an error."""
+        shape = tuple(int(n) for n in shape)
+        assert not (zero and flat), "flat scratch is written before it is read"
+        if not self.variant:
+            t = (torch.zeros if zero else torch.empty)(shape, dtype=dtype, device=self.device)
+            self.keep.append(t)
+            if self.family is not None:
+                self.family.allocs.append((t, bool(zero), bool(flat)))
+            return t
+        allocs = self.family.allocs
+        assert self._n_alloc < len(allocs), "a variant allocates more tensors than its capacity plan"
+        t, z, f = allocs[self._n_alloc]
+        self._n_alloc += 1
+        same = t.dtype == dtype and z == bool(zero) and f == bool(flat) and len(shape) == t.dim()
+        if same and shape == tuple(t.shape):
+            return t
+        if same and (t.dim() > 1 or flat) and shape[1:] == tuple(t.shape[1:]) and shape[0] <= t.shape[0]:
+            return t[:shape[0]]
+        raise AssertionError("allocation %d of a variant, %s %s (zero=%s, flat=%s), does not fit the capacity plan's "
+                             "%s %s (zero=%s, flat=%s)" % (self._n_alloc - 1, shape, dtype, zero, flat,
+                                                           tuple(t.shape), t.dtype, z, f))
+
+    def once(self, fn, *args):
+        """fn(*args), for host-side weight preparation (folding, packing, uploads).  A variant of a Family does not run
+        it: it gets the capacity plan's result of the same call, by call order -- device tensors themselves, host
+        tensors as meta tensors of their shape (a variant's host code reads only the shapes of folded weights)."""
+        if not self.variant:
+            out = fn(*args)
+            if self.family is not None:
+                self.family.memo.append((fn.__name__, _shape_only(out)))
+            return out
+        memo = self.family.memo
+        assert self._n_memo < len(memo), "a variant prepares more weights than its capacity plan"
+        name, out = memo[self._n_memo]
+        self._n_memo += 1
+        assert name == fn.__name__, "weight preparation %d: the variant calls %s, the capacity plan called %s" % (
+            self._n_memo - 1, fn.__name__, name)
+        return out
+
+    def end_compile(self):
+        """A family's plan is compiled: the capacity plan's lists are complete, a variant has used all of them."""
+        if self.variant:
+            assert (self._n_alloc, self._n_memo) == (len(self.family.allocs), len(self.family.memo)), \
+                "a variant made %d allocations and %d weight preparations, its capacity plan %d and %d" % (
+                    self._n_alloc, self._n_memo, len(self.family.allocs), len(self.family.memo))
+        elif self.family is not None:
+            self.family.built = True
+
     def act(self, B, T, H, W, C, name=None, dtype=None, role=None):
         """role: a hint for the FP32-accurate plan (engine_fp32.PrecisePlan.act); 16-bit activations have one form."""
         dtype = dtype or self.adt
@@ -248,8 +352,7 @@ class Plan:
         # buffer -- also with C = 27, 36, 180, 540 ... of the efficient backbones -- is addressable by TMA and by
         # 16-byte vector accesses; the logical tensor is the [..., :C] view
         Cp = C if (dtype != self.adt or C < 8) else (C + 7) // 8 * 8
-        t = torch.empty((B, T, H, W, Cp), dtype=dtype, device=self.device)
-        self.keep.append(t)
+        t = self.alloc((B, T, H, W, Cp), dtype)
         if Cp != C:
             self.padded[t.data_ptr()] = (C, Cp)     # channels [C, Cp) of every row are padding owned by this tensor
             t = t[..., :C]
@@ -270,6 +373,9 @@ class Plan:
 
     def tensor(self, t, dtype=torch.float32):
         """Plan-lifetime device copy of a (small) parameter-derived tensor; host tensors are converted on the host."""
+        return self.once(self._upload, t, dtype)
+
+    def _upload(self, t, dtype):
         if t.device.type == "cpu":
             t = to_device(t, self.device, dtype)
         else:
@@ -351,7 +457,7 @@ class Plan:
     # ---------------------------------------------------------------- ops
     def conv_igemm(self, x, y, w_folded, bias, stride=(1, 1, 1), padding=(0, 0, 0), dilation=(1, 1, 1), act=rt.ACT_NONE,
                    res=None, out_dtype=None):
-        wp, bp = pack_igemm_weight(w_folded, bias, self.device, self.adt)
+        wp, bp = self.once(pack_igemm_weight, w_folded, bias, self.device, self.adt)
         kt, kh, kw = w_folded.shape[2:]
         h = self._create("esf_conv_igemm_create",
                          self._conv_desc(x, y, res, wp, bp, (kt, kh, kw), stride, padding, dilation, 1, act))
@@ -375,19 +481,17 @@ class Plan:
         self._launch("esf_op_launch", h, kind=kind, label=label, flops=2.0 * m * cout * cin,
                      nbytes=self._nbytes(x, y) + x.shape[0] * cout * cin * 2)
 
-    def scratch(self, shape, dtype, zero=False):
+    def scratch(self, shape, dtype, zero=False, flat=False):
         """Plan-lifetime scratch tensor shared by every op that asks for the same (shape, dtype): the launches of a
-        plan are serialised on one stream, so the Non-local blocks of a model reuse one affinity matrix."""
-        key = (tuple(shape), dtype, bool(zero))
+        plan are serialised on one stream, so the Non-local blocks of a model reuse one affinity matrix.  `zero`,
+        `flat`: as in alloc."""
+        key = (tuple(shape), dtype, bool(zero), bool(flat))
         if key not in self._scratch:
-            t = (torch.zeros if zero else torch.empty)(tuple(shape), dtype=dtype, device=self.device)
-            self.keep.append(t)
-            self._scratch[key] = t
+            self._scratch[key] = self.alloc(shape, dtype, zero, flat)
         return self._scratch[key]
 
-    @staticmethod
-    def _weight_bias(conv):
-        return host64(conv.weight), host64(conv.bias)
+    def _weight_bias(self, conv):
+        return self.once(conv_weight_bias, conv)
 
     def _nonlocal_keys(self, x, nln):
         """Key side of a Non-local block on the (group-folded) input x: x max-pooled by nln.pool_size when nln.use_pool,
@@ -418,7 +522,6 @@ class Plan:
             x, y = fold_time_groups(x, group), fold_time_groups(y, group)
         B, T, H, W, C = x.shape
         d = nln.dim_inner
-        f64 = torch.float64
         xp, softmax = self._nonlocal_keys(x, nln)
         Tp, Hp, Wp = xp.shape[1:4]
         Nq, Nk = T * H * W, Tp * Hp * Wp
@@ -428,13 +531,8 @@ class Plan:
         # amplified by |mean| / std.  conv_out is linear, so a per-channel offset mu can be subtracted in the FP32
         # epilogue of the last product (its bias) and added back through conv_out's bias: W (att - mu) + (W mu + b).
         # mu = least-squares solution of W mu = running_mean - b, the att-space mean the BN statistics imply.
-        w_out = host64(nln.conv_out.weight).reshape(C, d)
-        rhs = (host64(nln.bn.running_mean) - host64(nln.conv_out.bias)).reshape(C, 1)
-        mu = torch.linalg.lstsq(w_out, rhs).solution.reshape(d)
         _, _, _, npad_d = rt.igemm_geometry(Nk if softmax else d, d)
-        bias2_h = torch.zeros(npad_d, dtype=torch.float32)
-        bias2_h[:d] = (-mu).to(torch.float32)
-        mu = -bias2_h[:d].to(f64)                    # the value actually subtracted (FP32-rounded)
+        mu, bias2_h = self.once(nonlocal_offset, nln, d, npad_d)
         bias2 = self.tensor(bias2_h)
         att = self.act(B, T, H, W, d)
 
@@ -443,7 +541,7 @@ class Plan:
             GEMM that contracts over the keys."""
             kc, kch, _, npad = rt.igemm_geometry(Nk, d)
             kpad = kc * kch
-            tT = torch.zeros((B, npad, kpad), dtype=self.adt, device=self.device)
+            tT = self.alloc((B, npad, kpad), self.adt, zero=True)
             self._launch("esf_transpose16", t, B, Nk, d, t.stride(0), t.stride(3), tT, npad * kpad, kpad,
                          kind="nl_transpose", label=name, nbytes=2 * self._nbytes(t))
             return tT
@@ -454,10 +552,9 @@ class Plan:
             assert kc1 * kch1 == d, "dim_inner must fill whole K chunks"
             theta = self.act(B, T, H, W, d)
             self.conv(x, theta, *wb(nln.conv_theta))
-            phi_rows = torch.zeros((B, npad1, d), dtype=self.adt, device=self.device)
+            phi_rows = self.alloc((B, npad1, d), self.adt, zero=True)
             phi = phi_rows.as_strided((B, Tp, Hp, Wp, d), (npad1 * d, Hp * Wp * d, Wp * d, d, 1))
             g = self.act(B, Tp, Hp, Wp, d)
-            self.keep += [phi_rows]
             self.conv(xp, phi, *wb(nln.conv_phi))
             self.conv(xp, g, *wb(nln.conv_g))
             gT = transposed(g, "g")
@@ -486,20 +583,19 @@ class Plan:
             wg, bg = wb(nln.conv_g)
             self.conv(xp, g, wg / Nk, bg / Nk)
             phiT, gT = transposed(phi, "phi"), transposed(g, "g")
-            MT = torch.zeros((B, 1, 1, d, d), dtype=self.adt, device=self.device)
-            self.keep.append(MT)
+            MT = self.alloc((B, 1, 1, d, d), self.adt, zero=True)
             zero_d = self.scratch((d,), torch.float32, zero=True)
             kpad = gT.shape[2]
             gT_act = gT.as_strided((B, 1, 1, d, Nk), (gT.stride(0), d * kpad, d * kpad, kpad, 1))
             self.gemm_rows(gT_act, MT, phiT, zero_d, "nl_gemm", "g^T.phi d=%d Nk=%d" % (d, Nk))
             self.gemm_rows(theta, att, MT.reshape(B, d, d), bias2, "nl_gemm", "theta.M N=%d d=%d" % (Nq, d))
-        w, bias = fold_conv_bn(nln.conv_out.weight, nln.conv_out.bias, nln.bn)
+        w, bias = self.once(fold_conv_bn, nln.conv_out.weight, nln.conv_out.bias, nln.bn)
         bias = bias + w.reshape(C, d) @ mu
         self.conv(att, y, w, bias, res=x)
 
     def conv_wfold(self, x, y, w_folded, bias, WB, stride=(1, 1, 1), padding=(0, 0, 0), act=rt.ACT_NONE, res=None):
         """Thin-layer (C_in <= 32) conv as a W-folded banded GEMM: see esf_conv_wfold_create."""
-        wp, bp = pack_wfold_band(w_folded, bias, WB, stride[2], self.device, self.adt)
+        wp, bp = self.once(pack_wfold_band, w_folded, bias, WB, stride[2], self.device, self.adt)
         kt, kh, kw = w_folded.shape[2:]
         h = self._create("esf_conv_wfold_create",
                          self._conv_desc(x, y, res, wp, bp, (kt, kh, kw), stride, padding, act=act), WB)
@@ -630,9 +726,9 @@ class Plan:
         cout = w_folded.shape[0]
         kt, kh, kw = w_folded.shape[2:]
         if twb:
-            wb, bt = pack_stem_tband(w_folded, bias, twb, stride[2], self.device, self.adt)
+            wb, bt = self.once(pack_stem_tband, w_folded, bias, twb, stride[2], self.device, self.adt)
         else:
-            wb, bt = pack_stem_band(w_folded, bias, stride[2], self.device, self.adt)
+            wb, bt = self.once(pack_stem_band, w_folded, bias, stride[2], self.device, self.adt)
         h = self._create("esf_stem_tband_create" if twb else "esf_stem_igemm_create", xp, B, Cin, T, H, W, pitch, wb, bt,
                          cout, kt, kh, kw, stride[1], stride[2], padding[0], padding[1], padding[2], act, y)
         label = "%dx%dx%d %d->%d %s" % (kt, kh, kw, Cin, cout, "t-band" if twb else "banded")
@@ -644,8 +740,7 @@ class Plan:
         """Stem on the tensor cores: the clip is packed into 16-bit rows (`pitch`, `lpad`: esf_stem_geometry), then one
         GEMM -- temporal-band for twb > 0, banded for twb == 0 (see stem_route)."""
         B, Cin, T, H, W = x_nc.shape
-        xp = torch.empty((B, T, H, pitch), dtype=self.adt, device=self.device)
-        self.keep.append(xp)
+        xp = self.alloc((B, T, H, pitch), self.adt)
         self.stem_routes[x_nc.data_ptr()] = (xp, pitch, lpad)   # the uint8 frame route writes xp itself (frames.py)
 
         def pack(s):
@@ -676,9 +771,9 @@ class Plan:
         -> channel scale.  Reuses the head kernels for the pooled MLP."""
         B, C = x.shape[0], x.shape[4]
         R = se.conv_reduce.out_channels
-        feat = torch.empty((B, C), dtype=torch.float32, device=self.device)
-        hid = torch.empty((B, R), dtype=torch.float32, device=self.device)
-        gate = torch.empty((B, C), dtype=torch.float32, device=self.device)
+        feat = self.alloc((B, C), torch.float32)
+        hid = self.alloc((B, R), torch.float32)
+        gate = self.alloc((B, C), torch.float32)
         w1, b1 = self.tensor(se.conv_reduce.weight.reshape(R, C)), self.tensor(se.conv_reduce.bias)
         w2, b2 = self.tensor(se.conv_expand.weight.reshape(C, R)), self.tensor(se.conv_expand.bias)
         self.global_mean(x, feat, C, 0, "se_pool")
@@ -691,7 +786,7 @@ class Plan:
         single-block head kernel for the small ones."""
         B, T, H, W, C = x.shape
         if T * H * W >= 1024 and (C % 8 == 0 or C <= 256):
-            scratch = self.scratch((self._size("esf_global_mean_scratch_floats", B, C),), torch.float32)
+            scratch = self.scratch((self._size("esf_global_mean_scratch_floats", B, C),), torch.float32, flat=True)
             self._launch("esf_global_mean", x, scratch, feat, feat_stride, feat_off, kind=kind, label="two-pass",
                          nbytes=self._nbytes(x), launches=2)
         else:
@@ -704,11 +799,11 @@ class Plan:
 
     def _eca_fuse(self, fn_name, scratch_fn_name, kind, x_fast, y_slice, alpha, eca_weight, bn):
         """eca_fuse on the entry point `fn_name` (the 16-bit one or its FP32 form) and its partial-sum scratch."""
-        scale, shift = bn_affine(bn)
+        scale, shift = self.once(bn_affine, bn)
         w = self.tensor(eca_weight.reshape(-1))
         sc, sh = self.tensor(scale), self.tensor(shift)
         B, C = x_fast.shape[0], x_fast.shape[4]
-        scratch = torch.empty(self._size(scratch_fn_name, B, C), dtype=torch.float32, device=self.device)
+        scratch = self.alloc((self._size(scratch_fn_name, B, C),), torch.float32, flat=True)
         self._launch(fn_name, x_fast, alpha, w, int(w.numel()), sc, sh, scratch, y_slice, kind=kind, label="C=%d" % C,
                      nbytes=2 * self._nbytes(x_fast) + self._nbytes(y_slice), launches=2)
 
@@ -717,10 +812,10 @@ class Plan:
         [x_d | q | k | v], and the (B, T, H, W, d, gamma, bn scale, bn shift, alpha) arguments that every attention entry
         point takes after its operand."""
         B, T, H, W, C = x_slow.shape
-        w_all, b_all, d = attention_projection(w_down, att)
+        w_all, b_all, d = self.once(attention_projection, w_down, att)
         proj = self.act(B, T, H, W, 4 * d, dtype=torch.float32)
         self.conv(x_slow, proj, w_all, b_all)
-        scale, shift = bn_affine(bn)
+        scale, shift = self.once(bn_affine, bn)
         sc, sh = self.tensor(scale), self.tensor(shift)
         gamma = float(att.gamma.detach().float().item())
         return proj, (B, T, H, W, d, gamma, sc, sh, alpha)
@@ -742,7 +837,7 @@ class Plan:
         if d > 128:
             return self._attention_generic(proj, geo, y_slice)
         nbytes = self._size("esf_attn_tc_pack_bytes", B, N, d)
-        packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        packed = self.alloc((nbytes,), torch.uint8, flat=True)
         h = self._create("esf_attn_tc_create", packed, *geo, y_slice)
         self._launch("esf_attn_tc_pack", proj, B, N, d, self.a16, packed, kind="attn_pack", label="N=%d d=%d" % (N, d),
                      nbytes=self._nbytes(proj) + nbytes)
@@ -753,8 +848,8 @@ class Plan:
         B = xs[0].shape[0]
         cin = sum(x.shape[4] for x in xs)
         K = weight.shape[0]
-        feat = torch.empty((B, cin), dtype=torch.float32, device=self.device)
-        out = torch.empty((B, K), dtype=torch.float32, device=self.device)
+        feat = self.alloc((B, cin), torch.float32)
+        out = self.alloc((B, K), torch.float32)
         w, b = self.tensor(weight), self.tensor(bias)
         self._head_pool(xs, feat)
         self._head_fc(feat, w, b, act, out, flops=2.0 * B * cin * K, nbytes=self._nbytes(feat, w, out))
@@ -797,7 +892,7 @@ class Plan:
                                      y.storage_offset()))
         per_pos = self.head(rows, weight, bias, act)
         K = weight.shape[0]
-        out = torch.empty((B, K), dtype=torch.float32, device=self.device)
+        out = self.alloc((B, K), torch.float32)
         self._launch("esf_group_mean", per_pos, B, P, K, out, kind="head_mean", label="P=%d" % P,
                      nbytes=self._nbytes(per_pos, out))
         self.out = out
@@ -808,14 +903,14 @@ class Plan:
         the `avg_pool3d -> conv_head_{slow,fast} -> ReLU` tail of GhostNetBasicHead (head_helper.py:676-688)."""
         B, C = x.shape[0], x.shape[4]
         K = weight.shape[0]
-        feat = torch.empty((B, C), dtype=torch.float32, device=self.device)
+        feat = self.alloc((B, C), torch.float32)
         w, b = self.tensor(weight.reshape(K, C)), self.tensor(bias)
         self._head_pool([x], feat)
         self._head_fc(feat, w, b, act, out, out_stride)
 
     def fc(self, feat, weight, bias, act):
         """out = act(feat @ weight^T + bias) on FP32 rows (final classifier of the GhostNet head)."""
-        out = torch.empty((feat.shape[0], weight.shape[0]), dtype=torch.float32, device=self.device)
+        out = self.alloc((feat.shape[0], weight.shape[0]), torch.float32)
         self._head_fc(feat, self.tensor(weight), self.tensor(bias), act, out)
         self.out = out
         return out
@@ -824,7 +919,7 @@ class Plan:
         """ResNetRoIHead's temporal AvgPool3d([T, 1, 1]) where it leaves one frame: 16-bit (B, T, H, W, C) -> dense FP32
         (B, H, W, C) map, the input of esf_roi_align_max.  A graph op: it reads plan-owned activations only."""
         B, T, H, W, C = x.shape
-        y = torch.empty((B, H, W, C), dtype=torch.float32, device=self.device)
+        y = self.alloc((B, H, W, C), torch.float32)
         self._launch("esf_temporal_mean", x, y, kind="roi_tpool", label="T=%d C=%d @%s" % (T, C, (H, W)),
                      nbytes=self._nbytes(x, y))
         return y
@@ -841,23 +936,25 @@ class Plan:
     def run_boxes(self, boxes):
         """`boxes`: (K, 5) contiguous FP32 on this plan's device, K >= 1, rows [batch index, x1, y1, x2, y2].  Launches
         esf_roi_align_max per pathway (both write slices of the same feature row) and esf_head_fc on the current
-        stream; the feat / out buffers grow to the largest K seen and are reused.  Returns a view of the first K rows."""
+        stream; the feat / out buffers grow to the largest K seen and are reused (by every plan of a Family).  Returns a
+        view of the first K rows."""
         r = self.roi
         K = boxes.shape[0]
-        if self.roi_out is None or self.roi_out.shape[0] < K:
-            self.roi_feat = torch.empty((K, r["cin"]), dtype=torch.float32, device=self.device)
-            self.roi_out = torch.empty((K, r["ncls"]), dtype=torch.float32, device=self.device)
+        rows = self.shared
+        if rows.roi_out is None or rows.roi_out.shape[0] < K:
+            rows.roi_feat = torch.empty((K, r["cin"]), dtype=torch.float32, device=self.device)
+            rows.roi_out = torch.empty((K, r["ncls"]), dtype=torch.float32, device=self.device)
         L = rt.lib()
         s = rt.current_stream_ptr()
         off = 0
         for m, scale, res in zip(r["maps"], r["scales"], r["res"]):
             B, H, W, C = m.shape
             rt.check(L.esf_roi_align_max(m.data_ptr(), B, H, W, C, boxes.data_ptr(), K, scale, res, r["aligned"],
-                                         self.roi_feat.data_ptr(), r["cin"], off, s), "esf_roi_align_max")
+                                         rows.roi_feat.data_ptr(), r["cin"], off, s), "esf_roi_align_max")
             off += C
-        rt.check(L.esf_head_fc(self.roi_feat.data_ptr(), K, r["cin"], r["cin"], r["w"].data_ptr(), r["b"].data_ptr(),
-                               r["ncls"], r["act"], self.roi_out.data_ptr(), r["ncls"], s), "esf_head_fc")
-        return self.roi_out[:K]
+        rt.check(L.esf_head_fc(rows.roi_feat.data_ptr(), K, r["cin"], r["cin"], r["w"].data_ptr(), r["b"].data_ptr(),
+                               r["ncls"], r["act"], rows.roi_out.data_ptr(), r["ncls"], s), "esf_head_fc")
+        return rows.roi_out[:K]
 
     # ---------------------------------------------------------------- execution
     def launch_all(self):

@@ -82,11 +82,24 @@ def split_weight_rows(w):
     return hi, lo, 1.0 / s
 
 
+def split_operand_weight(w, plane, c0):
+    """Folded FP64 weight (Cout, Cin, kT, kH, kW) of a conv that reads channels [c0, c0 + Cin) of every [hi|lo|hi] plane
+    of a buffer of plane width `plane` -> the [w_hi | w_hi | w_lo] weight over the whole 3 * plane channels (zero
+    elsewhere) and the inv_scale of split_weight_rows."""
+    cout, cin = w.shape[:2]
+    hi, lo, inv_scale = split_weight_rows(w)
+    w3 = torch.zeros((cout, 3 * plane) + tuple(w.shape[2:]), dtype=torch.float64)
+    w3[:, c0:c0 + cin] = hi
+    w3[:, plane + c0:plane + c0 + cin] = hi
+    w3[:, 2 * plane + c0:2 * plane + c0 + cin] = lo
+    return w3, inv_scale
+
+
 class PrecisePlan(Plan):
     wfold = False    # the banded thin-layer GEMM has no FP32 output; every conv is the plain igemm
 
-    def __init__(self, device, precision="fp32"):
-        super().__init__(device, precision="fp32")
+    def __init__(self, device, precision="fp32", family=None):
+        super().__init__(device, precision="fp32", family=family)
         self.precise = True
 
     # ---------------------------------------------------------------- memory
@@ -98,10 +111,10 @@ class PrecisePlan(Plan):
         assert role in (None, "operand", "residual") and not (name and role)
         plane = (C + 7) // 8 * 8
         has_f32, has_planes = role != "operand", role != "residual"
-        f32 = torch.empty((B, T, H, W, C), dtype=torch.float32, device=self.device if has_f32 else "meta")
+        f32 = (self.alloc((B, T, H, W, C), torch.float32) if has_f32 else
+               torch.empty((B, T, H, W, C), dtype=torch.float32, device="meta"))
         # zero-filled: the row padding [C, plane) of every plane meets zero weights in the GEMM and must stay finite
-        x3 = torch.zeros((B, T, H, W, 3 * plane), dtype=torch.float16, device=self.device) if has_planes else None
-        self.keep += [f32, x3]
+        x3 = self.alloc((B, T, H, W, 3 * plane), torch.float16, zero=True) if has_planes else None
         if name:
             self.buffers[name] = f32
         return Act32(f32, x3, plane, 0, C, has_f32=has_f32, has_planes=has_planes)
@@ -140,13 +153,8 @@ class PrecisePlan(Plan):
         w = w_folded.to(torch.float64)
         cout, cin = w.shape[:2]
         assert cin == x.shape[4]
-        hi, lo, inv_scale = split_weight_rows(w)
         # the GEMM reads the WHOLE parent buffer: a channel slice (x_s of a concat buffer) gets zero weights elsewhere
-        plane = x.plane
-        w3 = torch.zeros((cout, 3 * plane) + tuple(w.shape[2:]), dtype=torch.float64)
-        w3[:, x.c0:x.c0 + cin] = hi
-        w3[:, plane + x.c0:plane + x.c0 + cin] = hi
-        w3[:, 2 * plane + x.c0:2 * plane + x.c0 + cin] = lo
+        w3, inv_scale = self.once(split_operand_weight, w, x.plane, x.c0)
         yshape = tuple(y.shape)
         acc = self.scratch(yshape, torch.float32)
         zero = torch.zeros(cout, dtype=torch.float64)
@@ -167,7 +175,7 @@ class PrecisePlan(Plan):
         pitch, lpad, twb = route
         B, Cin, T, H, W = x_nc.shape
         cout = w_folded.shape[0]
-        hi, lo, inv_scale = split_weight_rows(w_folded.to(torch.float64))
+        hi, lo, inv_scale = self.once(split_weight_rows, w_folded.to(torch.float64))
         zero = torch.zeros(cout, dtype=torch.float64)
 
         def pack(fn_name, xp):      # reads the caller's clip: its pointer is looked up at launch time
@@ -175,13 +183,11 @@ class PrecisePlan(Plan):
 
         xps, accs = [], []
         for fn_name, part in (("esf_stem_pack", "hi"), ("esf_stem_pack_lo", "lo")):
-            xp = torch.empty((B, T, H, pitch), dtype=torch.float16, device=self.device)
-            self.keep.append(xp)
+            xp = self.alloc((B, T, H, pitch), torch.float16)
             self._add(pack(fn_name, xp), "stem_pack", part, nbytes=self._nbytes(x_nc, xp), eager=True)
             xps.append(xp)
         for name, xp, wpart in (("hi.hi", xps[0], hi), ("lo.hi", xps[1], hi), ("hi.lo", xps[0], lo)):
-            acc = torch.empty(tuple(y.shape), dtype=torch.float32, device=self.device)
-            self.keep.append(acc)
+            acc = self.alloc(tuple(y.shape), torch.float32)
             self._stem_gemm_op(xp, x_nc.shape, acc, wpart, zero, stride, padding, rt.ACT_NONE, pitch, twb, name)
             accs.append(acc)
         self._launch("esf_p32_post3", *accs, self.tensor(inv_scale), self.tensor(bias), act, y.f32, y.hi, y.plane,
@@ -216,8 +222,8 @@ class PrecisePlan(Plan):
             # (esf_attn_tc_create_split: O += P_hi V_hi + P_lo V_hi + P_hi V_lo, row sums in FP32 registers)
             nbytes = self._size("esf_attn_tc_pack_bytes", B, N, d)
             nlo = self._size("esf_attn_tc_vlo_bytes", B, N, d)
-            packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-            vlo = torch.empty(nlo, dtype=torch.uint8, device=self.device)
+            packed = self.alloc((nbytes,), torch.uint8, flat=True)
+            vlo = self.alloc((nlo,), torch.uint8, flat=True)
             h = self._create("esf_attn_tc_create_split", packed, vlo, *geo, y)
             pack = self._bind("esf_attn_tc_pack", proj, B, N, d, rt.F16, packed)
             pack_vlo = self._bind("esf_attn_tc_pack_vlo", proj, B, N, d, vlo)
@@ -272,14 +278,13 @@ class PrecisePlan(Plan):
         # inside a zero-padded (B, n_pad, 3 dp) matrix and view its first Nk rows as the activation
         kc1, kch1, _, npad1 = rt.igemm_geometry(3 * dp, Nk)
         assert kc1 * kch1 == 3 * dp, "3 x dim_inner must fill whole K chunks"
-        phi_rows = torch.zeros((B, npad1, 3 * dp), dtype=torch.float16, device=self.device)
-        phi32 = torch.empty((B, Tp, Hp, Wp, d), dtype=torch.float32, device=self.device)
+        phi_rows = self.alloc((B, npad1, 3 * dp), torch.float16, zero=True)
+        phi32 = self.alloc((B, Tp, Hp, Wp, d), torch.float32)
         phi_x3 = phi_rows.as_strided((B, Tp, Hp, Wp, 3 * dp), (npad1 * 3 * dp, Hp * Wp * 3 * dp, Wp * 3 * dp, 3 * dp, 1))
         phi = Act32(phi32, phi_x3, dp, 0, d, weight_order=True)
-        g32 = torch.empty((B, Tp, Hp, Wp, d), dtype=torch.float32, device=self.device)
-        g_x3 = torch.zeros((B, Tp, Hp, Wp, 3 * dp), dtype=torch.float16, device=self.device)
+        g32 = self.alloc((B, Tp, Hp, Wp, d), torch.float32)
+        g_x3 = self.alloc((B, Tp, Hp, Wp, 3 * dp), torch.float16, zero=True)
         g = Act32(g32, g_x3, dp, 0, d, weight_order=True)
-        self.keep += [phi_rows, phi32, g32, g_x3]
         self.conv(xp, phi, *wb(nln.conv_phi))
         self.conv(xp, g, *wb(nln.conv_g))
         # affinity S = theta^T phi (FP32), one launch for the whole batch
@@ -295,8 +300,7 @@ class PrecisePlan(Plan):
         # g^T in weight order: gT3[b][c][plane * nkp + k] = plane(g)[b, k, c], planes (hi, hi, lo)
         kc2, kch2, _, npad2 = rt.igemm_geometry(3 * nkp, d)
         kpad = kc2 * kch2
-        gT3 = torch.zeros((B, npad2, kpad), dtype=torch.float16, device=self.device)
-        self.keep.append(gT3)
+        gT3 = self.alloc((B, npad2, kpad), torch.float16, zero=True)
         for pl in range(3):
             self._launch("esf_transpose16", g_x3.data_ptr() + 2 * pl * dp, B, Nk, d, Nk * 3 * dp, 3 * dp,
                          gT3.data_ptr() + 2 * pl * nkp, npad2 * kpad, kpad, kind="nl_transpose", label="g plane %d" % pl,
@@ -306,5 +310,5 @@ class PrecisePlan(Plan):
         zero2 = self.scratch((npad2,), torch.float32, zero=True)
         self.gemm_rows(P3, acc, gT3, zero2, "nl_gemm", "p.g x3 N=%dx%d d=%d" % (Nq, Nk, d))
         self._post(acc, att, label="split")
-        w, bias = fold_conv_bn(nln.conv_out.weight, nln.conv_out.bias, nln.bn)
+        w, bias = self.once(fold_conv_bn, nln.conv_out.weight, nln.conv_out.bias, nln.bn)
         self.conv(att, y, w, bias, res=x)

@@ -431,13 +431,14 @@ def launch_clip_list(plan, fin, clips, alpha):
 
 def launch_video_list(plan, fin, videos):
     """Fill the stem inputs of `plan` from a VideoList on the current stream: row (v * num_clips + j) * V + s is video
-    v, temporal clip j, crop s.  The frame tables go to a plan-owned device buffer with one copy from pinned memory."""
+    v, temporal clip j, crop s.  The frame tables go to a device buffer of the plan (of its family: Plan.shared) with one
+    copy from pinned memory."""
     L = rt.lib()
     s = rt.current_stream_ptr()
     need = sum(own.shape[0] * own.shape[2] for own in plan.inputs)   # >= B * T_p of every pathway
-    dev = getattr(plan, "video_index", None)
+    dev = getattr(plan.shared, "video_index", None)
     if dev is None or dev.numel() < need:
-        dev = plan.video_index = torch.empty(need, dtype=torch.int32, device=plan.inputs[0].device)
+        dev = plan.shared.video_index = torch.empty(need, dtype=torch.int32, device=plan.inputs[0].device)
     n = videos.index.numel()
     assert n <= dev.numel()
     dev[:n].copy_(videos.index, non_blocking=True)

@@ -54,7 +54,7 @@ class _EfficientBase(_PlannedModel):
                       _conv_out(W, k[2], s[2], p[2], d[2]))
         if y is None:
             y = plan.act(B, To, Ho, Wo, conv.out_channels, name=name)
-        w, b = fold_conv_bn(conv.weight, conv.bias, bn)
+        w, b = plan.once(fold_conv_bn, conv.weight, conv.bias, bn)
         plan.conv(x, y, w, b, stride=tuple(s), padding=tuple(p), dilation=tuple(d), groups=conv.groups, act=act, res=res)
         return y
 
@@ -64,7 +64,7 @@ class _EfficientBase(_PlannedModel):
         B, _, T, H, W = x_nc.shape
         k, s, p = conv.kernel_size, conv.stride, conv.padding
         To, Ho, Wo = _conv_out(T, k[0], s[0], p[0]), _conv_out(H, k[1], s[1], p[1]), _conv_out(W, k[2], s[2], p[2])
-        w, b = fold_conv_bn(conv.weight, conv.bias, bn)
+        w, b = plan.once(fold_conv_bn, conv.weight, conv.bias, bn)
         pool = seq[3] if len(seq) > 3 else None
         if pool is None:
             y = plan.act(B, To, Ho, Wo, conv.out_channels)
@@ -410,7 +410,7 @@ class SlowFastShuffleNet(_EfficientBase):
             # the weight rows.  A permuted grouped conv is no longer grouped, so the layer runs as one dense implicit
             # GEMM over a block-diagonal weight (the layers are HBM bound; `groups`-fold MACs on structural zeros) --
             # one launch instead of a GEMM per group plus the shuffle kernel (1.6 ms of the 12.3 ms ShuffleNet step).
-            w, b = fold_conv_bn(conv1.weight, conv1.bias, blk.bn1)
+            w, b = plan.once(fold_conv_bn, conv1.weight, conv1.bias, blk.bn1)
             cout, cin_g, g = w.shape[0], w.shape[1], conv1.groups
             wd = torch.zeros((cout, cin_g * g, 1, 1, 1), dtype=w.dtype, device=w.device)
             for i in range(g):
@@ -685,7 +685,7 @@ class SlowFastMoibleNetV2(_EfficientBase):
             _, _, T, H, W = xs_in[p].shape
             T, H, W = self._pooled_shape(T, H, W, seq)
             buf = plan.act(B, T, H, W, seq[0].out_channels, name="s1_cat%d" % p)
-            w, b = fold_conv_bn(seq[0].weight, None, seq[1])
+            w, b = plan.once(fold_conv_bn, seq[0].weight, None, seq[1])
             plan.stem(xs_in[p], buf, w, b, tuple(seq[0].stride), tuple(seq[0].padding), act=rt.ACT_RELU6)
             cur.append(buf)
         order = [("s2", True, "s3_fuse"), ("s4", True, "s4_fuse"), ("s5", True, "s5_fuse"), ("s6", False, None),
@@ -907,7 +907,7 @@ class SlowFastGhostNet(_EfficientBase):
         x1 = out[..., :init] if res is None else plan.act(B, T, H, W, init)
         self._emit_conv(plan, x, pc, pbn, act, y=x1)
         if keep > 0:
-            w, b = fold_conv_bn(cc.weight, cc.bias, cbn)
+            w, b = plan.once(fold_conv_bn, cc.weight, cc.bias, cbn)
             # depthwise with channel multiplier 1: output channel j reads input channel j -> truncating is exact
             plan.conv(x1[..., :keep], out[..., init:init + keep], w[:keep], b[:keep], stride=tuple(cc.stride),
                       padding=tuple(cc.padding), groups=keep, act=act, res=None if res is None else res[..., init:init + keep])
@@ -983,7 +983,7 @@ class SlowFastGhostNet(_EfficientBase):
             _, _, T, H, W = xs_in[p].shape
             T, H, W = self._pooled_shape(T, H, W, seq)
             buf = plan.act(B, T, H, W, seq[0].out_channels, name="s0_cat%d" % p)
-            w, b = fold_conv_bn(seq[0].weight, None, seq[1])
+            w, b = plan.once(fold_conv_bn, seq[0].weight, None, seq[1])
             plan.stem(xs_in[p], buf, w, b, tuple(seq[0].stride), tuple(seq[0].padding), act=rt.ACT_RELU)
             cur.append(buf)
         for i in range(1, 6):
@@ -994,7 +994,7 @@ class SlowFastGhostNet(_EfficientBase):
             cur = [b[0] for b in bufs]
         h = self.head
         outs = [h.conv_head_slow.out_channels, h.conv_head_fast.out_channels]
-        feat = torch.empty((B, sum(outs)), dtype=torch.float32, device=plan.device)
+        feat = plan.alloc((B, sum(outs)), torch.float32)
         col = 0
         for p, (cba, ch) in enumerate(((h.stage5_conv_slow, h.conv_head_slow), (h.stage5_conv_fast, h.conv_head_fast))):
             t = self._emit_conv(plan, cur[p], cba.conv, cba.bn1, rt.ACT_RELU)

@@ -18,7 +18,7 @@ import torch.nn as nn
 
 from . import runtime as rt
 from .build import MODEL_REGISTRY
-from .engine import Plan, fold_conv_bn
+from .engine import Family, Plan, fold_conv_bn
 
 # video_model_builder.py:16-90 / custom_video_model_builder.py:151-168
 _MODEL_STAGE_DEPTH = {50: (3, 4, 6, 3), 101: (3, 4, 23, 3), 18: (2, 2, 2, 2), 34: (3, 4, 6, 3)}   # 18 / 34: the fork's additions
@@ -314,6 +314,10 @@ class _PlannedModel(nn.Module):
         # live plans kept per model: the activation arena of a plan is large (25 GB at batch 64), but a test loader
         # alternates between the full batch and a short last one, and the demo between window and batch shapes
         self._max_plans = max(1, int(esf.get("MAX_PLANS", 2)))
+        # batch capacity (0: off): one plan family per per-clip input shape serves every batch of up to MAX_BATCH rows
+        self._max_batch = int(esf.get("MAX_BATCH", 0) or 0)
+        if self._max_batch < 0:
+            raise ValueError("cfg.ESF.MAX_BATCH must be >= 0 (0: off), got %d" % self._max_batch)
 
     def _weights_stamp(self):
         """Identity of the weights a plan was compiled from: (storage address, version counter) of every parameter
@@ -337,12 +341,20 @@ class _PlannedModel(nn.Module):
         return out
 
     def _get_plan(self, shapes, device):
-        key = (tuple(tuple(s) for s in shapes), str(device))
+        """The plan for input `shapes` on `device`, compiled on first use.  With cfg.ESF.MAX_BATCH = N the key leaves
+        out the batch rows (dim 0): the first call compiles the family's capacity plan at N rows, a call with b < N rows
+        gets the family's variant for b (engine.Family), and b > N raises EsfError before anything is launched."""
+        shapes = [tuple(int(n) for n in s) for s in shapes]
+        cap = self._max_batch
+        if cap and shapes[0][0] > cap:
+            raise rt.EsfError("a batch of %d rows exceeds cfg.ESF.MAX_BATCH = %d, the capacity of the compiled plans"
+                              % (shapes[0][0], cap))
+        key = (tuple(s[1:] if cap else s for s in shapes), str(device))
         stamp = self._weights_stamp()
         ent = self._plans.get(key)
         if ent is not None and ent[0] == stamp:
             self._plans.move_to_end(key)
-            return ent[1]
+            return self._variant(ent[1], shapes) if cap else ent[1]
         self._check_roi_time_axis(shapes)            # before any cached plan is evicted for this shape
         if ent is not None or any(st != stamp for st, _ in self._plans.values()):
             self._plans.clear()                      # the weights changed: every compiled plan is stale
@@ -354,21 +366,40 @@ class _PlannedModel(nn.Module):
                                       "detection models with 'fp16' / 'bf16'")
         while len(self._plans) >= self._max_plans:
             self._plans.popitem(last=False)          # frees the arena of the least recently used shape
+        if cap:
+            plan = self._compile_plan([(cap,) + s[1:] for s in shapes], device, prec, Family())
+        else:
+            plan = self._compile_plan(shapes, device, prec)
+        self._plans[key] = (stamp, plan)
+        return self._variant(plan, shapes) if cap else plan
+
+    def _variant(self, plan, shapes):
+        """The plan of the family of capacity plan `plan` for `shapes` (their batch rows at most the capacity)."""
+        b = shapes[0][0]
+        if b == plan.inputs[0].shape[0]:
+            return plan
+        if b not in plan.variants:
+            plan.variants[b] = self._compile_plan(shapes, plan.device, plan.precision, plan.family)
+        return plan.variants[b]
+
+    def _compile_plan(self, shapes, device, prec, family=None):
+        """Compile a plan for input `shapes` at precision `prec`, as a member of `family` when given."""
         with torch.cuda.device(device):
             if prec == "fp32":
                 if not self.supports_fp32:
                     raise NotImplementedError("ESF.PRECISION = 'fp32' (FP32-accurate plan) covers the ResNet based "
                                               "models; %s runs with 'fp16' / 'bf16'" % type(self).__name__)
                 from .engine_fp32 import PrecisePlan
-                plan = PrecisePlan(device)
+                plan = PrecisePlan(device, family=family)
             else:
-                plan = Plan(device, precision=prec)
-            plan.inputs = [torch.empty(s, dtype=torch.float32, device=device) for s in shapes]
+                plan = Plan(device, precision=prec, family=family)
+            plan.inputs = [plan.alloc(s, torch.float32) for s in shapes]
             with torch.no_grad():
                 self._compile(plan)
+            if family is not None:
+                plan.end_compile()
             if self._use_graph:
                 plan.capture()
-        self._plans[key] = (stamp, plan)
         return plan
 
     def input_buffers(self, shapes, device=None):
@@ -425,9 +456,9 @@ class _PlannedModel(nn.Module):
             return self._empty(dev)
         alpha = self._cfg.SLOWFAST.ALPHA
         plan = self._get_plan([(B, C, T // alpha, H, W), (B, C, T, H, W)], dev)
-        idx = getattr(plan, "slow_index", None)
+        idx = getattr(plan.shared, "slow_index", None)
         if idx is None:
-            idx = plan.slow_index = torch.linspace(0, T - 1, T // alpha).long().to(torch.int32).to(dev)
+            idx = plan.shared.slow_index = torch.linspace(0, T - 1, T // alpha).long().to(torch.int32).to(dev)
         with torch.cuda.device(dev):
             if plan.inputs[0].data_ptr() in plan.stem_routes:
                 out = plan.run([None, fast], gather={0: (fast, idx)})
@@ -501,9 +532,9 @@ class _PlannedModel(nn.Module):
         """The plan for `shapes` and its FrameInput (frames.py) for frames of `channels` channels."""
         from . import frames as esf_frames
         plan = self._get_plan(shapes, dev)
-        fin = getattr(plan, "frame_input", None)
+        fin = getattr(plan.shared, "frame_input", None)
         if fin is None:
-            fin = plan.frame_input = esf_frames.FrameInput(self._cfg, dev, plan.adt, channels=channels)
+            fin = plan.shared.frame_input = esf_frames.FrameInput(self._cfg, dev, plan.adt, channels=channels)
         return plan, fin
 
     def _forward_clip_list(self, clips, bboxes, frame_index, crop_size, spatial_idx):
@@ -652,7 +683,7 @@ class _PlannedModel(nn.Module):
                                     fuse.attention_spatial_s2f, fuse.bn_s2f)
         else:
             conv = fuse.conv_f2s
-            w, b = fold_conv_bn(conv.weight, None, fuse.bn)
+            w, b = plan.once(fold_conv_bn, conv.weight, None, fuse.bn)
             plan.conv(x_f, sbuf[..., cs:cs + conv.out_channels], w, b, stride=tuple(conv.stride),
                       padding=tuple(conv.padding), act=rt.ACT_RELU)
 
@@ -785,7 +816,7 @@ class _TwoStreamResNet(_PlannedModel):
             To, Ho, Wo = conv_out(T, k[0], s[0], p[0]), conv_out(H, k[1], s[1], p[1]), conv_out(W, k[2], s[2], p[2])
             cout = stem.conv.out_channels
             y = plan.act(B, To, Ho, Wo, cout)
-            w, b = fold_conv_bn(stem.conv.weight, None, stem.bn)
+            w, b = plan.once(fold_conv_bn, stem.conv.weight, None, stem.bn)
             plan.stem(x, y, w, b, tuple(s), tuple(p), act=rt.ACT_RELU)
             Hp, Wp = conv_out(Ho, 3, 2, 1), conv_out(Wo, 3, 2, 1)
             buf = plan.act(B, To, Hp, Wp, cs_tot if pw == 0 else cf_tot, name="s1_cat%d" % pw)
@@ -893,19 +924,19 @@ class _TwoStreamResNet(_PlannedModel):
         tb = plan.act(B, T, Ho, Wo, ci, role="operand")
         if hasattr(blk, "branch1"):
             sc = plan.act(B, T, Ho, Wo, co, role="residual")  # read by conv c's residual add only
-            w, b = fold_conv_bn(blk.branch1.weight, None, blk.branch1_bn)
+            w, b = plan.once(fold_conv_bn, blk.branch1.weight, None, blk.branch1_bn)
             plan.conv(x, sc, w, b, stride=tuple(blk.branch1.stride))
         else:
             sc = x
-        w, b = fold_conv_bn(t.a.weight, None, t.a_bn)
+        w, b = plan.once(fold_conv_bn, t.a.weight, None, t.a_bn)
         plan.conv(x, ta, w, b, stride=tuple(t.a.stride), padding=tuple(t.a.padding), act=rt.ACT_RELU)
         # RESNET.NUM_GROUPS > 1 (ResNeXt, resnet_helper.py:196-205): Plan.conv runs one implicit GEMM per group on
         # channel slices, or one dense GEMM over a block-diagonal weight when the slices are thinner than a TMA row;
         # PrecisePlan.conv always takes the block-diagonal weight
-        w, b = fold_conv_bn(t.b.weight, None, t.b_bn)
+        w, b = plan.once(fold_conv_bn, t.b.weight, None, t.b_bn)
         plan.conv(ta, tb, w, b, stride=tuple(t.b.stride), padding=tuple(t.b.padding),
                   dilation=tuple(t.b.dilation), groups=t.b.groups, act=rt.ACT_RELU)
-        w, b = fold_conv_bn(t.c.weight, None, t.c_bn)
+        w, b = plan.once(fold_conv_bn, t.c.weight, None, t.c_bn)
         plan.conv(tb, y, w, b, act=rt.ACT_RELU, res=sc)
 
 @MODEL_REGISTRY.register()
@@ -993,7 +1024,7 @@ class ResNet(_TwoStreamResNet):
         k, s, p = stem.kernel, stem.stride, stem.padding
         To, Ho, Wo = conv_out(T, k[0], s[0], p[0]), conv_out(H, k[1], s[1], p[1]), conv_out(W, k[2], s[2], p[2])
         y = plan.act(B, To, Ho, Wo, wpg)
-        w, b = fold_conv_bn(stem.conv.weight, None, stem.bn)
+        w, b = plan.once(fold_conv_bn, stem.conv.weight, None, stem.bn)
         plan.stem(x, y, w, b, tuple(s), tuple(p), act=rt.ACT_RELU)
         cur = plan.act(B, To, conv_out(Ho, 3, 2, 1), conv_out(Wo, 3, 2, 1), wpg, name="s1_cat0")
         plan.pool(y, cur, (1, 3, 3), (1, 2, 2), (0, 1, 1))

@@ -101,7 +101,8 @@ class ClipStream:
         cur = torch.cuda.current_stream(self.device)
         # A loader with drop_last=False (the reference's test loader, datasets/loader.py) ends on a SHORT batch: it is
         # copied into the leading rows of the staging slot (a leading-dim slice of a contiguous tensor is contiguous)
-        # and the forward runs on those views -- the model compiles a second plan for that batch size and keeps both.
+        # and the forward runs on those views -- the model compiles a second plan for that batch size and keeps both
+        # (with cfg.ESF.MAX_BATCH, a variant of the same plan family, on the same arena).
         if self.slow_from_fast:
             if len(host_inputs) == 2:
                 if not self._sff_checked:   # once: the promise the flag makes
