@@ -29,6 +29,11 @@
 // pair: its source is the whole video (Tsrc_b, H0, W0, C), shared by the video's views, and its frames are row b of a
 // device frame table t_index[B][T], each entry clamped to the clip's own Tsrc_b.  The chunk (CropVideoChunk) is the
 // ragged one plus the per-clip Tsrc; the kernel body is the ragged kernel's, instantiated for that chunk.
+//
+// AVA detection (esf_*_ava, esf_ava_boxes).  The test split of the AVA loader (datasets/ava_dataset.py
+// _images_and_boxes_preprocessing, PyTorch backend) resizes the [0, 1] values (table u / 255) to short side S with no
+// crop and normalises after the resize, before its BGR -> RGB swap.  The same crop_rows body writes the whole Hr x Wr
+// frame as one view at (0, 0) under the AvaEmit policy; the boxes get the loader's FP64 numpy arithmetic on the device.
 #include <algorithm>
 #include <type_traits>
 
@@ -131,12 +136,30 @@ __device__ __forceinline__ int source_frame(const CropShared& s, int row, int t,
   return s.t_index ? min(max(__ldg(s.t_index + row * s.T + t), 0), Tsrc - 1) : t;
 }
 
-// All V crops of output row y of frame t of output clip oc, from the source frame `frame` of geometry g.
-// PACKED: rows [B*V][T][S][pitch] of 16-bit stem input (layout of esf_stem_pack), else FP32 NCDHW (B*V, C, T, S, S)
-template <bool RESIZE, bool PACKED>
+// What a route emits: the size of its output frames and the final value of output channel c from the resized value v.
+// CropEmit: the S x S crops of the classification routes, whose table already holds normalised values.
+struct CropEmit {
+  __device__ __forceinline__ int height(const CropShared& s, const CropClip&) const { return s.S; }
+  __device__ __forceinline__ int width(const CropShared& s, const CropClip&) const { return s.S; }
+  __device__ __forceinline__ float value(float v, int) const { return v; }
+};
+
+// AvaEmit: the whole resized Hr x Wr frame of the AVA test branch, which resizes the [0, 1] values (table u / 255) and
+// normalises afterwards: (v - mean[c]) / std[c] with the statistics of output channel c (those of its source channel).
+struct AvaEmit {
+  float mean[4], std[4];
+  __device__ __forceinline__ int height(const CropShared&, const CropClip& g) const { return g.Hr; }
+  __device__ __forceinline__ int width(const CropShared&, const CropClip& g) const { return g.Wr; }
+  __device__ __forceinline__ float value(float v, int c) const { return __fdiv_rn(__fsub_rn(v, mean[c]), std[c]); }
+};
+
+// All V crops of output row y of frame t of output clip oc, from the source frame `frame` of geometry g.  The output
+// frames are Ho x Wo = e.height x e.width (S x S for the crops).
+// PACKED: rows [B*V][T][Ho][pitch] of 16-bit stem input (layout of esf_stem_pack), else FP32 NCDHW (B*V, C, T, Ho, Wo)
+template <bool RESIZE, bool PACKED, class Emit = CropEmit>
 __device__ __forceinline__ void crop_rows(const CropShared& s, const CropClip& g, const uint8_t* frame, int oc, int t,
                                           int y, const float* lut_s, uint8_t* rows_s, int pitch, int lpad, int f16,
-                                          void* __restrict__ out) {
+                                          void* __restrict__ out, const Emit& e = Emit()) {
   const int row_bytes = g.W0 * s.C;
   const int row_pitch = ((row_bytes + 15) & ~15) + 16;   // + 16: room for the source's 16-byte phase
   const uint8_t* r0 = rows_s;
@@ -161,20 +184,21 @@ __device__ __forceinline__ void crop_rows(const CropShared& s, const CropClip& g
       const float2 yw = __ldg(reinterpret_cast<const float2*>(g.y_wt) + yr);
       l0 = yw.x, l1 = yw.y;
     }
-    const long long orow = ((long long)(oc * s.V + v) * s.T + t) * s.S + y;   // (clip row, t, y) of the output
+    const long long orow = ((long long)(oc * s.V + v) * s.T + t) * e.height(s, g) + y;   // (clip row, t, y) of the output
     const int x0 = g.x0[v];
     if (PACKED) {
       uint16_t* dst = static_cast<uint16_t*>(out) + orow * pitch;
-      const int SC = s.S * s.C;
+      const int SC = e.width(s, g) * s.C;
       for (int ck = threadIdx.x; ck < pitch / 8; ck += blockDim.x) {
         const int j0 = ck * 8 - lpad;
         int x = j0 >= 0 ? j0 / s.C : -1 - ((-1 - j0) / s.C);   // floor division: lpad need not be a multiple of C
         int c = j0 - x * s.C;
         float f[8];
 #pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const int j = j0 + e;
-          f[e] = (j >= 0 && j < SC) ? crop_value<RESIZE>(g, s.C, r0, r1, lut_s, x0 + x, c, s.chan_src[c], l0, l1) : 0.f;
+        for (int k = 0; k < 8; ++k) {
+          const int j = j0 + k;
+          f[k] = (j >= 0 && j < SC) ? e.value(crop_value<RESIZE>(g, s.C, r0, r1, lut_s, x0 + x, c, s.chan_src[c], l0, l1), c)
+                                     : 0.f;
           if (++c == s.C) c = 0, ++x;
         }
         uint4 o;
@@ -185,22 +209,24 @@ __device__ __forceinline__ void crop_rows(const CropShared& s, const CropClip& g
         *reinterpret_cast<uint4*>(dst + ck * 8) = o;
       }
     } else {
-      // out[(oc*V + v), c, t, y, :]: one thread = 4 consecutive x of one channel (16-byte store when S % 4 == 0)
-      const int S4 = (s.S + 3) / 4;
-      const bool vec = (s.S & 3) == 0;
+      // out[(oc*V + v), c, t, y, :]: one thread = 4 consecutive x of one channel (16-byte store when Wo % 4 == 0)
+      const int S4 = (e.width(s, g) + 3) / 4;
+      const bool vec = (e.width(s, g) & 3) == 0;
       for (int i = threadIdx.x; i < s.C * S4; i += blockDim.x) {
         const int c = i / S4, xs = (i - c * S4) * 4;
         float f[4];
 #pragma unroll
-        for (int e = 0; e < 4; ++e)
-          f[e] = xs + e < s.S ? crop_value<RESIZE>(g, s.C, r0, r1, lut_s, x0 + xs + e, c, s.chan_src[c], l0, l1) : 0.f;
-        float* dst = static_cast<float*>(out) + ((((long long)(oc * s.V + v) * s.C + c) * s.T + t) * s.S + y) * s.S + xs;
+        for (int k = 0; k < 4; ++k)
+          f[k] = xs + k < e.width(s, g)
+                     ? e.value(crop_value<RESIZE>(g, s.C, r0, r1, lut_s, x0 + xs + k, c, s.chan_src[c], l0, l1), c)
+                     : 0.f;
+        float* dst = static_cast<float*>(out) + ((((long long)(oc * s.V + v) * s.C + c) * s.T + t) * e.height(s, g) + y) * e.width(s, g) + xs;
         if (vec) {
           *reinterpret_cast<float4*>(dst) = make_float4(f[0], f[1], f[2], f[3]);
         } else {
 #pragma unroll
-          for (int e = 0; e < 4; ++e)
-            if (xs + e < s.S) dst[e] = f[e];
+          for (int k = 0; k < 4; ++k)
+            if (xs + k < e.width(s, g)) dst[k] = f[k];
         }
       }
     }
@@ -240,6 +266,57 @@ __global__ void __launch_bounds__(kCropThreads, 6) crop_frames_ragged_kernel(con
     crop_rows<true, PACKED>(p.s, g, frame, p.clip0 + b, t, y, lut_s, rows_s, pitch, lpad, f16, out);
   else
     crop_rows<false, PACKED>(p.s, g, frame, p.clip0 + b, t, y, lut_s, rows_s, pitch, lpad, f16, out);
+}
+
+// The AVA test branch on B clips of one geometry: every output row y < Hr of the whole resized frame, one block each;
+// normalisation after the resize (AvaEmit).  Frames whose short side already is the target size take the pure window.
+struct AvaParams {
+  CropShared s;   // V = 1, S = min(Hr, Wr)
+  CropClip g;     // one view at (0, 0)
+  AvaEmit e;
+  int B;
+};
+
+template <bool RESIZE, bool PACKED>
+__global__ void __launch_bounds__(kCropThreads) ava_frames_kernel(const __grid_constant__ AvaParams p, int pitch,
+                                                                  int lpad, int f16, void* __restrict__ out) {
+  __shared__ float lut_s[4 * 256];
+  extern __shared__ __align__(16) uint8_t rows_s[];
+  for (int i = threadIdx.x; i < p.s.C * 256; i += blockDim.x) lut_s[i] = p.s.lut[i];
+  const int y = blockIdx.x % p.g.Hr;
+  const int t = (blockIdx.x / p.g.Hr) % p.s.T;
+  const int b = blockIdx.x / (p.g.Hr * p.s.T);
+  const int ts = source_frame(p.s, 0, t, p.s.Tsrc);
+  const uint8_t* frame = p.g.frames + ((long long)b * p.s.Tsrc + ts) * p.g.H0 * (p.g.W0 * p.s.C);
+  crop_rows<RESIZE, PACKED, AvaEmit>(p.s, p.g, frame, b, t, y, lut_s, rows_s, pitch, lpad, f16, out, p.e);
+}
+
+// numpy's maximum(lo, x) / minimum(hi, x) of a non-NaN bound: a NaN x stays NaN, -0.0 against 0.0 gives the bound
+__device__ __forceinline__ double np_max(double lo, double x) { return lo >= x ? lo : x; }
+__device__ __forceinline__ double np_min(double hi, double x) { return hi <= x ? hi : x; }
+
+// The loader's box arithmetic of the AVA test branch (FP64, as numpy runs it on the float64 boxes of ava_helper), one
+// thread per box: [0, 1] coordinates times (W0, H0), clip_boxes_to_image(H0, W0), the short-side scale factor
+// new / old of random_short_side_scale_jitter (none for a pure window), clip_boxes_to_image(S, S), then FP32 as the
+// detection collate makes it.  Column 0 (the batch index) is passed through.
+__global__ void __launch_bounds__(128) ava_boxes_kernel(const void* __restrict__ in, int f64, int K, int H0, int W0,
+                                                        int Hr, int Wr, int S, float* __restrict__ out) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= K) return;
+  const bool resize = Hr != H0 || Wr != W0;
+  const double num = W0 < H0 ? (double)Hr : (double)Wr, den = W0 < H0 ? (double)H0 : (double)W0;
+  for (int j = 0; j < 5; ++j) {
+    double v = f64 ? __ldg(static_cast<const double*>(in) + 5LL * k + j)
+                   : (double)__ldg(static_cast<const float*>(in) + 5LL * k + j);
+    if (j > 0) {
+      const bool x = (j & 1) != 0;   // columns 1, 3: x1, x2; 2, 4: y1, y2
+      v = __dmul_rn(v, x ? (double)W0 : (double)H0);
+      v = np_min((x ? W0 : H0) - 1.0, np_max(0.0, v));
+      if (resize) v = __ddiv_rn(__dmul_rn(v, num), den);
+      v = np_min(S - 1.0, np_max(0.0, v));
+    }
+    out[5LL * k + j] = __double2float_rn(v);
+  }
 }
 
 static int crop_shared(CropShared* s, const char* who, int32_t B, int32_t Tsrc, int32_t C, const int32_t* t_index,
@@ -375,6 +452,39 @@ static int check_frame_table(const char* who, const int32_t* t_index) {
   return ESF_OK;
 }
 
+// Geometry of the AVA test branch: one view of the whole Hr x Wr frame, the statistics of every output channel.
+static int ava_params(AvaParams* p, const char* who, const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0,
+                      int32_t W0, int32_t C, const int32_t* t_index, int32_t T, const int32_t* chan_src,
+                      const float* lut32, const float* mean_host, const float* std_host, const int32_t* y_index,
+                      const float* y_weight, int32_t Hr, const int32_t* x_index, const float* x_weight, int32_t Wr) {
+  static const int32_t kWhole[2] = {0, 0};
+  int rc = crop_shared(&p->s, who, B, Tsrc, C, t_index, T, chan_src, lut32, 1, std::max(1, std::min(Hr, Wr)));
+  if (rc != ESF_OK) return rc;
+  rc = crop_clip(&p->g, who, -1, p->s, frames, H0, W0, y_index, y_weight, Hr, x_index, x_weight, Wr, kWhole);
+  if (rc != ESF_OK) return rc;
+  ESF_CHECK_ARG(mean_host && std_host, "%s: null mean / std", who);
+  ESF_CHECK_ARG((long long)B * T * Hr < (1LL << 31), "%s: grid too large", who);
+  for (int c = 0; c < 4; ++c) {   // normalised before the channel swap: output c takes its source channel's statistics
+    p->e.mean[c] = c < C ? mean_host[p->s.chan_src[c]] : 0.f;
+    p->e.std[c] = c < C ? std_host[p->s.chan_src[c]] : 1.f;
+  }
+  p->B = B;
+  return ESF_OK;
+}
+
+template <bool PACKED>
+static int ava_launch(const char* who, const AvaParams& p, int pitch, int lpad, int f16, void* out, void* stream) {
+  const bool resize = p.g.Hr != p.g.H0 || p.g.Wr != p.g.W0;
+  const size_t smem = crop_smem(p.g.W0, p.s.C);
+  const unsigned grid = (unsigned)((long long)p.B * p.s.T * p.g.Hr);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (resize)
+    ava_frames_kernel<true, PACKED><<<grid, kCropThreads, smem, s>>>(p, pitch, lpad, f16, out);
+  else
+    ava_frames_kernel<false, PACKED><<<grid, kCropThreads, smem, s>>>(p, pitch, lpad, f16, out);
+  return check_launch(who);
+}
+
 }  // namespace esf
 
 using namespace esf;
@@ -453,4 +563,41 @@ extern "C" int esf_frames_to_clip_crop_videos(const void* frames_host, int32_t B
   return crop_ragged<false, CropVideoChunk>("esf_frames_to_clip_crop_videos", "crop_frames_ragged_kernel (videos, clip)",
                                             frames_host, B, T, C, t_index, T, chan_src, lut32, geom_host, tables_host,
                                             crop_yx_host, V, S, 0, 0, 0, clip, stream);
+}
+
+extern "C" int esf_stem_pack_u8_ava(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0, int32_t W0, int32_t C,
+                                    const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
+                                    const float* mean_host, const float* std_host, const int32_t* y_index,
+                                    const float* y_weight, int32_t Hr, const int32_t* x_index, const float* x_weight,
+                                    int32_t Wr, int32_t dtype, int32_t pitch, int32_t lpad, void* xp, void* stream) {
+  AvaParams p;
+  int rc = ava_params(&p, "esf_stem_pack_u8_ava", frames, B, Tsrc, H0, W0, C, t_index, T, chan_src, lut32, mean_host,
+                      std_host, y_index, y_weight, Hr, x_index, x_weight, Wr);
+  if (rc != ESF_OK) return rc;
+  if ((rc = check_packed_out("esf_stem_pack_u8_ava", dtype, pitch, lpad, Wr, C, xp)) != ESF_OK) return rc;
+  return ava_launch<true>("ava_frames_kernel (packed)", p, pitch, lpad, dtype == ESF_F16, xp, stream);
+}
+
+extern "C" int esf_frames_to_clip_ava(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0, int32_t W0, int32_t C,
+                                      const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
+                                      const float* mean_host, const float* std_host, const int32_t* y_index,
+                                      const float* y_weight, int32_t Hr, const int32_t* x_index, const float* x_weight,
+                                      int32_t Wr, float* clip, void* stream) {
+  AvaParams p;
+  int rc = ava_params(&p, "esf_frames_to_clip_ava", frames, B, Tsrc, H0, W0, C, t_index, T, chan_src, lut32, mean_host,
+                      std_host, y_index, y_weight, Hr, x_index, x_weight, Wr);
+  if (rc != ESF_OK) return rc;
+  if ((rc = check_clip_out("esf_frames_to_clip_ava", Wr, clip)) != ESF_OK) return rc;
+  return ava_launch<false>("ava_frames_kernel (clip)", p, 0, 0, 0, clip, stream);
+}
+
+extern "C" int esf_ava_boxes(const void* boxes, int32_t f64, int32_t K, int32_t H0, int32_t W0, int32_t Hr, int32_t Wr,
+                             int32_t S, float* out, void* stream) {
+  ESF_CHECK_ARG(K >= 0 && (K == 0 || (boxes && out)), "esf_ava_boxes: null/bad argument");
+  ESF_CHECK_ARG(H0 > 0 && W0 > 0 && Hr > 0 && Wr > 0 && S > 0, "esf_ava_boxes: bad geometry %d x %d -> %d x %d, size %d",
+                H0, W0, Hr, Wr, S);
+  if (K == 0) return ESF_OK;
+  ava_boxes_kernel<<<(K + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(boxes, f64 != 0, K, H0, W0, Hr, Wr,
+                                                                                   S, out);
+  return check_launch("ava_boxes_kernel");
 }

@@ -24,6 +24,12 @@ temporal clips x TEST.NUM_SPATIAL_CROPS crops.  Its decoder samples temporal cli
 (datasets/decoder.py decode with the whole video decoded: get_start_end_idx + temporal_sampling).  `temporal_index`
 evaluates those expressions here, and the whole video (N, H, W, C) uint8 goes to the device once; the kernel reads
 every view's frames through a per-clip frame table (esf_*_crop_videos).
+
+AVA detection (`forward_ava_frames(frames, boxes)`): the test split of the reference's AVA loader
+(datasets/ava_dataset.py _images_and_boxes_preprocessing, PyTorch backend) scales the clip's [0, 1] values so that the
+short side is DATA.TEST_CROP_SIZE, with no crop, and normalises AFTER the resize; the boxes go through the same
+scale and two clips.  `esf_*_ava` writes the whole resized frame with that order (table u / 255, statistics applied to
+the blended value), and `esf_ava_boxes` maps the loader's [0, 1] boxes to resized pixels on the device.
 """
 import ctypes
 import math
@@ -315,6 +321,94 @@ class VideoList:
         torch.cat(parts, out=self.index)
 
 
+def unit_table(channels):
+    """FP32 [C][256]: `imgs.float() / 255.0` of every byte value (the AVA branch's first step), per channel."""
+    u = torch.arange(256, dtype=torch.uint8).float() / 255.0
+    return u.reshape(1, 256).repeat(channels, 1).contiguous()
+
+
+def ava_channel_source(channels, bgr=False, reverse=False):
+    """Source channel of every output channel of the AVA branch: the loader swaps BGR -> RGB when AVA.BGR is false
+    (after colour normalisation), and pack_pathway_output reverses again under DATA.REVERSE_INPUT_CHANNEL."""
+    swap = (not bgr) != bool(reverse)
+    if not swap:
+        return list(range(channels))
+    if channels != 3:
+        raise ValueError("the AVA loader's channel swap needs 3 channels, got %d (set AVA.BGR)" % channels)
+    return [2, 1, 0]
+
+
+def check_ava_frames(frames):
+    """(B, T, H, W, C) of the uint8 frames of forward_ava_frames; ValueError unless they are one contiguous uint8 tensor
+    of 5 dimensions whose rows fit the frame kernel."""
+    if not isinstance(frames, torch.Tensor) or frames.dtype != torch.uint8 or frames.dim() != 5 \
+            or not frames.is_contiguous():
+        raise ValueError("forward_ava_frames takes contiguous uint8 frames (B, T, H, W, C), got %s"
+                         % (("%s %s" % (frames.dtype, tuple(frames.shape))) if isinstance(frames, torch.Tensor)
+                            else type(frames).__name__))
+    B, T, H, W, C = (int(n) for n in frames.shape)
+    if min(T, H, W, C) < 1 or C > 4:
+        raise ValueError("forward_ava_frames: bad frame shape %s" % ((B, T, H, W, C),))
+    if W * C > MAX_ROW_BYTES:
+        raise ValueError("frame rows of %d x %d bytes exceed the frame kernel's %d" % (W, C, MAX_ROW_BYTES))
+    return B, T, H, W, C
+
+
+def check_ava_boxes(boxes, batch):
+    """The loader's normalised boxes (K, 5) [batch index, x1, y1, x2, y2] as the tensor esf_ava_boxes reads: FP64 kept,
+    any other floating type as FP32, contiguous.  ValueError for a wrong type or shape and, for host boxes, for batch
+    indices outside [0, batch) (device boxes are not read: that would synchronise)."""
+    if not torch.is_tensor(boxes) or not boxes.is_floating_point() or boxes.dim() != 2 or boxes.shape[1] != 5:
+        raise ValueError("boxes must be a floating-point (K, 5) tensor of [batch index, x1, y1, x2, y2] in [0, 1]; got %s"
+                         % ((tuple(boxes.shape), boxes.dtype) if torch.is_tensor(boxes) else type(boxes).__name__,))
+    b = boxes.detach()
+    b = b if b.dtype == torch.float64 else b.to(torch.float32)
+    if b.device.type == "cpu":
+        idx = b[:, 0]
+        bad = ~((idx >= 0) & (idx < batch))
+        if bool(bad.any()):
+            raise ValueError("boxes[:, 0] must be batch indices in [0, %d); got %s" % (batch, idx[bad][:4].tolist()))
+    return b.contiguous()
+
+
+def ava_boxes(boxes, height, width, size):
+    """The arithmetic of esf_ava_boxes on the host: the loader's boxes (K, 5) [batch index, x1, y1, x2, y2] in [0, 1]
+    of height x width frames -> FP32 (K, 5) in pixels of the frames resized to resized_size(height, width, size).  FP64
+    as numpy runs it: times (width, height), clip_boxes_to_image(height, width), times new / old of the short-side
+    resize (random_short_side_scale_jitter; none when the short side already is `size`), clip_boxes_to_image(size,
+    size), then FP32 as detection_collate makes it."""
+    b = np.array(boxes, dtype=np.float64).reshape(-1, 5)
+    Hr, Wr = resized_size(height, width, size)
+    out = b.copy()
+    for j, extent in ((1, width), (2, height), (3, width), (4, height)):
+        v = np.minimum(extent - 1.0, np.maximum(0.0, b[:, j] * extent))
+        if (Hr, Wr) != (height, width):
+            v = v * float(Hr if width < height else Wr) / (height if width < height else width)
+        out[:, j] = np.minimum(size - 1.0, np.maximum(0.0, v))
+    return torch.from_numpy(out.astype(np.float32))
+
+
+class AvaInput:
+    """Per-(model, device) state of the AVA frame route: the u / 255 table on the device, the channel order and the
+    statistics of every source channel (host arrays of esf_*_ava)."""
+
+    def __init__(self, cfg, device, channels):
+        data = cfg.DATA
+        ava = cfg.get("AVA", None) if hasattr(cfg, "get") else getattr(cfg, "AVA", None)
+        get = (lambda node, k, d: node.get(k, d) if node is not None and hasattr(node, "get") else d)
+        mean = list(get(data, "MEAN", [0.45] * channels))
+        std = list(get(data, "STD", [0.225] * channels))
+        if len(mean) != channels or len(std) != channels:
+            raise ValueError("DATA.MEAN / DATA.STD have %d / %d entries for %d channels (color_normalization asserts "
+                             "one per channel)" % (len(mean), len(std), channels))
+        src = ava_channel_source(channels, bool(get(ava, "BGR", False)), bool(get(data, "REVERSE_INPUT_CHANNEL", False)))
+        self.lut32 = unit_table(channels).to(device)
+        self.chan_src = (ctypes.c_int32 * channels)(*src)
+        # np.array(..., dtype=np.float32) in the loader: the statistics are FP32 numbers
+        self.mean = (ctypes.c_float * channels)(*[float(np.float32(m)) for m in mean])
+        self.std = (ctypes.c_float * channels)(*[float(np.float32(v)) for v in std])
+
+
 class FrameInput:
     """Per-(model, device) state of the frame route: look-up tables and frame indices on the device."""
 
@@ -340,6 +434,12 @@ class FrameInput:
         self._index = {}
         self._crops = {}
         self._videos = {}
+
+    def ava(self, cfg):
+        """AvaInput of this device (built on first use)."""
+        if getattr(self, "_ava", None) is None:
+            self._ava = AvaInput(cfg, self.device, self.channels)
+        return self._ava
 
     def crop(self, H0, W0, size, views):
         """CropTables of frames H0 x W0 cropped to size x size at `views` (cached per geometry)."""
@@ -456,3 +556,33 @@ def launch_video_list(plan, fin, videos):
                      "esf_stem_pack_u8_crop_videos")
         else:
             rt.check(L.esf_frames_to_clip_crop_videos(*args, own.data_ptr(), s), "esf_frames_to_clip_crop_videos")
+
+
+def launch_ava(plan, fin, ava, frames, crop, alpha):
+    """Fill the stem inputs of `plan` from uint8 frames (B, T, H, W, C) with the AVA test branch on the current stream:
+    every clip's whole frame resized to crop.Hr x crop.Wr (CropTables without views), normalised after the resize."""
+    L = rt.lib()
+    s = rt.current_stream_ptr()
+    B, Tsrc, H, W, C = frames.shape
+    for own in plan.inputs:
+        b, c, T, h, w = own.shape
+        assert (b, c, h, w) == (B, C, crop.Hr, crop.Wr) and (H, W) == (crop.H0, crop.W0)
+        idx = fin.index(Tsrc, T, alpha)
+        args = (frames.data_ptr(), B, Tsrc, H, W, C, idx.data_ptr() if idx is not None else None, T, ava.chan_src,
+                ava.lut32.data_ptr(), ava.mean, ava.std) + crop.pointers()
+        route = plan.stem_routes.get(own.data_ptr())
+        if route is not None:
+            xp, pitch, lpad = route
+            rt.check(L.esf_stem_pack_u8_ava(*args, rt.dtype_code(xp), pitch, lpad, xp.data_ptr(), s),
+                     "esf_stem_pack_u8_ava")
+        else:
+            rt.check(L.esf_frames_to_clip_ava(*args, own.data_ptr(), s), "esf_frames_to_clip_ava")
+
+
+def launch_ava_boxes(boxes, crop, out):
+    """esf_ava_boxes on the current stream: the loader's [0, 1] boxes (check_ava_boxes, on the device) to FP32 pixels of
+    the crop.Hr x crop.Wr frames in `out` (K, 5)."""
+    K = boxes.shape[0]
+    assert boxes.is_cuda and boxes.is_contiguous() and out.shape == (K, 5) and out.dtype == torch.float32
+    rt.check(rt.lib().esf_ava_boxes(boxes.data_ptr(), int(boxes.dtype == torch.float64), K, crop.H0, crop.W0, crop.Hr,
+                                    crop.Wr, crop.S, out.data_ptr(), rt.current_stream_ptr()), "esf_ava_boxes")

@@ -610,6 +610,62 @@ class _PlannedModel(nn.Module):
             out = plan.run_frames(lambda: esf_frames.launch_video_list(plan, fin, batch))
             return self._finish(plan, out, None)
 
+    def forward_ava_frames(self, frames, boxes, crop_size=None, return_boxes=False):
+        """AVA detection from the decoder's uint8 frames: the same result as `forward(clips, bboxes)` on what the test
+        split of the reference's AVA loader makes of them (datasets/ava_dataset.py _images_and_boxes_preprocessing,
+        PyTorch backend): `frames / 255`, the boxes times (W, H) and clipped to the frame, a bilinear short-side resize to
+        `crop_size` (default cfg.DATA.TEST_CROP_SIZE) with the boxes scaled alike and no crop, color_normalization with
+        DATA.MEAN / DATA.STD, the BGR -> RGB swap unless cfg.AVA.BGR, the boxes clipped to crop_size x crop_size, and
+        pack_pathway_output.  All of it runs on the device (csrc/esf_crop.cu): frames and boxes are read in place.
+
+        `frames`: contiguous uint8 (B, T, H, W, C) on a CUDA device, the loader's sampled frames at decode size.
+        `boxes`: floating (K, 5) rows [batch index, x1, y1, x2, y2] with coordinates in [0, 1] (the annotation format), on
+        the host (checked before anything runs) or on the device (read by the kernel, no synchronisation); FP64 boxes
+        keep the loader's FP64 arithmetic exactly.  Returns the (K, NUM_CLASSES) scores, and with `return_boxes` also
+        the transformed FP32 (K, 5) boxes in resized-frame pixels.  The plan is that of `forward(clips, bboxes)` on clips
+        of the resized size, and any number of boxes reuses its graph.  AVA.TEST_FORCE_FLIP is not covered."""
+        from . import frames as esf_frames
+        if self.training:
+            raise NotImplementedError("eval-mode forward path only")
+        if not self.enable_detection:
+            raise NotImplementedError("forward_ava_frames needs a detection model (cfg.DETECTION.ENABLE, ResNetRoIHead)")
+        cfg = self._cfg
+        ava = cfg.get("AVA", None) if hasattr(cfg, "get") else None
+        if ava is not None and hasattr(ava, "get") and bool(ava.get("TEST_FORCE_FLIP", False)):
+            raise NotImplementedError("AVA.TEST_FORCE_FLIP (the test branch's horizontal flip) is not covered by "
+                                      "forward_ava_frames")
+        B, T, H, W, C = esf_frames.check_ava_frames(frames)
+        b = esf_frames.check_ava_boxes(boxes, B)
+        S = int(cfg.DATA.TEST_CROP_SIZE if crop_size is None else crop_size)
+        if S < 1:
+            raise ValueError("crop_size must be >= 1, got %d" % S)
+        dev = frames.device
+        if dev.type != "cuda":
+            raise rt.EsfError("the forward path is CUDA-only (sm_100a); got frames on %s -- there is no CPU fallback"
+                              % dev)
+        Hr, Wr = esf_frames.resized_size(H, W, S)
+        shapes = self.frame_shapes((B, T, Hr, Wr, C))
+        K = b.shape[0]
+        if B == 0 or K == 0:
+            out = self._empty(dev)
+            return (out, torch.empty((0, 5), dtype=torch.float32, device=dev)) if return_boxes else out
+        alpha = cfg.SLOWFAST.ALPHA if self.num_pathways > 1 else 1
+        plan, fin = self._frame_plan(shapes, dev, C)
+        state = fin.ava(cfg)
+        tabs = fin.crop(H, W, S, ())
+        with torch.cuda.device(dev):
+            if b.device.type == "cpu":   # staged through pinned memory, as forward's boxes: no wait for earlier work
+                staged = torch.empty(b.shape, dtype=b.dtype, pin_memory=True)
+                staged.copy_(b)
+                b = staged.to(dev, non_blocking=True)
+            elif b.device != dev:
+                b = b.to(dev)
+            px = torch.empty((K, 5), dtype=torch.float32, device=dev)
+            esf_frames.launch_ava_boxes(b, tabs, px)
+            out = plan.run_frames(lambda: esf_frames.launch_ava(plan, fin, state, frames, tabs, alpha))
+            out = self._finish(plan, out, px)
+        return (out, px) if return_boxes else out
+
     def _empty(self, dev):
         return torch.empty((0, int(self._cfg.MODEL.NUM_CLASSES)), dtype=torch.float32, device=dev)
 

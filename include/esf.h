@@ -191,6 +191,32 @@ int esf_frames_to_clip_crop_videos(const void* frames_host, int32_t B, int32_t C
                                    const int32_t* chan_src, const float* lut32, const int32_t* geom_host,
                                    const void* tables_host, const int32_t* crop_yx_host, int32_t V, int32_t S,
                                    float* clip, void* stream);
+/* ---- AVA detection from uint8 frames (csrc/esf_crop.cu) ----------------------------------------------------------------
+ * The test split of the reference's AVA loader (SlowFast/slowfast/datasets/ava_dataset.py _images_and_boxes_preprocessing,
+ * PyTorch backend): u / 255 -> short-side bilinear resize to Hr x Wr (transform.random_short_side_scale_jitter, no
+ * crop) -> color_normalization -> channel swap -> pack_pathway_output, from frames at decode size (B, Tsrc, H0, W0, C).
+ * The resize runs on the [0, 1] values and the normalisation after it: lut32 is the [C][256] table of u / 255 (per
+ * OUTPUT channel, as esf_frames_to_clip), mean_host / std_host: host float[C], the statistics of every SOURCE channel
+ * (output channel c = source channel chan_src[c] takes those of its source).  Resize tables as esf_stem_pack_u8_crop
+ * (null when Hr == H0 and Wr == W0).  Output row b is clip b's whole Hr x Wr frame: packed stem rows [B][T][Hr][pitch]
+ * (pitch >= lpad + Wr * C) or the FP32 (B, C, T, Hr, Wr) clip. */
+int esf_stem_pack_u8_ava(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0, int32_t W0, int32_t C,
+                         const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
+                         const float* mean_host, const float* std_host, const int32_t* y_index, const float* y_weight,
+                         int32_t Hr, const int32_t* x_index, const float* x_weight, int32_t Wr, int32_t dtype,
+                         int32_t pitch, int32_t lpad, void* xp, void* stream);
+int esf_frames_to_clip_ava(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0, int32_t W0, int32_t C,
+                           const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,
+                           const float* mean_host, const float* std_host, const int32_t* y_index, const float* y_weight,
+                           int32_t Hr, const int32_t* x_index, const float* x_weight, int32_t Wr, float* clip,
+                           void* stream);
+/* The same branch's boxes: boxes (K, 5) on the device, FP32 (f64 = 0) or FP64 (f64 = 1), rows [batch index, x1, y1, x2,
+ * y2] with coordinates in [0, 1] of the H0 x W0 frames; out: FP32 (K, 5) in pixels of the Hr x Wr frames.  FP64 as the
+ * loader's numpy: times (W0, H0), clip_boxes_to_image(H0, W0), times new / old of the short-side resize (none when
+ * Hr == H0 and Wr == W0), clip_boxes_to_image(S, S) with S the crop size; the batch index is passed through.  No
+ * host synchronisation. */
+int esf_ava_boxes(const void* boxes, int32_t f64, int32_t K, int32_t H0, int32_t W0, int32_t Hr, int32_t Wr, int32_t S,
+                  float* out, void* stream);
 int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int32_t T, int32_t H, int32_t W, int32_t pitch,
                           const void* w_band, const float* bias_tiled, int32_t Cout, int32_t kT, int32_t kH,
                           int32_t kW, int32_t sH, int32_t sW, int32_t pT, int32_t pH, int32_t pW, int32_t act,
