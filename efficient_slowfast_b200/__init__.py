@@ -8,7 +8,7 @@ from .config import (CfgNode, ava_slow_8x8_r50_cfg, ava_slowfast_32x2_r50_cfg, g
                      slowfast_ghostnet_cfg, slowfast_mobilenetv2_cfg, slowfast_shufflenet_cfg,
                      slowfast_shufflenetv2_cfg)
 from .pipeline import ClipStream  # noqa: F401
-from .demo import SlidingWindow  # noqa: F401
+from .demo import CameraWindows, SlidingWindow  # noqa: F401
 from .testing import TestMeter, perform_test, topks_correct  # noqa: F401
 from .checkpoint import load_checkpoint, save_checkpoint  # noqa: F401
 from . import nets_resnet  # noqa: F401  (registers SlowFast, SlowFastDualAttention)

@@ -276,9 +276,32 @@ struct FramesParams {
   int chan_src[4];
 };
 
+// Frame addressing policies: the frame (index into `frames`, H * W * C bytes each) that output row b reads for pathway
+// frame t.  ClipFrames: B clips of Tsrc frames, t_index (or the identity) picks the frame of each clip.  RingFrames: a
+// bank of rings of Tsrc = L frames per camera; rows[b] = (camera, oldest slot) and t_index holds the window positions
+// (oldest frame = 0), so the frame is ring slot (pos[t] + oldest) % L of that camera.  The host checks camera < N and
+// pos, oldest in [0, L), hence one conditional subtraction is the modulo.
+struct ClipFrames {
+  __device__ __forceinline__ long long operator()(const FramesParams& p, int b, int t) const {
+    const int ts = p.t_index ? __ldg(p.t_index + t) : t;
+    return (long long)b * p.Tsrc + ts;
+  }
+};
+
+struct RingFrames {
+  const int32_t* rows;
+  __device__ __forceinline__ long long operator()(const FramesParams& p, int b, int t) const {
+    const int camera = __ldg(rows + 2 * b), oldest = __ldg(rows + 2 * b + 1);
+    int slot = __ldg(p.t_index + t) + oldest;
+    if (slot >= p.Tsrc) slot -= p.Tsrc;
+    return (long long)camera * p.Tsrc + slot;
+  }
+};
+
 // -> packed 16-bit stem rows [B][T][H][pitch] (see stem_pack_kernel): one thread = 8 consecutive row elements
+template <class Frames>
 __global__ void __launch_bounds__(256) stem_pack_u8_kernel(const FramesParams p, const uint16_t* __restrict__ lut, int pitch,
-                                                           int lpad, uint16_t* __restrict__ xp) {
+                                                           int lpad, uint16_t* __restrict__ xp, const Frames frame_of) {
   __shared__ uint16_t lut_s[4 * 256];
   for (int i = threadIdx.x; i < p.C * 256; i += blockDim.x) lut_s[i] = lut[i];
   __syncthreads();
@@ -294,8 +317,7 @@ __global__ void __launch_bounds__(256) stem_pack_u8_kernel(const FramesParams p,
     r /= p.H;
     const int t = r % p.T;
     const int b = r / p.T;
-    const int ts = p.t_index ? __ldg(p.t_index + t) : t;
-    const uint8_t* row = p.frames + (((long long)b * p.Tsrc + ts) * p.H + h) * WC;
+    const uint8_t* row = p.frames + (frame_of(p, b, t) * p.H + h) * WC;
     const int j0 = ck * 8 - lpad;
     int c = ((j0 % p.C) + p.C) % p.C;
     uint16_t v[8];
@@ -321,8 +343,9 @@ __global__ void __launch_bounds__(256) stem_pack_u8_kernel(const FramesParams p,
 
 // -> FP32 NCDHW clip (B, C, T, H, W): the generic route for stems that do not take packed rows.  One thread = 4
 // consecutive w of one (b, c, t, h) row (16-byte store).
+template <class Frames>
 __global__ void __launch_bounds__(256) frames_to_clip_kernel(const FramesParams p, const float* __restrict__ lut,
-                                                             float* __restrict__ clip) {
+                                                             float* __restrict__ clip, const Frames frame_of) {
   __shared__ float lut_s[4 * 256];
   for (int i = threadIdx.x; i < p.C * 256; i += blockDim.x) lut_s[i] = lut[i];
   __syncthreads();
@@ -339,8 +362,7 @@ __global__ void __launch_bounds__(256) frames_to_clip_kernel(const FramesParams 
     r /= p.T;
     const int c = r % p.C;
     const int b = r / p.C;
-    const int ts = p.t_index ? __ldg(p.t_index + t) : t;
-    const uint8_t* src = p.frames + ((((long long)b * p.Tsrc + ts) * p.H + h) * p.W + w0) * p.C + p.chan_src[c];
+    const uint8_t* src = p.frames + ((frame_of(p, b, t) * p.H + h) * p.W + w0) * p.C + p.chan_src[c];
     float v[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) v[e] = (w0 + e < p.W) ? lut_s[c * 256 + __ldg(src + e * p.C)] : 0.f;
@@ -2292,7 +2314,7 @@ extern "C" int esf_stem_pack_u8(const uint8_t* frames, int32_t B, int32_t Tsrc, 
   ESF_CHECK_ARG(pitch % 8 == 0 && lpad >= 0 && pitch >= lpad + W * C, "esf_stem_pack_u8: bad pitch %d", pitch);
   const long long total = (long long)B * T * H * (pitch / 8);
   stem_pack_u8_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      p, static_cast<const uint16_t*>(lut16), pitch, lpad, static_cast<uint16_t*>(xp));
+      p, static_cast<const uint16_t*>(lut16), pitch, lpad, static_cast<uint16_t*>(xp), ClipFrames{});
   return check_launch("stem_pack_u8_kernel");
 }
 
@@ -2304,8 +2326,59 @@ extern "C" int esf_frames_to_clip(const uint8_t* frames, int32_t B, int32_t Tsrc
   if (rc != ESF_OK) return rc;
   ESF_CHECK_ARG(lut32 && clip, "esf_frames_to_clip: null argument");
   const long long total = (long long)B * C * T * H * ((W + 3) / 4);
-  frames_to_clip_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(p, lut32, clip);
+  frames_to_clip_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(p, lut32, clip,
+                                                                                             ClipFrames{});
   return check_launch("frames_to_clip_kernel");
+}
+
+// Ring bank (N, L, H, W, C): frames_params with B = R output rows and Tsrc = L, then the range checks that make the
+// device-side slot arithmetic of RingFrames safe, on the host copies of the tables the kernel reads.
+static int rings_params(FramesParams* p, const char* who, const uint8_t* bank, int32_t N, int32_t L, int32_t H, int32_t W,
+                        int32_t C, const int32_t* rows, const int32_t* rows_host, int32_t R, const int32_t* pos,
+                        const int32_t* pos_host, int32_t T, const int32_t* chan_src) {
+  ESF_CHECK_ARG(N >= 1 && R >= 1 && rows && rows_host && pos && pos_host, "%s: null/bad argument (N %d, R %d)", who, N, R);
+  const int rc = frames_params(p, bank, R, L, H, W, C, pos, T, chan_src, who);
+  if (rc != ESF_OK) return rc;
+  for (int r = 0; r < R; ++r) {
+    ESF_CHECK_ARG(rows_host[2 * r] >= 0 && rows_host[2 * r] < N, "%s: row %d: camera %d not in [0, %d)", who, r,
+                  rows_host[2 * r], N);
+    ESF_CHECK_ARG(rows_host[2 * r + 1] >= 0 && rows_host[2 * r + 1] < L, "%s: row %d: oldest slot %d not in [0, %d)", who,
+                  r, rows_host[2 * r + 1], L);
+  }
+  for (int t = 0; t < T; ++t)
+    ESF_CHECK_ARG(pos_host[t] >= 0 && pos_host[t] < L, "%s: pos[%d] = %d not in [0, %d)", who, t, pos_host[t], L);
+  return ESF_OK;
+}
+
+extern "C" int esf_stem_pack_u8_rings(const uint8_t* bank, int32_t N, int32_t L, int32_t H, int32_t W, int32_t C,
+                                      const int32_t* rows, const int32_t* rows_host, int32_t R, const int32_t* pos,
+                                      const int32_t* pos_host, int32_t T, const int32_t* chan_src, const void* lut16,
+                                      int32_t pitch, int32_t lpad, void* xp, void* stream) {
+  FramesParams p;
+  const int rc = rings_params(&p, "esf_stem_pack_u8_rings", bank, N, L, H, W, C, rows, rows_host, R, pos, pos_host, T,
+                              chan_src);
+  if (rc != ESF_OK) return rc;
+  ESF_CHECK_ARG(pitch % 8 == 0 && lpad >= 0 && pitch >= lpad + W * C, "esf_stem_pack_u8_rings: bad pitch %d", pitch);
+  ESF_CHECK_ARG(lut16 && xp, "esf_stem_pack_u8_rings: null argument");
+  const long long total = (long long)R * T * H * (pitch / 8);
+  stem_pack_u8_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      p, static_cast<const uint16_t*>(lut16), pitch, lpad, static_cast<uint16_t*>(xp), RingFrames{rows});
+  return check_launch("stem_pack_u8_kernel (rings)");
+}
+
+extern "C" int esf_frames_to_clip_rings(const uint8_t* bank, int32_t N, int32_t L, int32_t H, int32_t W, int32_t C,
+                                        const int32_t* rows, const int32_t* rows_host, int32_t R, const int32_t* pos,
+                                        const int32_t* pos_host, int32_t T, const int32_t* chan_src, const float* lut32,
+                                        float* clip, void* stream) {
+  FramesParams p;
+  const int rc = rings_params(&p, "esf_frames_to_clip_rings", bank, N, L, H, W, C, rows, rows_host, R, pos, pos_host, T,
+                              chan_src);
+  if (rc != ESF_OK) return rc;
+  ESF_CHECK_ARG(lut32 && clip, "esf_frames_to_clip_rings: null argument");
+  const long long total = (long long)R * C * T * H * ((W + 3) / 4);
+  frames_to_clip_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(p, lut32, clip,
+                                                                                             RingFrames{rows});
+  return check_launch("frames_to_clip_kernel (rings)");
 }
 
 extern "C" int esf_row_softmax(const float* S, int64_t rows, int32_t n, int64_t s_pitch, float scale, int32_t mode,

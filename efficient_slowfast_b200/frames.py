@@ -510,6 +510,34 @@ def launch_frames(plan, fin, frames, alpha, frame_index=None, crop=None):
                                           fin.lut32.data_ptr(), own.data_ptr(), s), "esf_frames_to_clip")
 
 
+def launch_rings(plan, fin, bank, rows, positions):
+    """Fill the stem inputs of `plan` from a bank of per-camera frame rings (N, L, H, W, C) uint8 on the current stream
+    (demo.CameraWindows): output row r, frame t of pathway p is ring slot (positions[p][t] + oldest_r) % L of camera
+    camera_r.  `rows`: (device, host) contiguous int32 tables (R, 2) of (camera, oldest slot), R = the plan's rows;
+    the library's range checks read the host copy.  `positions`: one (device tensor, host ctypes int32 array) pair of
+    window positions [T_p] per pathway (demo.window_indices)."""
+    L = rt.lib()
+    s = rt.current_stream_ptr()
+    N, Lr, H, W, C = bank.shape
+    dev_rows, host_rows = rows
+    assert host_rows.device.type == "cpu" and host_rows.is_contiguous() and host_rows.dtype == torch.int32
+    rows_host = ctypes.cast(host_rows.data_ptr(), ctypes.POINTER(ctypes.c_int32))
+    for own, (dev_pos, host_pos) in zip(plan.inputs, positions):
+        R, c, T, h, w = own.shape
+        assert (c, h, w) == (C, H, W) and dev_pos.numel() == len(host_pos) == T
+        assert dev_rows.shape[0] >= R and host_rows.shape[0] >= R
+        args = (bank.data_ptr(), N, Lr, H, W, C, dev_rows.data_ptr(), rows_host, R, dev_pos.data_ptr(), host_pos, T,
+                fin.chan_src)
+        route = plan.stem_routes.get(own.data_ptr())
+        if route is not None:
+            xp, pitch, lpad = route
+            rt.check(L.esf_stem_pack_u8_rings(*args, fin.lut16.data_ptr(), pitch, lpad, xp.data_ptr(), s),
+                     "esf_stem_pack_u8_rings")
+        else:
+            rt.check(L.esf_frames_to_clip_rings(*args, fin.lut32.data_ptr(), own.data_ptr(), s),
+                     "esf_frames_to_clip_rings")
+
+
 def launch_clip_list(plan, fin, clips, alpha):
     """Fill the stem inputs of `plan` from a ClipList on the current stream: row b * V + v is clip b at view v."""
     L = rt.lib()

@@ -85,6 +85,10 @@ def lib():
     L.esf_group_mean.argtypes = [vp, i32, i32, i32, vp, vp]
     L.esf_stem_pack_u8.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, P(i32), vp, i32, i32, vp, vp]
     L.esf_frames_to_clip.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, P(i32), vp, vp, vp]
+    L.esf_stem_pack_u8_rings.argtypes = [vp, i32, i32, i32, i32, i32, vp, P(i32), i32, vp, P(i32), i32, P(i32), vp, i32,
+                                         i32, vp, vp]
+    L.esf_frames_to_clip_rings.argtypes = [vp, i32, i32, i32, i32, i32, vp, P(i32), i32, vp, P(i32), i32, P(i32), vp,
+                                           vp, vp]
     L.esf_stem_pack_u8_crop.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, P(i32), vp, vp, vp, i32, vp, vp, i32,
                                         P(i32), i32, i32, i32, i32, i32, vp, vp]
     L.esf_frames_to_clip_crop.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, P(i32), vp, vp, vp, i32, vp, vp, i32,

@@ -142,6 +142,21 @@ int esf_stem_pack_u8(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H, 
 int esf_frames_to_clip(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H, int32_t W, int32_t C,
                        const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32, float* clip,
                        void* stream);
+/* The same two outputs gathered from a bank of per-camera frame rings (the demo loop over many cameras,
+ * efficient_slowfast_b200/demo.py CameraWindows): bank: device uint8 (N, L, H, W, C) contiguous, camera n's ring of its
+ * last L frames.  rows: device int32[R][2], (camera, oldest ring slot) of every output row.  pos: device int32[T], the
+ * pathway's window positions (oldest frame = 0, demo.window_indices).  Output row r, frame t is ring slot
+ * (pos[t] + oldest_r) % L of camera camera_r, so a call uploads only the 8 * R bytes of rows.  rows_host / pos_host:
+ * the same tables on the host, read for the range checks before the launch: R >= 1, camera in [0, N), oldest and pos
+ * entries in [0, L).  chan_src, tables and outputs as esf_stem_pack_u8 / esf_frames_to_clip with B = R rows. */
+int esf_stem_pack_u8_rings(const uint8_t* bank, int32_t N, int32_t L, int32_t H, int32_t W, int32_t C,
+                           const int32_t* rows, const int32_t* rows_host, int32_t R, const int32_t* pos,
+                           const int32_t* pos_host, int32_t T, const int32_t* chan_src, const void* lut16, int32_t pitch,
+                           int32_t lpad, void* xp, void* stream);
+int esf_frames_to_clip_rings(const uint8_t* bank, int32_t N, int32_t L, int32_t H, int32_t W, int32_t C,
+                             const int32_t* rows, const int32_t* rows_host, int32_t R, const int32_t* pos,
+                             const int32_t* pos_host, int32_t T, const int32_t* chan_src, const float* lut32,
+                             float* clip, void* stream);
 /* ---- test-time spatial sampling of uint8 frames (csrc/esf_crop.cu) -------------------------------------------------
  * The same chain with the reference's test-mode spatial_sampling in between (SlowFast/slowfast/datasets/utils.py
  * spatial_sampling -> transform.random_short_side_scale_jitter with min = max = crop size S, bilinear
