@@ -485,9 +485,104 @@ static int ava_launch(const char* who, const AvaParams& p, int pitch, int lpad, 
   return check_launch(who);
 }
 
+// The demo's frame resize (tools/demo_net.py -> datasets/cv2_transform.scale: cv2.resize(frame, (Ws, Hs),
+// interpolation=cv2.INTER_LINEAR) on uint8), OpenCV's fixed-point arithmetic in integers only.  Every axis is a host
+// table (efficient_slowfast_b200/frames.py cv2_axis_table) of (source index s, weights w0 | w1 << 16), 11-bit weights;
+// the x table holds OpenCV's clamped (s, f), the y table its unclamped s.  Both read s and s + 1 clamped to the frame:
+//   row_k[x] = p_k[s_x] * w0_x + p_k[s_x + 1] * w1_x                                       (k = source rows s_y, s_y + 1)
+//   out = (((w0_y * (row_0 >> 4)) >> 16) + ((w1_y * (row_1 >> 4)) >> 16) + 2) >> 2,  saturated   (VResizeLinear, uint8)
+// One block per output row of one frame (grid.y: the frame of the chunk): the two source rows go to shared memory with
+// 16-byte loads, then one thread per output byte.  A launch takes up to kResizeChunk frames of their own geometry, source
+// and destination, by value in the parameter block.
+constexpr int kResizeChunk = 64;
+
+struct ResizeFrame {
+  const uint8_t* src;    // (H, W, C)
+  uint8_t* dst;          // (Hs, Ws, C)
+  const int2* y_tab;     // [Hs]
+  const int2* x_tab;     // [Ws]
+  int H, W, Hs, Ws;
+};
+
+struct ResizeChunk {
+  int C;
+  ResizeFrame f[kResizeChunk];
+};
+static_assert(sizeof(ResizeChunk) <= 4096, "ResizeChunk must fit the 4 KB parameters");
+
+__global__ void __launch_bounds__(kCropThreads) resize_u8_cv2_kernel(const __grid_constant__ ResizeChunk p) {
+  extern __shared__ __align__(16) uint8_t rows_s[];
+  const ResizeFrame& f = p.f[blockIdx.y];
+  const int y = blockIdx.x;
+  if (y >= f.Hs) return;
+  const int C = p.C;
+  const int row_bytes = f.W * C;
+  const int row_pitch = ((row_bytes + 15) & ~15) + 16;   // + 16: room for the source's 16-byte phase
+  const int2 yt = __ldg(f.y_tab + y);
+  const int s0 = min(max(yt.x, 0), f.H - 1), s1 = min(max(yt.x + 1, 0), f.H - 1);
+  const uint8_t* r0 = load_row_bytes(rows_s, f.src + (long long)s0 * row_bytes, row_bytes);
+  const uint8_t* r1 = load_row_bytes(rows_s + row_pitch, f.src + (long long)s1 * row_bytes, row_bytes);
+  __syncthreads();
+  const int b0 = yt.y & 0xffff, b1 = (int)((unsigned)yt.y >> 16);
+  const int n = f.Ws * C;
+  uint8_t* dst = f.dst + (long long)y * n;
+  for (int j = threadIdx.x; j < n; j += blockDim.x) {
+    const int x = j / C, c = j - x * C;
+    const int2 xt = __ldg(f.x_tab + x);
+    const int a = min(max(xt.x, 0), f.W - 1) * C + c, b = min(max(xt.x + 1, 0), f.W - 1) * C + c;
+    const int a0 = xt.y & 0xffff, a1 = (int)((unsigned)xt.y >> 16);
+    const int v0 = r0[a] * a0 + r0[b] * a1;
+    const int v1 = r1[a] * a0 + r1[b] * a1;
+    const int v = (((b0 * (v0 >> 4)) >> 16) + ((b1 * (v1 >> 4)) >> 16) + 2) >> 2;
+    dst[j] = (uint8_t)min(max(v, 0), 255);
+  }
+}
+
 }  // namespace esf
 
 using namespace esf;
+
+extern "C" int esf_resize_u8_cv2(const void* frames_host, const void* dst_host, const int32_t* geom_host,
+                                 const void* tables_host, int32_t B, int32_t C, void* stream) {
+  ESF_CHECK_ARG(B >= 1 && frames_host && dst_host && geom_host && tables_host, "esf_resize_u8_cv2: null/bad argument");
+  // C = 2: OpenCV resizes exact 2x downscales of 2-channel frames with INTER_AREA, which this kernel does not restate
+  ESF_CHECK_ARG(C == 1 || C == 3 || C == 4, "esf_resize_u8_cv2: %d channels (1, 3 or 4)", C);
+  const void* const* src = static_cast<const void* const*>(frames_host);
+  void* const* dst = static_cast<void* const*>(const_cast<void*>(dst_host));
+  const void* const* tb = static_cast<const void* const*>(tables_host);
+  for (int b = 0; b < B; ++b) {   // a bad frame anywhere: nothing is written
+    const int32_t* g = geom_host + 4 * b;
+    ESF_CHECK_ARG(src[b] && dst[b] && tb[2 * b] && tb[2 * b + 1], "esf_resize_u8_cv2: frame %d: null address", b);
+    ESF_CHECK_ARG(((reinterpret_cast<uintptr_t>(tb[2 * b]) | reinterpret_cast<uintptr_t>(tb[2 * b + 1])) & 7) == 0,
+                  "esf_resize_u8_cv2: frame %d: misaligned axis table", b);
+    ESF_CHECK_ARG(g[0] > 0 && g[1] > 0 && g[2] > 0 && g[3] > 0, "esf_resize_u8_cv2: frame %d: bad size %d x %d -> %d x %d",
+                  b, g[0], g[1], g[2], g[3]);
+    ESF_CHECK_ARG((long long)g[1] * C <= kCropMaxRowBytes, "esf_resize_u8_cv2: frame %d: source rows of %lld bytes exceed %d",
+                  b, (long long)g[1] * C, kCropMaxRowBytes);
+    ESF_CHECK_ARG((long long)g[2] * g[3] * C < (1LL << 31), "esf_resize_u8_cv2: frame %d: output too large", b);
+  }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  ResizeChunk p{};
+  p.C = C;
+  for (int b0 = 0; b0 < B; b0 += kResizeChunk) {
+    const int n = std::min(B - b0, kResizeChunk);
+    int hs = 0, w0 = 0;
+    for (int i = 0; i < n; ++i) {
+      const int32_t* g = geom_host + 4 * (b0 + i);
+      ResizeFrame& f = p.f[i];
+      f.src = static_cast<const uint8_t*>(src[b0 + i]);
+      f.dst = static_cast<uint8_t*>(dst[b0 + i]);
+      f.y_tab = static_cast<const int2*>(tb[2 * (b0 + i)]);
+      f.x_tab = static_cast<const int2*>(tb[2 * (b0 + i) + 1]);
+      f.H = g[0], f.W = g[1], f.Hs = g[2], f.Ws = g[3];
+      hs = std::max(hs, f.Hs), w0 = std::max(w0, f.W);
+    }
+    resize_u8_cv2_kernel<<<dim3((unsigned)hs, (unsigned)n), kCropThreads, crop_smem(w0, C), s>>>(p);
+    const int rc = check_launch("resize_u8_cv2_kernel");
+    if (rc != ESF_OK) return rc;
+  }
+  return ESF_OK;
+}
 
 extern "C" int esf_stem_pack_u8_crop(const uint8_t* frames, int32_t B, int32_t Tsrc, int32_t H0, int32_t W0, int32_t C,
                                      const int32_t* t_index, int32_t T, const int32_t* chan_src, const float* lut32,

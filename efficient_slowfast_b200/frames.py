@@ -430,6 +430,9 @@ class FrameInput:
             self.lut32 = self.lut32[src].contiguous()
             self.lut16 = self.lut16[src].contiguous()
         self.chan_src = (ctypes.c_int32 * channels)(*src)
+        # BGR frames (cv2.VideoCapture's order; the demo swaps with COLOR_BGR2RGB before everything else): RGB channel k
+        # is frame channel 2 - k, and the tables stay those of the RGB channels
+        self.chan_src_bgr = (ctypes.c_int32 * 3)(*[2 - k for k in src]) if channels == 3 else None
         self.device = device
         self._index = {}
         self._crops = {}
@@ -510,12 +513,12 @@ def launch_frames(plan, fin, frames, alpha, frame_index=None, crop=None):
                                           fin.lut32.data_ptr(), own.data_ptr(), s), "esf_frames_to_clip")
 
 
-def launch_rings(plan, fin, bank, rows, positions):
+def launch_rings(plan, fin, bank, rows, positions, bgr=False):
     """Fill the stem inputs of `plan` from a bank of per-camera frame rings (N, L, H, W, C) uint8 on the current stream
     (demo.CameraWindows): output row r, frame t of pathway p is ring slot (positions[p][t] + oldest_r) % L of camera
     camera_r.  `rows`: (device, host) contiguous int32 tables (R, 2) of (camera, oldest slot), R = the plan's rows;
     the library's range checks read the host copy.  `positions`: one (device tensor, host ctypes int32 array) pair of
-    window positions [T_p] per pathway (demo.window_indices)."""
+    window positions [T_p] per pathway (demo.window_indices).  `bgr`: the rings hold BGR frames (FrameInput.chan_src_bgr)."""
     L = rt.lib()
     s = rt.current_stream_ptr()
     N, Lr, H, W, C = bank.shape
@@ -527,7 +530,7 @@ def launch_rings(plan, fin, bank, rows, positions):
         assert (c, h, w) == (C, H, W) and dev_pos.numel() == len(host_pos) == T
         assert dev_rows.shape[0] >= R and host_rows.shape[0] >= R
         args = (bank.data_ptr(), N, Lr, H, W, C, dev_rows.data_ptr(), rows_host, R, dev_pos.data_ptr(), host_pos, T,
-                fin.chan_src)
+                fin.chan_src_bgr if bgr else fin.chan_src)
         route = plan.stem_routes.get(own.data_ptr())
         if route is not None:
             xp, pitch, lpad = route
@@ -605,6 +608,67 @@ def launch_ava(plan, fin, ava, frames, crop, alpha):
                      "esf_stem_pack_u8_ava")
         else:
             rt.check(L.esf_frames_to_clip_ava(*args, own.data_ptr(), s), "esf_frames_to_clip_ava")
+
+
+# one entry of a cv2_axis_table: the layout esf_resize_u8_cv2 reads (8 bytes, little-endian)
+CV2_AXIS = np.dtype([("index", "<i4"), ("w0", "<i2"), ("w1", "<i2")])
+
+
+def cv2_axis_table(n_in, n_out, clamp):
+    """One axis of OpenCV's cv2.resize(..., interpolation=cv2.INTER_LINEAR) on uint8 (imgproc resize.cpp, fixed point
+    with 11-bit weights), as a CV2_AXIS array [n_out].  With scale = 1 / (n_out / n_in) in double: f = float32((d + 0.5)
+    * scale - 0.5), s = floor(f), f -= s; w0 = rint(float32((1 - f) * 2048)), w1 = rint(float32(f * 2048)).  `clamp` (the
+    x axis) is OpenCV's column rule: s < 0 gives (0, f = 0) and s >= n_in - 1 gives (n_in - 1, f = 0).  The y axis keeps
+    s and f as they are; its rows are s and s + 1 clamped to the frame (which the kernel applies to both axes)."""
+    scale = 1.0 / (float(n_out) / n_in)
+    f = ((np.arange(n_out, dtype=np.float64) + 0.5) * scale - 0.5).astype(np.float32)
+    s = np.floor(f)
+    f = (f - s).astype(np.float32)
+    s = s.astype(np.int64)
+    if clamp:
+        for edge, value in ((s < 0, 0), (s >= n_in - 1, n_in - 1)):
+            s[edge], f[edge] = value, np.float32(0)
+    out = np.empty(n_out, CV2_AXIS)
+    out["index"] = s
+    out["w0"] = np.rint((np.float32(1) - f) * np.float32(2048)).astype(np.int16)
+    out["w1"] = np.rint(f * np.float32(2048)).astype(np.int16)
+    return out
+
+
+def scale_boxes(size, boxes, height, width):
+    """datasets/cv2_transform.scale_boxes on a copy of FP32 `boxes` (K, 4) in pixels of height x width frames: unchanged
+    when the short side already is `size`, else times float(new long side) / long side, the reference's own torch
+    expression (the multiplication runs in FP32 on the boxes' device)."""
+    boxes = boxes.detach().to(torch.float32).clone()
+    Hs, Ws = resized_size(height, width, size)
+    if (Hs, Ws) == (height, width):
+        return boxes
+    if width < height:
+        boxes *= float(Hs) / height
+    else:
+        boxes *= float(Ws) / width
+    return boxes
+
+
+class Cv2Resize:
+    """Device tables of the demo's resize of height x width frames to short side `size` (cv2_transform.scale): the y and
+    x cv2_axis_table, uploaded once."""
+
+    def __init__(self, height, width, size, device):
+        self.H, self.W = int(height), int(width)
+        self.Hs, self.Ws = resized_size(self.H, self.W, int(size))
+        self.y = torch.from_numpy(cv2_axis_table(self.H, self.Hs, False).view(np.int32)).to(device)
+        self.x = torch.from_numpy(cv2_axis_table(self.W, self.Ws, True).view(np.int32)).to(device)
+
+
+def launch_resize_cv2(sources, destinations, resizes, channels):
+    """esf_resize_u8_cv2 on the current stream: frame b at device address sources[b] (H, W, C) resized by resizes[b]
+    (Cv2Resize) into destinations[b] (Hs, Ws, C), in one call."""
+    B = len(sources)
+    geom = (ctypes.c_int32 * (4 * B))(*[n for r in resizes for n in (r.H, r.W, r.Hs, r.Ws)])
+    tables = (ctypes.c_void_p * (2 * B))(*[a for r in resizes for a in (r.y.data_ptr(), r.x.data_ptr())])
+    rt.check(rt.lib().esf_resize_u8_cv2((ctypes.c_void_p * B)(*sources), (ctypes.c_void_p * B)(*destinations), geom,
+                                        tables, B, channels, rt.current_stream_ptr()), "esf_resize_u8_cv2")
 
 
 def launch_ava_boxes(boxes, crop, out):

@@ -232,6 +232,18 @@ int esf_frames_to_clip_ava(const uint8_t* frames, int32_t B, int32_t Tsrc, int32
  * host synchronisation. */
 int esf_ava_boxes(const void* boxes, int32_t f64, int32_t K, int32_t H0, int32_t W0, int32_t Hr, int32_t Wr, int32_t S,
                   float* out, void* stream);
+/* ---- the demo's frame resize (csrc/esf_crop.cu) -------------------------------------------------------------------------
+ * cv2.resize(frame, (Ws, Hs), interpolation=cv2.INTER_LINEAR) on uint8 frames, as the reference demo's
+ * datasets/cv2_transform.scale runs it on every captured frame: OpenCV's fixed-point arithmetic (11-bit weights) in
+ * integers, bit for bit.  One call resizes B frames of their own sizes: frames_host / dst_host are host arrays of B
+ * device addresses, frame b being (H, W, C) uint8 contiguous and its output (Hs, Ws, C) uint8 contiguous (a camera's
+ * ring slot).  geom_host: host int32[B][4], (H, W, Hs, Ws).  tables_host: host array [B][2] of the device addresses
+ * (8-byte aligned) of the y table [Hs] and the x table [Ws], entries {int32 source index; int16 w0; int16 w1} as
+ * efficient_slowfast_b200/frames.py cv2_axis_table makes them.  C is 1, 3 or 4 (OpenCV takes another route for the
+ * exact 2x downscale of 2-channel frames); W * C <= 16384.  Every frame is checked before anything is launched; the
+ * host arrays are read before the call returns. */
+int esf_resize_u8_cv2(const void* frames_host, const void* dst_host, const int32_t* geom_host, const void* tables_host,
+                      int32_t B, int32_t C, void* stream);
 int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int32_t T, int32_t H, int32_t W, int32_t pitch,
                           const void* w_band, const float* bias_tiled, int32_t Cout, int32_t kT, int32_t kH,
                           int32_t kW, int32_t sH, int32_t sW, int32_t pT, int32_t pH, int32_t pW, int32_t act,
