@@ -9,10 +9,11 @@ from .config import (CfgNode, ava_slow_8x8_r50_cfg, ava_slowfast_32x2_r50_cfg, g
                      slowfast_shufflenetv2_cfg)
 from .pipeline import ClipStream  # noqa: F401
 from .demo import CameraWindows, SlidingWindow  # noqa: F401
+from .jpeg import decode_jpeg  # noqa: F401
 from .testing import TestMeter, perform_test, topks_correct  # noqa: F401
 from .checkpoint import load_checkpoint, save_checkpoint  # noqa: F401
 from . import nets_resnet  # noqa: F401  (registers SlowFast, SlowFastDualAttention)
 from . import nets_efficient  # noqa: F401  (registers SlowFastShuffleNetV2, SlowFastShuffleNet, ...)
 
-__all__ = ["MODEL_REGISTRY", "build_model", "get_cfg", "CfgNode", "ClipStream", "slowfast_4x16_r50_cfg",
+__all__ = ["MODEL_REGISTRY", "build_model", "get_cfg", "CfgNode", "ClipStream", "decode_jpeg", "slowfast_4x16_r50_cfg",
            "slowfast_dual_8x8_r50_cfg"]

@@ -11,7 +11,8 @@ import subprocess
 
 CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc")
 LIB = os.path.join(CSRC, "libesf_b200.so")
-SOURCES = ["esf_api.cu", "esf_igemm.cu", "esf_simt.cu", "esf_attention.cu", "esf_attn_tc.cu", "esf_precise.cu", "esf_roi.cu", "esf_crop.cu"]
+SOURCES = ["esf_api.cu", "esf_igemm.cu", "esf_simt.cu", "esf_attention.cu", "esf_attn_tc.cu", "esf_precise.cu", "esf_roi.cu", "esf_crop.cu",
+           "esf_jpeg.cu"]
 HEADERS = ["esf_common.cuh", "esf_host.h", os.path.join("..", "..", "include", "esf.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -106,6 +106,8 @@ def lib():
                                          i32, vp, vp]
     L.esf_ava_boxes.argtypes = [vp, i32, i32, i32, i32, i32, i32, i32, vp, vp]
     L.esf_resize_u8_cv2.argtypes = [vp, vp, P(i32), vp, i32, i32, vp]
+    L.esf_jpeg_scratch_bytes.argtypes = [vp, i32, i32, vp]
+    L.esf_jpeg_decode.argtypes = [vp, i64, vp, i32, vp, i32, i32, i32, vp, i64, vp, i32, i32, i32, i32, vp, vp]
     L.esf_stem_igemm_create.argtypes = [vp, i32, i32, i32, i32, i32, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32,
                                         i32, i32, i32, P(EsfView), P(vp)]
     L.esf_stem_tband_create.argtypes = L.esf_stem_igemm_create.argtypes

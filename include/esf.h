@@ -244,6 +244,36 @@ int esf_ava_boxes(const void* boxes, int32_t f64, int32_t K, int32_t H0, int32_t
  * host arrays are read before the call returns. */
 int esf_resize_u8_cv2(const void* frames_host, const void* dst_host, const int32_t* geom_host, const void* tables_host,
                       int32_t B, int32_t C, void* stream);
+/* ---- baseline JPEG decoding (csrc/esf_jpeg.cu) --------------------------------------------------------------------------
+ * cv2.imdecode(buf, cv2.IMREAD_COLOR) (BGR) or, with gray, cv2.IMREAD_GRAYSCALE, bit for bit (OpenCV's libjpeg-turbo with
+ * its defaults: islow IDCT, fancy upsampling), for the frame-directory loaders' cv2.imread.  Baseline / extended
+ * sequential Huffman files of 8-bit precision, one interleaved scan, 1 component or 3 YCbCr components with luma
+ * sampling 1x1, 2x1, 2x2, 1x2 or 4x1 and 1x1 chroma.  efficient_slowfast_b200/jpeg.py parses the files and packs `blob`
+ * (device, 16-byte aligned, blob_bytes long), sections 16-byte aligned in this order:
+ *   esf_jpeg_file[n_files], esf_jpeg_segment[n_segs], n_huff Huffman tables of 1424 bytes (uint16 look[512]: code
+ *   length << 8 | symbol of the 9-bit codes' prefixes, 0 for longer codes; int32 maxcode[18]; int32 valoffset[18];
+ *   uint8 values[256], as libjpeg's jpeg_make_d_derived_tbl), n_quant quantisation tables (int16[64], natural order),
+ *   then the files' bytes, which segment offsets count from.
+ * files_host / segs_host are host copies of the first two sections; every descriptor is checked on them before anything
+ * is launched.  Segments are grouped by file in file order, one per restart interval (first_mcu = k * restart) or one per
+ * scan.  scratch: esf_jpeg_scratch_bytes bytes (16-byte aligned).  out: (n_files, H, W, C) uint8 contiguous, C = 3 or
+ * C = 1 with gray; every file is H x W.  status: device int32[n_files], zeroed, then nonzero for a file whose scan holds
+ * an invalid Huffman code (its pixels are then unspecified; nothing is written outside its frame). */
+typedef struct esf_jpeg_file {
+  int32_t H, W, ncomp, restart; /* restart interval in MCUs, 0: the scan is one segment */
+  int32_t h[3], v[3];           /* sampling factors (1, 1 for a one-component file) */
+  int32_t qt[3], dc[3], ac[3];  /* per component: quantisation and Huffman table indices into the blob's sections */
+  int32_t pad;
+} esf_jpeg_file;
+typedef struct esf_jpeg_segment {
+  int64_t begin, end;           /* entropy-coded bytes, markers and fill bytes excluded */
+  int32_t file, first_mcu;
+} esf_jpeg_segment;
+int esf_jpeg_scratch_bytes(const esf_jpeg_file* files_host, int32_t n_files, int32_t gray, int64_t* bytes);
+int esf_jpeg_decode(const void* blob, int64_t blob_bytes, const esf_jpeg_file* files_host, int32_t n_files,
+                    const esf_jpeg_segment* segs_host, int32_t n_segs, int32_t n_huff, int32_t n_quant, void* scratch,
+                    int64_t scratch_bytes, uint8_t* out, int32_t H, int32_t W, int32_t C, int32_t gray, void* status,
+                    void* stream);
 int esf_stem_igemm_create(const void* xp, int32_t B, int32_t Cin, int32_t T, int32_t H, int32_t W, int32_t pitch,
                           const void* w_band, const float* bias_tiled, int32_t Cout, int32_t kT, int32_t kH,
                           int32_t kW, int32_t sH, int32_t sW, int32_t pT, int32_t pH, int32_t pW, int32_t act,
